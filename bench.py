@@ -2,6 +2,7 @@
 """bench.py -- refined samples / second of the collaborative-sampling hot path.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--sweep]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic proposals: K_refine refinement steps through
 G-tail + D (sampling/collaborator.py:41-88) followed by the MH-GAN accept-reject pass (sampling/idpsampler.py) on
@@ -65,7 +66,36 @@ def parse_args():
     ap.add_argument("--no-graph", action="store_true", help="launch the K-step sequence eagerly instead of replaying a CUDA graph")
     ap.add_argument("--sweep", action="store_true", help="BASELINE configs C3/C4/C5 at this world size -> gpurun_out/sweep_N<world>.json")
     ap.add_argument("--sweep-max-seconds", type=float, default=60.0, help="skip sweep points whose estimated step time exceeds this")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one returned as "
+                    "DIR/<name>.npy (float32 / float64, at most 60 MiB in all) to compare builds output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.sweep):
+        ap.error("--dump-outputs applies to the timed hot path of --impl ours (not --sweep)")
+    return args
+
+
+DUMP_BYTES = 60 << 20           # under 64 MB in all, .npy headers included
+
+
+def dump_outputs(out_dir, arrays):
+    """Write {name: array} as out_dir/<name>.npy, at most DUMP_BYTES in all.  Arrays are written smallest first; one
+    larger than an equal share of the bytes still free keeps a fixed, seeded sample of its rows (sorted), so two runs
+    with the same arguments write the same rows."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    free, left = DUMP_BYTES, len(arrays)
+    for name in sorted(arrays, key=lambda k: arrays[k].nbytes):
+        a = arrays[name]
+        share = free // left
+        if a.nbytes > share:
+            keep = share // (a.nbytes // a.shape[0])
+            a = a[np.sort(np.random.RandomState(0).choice(a.shape[0], keep, replace=False))]
+            print("bench: %s.npy holds a seeded sample of %d of its %d rows" % (name, keep, arrays[name].shape[0]),
+                  file=sys.stderr)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+        free, left = free - a.nbytes, left - 1
 
 
 # ----------------------------------------------------------------------------------------------------------
@@ -606,6 +636,12 @@ def run_ours(args, wl):
     launches = (lib.cgs_launch_count() + refiner.replayed_launches - launches0) // max(args.steps + args.warmup, 1)
     clk = clocks.stop() if rank == 0 else None
     n_acc = int(cnt.item())
+    if args.dump_outputs and rank == 0:
+        # what a caller of the hot path receives from the last timed step: this rank's refined batch and its scores,
+        # and the accepted rows of the whole batch (the padding past the count is undefined and left out)
+        dump_outputs(args.dump_outputs, {"refined": x.cpu().numpy(), "scores": sig_local.cpu().numpy(),
+                                         "accepted": acc[:n_acc].cpu().numpy(),
+                                         "accepted_count": np.array([n_acc], dtype=np.float64)})
     value = world * batch * args.steps / total_s
 
     # ---- end-to-end through the public API: pinned host inputs, host outputs ------------------------------

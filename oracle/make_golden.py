@@ -1,4 +1,5 @@
-"""Generate tests/golden/*.npz (TEST INFRASTRUCTURE).  Run in the build container, where /root/reference exists:
+"""Generate tests/golden/*.npz (TEST INFRASTRUCTURE).  Needs a checkout of the original project (/root/reference, or
+the directory CGS_REFERENCE_ROOT names):
 
     python -m oracle.make_golden
 
@@ -6,18 +7,23 @@
                         (imported with the shims of oracle/ref_shims.py) on seeded inputs: these PIN the oracle.
 * graph_refiner.npz  -- outputs of the oracle's torch restatement of sampling/collaborator.py on seeded inputs
                         (parity unpinned by the reference: it ships no vectors and TF 1.13 cannot run here).
+* reference_cases.npz -- outputs of the reference's OWN sampling/{policy,rejector,idpsampler}.py on the fixed-seed cases
+                        of tests/test_oracle_vs_reference.py and tests/test_fillup_cpu.py (oracle/ref_cases.py).
+* refine2d_scores.npz -- the MLP scores behind sampling_ref.npz's 2-D refiner runs, recorded on the host that made
+                        them (`python -m oracle.make_golden refine2d` records only these).
 Weights are regenerated from their seed; a checksum is stored to catch initialiser drift.
 """
 from __future__ import annotations
 
 import os
+import sys
 import types
 
 import numpy as np
 import torch
 
 from . import graph_refiner as gr
-from . import nets, ref_shims
+from . import nets, ref_cases, ref_shims, sampling_np
 
 OUT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden")
 
@@ -120,7 +126,47 @@ def graph_ref():
     return len(g)
 
 
+def reference_cases():
+    g = ref_cases.record(ref_shims.load_reference_sampling())
+    np.savez_compressed(ref_cases.GOLDEN, **g)
+    return len(g)
+
+
+def refine2d_scores():
+    """The MLP scores the reference's 2-D refiner was fed at every step of sampling_ref.npz's r2d_* runs.
+
+    The oracle MLP runs in float32 on torch-CPU, whose last bits depend on the host's BLAS kernel and thread count, so
+    the recorded r2d_*_out reproduce only on a host like the one that made them.  Run on such a host (checked below),
+    this stores what the MLP returned there; the test replays it, which pins the refinement loop on any host.  The
+    loop treats rows independently, so the K=50 run keeps a seeded sample of its rows (the file stays small)."""
+    gold = np.load(os.path.join(OUT, "sampling_ref.npz"))
+    ws = nets.init_mlp2d(64, 6, seed=2019, gain=1.5)
+    g = {}
+    for K, n_rows in ((10, None), (50, 200)):
+        key = "r2d_K%d" % K
+        calls = []
+
+        def score(x):
+            calls.append(nets.mlp2d_sigmoid_saliency(x, ws))
+            return calls[-1]
+        real_sig, _ = nets.mlp2d_sigmoid_saliency(gold[key + "_real"], ws)
+        o = sampling_np.refine_2d(gold[key + "_x0"], score, np.mean(real_sig), K, 0.1, "ladam")
+        if not np.array_equal(o["optimal_batch"], gold[key + "_out"]):
+            raise RuntimeError("this host's float32 MLP does not reproduce %s_out: record on the host that made it" % key)
+        n = len(gold[key + "_x0"])
+        rows = np.arange(n) if n_rows is None else np.sort(np.random.RandomState(K).choice(n, n_rows, replace=False))
+        g[key + "_rows"] = rows
+        g[key + "_real_mean"] = np.asarray(np.mean(real_sig))
+        g[key + "_sig"] = np.stack([s[rows] for s, _ in calls])
+        g[key + "_sal"] = np.stack([a[rows] for _, a in calls])
+    np.savez_compressed(os.path.join(OUT, "refine2d_scores.npz"), **g)
+    return len(g)
+
+
 if __name__ == "__main__":
     os.makedirs(OUT, exist_ok=True)
-    print("sampling_ref.npz:", sampling_ref(), "arrays")
-    print("graph_refiner.npz:", graph_ref(), "arrays")
+    if sys.argv[1:] != ["refine2d"]:          # `refine2d`: only re-record the scores (no reference checkout needed)
+        print("sampling_ref.npz:", sampling_ref(), "arrays")
+        print("graph_refiner.npz:", graph_ref(), "arrays")
+        print("reference_cases.npz:", reference_cases(), "arrays")
+    print("refine2d_scores.npz:", refine2d_scores(), "arrays")

@@ -1,9 +1,10 @@
-"""Import the reference's own ``sampling/*.py`` (numpy code) in the build container.
+"""Import the reference's own ``sampling/*.py`` (numpy code) from a checkout of the original project.
 
-TEST INFRASTRUCTURE ONLY (see ``oracle/__init__.py``).  ``/root/reference`` only
-exists in the build container, never on the GPU box, so this module is used by
-``oracle/make_golden.py`` (fixture generation) and by ``-m "not gpu"`` tests
-that skip themselves when the reference tree is absent.
+TEST INFRASTRUCTURE ONLY (see ``oracle/__init__.py``).  The original project is
+not part of this repository; it is taken from ``/root/reference`` unless
+``CGS_REFERENCE_ROOT`` names another checkout.  This module is used by
+``oracle/make_golden.py`` (fixture generation) and by ``-m "not gpu"`` tests,
+which fall back to the outputs make_golden stored when no checkout is present.
 
 Shims (SURVEY.md §8c), none of which touches the reference's arithmetic:
   1. ``np.float = float``  -- ``sampling/rejector.py:12,18`` use the alias that
@@ -24,6 +25,7 @@ import types
 import numpy as np
 
 REFERENCE_ROOT = os.environ.get("CGS_REFERENCE_ROOT", "/root/reference")
+SKIP_REASON = "no checkout of the original project (/root/reference or CGS_REFERENCE_ROOT)"
 
 
 def reference_available() -> bool:
@@ -38,7 +40,7 @@ def load_reference_sampling():
     if "ns" in _CACHE:
         return _CACHE["ns"]
     if not reference_available():
-        raise RuntimeError("reference tree not present at %s" % REFERENCE_ROOT)
+        raise RuntimeError(SKIP_REASON)
     if not hasattr(np, "float"):
         np.float = float  # shim 1
     if "tensorflow" not in sys.modules:

@@ -5,7 +5,7 @@ import numpy as np
 import pytest
 
 from oracle import fillup_np as F
-from oracle import ref_shims
+from oracle import ref_cases, ref_shims
 
 
 def _stream(seed, dim=3):
@@ -18,29 +18,15 @@ def _stream(seed, dim=3):
     return propose
 
 
-@pytest.mark.skipif(not ref_shims.reference_available(), reason="reference tree not present")
 @pytest.mark.parametrize("kind", ["rejection", "hastings"])
 def test_oracle_loop_with_reference_samplers_equals_oracle_samplers(kind):
-    ref = ref_shims.load_reference_sampling()
-    outs = []
-    for impl in ("reference", "oracle"):
-        propose = _stream(3)
-        base_x, base_s = propose(200)
-        np.random.seed(11)
-        if kind == "rejection":
-            smp = ref.rejector.Rejector() if impl == "reference" else F.OracleRejector()
-            smp.set_score_max(np.float32(0.9))
-            sampling = lambda x, s, smp=smp: smp.sampling(x, s, shift_percent=100.0)
-            guard = "running"
-        else:
-            smp = ref.idpsampler.IndependenceSampler(T=3) if impl == "reference" else F.OracleIndependenceSampler(T=3)
-            smp.set_score_curr(np.float32(0.3))
-            sampling = smp.sampling
-            guard = "batch"
-        outs.append(F.fill_up_nsgan(base_x, base_s, propose, sampling, 200, 32, store_guard=guard))
-    a, b = outs
-    assert a["cnt"] == b["cnt"] and a["cnt_propose"] == b["cnt_propose"] and a["n_backfilled"] == b["n_backfilled"]
-    assert np.array_equal(a["samples"], b["samples"]) and a["cnt"] >= 200
+    exp = ref_cases.expected("fillup_%s" % kind)       # the loop over the reference's own sampler classes
+    if exp is None:
+        pytest.skip(ref_shims.SKIP_REASON + " and no recorded outputs (python -m oracle.make_golden)")
+    b = ref_cases.fillup_run(kind, F.OracleRejector, F.OracleIndependenceSampler)
+    assert int(exp["cnt"]) == b["cnt"] and int(exp["cnt_propose"]) == b["cnt_propose"]
+    assert int(exp["n_backfilled"]) == b["n_backfilled"]
+    assert np.array_equal(exp["samples"], b["samples"]) and b["cnt"] >= 200
 
 
 def test_backfill_starts_at_the_efficiency_cap_and_efficiency_may_overshoot():

@@ -1,61 +1,58 @@
-"""Oracle vs the reference's own modules executed in place (build container only: /root/reference must exist)."""
+"""Oracle vs the reference's own modules: executed in place where the original project is checked out, else through
+the outputs oracle/make_golden.py recorded from it (tests/golden/reference_cases.npz, see oracle/ref_cases.py)."""
 import types
 
 import numpy as np
 import pytest
 
 from oracle import nets as onets
+from oracle import ref_cases as rc
 from oracle import ref_shims
 from oracle import sampling_np as snp
-
-pytestmark = pytest.mark.skipif(not ref_shims.reference_available(), reason="reference tree not present")
 
 
 @pytest.fixture(scope="module")
 def ref():
+    if not ref_shims.reference_available():
+        pytest.skip(ref_shims.SKIP_REASON)
     return ref_shims.load_reference_sampling()
 
 
+def expected(name):
+    out = rc.expected(name)
+    if out is None:
+        pytest.skip(ref_shims.SKIP_REASON + " and no recorded outputs (python -m oracle.make_golden)")
+    return out
+
+
 @pytest.mark.parametrize("dt", [np.float32, np.float64])
-def test_drs_bit_exact(ref, dt):
-    rng = np.random.RandomState(1)
-    R = ref.rejector.Rejector()
-    R.set_score_max(np.amax(rng.beta(2, 5, size=200).astype(dt)))
-    m = R.D_tilde_M
-    samples = rng.randn(1000, 2).astype(np.float32)
-    for call, sp in enumerate((100.0, 60.0, None, 100.0, 12.5)):
-        sig = rng.beta(2, 5, size=(1000, 1)).astype(dt)
-        if call == 3:
-            sig[17] = 1.0 - 1e-9
-        np.random.seed(call)
-        good = R.sampling(samples, sig, shift_percent=sp)
+def test_drs_bit_exact(dt):
+    exp = expected("drs_%s" % ("f32" if dt == np.float32 else "f64"))
+    _, samples, calls = rc.drs_case(dt)
+    m = exp["M0"][()]
+    for call, (sig, sp) in enumerate(calls):
         np.random.seed(call)
         acc, m = snp.drs_accept(sig, np.random.rand(1000), m, shift_percent=sp)
-        assert np.array_equal(samples[acc], good)
-        assert float(m) == float(R.D_tilde_M)
+        assert np.array_equal(samples[acc], exp["%d_good" % call])
+        assert float(m) == float(exp["%d_M" % call])
 
 
 @pytest.mark.parametrize("dt", [np.float32, np.float64])
 @pytest.mark.parametrize("T,B", [(0, 0), (1, 0), (5, 2), (20, 0), (20, 5)])
-def test_mh_bit_exact_with_carried_state(ref, dt, T, B):
-    rng = np.random.RandomState(T + 7 * B)
-    S = ref.idpsampler.IndependenceSampler(T=T, B=B)
-    S.set_score_curr(np.mean(rng.beta(2, 5, size=64).astype(dt)))
-    d, cnt = S.d_curr, S.cnt_chain
-    for call in range(4):
-        n = (900, 1, 333, 64)[call]
-        sig = rng.beta(2, 5, size=(n, 1)).astype(dt)
-        samples = rng.randn(n, 3).astype(np.float32)
-        np.random.seed(call)
-        good = S.sampling(samples, sig)
+def test_mh_bit_exact_with_carried_state(dt, T, B):
+    exp = expected("mh_%s_T%d_B%d" % ("f32" if dt == np.float32 else "f64", T, B))
+    _, calls = rc.mh_case(dt, T, B)
+    d, cnt = exp["d0"][()], int(exp["cnt0"])
+    for call, (sig, samples) in enumerate(calls):
+        n = len(sig)
         np.random.seed(call)
         emit, d, cnt, _ = snp.mh_chain(sig, np.random.rand(n), d, cnt, T, B)
-        exp = samples[emit] if len(emit) else np.zeros((0,), np.float32)
-        assert np.array_equal(exp.astype(np.float32), good)
-        assert cnt == S.cnt_chain and float(np.squeeze(d)) == float(np.squeeze(S.d_curr))
+        got = samples[emit] if len(emit) else np.zeros((0,), np.float32)
+        assert np.array_equal(got.astype(np.float32), exp["%d_good" % call])
+        assert cnt == int(exp["%d_cnt" % call]) and float(np.squeeze(d)) == float(exp["%d_d" % call])
 
 
-def test_mh_uniform_stream_equals_rand(ref):
+def test_mh_uniform_stream_equals_rand():
     np.random.seed(3)
     a = np.array([np.random.uniform(0, 1) for _ in range(50)])
     np.random.seed(3)
@@ -63,20 +60,16 @@ def test_mh_uniform_stream_equals_rand(ref):
 
 
 @pytest.mark.parametrize("method", ["sgd", "momentum", "ladam"])
-def test_policy_bit_exact(ref, method):
-    rng = np.random.RandomState(5)
-    P = ref.policy.PolicyAdaptive(0.1, method)
-    a = (rng.randn(100, 2)).astype(np.float32)
-    b = a.copy()
+def test_policy_bit_exact(method):
+    exp = expected("policy_%s" % method)
+    b, steps = rc.policy_case()
     st = snp.policy_new_state()
-    for _ in range(4):
-        g = rng.randn(100, 2).astype(np.float32) * 1e-3
-        l = (rng.rand(100) - .5).astype(np.float32)
-        P.apply_gradient(a, g, l)
+    for i, (g, l) in enumerate(steps):
         snp.policy_step(method, b, g, st, 0.1, l)
-        assert np.array_equal(a, b)
+        assert np.array_equal(exp["%d_theta" % i], b)
+    assert bool(exp["unknown_method_raises"])
     with pytest.raises(NotImplementedError):
-        ref.policy.PolicyAdaptive(0.1, "nope").apply_gradient(a, a)
+        snp.policy_step("nope", b, b, snp.policy_new_state(), 0.1)
 
 
 @pytest.mark.parametrize("mode", ["deterministic", "probabilistic"])
