@@ -5,6 +5,7 @@ and every compute entry point returns CGS_ERR_CUDA on a machine without a B200.
 """
 from __future__ import annotations
 
+import contextlib
 import ctypes as C
 import os
 
@@ -23,6 +24,30 @@ MATH_TF32_TENSOR, MATH_FP32_SIMT = 0, 1
 MATH_IDS = {"tf32": MATH_TF32_TENSOR, "fp32": MATH_FP32_SIMT}
 MLP_MAX_LAYERS = 8
 MAX_LAYERS = 8
+
+# developer knobs, enum cgs_debug_flag of include/cgs.h (the comments there say what each one does)
+DEBUG_SKIP_A_GATHER = 1
+DEBUG_SKIP_WEIGHT_TMA = 2
+DEBUG_SKIP_MMA = 4
+DEBUG_SKIP_A_TMA = 8
+DEBUG_SKIP_EPILOGUE = 16
+DEBUG_TRACE = 256
+DEBUG_GATHER_A = 512
+DEBUG_SKIP_STORES = 1024
+DEBUG_NO_PREFETCH = 2048
+DEBUG_EDGE_GENERAL = 4096
+DEBUG_NO_FC_SPLIT = 16384
+DEBUG_PDL_ON = 32768
+DEBUG_NO_EDGE_PAIR = 65536
+DEBUG_NO_HEAD_PARTIALS = 131072
+DEBUG_NO_FUSION = 524288
+DEBUG_FORCE_FUSION = 1048576
+DEBUG_NO_MTILE_PAIRS = 4194304
+DEBUG_FORCE_MTILE_PAIRS = 8388608
+DEBUG_NO_CTA_PAIRS = 16777216
+DEBUG_FORCE_CTA_PAIRS = 33554432
+DEBUG_MLP2D_ONE_THREAD = 134217728
+DEBUG_PDL_OFF = 536870912
 
 
 class PolicyCfg(C.Structure):
@@ -127,6 +152,17 @@ def load():
         raise ImportError("libcgs ABI version mismatch")
     _lib = lib
     return lib
+
+
+@contextlib.contextmanager
+def debug_flags(flags):
+    """Run the body with the CGS_DEBUG knobs set to `flags` (process-wide), then restore the previous value."""
+    lib = load()
+    old = lib.cgs_debug_set_flags(flags)
+    try:
+        yield
+    finally:
+        lib.cgs_debug_set_flags(old)
 
 
 def last_error():

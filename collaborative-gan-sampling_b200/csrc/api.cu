@@ -30,8 +30,8 @@ void set_debug_flags(int v) { g_debug.store(v < 0 ? 0 : v, std::memory_order_rel
 static thread_local bool tl_pdl = false;
 bool pdl_enabled() {
   const int f = debug_flags();
-  if (f & 536870912) return false;
-  return tl_pdl || (f & 32768) != 0;
+  if (f & CGS_DEBUG_PDL_OFF) return false;
+  return tl_pdl || (f & CGS_DEBUG_PDL_ON) != 0;
 }
 PdlScope::PdlScope(bool on) : prev(tl_pdl) { tl_pdl = on; }
 PdlScope::~PdlScope() { tl_pdl = prev; }
@@ -78,14 +78,14 @@ extern "C" int cgs_version(void) { return CGS_ABI_VERSION; }
 extern "C" const char* cgs_last_error(void) { return cgs::error_buffer(); }
 
 namespace cgs { int debug_trace_read(unsigned long long* out, int cap); }
-// Developer aid: read (and reset) the CTA-0 pipeline event trace recorded when CGS_DEBUG has bit 256 set.
+// Developer aid: read (and reset) the CTA-0 pipeline event trace recorded under CGS_DEBUG_TRACE.
 extern "C" __attribute__((visibility("default"))) int cgs_debug_trace(unsigned long long* out_host, int capacity) {
   return cgs::debug_trace_read(out_host, capacity);
 }
 
 namespace cgs { void set_debug_flags(int v); }
-// Developer aid: replace the CGS_DEBUG knobs at run time (bit 4096 = image-edge passes on the general tcgen05
-// lowerings, used by the parity tests to keep both implementations covered).  Returns the previous value.
+// Developer aid: replace the CGS_DEBUG knobs (cgs_debug_flag) at run time; the parity tests use it to keep every
+// lowering covered.  Returns the previous value.
 extern "C" __attribute__((visibility("default"))) int cgs_debug_set_flags(int flags) {
   const int old = cgs::debug_flags();
   cgs::set_debug_flags(flags);
@@ -93,5 +93,5 @@ extern "C" __attribute__((visibility("default"))) int cgs_debug_set_flags(int fl
 }
 
 namespace cgs { int debug_trace_tc(long long* out_host); }
-// Developer aid: CTA-0 event clocks of the last edge_wide_tc launch run with CGS_DEBUG bit 256 ([8 roles][64 tiles]).
+// Developer aid: CTA-0 event clocks of the last edge_wide_tc launch run under CGS_DEBUG_TRACE ([8 roles][64 tiles]).
 extern "C" CGS_API int cgs_debug_trace_tc(long long* out_host) { return cgs::debug_trace_tc(out_host); }

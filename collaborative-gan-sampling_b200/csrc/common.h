@@ -54,7 +54,7 @@ inline cudaError_t ensure_dyn_smem(K kernel, size_t smem, DynSmemCache& c) {
   return e;
 }
 
-// Developer knobs: env CGS_DEBUG at first use, overridable with cgs_debug_set_flags (api.cu).
+// Developer knobs (cgs_debug_flag in cgs.h): env CGS_DEBUG at first use, overridable with cgs_debug_set_flags (api.cu).
 int debug_flags();
 
 // Process-wide count of kernels launched by the library (cgs_launch_count).
@@ -65,8 +65,8 @@ void count_launch(int n = 1);
 // kernel's set-up -- barrier init, TMEM allocation, tensor-map prefetch -- overlaps the previous kernel's drain).
 // Measured on B200 inside the replayed CUDA graph: +1.5 % on the DCGAN-64 step, +1.1 % on DCGAN-32, -0.8 % on the
 // MNIST-sized nets (their kernels are 20-45 us; an early-resident successor only gets in the way), so the refinement
-// loop switches it on per call from its average work per launch (refine_conv.cu).  CGS_DEBUG bit 32768 forces it on
-// everywhere, 536870912 off.
+// loop switches it on per call from its average work per launch (refine_conv.cu).  CGS_DEBUG_PDL_ON forces it on
+// everywhere, CGS_DEBUG_PDL_OFF off.
 bool pdl_enabled();
 struct PdlScope {            // switches programmatic dependent launch on for the launches of the calling thread
   explicit PdlScope(bool on);

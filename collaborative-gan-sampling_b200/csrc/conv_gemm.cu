@@ -13,8 +13,8 @@
 //   warp  14    TMA producer for the A tile (one 4-D box per K atom with traversal strides, or the window map)
 // Pipelines: full/empty mbarriers per smem stage (3-8 stages, 1-2 K atoms each), tmem_full/tmem_empty per
 // accumulator buffer (ring of 4 x BN TMEM columns, 2 at BN = 256: tile epilogues overlap the following main loops).
-// CGS_DEBUG knobs (cgs_debug_set_flags): 1 skip A gather, 2 skip weight TMA, 8 skip A TMA, 4 skip MMA issue,
-// 16 skip epilogue work, 512 force gather mode, 1024 skip stores, 2048 no operand prefetch, 256 event trace (CGS_TRACE).
+// CGS_DEBUG knobs (cgs_debug_flag): CGS_DEBUG_GATHER_A forces gather mode; profiling: CGS_DEBUG_SKIP_A_GATHER,
+// _SKIP_WEIGHT_TMA, _SKIP_A_TMA, _SKIP_MMA, _SKIP_EPILOGUE, _SKIP_STORES, _NO_PREFETCH, _TRACE (built with CGS_TRACE).
 #include "conv_gemm.cuh"
 #include "ptx.cuh"
 #include "common.h"
@@ -25,13 +25,13 @@
 
 namespace cgs {
 
-// ---- optional event trace of CTA 0 (CGS_DEBUG bit 256): (role, event, index, clock) records for pipeline analysis
+// ---- optional event trace of CTA 0 (CGS_DEBUG_TRACE): (role, event, index, clock) records for pipeline analysis
 __device__ unsigned long long g_trace[32768];
 __device__ unsigned int g_trace_n;
 __device__ __forceinline__ void trace(const ConvGemmParams& p, int role, int ev, unsigned idx) {
 #ifdef CGS_TRACE
   // fixed slot per (role, event, index): a plain store, no atomics, so the traced thread is barely perturbed
-  if ((p.debug & 256) && blockIdx.x == 0 && idx < 1024) {
+  if ((p.debug & CGS_DEBUG_TRACE) && blockIdx.x == 0 && idx < 1024) {
     const unsigned slot = ((unsigned)(role * 4 + ev) << 10) + idx;
     g_trace[slot & 32767] = ((unsigned long long)role << 60) | ((unsigned long long)ev << 56) |
                             ((unsigned long long)(idx & 0xffffff) << 32) | (unsigned long long)(unsigned)clock64();
@@ -234,7 +234,7 @@ conv_gemm_tc_kernel(const __grid_constant__ ConvGemmParams p, const __grid_const
             off = tap_off + (cb + gc.cb0) * BK + chunk * 4;
           }
           const uint32_t atom_base = smem_a_u32 + s * C::A_STAGE_BYTES + a * A_ATOM_BYTES;
-          if (!(p.debug & 1)) {
+          if (!(p.debug & CGS_DEBUG_SKIP_A_GATHER)) {
 #pragma unroll
             for (int it = 0; it < kRowsPerThread; ++it) {
               const bool ok = (vmask[it] >> tt) & 1u;
@@ -263,7 +263,7 @@ conv_gemm_tc_kernel(const __grid_constant__ ConvGemmParams p, const __grid_const
       // the whole warp walks the loop: lane 0 waits for the slot and posts the byte count, then lane q issues the box
       // of the q-th class with a tap at the shift (a single thread issuing up to four boxes per stage was the slowest
       // role of the fused tiles: 45 us of a 210 us pass)
-      const bool skip = (p.debug & 2) != 0;
+      const bool skip = (p.debug & CGS_DEBUG_SKIP_WEIGHT_TMA) != 0;
       uint32_t stage = 0, phase = 0;
       for (int tile = tile_first; tile < total_tiles; tile += tile_stride) {
         const int ci = fast_div(tile, fd_tpc);
@@ -298,7 +298,7 @@ conv_gemm_tc_kernel(const __grid_constant__ ConvGemmParams p, const __grid_const
     if (elect_one()) {                     // one thread walks the whole loop: no per-K-block election or warp sync
       uint32_t it_global = 0;
       uint32_t stage = 0, phase = 0;
-      const bool skip = (p.debug & 2) != 0;
+      const bool skip = (p.debug & CGS_DEBUG_SKIP_WEIGHT_TMA) != 0;
       for (int tile = tile_first; tile < total_tiles; tile += tile_stride) {
         const int ci = fast_div(tile, fd_tpc);
         const int rem = tile - ci * tiles_per_class;
@@ -330,7 +330,7 @@ conv_gemm_tc_kernel(const __grid_constant__ ConvGemmParams p, const __grid_const
       const uint32_t a_bytes = (uint32_t)p.rows_valid * 128u;
       if (elect_one()) {                   // one thread walks the whole loop
         uint32_t stage = 0, phase = 0;
-        const bool skip = (p.debug & 8) != 0;
+        const bool skip = (p.debug & CGS_DEBUG_SKIP_A_TMA) != 0;
         const int cblocks = p.cblocks;
         for (int tile = tile_first; tile < total_tiles; tile += tile_stride) {
           const int ci = fast_div(tile, fd_tpc);
@@ -440,7 +440,7 @@ conv_gemm_tc_kernel(const __grid_constant__ ConvGemmParams p, const __grid_const
     uint32_t tile_count = 0;
     uint32_t stage = 0, phase = 0;               // position in the smem ring
     const bool a_tma = p.a_tma != 0;
-    const bool skip_mma = (p.debug & 4) != 0;
+    const bool skip_mma = (p.debug & CGS_DEBUG_SKIP_MMA) != 0;
     for (int tile = tile_first; tile < total_tiles; tile += tile_stride, ++tile_count) {
       const int ci = fast_div(tile, fd_tpc);
       const uint32_t acc = tile_count % C::NACC;
@@ -543,7 +543,8 @@ conv_gemm_tc_kernel(const __grid_constant__ ConvGemmParams p, const __grid_const
     const int tile_groups = kSplitTiles ? ngroups : 1;       // groups that take separate tiles
     const int chunk_groups = kSplitTiles ? 1 : ngroups;      // groups that share the chunks of one tile
     float* stage = smem_epi + warp * 32 * EPI_PITCH;
-    const bool dbg_skip_epi = (p.debug & 16) != 0, dbg_skip_store = (p.debug & 1024) != 0, dbg_no_prefetch = (p.debug & 2048) != 0;
+    const bool dbg_skip_epi = (p.debug & CGS_DEBUG_SKIP_EPILOGUE) != 0, dbg_skip_store = (p.debug & CGS_DEBUG_SKIP_STORES) != 0;
+    const bool dbg_no_prefetch = (p.debug & CGS_DEBUG_NO_PREFETCH) != 0;
     const int c4 = lane % Q;
     const int rsub = lane / Q;
     // tile-invariant part of the row -> output offset map of the PASSES rows this lane stores
@@ -897,9 +898,9 @@ void build_fusion(ConvGemmParams& p, int NS) {
   }
 }
 
-// Can this launch run class-fused, and with how many slots per tile?  (CGS_DEBUG bit 524288 switches fusion off.)
+// Can this launch run class-fused, and with how many slots per tile?  (CGS_DEBUG_NO_FUSION switches fusion off.)
 int fusion_slots(const ConvGemmParams& p, int bn) {
-  if (debug_flags() & (524288 | 512)) return 0;
+  if (debug_flags() & (CGS_DEBUG_NO_FUSION | CGS_DEBUG_GATHER_A)) return 0;
   if (p.nclasses != 4 || p.S != 1 || p.os != 2 || p.cblocks <= 0 || p.window || bn != p.N) return 0;
   for (int c = 0; c < 4; ++c) {
     if (p.cls[c].cb0 != 0 || p.cls[c].k0 % BK) return 0;
@@ -978,7 +979,7 @@ int launch_tc_epi(ConvGemmParams p, const float* w, int w_rows, int w_cols, cuda
   p.hy_tiles = (p.MH + p.BH - 1) / p.BH;
   p.rows_valid = p.BB * p.BH * p.MW;
   p.m_tiles = ((p.B + p.BB - 1) / p.BB) * p.hy_tiles;
-  p.a_tma = (p.cblocks > 0) && !(p.debug & 512);
+  p.a_tma = (p.cblocks > 0) && !(p.debug & CGS_DEBUG_GATHER_A);
   CUtensorMap tmap_a;
   std::memset(&tmap_a, 0, sizeof(tmap_a));
   if (p.window) {
@@ -1046,12 +1047,12 @@ int launch_tc(const ConvGemmParams& p, const float* w, int w_rows, int w_cols, c
 }
 
 // CTA pairs (cta_group::2) are taken for the passes whose stages are widest in bytes per MMA cycle -- class-fused tiles
-// and 256-wide tiles -- when the TMA'd A operand is in use and every SM still gets a tile.  CGS_DEBUG bit 16777216
-// switches them off, 33554432 forces them whenever legal (parity tests at small batch).
+// and 256-wide tiles -- when the TMA'd A operand is in use and every SM still gets a tile.  CGS_DEBUG_NO_CTA_PAIRS
+// switches them off, CGS_DEBUG_FORCE_CTA_PAIRS forces them whenever legal (parity tests at small batch).
 bool use_cta_pairs(const ConvGemmParams& p, long long units_total, int num_sms) {
-  if (debug_flags() & (16777216 | 512)) return false;
+  if (debug_flags() & (CGS_DEBUG_NO_CTA_PAIRS | CGS_DEBUG_GATHER_A)) return false;
   if (p.cblocks <= 0 || p.window) return false;
-  if (debug_flags() & 33554432) return true;
+  if (debug_flags() & CGS_DEBUG_FORCE_CTA_PAIRS) return true;
   return 2 * units_total >= (num_sms & ~1);
 }
 
@@ -1104,11 +1105,11 @@ int launch_conv_gemm_tc(const ConvGemmParams& p_in, const float* w, int w_rows, 
     if (force) bn = force;
   }
   // class-fused instances of the transposed-type passes: taken when the fused tiles (4x / 2x fewer than class tiles)
-  // still give every SM one; CGS_DEBUG bit 1048576 forces them whenever they are legal (parity tests at small batch)
+  // still give every SM one; CGS_DEBUG_FORCE_FUSION forces them whenever they are legal (parity tests at small batch)
   if (!p.force_bn) {
     const int bn_full = pick_bn(p.N);
     const int ns = fusion_slots(p, bn_full);
-    if (ns && ((debug_flags() & 1048576) || count_m_tiles(p) * (ns == 2 ? 2 : 1) >= num_sms)) {
+    if (ns && ((debug_flags() & CGS_DEBUG_FORCE_FUSION) || count_m_tiles(p) * (ns == 2 ? 2 : 1) >= num_sms)) {
       const bool pairs = use_cta_pairs(p, (long long)((count_m_tiles(p) + 1) / 2) * (ns == 2 ? 2 : 1), num_sms);
       switch (ns * 1000 + bn_full) {
         case 4032: return launch_tc<32, 4>(p, w, w_rows, w_cols, stream);
@@ -1120,10 +1121,10 @@ int launch_conv_gemm_tc(const ConvGemmParams& p_in, const float* w, int w_rows, 
   }
   // M-tile pairs sharing the weight atoms (MT = 2): 64- / 128-wide one-class tiles with a TMA'd A operand, when the
   // pairs still give every SM a tile.  Bit-identical to single tiles (each accumulator sees the same MMA sequence).
-  // CGS_DEBUG bit 4194304 switches them off, 8388608 forces them whenever legal.
+  // CGS_DEBUG_NO_MTILE_PAIRS switches them off, CGS_DEBUG_FORCE_MTILE_PAIRS forces them whenever legal.
   // (64-wide pairs on one CTA save only 17 % of the bytes and measured slower on the MNIST nets; inside CTA pairs --
   //  four M tiles per weight atom, half of it per CTA -- they save 25 % and measured 3-7 % faster: taken only there)
-  if (!p.force_bn && (bn == 128 || bn == 64) && p.cblocks > 0 && !p.window && !(debug_flags() & (4194304 | 512)) &&
+  if (!p.force_bn && (bn == 128 || bn == 64) && p.cblocks > 0 && !p.window && !(debug_flags() & (CGS_DEBUG_NO_MTILE_PAIRS | CGS_DEBUG_GATHER_A)) &&
       p.N > bn / 2) {
     const long long nt = (long long)((p.N + bn - 1) / bn) * p.nclasses;
     const long long tiles = (long long)count_m_tiles(p) * nt, pairs = (long long)((count_m_tiles(p) + 1) / 2) * nt;
@@ -1131,7 +1132,7 @@ int launch_conv_gemm_tc(const ConvGemmParams& p_in, const float* w, int w_rows, 
     // whole rounds over the SMs: a pair round costs two tile rounds at 0.78x / 0.85x of their bytes
     const double cost_pair = (double)((pairs + num_sms - 1) / num_sms) * 2.0 * (bn == 128 ? 0.78 : 0.85);
     const double cost_single = (double)((tiles + num_sms - 1) / num_sms);
-    const bool forced = (debug_flags() & 8388608) != 0;
+    const bool forced = (debug_flags() & CGS_DEBUG_FORCE_MTILE_PAIRS) != 0;
     if (forced || (pairs >= num_sms && cost_pair < cost_single)) {
       // M-tile pairs inside CTA pairs: 40 KB instead of 48 KB of L2 -> SM traffic per 512 tensor cycles (BN = 128) on
       // passes that sit at the L2 throughput ceiling

@@ -103,7 +103,7 @@ struct ConvGemmParams {
   int m2;
   FuseGroup grp[2];
   FuseShift shf[kMaxShifts];
-  int debug;          // profiling knobs (env CGS_DEBUG): 1 = skip A gather, 2 = skip weight TMA, 4 = skip MMA issue
+  int debug;          // debug_flags() at launch: the profiling knobs of cgs_debug_flag (CGS_DEBUG_SKIP_*, _TRACE)
   // exact division of the persistent tile index by multiply-shift (filled by the launcher; see fast_div)
   unsigned long long fd_tiles_per_class, fd_n_tiles, fd_hy_tiles;
   GemmClass cls[kMaxClasses];

@@ -5,7 +5,6 @@
 #include "edge_conv.cuh"
 
 #include <cstdint>
-#include <type_traits>
 
 #include "common.h"
 #include "conv_gemm.cuh"
@@ -384,256 +383,6 @@ __global__ void __launch_bounds__(EN_THREADS) edge_narrow_kernel(const EdgeNarro
 }
 
 // ---------------------------------------------------------------------------------------------
-// edge_narrow2: the same pass (64 channels -> image-like output, stride-2 transposed type) in GATHER form with the
-// accumulators in registers -- no column buffer, no shared-memory col2im, no halo recompute.
-//
-// Output pixel (2j + py, 2i + px) sums the taps (ky, kx) of matching parity; tap ky reads input row j + dy with
-// dy = (py + pad - ky) / 2 in {-1, 0, 1} (pad = 1 for k = 4 and k = 5 under TF SAME), likewise dx.  So for the input
-// grid point (j, i) the 4 parity classes x 4 padded channels are 16 GEMM columns and the reduction runs over
-// (dy, dx, 64 channels): acc[(j, i)][(py, px, c)] += in[j + dy][i + dx][:] . Wshift[dy][dx][:][(py, px, c)], with
-// Wshift zero where a class has no tap at that shift.  n-tile 0 holds the py = 0 classes, n-tile 1 the py = 1 ones,
-// so (dy, n-tile) pairs without any tap are skipped at compile time: 15 of 18 (k = 5) / 12 of 18 (k = 4).
-//
-// A WARP owns a job = (image, band of R input rows) and sweeps the input rows once ("input stationary"): row r feeds
-// the accumulator sets of output-row pairs j = r + 1, r, r - 1 (three register sets, rotated by a compile-time phase),
-// so every A fragment is loaded once per dx instead of once per (dy, dx).  Rows are staged by the warp itself with
-// cp.async into a private double buffer (swizzled 16-byte chunks: conflict-free LDS.128 fragment loads); warps never
-// synchronise with each other.  When row r is done the pair j = r - 1 is complete: bias / tanh (or x tanh') and the
-// pitched store straight from the mma accumulator layout (a quad writes two adjacent pixels = 32 bytes, a warp
-// instruction 256 contiguous bytes).
-// ---------------------------------------------------------------------------------------------
-constexpr int N2_PX = 34;                      // staged pixels per row: zero | <= 32 data | zero
-constexpr int N2_ROW_FLOATS = N2_PX * 64;      // 8704 bytes
-constexpr int N2_BFRAG = 9 * EN_KSTEPS * 2 * 32;   // float2 per CTA: [shift][k-step][n-tile][lane]
-
-template <int KS>
-__host__ __device__ constexpr bool n2_need(int nt, int dyi) {       // does class row py = nt have a tap at dy = dyi - 1 ?
-  return (nt + 3 - 2 * dyi) >= 0 && (nt + 3 - 2 * dyi) < KS;         // ky = py + pad - 2 dy, pad = 1
-}
-
-// Four 8x4 TF32 sub-matrices (8 rows of 16 bytes each) -> the A fragment of mma.m16n8k8 in register order: lanes 0-7
-// address the rows of (pixels g, k 0-3), lanes 8-15 (pixels g+8, k 0-3), lanes 16-23 (g, k 4-7), lanes 24-31 (g+8, k 4-7).
-__device__ __forceinline__ void ldmatrix_x4(uint32_t (&r)[4], uint32_t addr) {
-  asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0,%1,%2,%3}, [%4];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"(addr));
-}
-
-__device__ __forceinline__ void n2_setup(const EdgeNarrowParams& p, float2* bfrag) {
-  for (int idx = threadIdx.x; idx < N2_BFRAG; idx += blockDim.x) {
-    const int l = idx & 31, nt = (idx >> 5) & 1, ks = (idx >> 6) & 7, sh = idx >> 9;
-    const int dy = sh / 3 - 1, dx = sh % 3 - 1;
-    const int g = l >> 2, t = l & 3;
-    const int py = nt, px = g >> 2, c = g & 3;
-    const int ky = py + p.pad_y - 2 * dy, kx = px + p.pad_x - 2 * dx;
-    float2 b = make_float2(0.f, 0.f);                                // b0 = W[k = t][n = g], b1 = W[k = t + 4][n = g]
-    if (c < p.cimg && ky >= 0 && ky < p.k && kx >= 0 && kx < p.k) {
-      const float* wr = p.w + (size_t)((ky * p.k + kx) * 4 + c) * p.K + 8 * ks + t;
-      b = make_float2(__ldg(wr), __ldg(wr + 4));
-    }
-    bfrag[idx] = b;
-  }
-}
-
-template <int KS, int MT>
-__global__ void __launch_bounds__(256, 1) edge_narrow2_kernel(const EdgeNarrowParams p, int njobs) {
-  extern __shared__ float4 n2_smem4[];
-  float2* bfrag = reinterpret_cast<float2*>(n2_smem4);
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nwarps = blockDim.x >> 5;
-  const int g = lane >> 2, t = lane & 3;
-  float* rowbuf = reinterpret_cast<float*>(bfrag + N2_BFRAG) + (size_t)warp * 2 * N2_ROW_FLOATS;   // [2][34][64]
-  n2_setup(p, bfrag);
-  for (int i = lane; i < 2 * N2_ROW_FLOATS / 4; i += 32) reinterpret_cast<float4*>(rowbuf)[i] = make_float4(0.f, 0.f, 0.f, 0.f);
-  __syncthreads();
-  pdl_launch_dependents();
-  pdl_wait();
-  if (p.e.live) njobs = min(njobs, live_images(p.e.live, p.B) * p.bands);
-  const uint32_t rowbuf_u32 = smem_u32(rowbuf);
-  const float4 bias4 = (p.e.epi == EPI_FWD && p.e.bias) ? __ldg(reinterpret_cast<const float4*>(p.e.bias))
-                                                        : make_float4(0.f, 0.f, 0.f, 0.f);
-  const float bias0 = (t & 1) ? bias4.z : bias4.x, bias1 = (t & 1) ? bias4.w : bias4.y;
-  const int c0 = (t & 1) * 2;                       // image channels this lane holds: c0, c0 + 1
-  const bool bwd = p.e.epi == EPI_BWD;
-  // ldmatrix row address of this lane: stored pixel (lane & 7) + 8 * bit 3 (+ 16 m + dx), 16-byte chunk 2 ks + bit 4
-  const int lm_px = (lane & 7) + ((lane >> 3) & 1) * 8;
-  const int lm_half = lane >> 4;
-
-  for (int job = blockIdx.x * nwarps + warp; job < njobs; job += gridDim.x * nwarps) {
-    const int b = job / p.bands;
-    const int j0 = (job - b * p.bands) * p.R;
-    const int j1 = min(p.IH, j0 + p.R);              // output-row pairs [j0, j1)
-    const float* src_img = p.in + (size_t)b * p.IH * p.IW * 64;
-    // three accumulator sets: output-row pairs j = r + 1, r, r - 1 of the input row r being swept
-    float acc[3][MT][2][4];
-#pragma unroll
-    for (int s3 = 0; s3 < 3; ++s3)
-#pragma unroll
-      for (int m = 0; m < MT; ++m)
-#pragma unroll
-        for (int nt = 0; nt < 2; ++nt)
-#pragma unroll
-          for (int q = 0; q < 4; ++q) acc[s3][m][nt][q] = 0.f;
-
-    // stage input row r into buffer `buf`: 16-byte chunk c of stored pixel x lands at chunk (c & 8) | ((c ^ x) & 7), so
-    // that the eight 16-byte rows of an ldmatrix sub-matrix (8 consecutive pixels, same chunk) hit distinct banks
-    auto stage_row = [&](int r, int buf) {
-      if ((unsigned)r < (unsigned)p.IH) {
-        const float* src = src_img + (size_t)r * p.IW * 64;
-        const uint32_t dst = rowbuf_u32 + buf * (N2_ROW_FLOATS * 4);
-        for (int q = lane; q < p.IW * 16; q += 32) {
-          const int px = (q >> 4) + 1, ck = q & 15;
-          cp_async_16(dst + px * 256 + (((ck & 8) | ((ck ^ px) & 7)) << 4), src + q * 4, 16u);
-        }
-      }
-      cp_async_commit();
-    };
-
-    // epilogue of the output-row pair j held in accumulator set `a` (stale sets are zeroed, never stored)
-    auto finalize = [&](int j, bool store, float (&a)[MT][2][4], const float2 (&aux)[MT][2][2]) {
-#pragma unroll
-      for (int nt = 0; nt < 2; ++nt) {
-        float* orow = p.out + ((size_t)b * p.OH + 2 * j + nt) * p.out_pitch * 4;
-#pragma unroll
-        for (int m = 0; m < MT; ++m)
-#pragma unroll
-          for (int h = 0; h < 2; ++h) {
-            const int i = 16 * m + 8 * h + g;
-            if (store && i < p.IW) {
-              const float x0a = bwd ? aux[m][nt][h].x : bias0, x0b = bwd ? aux[m][nt][h].y : bias1;
-              float unused;
-              float2 o;
-              o.x = c0 < p.cimg ? epilogue1(p.e, a[m][nt][2 * h], x0a, 0.f, &unused) : 0.f;
-              o.y = c0 + 1 < p.cimg ? epilogue1(p.e, a[m][nt][2 * h + 1], x0b, 0.f, &unused) : 0.f;
-              *reinterpret_cast<float2*>(orow + (size_t)(2 * i + (t >> 1) + p.out_xoff) * 4 + c0) = o;
-            }
-            a[m][nt][2 * h] = 0.f;
-            a[m][nt][2 * h + 1] = 0.f;
-          }
-        // margins of the pitched layout are zeros
-        const int nmargin = p.out_pitch - p.OW;
-        if (store && lane < nmargin) {
-          const int col = lane < p.out_xoff ? lane : p.OW + lane;
-          *reinterpret_cast<float4*>(orow + (size_t)col * 4) = make_float4(0.f, 0.f, 0.f, 0.f);
-        }
-      }
-    };
-
-    // one input row: PH = (r - (j0 - 1)) % 3 selects which register set belongs to which output-row pair.  All three
-    // targets are always accumulated (no branches around the MMAs: 10 independent accumulators per k-step hide the
-    // mma.sync latency with only two warps per scheduler); the set of a pair outside the band collects garbage and is
-    // zeroed, never stored, when its turn to be finalised comes.  The k-step loop is deliberately NOT fully unrolled:
-    // the fully unrolled kernel was 140 KB of code and spent 20 % of its issue slots on instruction-cache misses.
-    auto row_step = [&](int r, int buf, auto ph_tag) {
-      constexpr int PH = decltype(ph_tag)::value;
-      cp_async_wait<0>();
-      __syncwarp();                                   // row r has landed; every lane is done with the other buffer
-      if (r + 1 <= j1) stage_row(r + 1, buf ^ 1);
-      // derivative operand of the pair that completes after this row (prefetched: its latency hides behind the MMAs)
-      float2 aux[MT][2][2];
-      const int jf = r - 1;
-      const bool fin = jf >= j0 && jf < j1;
-      if (bwd && fin) {
-#pragma unroll
-        for (int nt = 0; nt < 2; ++nt) {
-          const float* arow = p.e.aux + ((size_t)b * p.OH + 2 * jf + nt) * p.out_pitch * 4;
-#pragma unroll
-          for (int m = 0; m < MT; ++m)
-#pragma unroll
-            for (int h = 0; h < 2; ++h) {
-              const int i = 16 * m + 8 * h + g;
-              aux[m][nt][h] = i < p.IW ? __ldg(reinterpret_cast<const float2*>(arow + (size_t)(2 * i + (t >> 1) + p.out_xoff) * 4 + c0))
-                                       : make_float2(0.f, 0.f);
-            }
-        }
-      }
-      if ((unsigned)r < (unsigned)p.IH) {
-        const uint32_t rb = rowbuf_u32 + buf * (N2_ROW_FLOATS * 4);
-        constexpr int kSetOf[3] = {(PH + 1) % 3, PH, (PH + 2) % 3};    // dy = -1, 0, +1  ->  pair j = r + 1, r, r - 1
-#pragma unroll
-        for (int dxi = 0; dxi < 3; ++dxi) {
-          const int swz = (lm_px + dxi) & 7;                            // low bits of the stored pixel index
-          const uint32_t abase = rb + (uint32_t)(lm_px + dxi) * 256u;
-          const float2* bsh = bfrag + (size_t)dxi * (EN_KSTEPS * 2 * 32) + lane;   // shift (dy, dx) at + dyi * 3 * 512
-#pragma unroll 2
-          for (int ks = 0; ks < EN_KSTEPS; ++ks) {
-            const int ck = 2 * ks + lm_half;
-            const uint32_t coff = (uint32_t)(((ck & 8) | ((ck ^ swz) & 7)) << 4);
-            uint32_t af[MT][4];
-#pragma unroll
-            for (int m = 0; m < MT; ++m) ldmatrix_x4(af[m], abase + (uint32_t)m * (16u * 256u) + coff);
-#pragma unroll
-            for (int dyi = 0; dyi < 3; ++dyi)
-#pragma unroll
-              for (int nt = 0; nt < 2; ++nt) {
-                if (!n2_need<KS>(nt, dyi)) continue;                    // compile time
-                const float2 bq = bsh[(size_t)dyi * (3 * EN_KSTEPS * 2 * 32) + (ks * 2 + nt) * 32];
-#pragma unroll
-                for (int m = 0; m < MT; ++m)
-                  mma_tf32(acc[kSetOf[dyi]][m][nt], af[m][0], af[m][1], af[m][2], af[m][3], __float_as_uint(bq.x),
-                           __float_as_uint(bq.y));
-              }
-          }
-        }
-      }
-      finalize(jf, fin, acc[(PH + 2) % 3], aux);      // store if the pair is in the band; zero the set either way
-    };
-
-    __syncwarp();                                     // previous job's reads of the row buffers are done
-    stage_row(j0 - 1, 0);
-    int buf = 0;
-    for (int r = j0 - 1; r <= j1; r += 3) {
-      row_step(r, buf, std::integral_constant<int, 0>());
-      buf ^= 1;
-      if (r + 1 > j1) break;
-      row_step(r + 1, buf, std::integral_constant<int, 1>());
-      buf ^= 1;
-      if (r + 2 > j1) break;
-      row_step(r + 2, buf, std::integral_constant<int, 2>());
-      buf ^= 1;
-    }
-    cp_async_wait<0>();
-  }
-}
-
-template <int KS, int MT>
-int launch_narrow2_inst(const EdgeNarrowParams& p, int warps, cudaStream_t st) {
-  const size_t smem = (size_t)N2_BFRAG * sizeof(float2) + (size_t)warps * 2 * N2_ROW_FLOATS * sizeof(float);
-  static DynSmemCache smem_cache;
-  cudaError_t e = ensure_dyn_smem(edge_narrow2_kernel<KS, MT>, smem, smem_cache);
-  if (e != cudaSuccess) return set_error(CGS_ERR_CUDA, "cudaFuncSetAttribute(edge_narrow2): %s", cudaGetErrorString(e));
-  const long long jobs = (long long)p.B * p.bands;
-  if (jobs >= (1ll << 31)) return set_error(CGS_ERR_UNSUPPORTED, "batch too large; split the batch");
-  long long grid = (jobs + warps - 1) / warps;
-  if (grid > device_num_sms()) grid = device_num_sms();
-  cudaError_t le = launch_pdl(edge_narrow2_kernel<KS, MT>, dim3((unsigned)grid), dim3(warps * 32), smem, st, p, (int)jobs);
-  count_launch();
-  if (le != cudaSuccess) return set_error(CGS_ERR_CUDA, "edge_narrow2_kernel: %s", cudaGetErrorString(le));
-  return check_launch("edge_narrow2_kernel");
-}
-
-// Rows per job and warps per CTA: as few bands as possible (a band re-reads two halo rows) while the jobs still fill
-// the machine in whole rounds.  Pure function of (batch, image height, SM count): never of the data.
-void narrow2_geometry(EdgeNarrowParams& p, int& warps) {
-  const int sms = device_num_sms();
-  double best = 1e30;
-  int best_bands = 1, best_w = 8;
-  for (int bands = 1; bands <= p.IH / 4 || bands == 1; bands *= 2) {
-    const int R = (p.IH + bands - 1) / bands;
-    const int nb = (p.IH + R - 1) / R;
-    const double per_job = 5.0 * R + 3.0 + 0.5 * (R + 2);           // MMA units of a band + staging of its rows
-    for (int w = 8; w >= 5; --w) {
-      const long long jobs = (long long)p.B * nb;
-      const long long slots = (long long)sms * w;
-      const long long rounds = (jobs + slots - 1) / slots;
-      const double cost = (double)rounds * per_job * (1.0 + 0.02 * (8 - w));   // a round takes a job's time
-      if (cost < best) { best = cost; best_bands = nb; best_w = w; p.R = R; }
-    }
-  }
-  p.bands = best_bands;
-  p.R = (p.IH + best_bands - 1) / best_bands;
-  warps = best_w;
-}
-
-// ---------------------------------------------------------------------------------------------
 // edge_pair: the narrow pass of one layer followed by the wide pass of the next on the same image, in one kernel:
 // forward   G's last deconv (-> image, tanh) + D's first conv (-> 64 channels, LeakyReLU)
 // backward  D's first conv data-gradient (x tanh') + G's last deconv data-gradient (x ReLU' / policy step)
@@ -841,17 +590,9 @@ int launch_edge_pair(EdgeNarrowParams pn, const EdgeWideParams& pw, int store_im
 
 int launch_edge_narrow(EdgeNarrowParams p, cudaStream_t st) {
   if (p.B <= 0) return CGS_OK;
-  // tcgen05 form with the input patch resident in shared memory (edge_tc.cu); CGS_DEBUG bit 2097152 keeps mma.sync
-  if (!(debug_flags() & 2097152) && p.IW >= 16 && edge_narrow_tc_supported(p)) return launch_edge_narrow_tc(p, st);
-  // gather form with register accumulators (edge_narrow2); CGS_DEBUG bit 262144 keeps the column-buffer kernel
-  // (rows narrower than 16 pixels leave half of every 16-row MMA tile empty: the MNIST-sized nets keep the other form)
-  if (!(debug_flags() & 262144) && p.K == 64 && p.pad_y == 1 && p.pad_x == 1 && p.IW >= 16 && p.IW <= 32 && (p.k == 4 || p.k == 5) &&
-      p.OW == 2 * p.IW && p.OH == 2 * p.IH && p.e.epi != EPI_UPDATE) {
-    int warps = 8;
-    narrow2_geometry(p, warps);
-    if (p.k == 5) return p.IW > 16 ? launch_narrow2_inst<5, 2>(p, warps, st) : launch_narrow2_inst<5, 1>(p, warps, st);
-    return p.IW > 16 ? launch_narrow2_inst<4, 2>(p, warps, st) : launch_narrow2_inst<4, 1>(p, warps, st);
-  }
+  // tcgen05 form with the input patch resident in shared memory (edge_tc.cu), else the column-buffer kernel
+  if (edge_narrow_tc_supported(p)) return launch_edge_narrow_tc(p, st);
+  if (p.s2d) return set_error(CGS_ERR_UNSUPPORTED, "s2d image layout needs the tcgen05 edge kernels");
   if (int rc = narrow_geometry(p)) return rc;
   if (p.k == 4 && p.cimg == 1) return launch_narrow_nt<2, 1>(p, st);
   if (p.k == 5 && p.cimg == 1) return launch_narrow_nt<4, 1>(p, st);

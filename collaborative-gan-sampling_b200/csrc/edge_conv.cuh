@@ -55,6 +55,8 @@ bool edge_wide_supported(int N, int k, int cimg);
 bool edge_narrow_supported(int K, int k, int cimg, int IW);
 int launch_edge_wide(const EdgeWideParams& p, cudaStream_t st);
 int launch_edge_narrow(EdgeNarrowParams p, cudaStream_t st);
+// the row widths the tcgen05 edge kernels take (narrow pass input = wide pass output = s2d grid width)
+bool edge_tc_width_supported(int w);
 // the same pass on tcgen05 with the input patch resident in shared memory (edge_tc.cu)
 bool edge_narrow_tc_supported(const EdgeNarrowParams& p);
 int launch_edge_narrow_tc(const EdgeNarrowParams& p, cudaStream_t st);

@@ -2,12 +2,14 @@
 // generator's last deconv forward, nsgan/ops.py:55, and the data-gradient of the discriminator's first conv,
 // sampling/collaborator.py:31) on the 5th-generation tensor cores, with the input PATCH RESIDENT in shared memory.
 //
-// Gather form (see edge_narrow2 in edge_conv.cu): for the input-grid point (j, i) the 4 output-parity classes x 4
-// padded channels are 16 GEMM columns and the reduction runs over (dy, dx, 64 channels), dy, dx in {-1, 0, 1}:
-//     acc[(j, i)][(py, px, c)] += in[j + dy][i + dx][:] . Wshift[dy][dx][:][(py, px, c)].
-// The legacy mma.sync path is throughput-bound on this part (one HMMA.1688.TF32 per ~23 cycles per SM sub-partition,
-// ~100 TFLOP/s chip-wide: profiles/round2_ncu_summary.md), so the 9x MMA inflation of the gather form made the
-// mma.sync kernels 4x slower than the HBM floor.  tcgen05 has the rate, and its shared-memory descriptors make the
+// Gather form: output pixel (2j + py, 2i + px) sums the taps (ky, kx) of matching parity; tap ky reads input row
+// j + dy with dy = (py + pad - ky) / 2 in {-1, 0, 1} (pad = 1 for k = 4 and k = 5 under TF SAME), likewise dx.  So for
+// the input-grid point (j, i) the 4 output-parity classes x 4 padded channels are 16 GEMM columns and the reduction
+// runs over (dy, dx, 64 channels):
+//     acc[(j, i)][(py, px, c)] += in[j + dy][i + dx][:] . Wshift[dy][dx][:][(py, px, c)],
+// with Wshift zero where a class has no tap at that shift.  mma.sync is throughput-bound on this part (one
+// HMMA.1688.TF32 per ~23 cycles per SM sub-partition, ~100 TFLOP/s chip-wide: profiles/round2_ncu_summary.md), so the
+// 9x MMA inflation of the gather form made an mma.sync version of it 4x slower than the HBM floor (it was removed).  tcgen05 has the rate, and its shared-memory descriptors make the
 // nine shifted A operands FREE: a band of input rows (+ one halo row / column each side, zero-filled by TMA) is loaded
 // once as [pixel][32 channels] 128-byte rows (SWIZZLE_128B, two channel halves); the A tile of shift (dy, dx) for the
 // 128 "virtual pixels" v .. v+127 is the same memory starting (1 + dy) * pitch + (1 + dx) rows later -- a descriptor
@@ -259,8 +261,10 @@ PFN_encodeTiledTc encode_fn() {
 
 }  // namespace
 
+bool edge_tc_width_supported(int w) { return w == 16 || w == 32 || w == 64; }
+
 bool edge_narrow_tc_supported(const EdgeNarrowParams& p) {
-  return p.K == 64 && p.pad_y == 1 && p.pad_x == 1 && (p.IW == 16 || p.IW == 32 || p.IW == 64) && (p.k == 4 || p.k == 5) &&
+  return p.K == 64 && p.pad_y == 1 && p.pad_x == 1 && edge_tc_width_supported(p.IW) && (p.k == 4 || p.k == 5) &&
          p.OW == 2 * p.IW && p.OH == 2 * p.IH && p.e.epi != EPI_UPDATE && p.cimg >= 1 && p.cimg <= 3;
 }
 
@@ -354,10 +358,10 @@ constexpr int WT_B_BYTES = 5 * 64 * 128;          // 18 k-steps of 8 floats -> f
 constexpr int WT_PITCH = 20;                      // floats per staged row of the epilogue transpose
 constexpr int WT_EPI_BYTES = WT_EPI_WARPS * 2 * 32 * WT_PITCH * 4;   // two staging tiles per warp
 
-// CTA-0 event trace (CGS_DEBUG bit 256): g_tc_trace[role][tile] = clock; dumped by cgs_debug_trace_tc
+// CTA-0 event trace (CGS_DEBUG_TRACE): g_tc_trace[role][tile] = clock; dumped by cgs_debug_trace_tc
 __device__ long long g_tc_trace[8][64];
 __device__ __forceinline__ void tc_trace(int debug, int role, unsigned tile) {
-  if ((debug & 256) && blockIdx.x == 0 && tile < 64) g_tc_trace[role][tile] = clock64();
+  if ((debug & CGS_DEBUG_TRACE) && blockIdx.x == 0 && tile < 64) g_tc_trace[role][tile] = clock64();
 }
 
 struct WideTcParams {
@@ -445,7 +449,7 @@ edge_wide_tc_kernel(const __grid_constant__ WideTcParams q, const __grid_constan
         if (++stage == (uint32_t)q.nstages) { stage = 0; phase ^= 1u; }
         mbar_wait(&empty_bar[s], ph ^ 1);
         tc_trace(ep.debug, 0, (unsigned)((tile - blockIdx.x) / gridDim.x));
-        if (ep.debug & 8) { mbar_arrive(&full_bar[s]); continue; }            // profiling knob: no loads
+        if (ep.debug & CGS_DEBUG_SKIP_A_TMA) { mbar_arrive(&full_bar[s]); continue; }   // profiling knob: no loads
         mbar_arrive_expect_tx(&full_bar[s], bytes);
         tma_load_4d(smem_u32(smem_a) + s * q.stage_bytes, &tmap_in, &full_bar[s], 0, -1, j0 - 1, b);
       }
@@ -466,7 +470,7 @@ edge_wide_tc_kernel(const __grid_constant__ WideTcParams q, const __grid_constan
         if (++stage == (uint32_t)q.nstages) { stage = 0; phase ^= 1u; }
         tcgen05_fence_after();
         const uint64_t da_stage = da0 + (uint64_t)((s * (uint32_t)q.stage_bytes) >> 4);
-        const bool no_mma = (ep.debug & 4) != 0;                              // profiling knob
+        const bool no_mma = (ep.debug & CGS_DEBUG_SKIP_MMA) != 0;             // profiling knob
         for (int mt = 0; mt < q.MT; ++mt) {
           const uint32_t tmem_d = tmem_base + (acc * TC_MAX_MT + mt) * 64;
           const uint64_t da_mt = da_stage + (uint64_t)(mt * ((128 * 64) >> 4));
@@ -519,7 +523,7 @@ edge_wide_tc_kernel(const __grid_constant__ WideTcParams q, const __grid_constan
           if (EPI == EPI_BWD) {
 #pragma unroll
             for (int ps = 0; ps < 4; ++ps)
-              x0[ch][ps] = (ro[ps] >= 0 && !(ep.debug & 2048)) ? __ldg(reinterpret_cast<const float4*>(ep.aux + ro[ps] + n))
+              x0[ch][ps] = (ro[ps] >= 0 && !(ep.debug & CGS_DEBUG_NO_PREFETCH)) ? __ldg(reinterpret_cast<const float4*>(ep.aux + ro[ps] + n))
                                                               : make_float4(1.f, 1.f, 1.f, 1.f);   // knob 2048: no operand loads
           } else if (EPI == EPI_FWD) {
             x0[ch][0] = ep.bias ? __ldg(reinterpret_cast<const float4*>(ep.bias + n)) : make_float4(0.f, 0.f, 0.f, 0.f);
@@ -566,7 +570,7 @@ edge_wide_tc_kernel(const __grid_constant__ WideTcParams q, const __grid_constan
                   if (!ep.sgd && !ep.first) xb = *reinterpret_cast<const float4*>(ep.mom + ro[ps] + n);
                 }
                 const float4 o = epilogue4_t<EPI>(ep, ro[ps] + n, v, xa, xb);
-                if (!(ep.debug & 1024)) *reinterpret_cast<float4*>(ep.out + ro[ps] + n) = o;      // knob 1024: no stores
+                if (!(ep.debug & CGS_DEBUG_SKIP_STORES)) *reinterpret_cast<float4*>(ep.out + ro[ps] + n) = o;
               }
             }
           }
@@ -625,7 +629,7 @@ int debug_trace_tc(long long* out_host) {
 
 bool edge_wide_tc_supported(const EdgeWideParams& p) {
   return p.N == 64 && p.ON == 64 && (p.k == 4 || p.k == 5) && p.cimg >= 1 && p.cimg <= 3 && p.pad_y == 1 && p.pad_x == 1 &&
-         (p.IH % 2) == 0 && p.OH * 2 == p.IH && (p.OW == 16 || p.OW == 32 || p.OW == 64);
+         (p.IH % 2) == 0 && p.OH * 2 == p.IH && edge_tc_width_supported(p.OW);
 }
 
 // p.in must be the s2d form of the image-like input; p.pitch / p.xoff are ignored

@@ -484,7 +484,7 @@ extern "C" int cgs_refine_mlp2d(const cgs_mlp_desc* d, const cgs_refine2d_cfg* c
   if (n == 0) return CGS_OK;
   if (!x_in || !best_x || !best_loss || !best_step) return set_error(CGS_ERR_INVALID, "null argument");
   const int64_t n_mean = cfg->n_mean > 0 ? cfg->n_mean : n;
-  if (!(debug_flags() & 134217728)) {
+  if (!(debug_flags() & CGS_DEBUG_MLP2D_ONE_THREAD)) {
     // split form: four threads per point; the points are dealt evenly over the SMs (at most 96 per CTA round)
     const int sms = device_num_sms();
     int64_t ppb64 = (n + sms - 1) / sms;

@@ -334,7 +334,7 @@ inline int fc_split(const cgs_layer_desc& L, bool backward) {
 }
 
 inline bool use_fc_split(const cgs_layer_desc& L, bool backward, int64_t B, int math, const float* scratch) {
-  return fc_split(L, backward) > 1 && math == CGS_MATH_TF32_TENSOR && scratch && !(debug_flags() & 16384) &&
+  return fc_split(L, backward) > 1 && math == CGS_MATH_TF32_TENSOR && scratch && !(debug_flags() & CGS_DEBUG_NO_FC_SPLIT) &&
          ((B + 127) / 128) * ((L.cout + 255) / 256) * fc_split(L, backward) <= 2 * 148;
 }
 
@@ -464,8 +464,8 @@ EdgeEpi make_edge_epi(const PassEpi& e, const float* bias) {
   return x;
 }
 
-// CGS_DEBUG bit 4096 (or cgs_debug_set_flags): keep the image-edge passes on the general tcgen05 lowerings
-bool edge_kernels_enabled() { return !(debug_flags() & 4096); }
+// CGS_DEBUG_EDGE_GENERAL: keep the image-edge passes on the general tcgen05 lowerings
+bool edge_kernels_enabled() { return !(debug_flags() & CGS_DEBUG_EDGE_GENERAL); }
 
 int launch_gemm(const ConvGemmParams& p, const float* w, int rows, int cols, int math, cudaStream_t stream) {
   if (math == CGS_MATH_FP32_SIMT) return launch_conv_gemm_simt(p, w, rows, cols, stream);
@@ -558,7 +558,7 @@ bool make_edge_wide(const cgs_layer_desc& L, bool backward, int64_t B, const flo
 // Returns 1 when the pair was launched, 0 when the caller should run the two passes separately, < 0 on error.
 int try_edge_pair(const cgs_layer_desc& ln, const cgs_layer_desc& lw, bool backward, int64_t B, const float* in,
                   float* mid, float* out, const PassEpi& en, const PassEpi& ew, int store_mid, int math, cudaStream_t st) {
-  if (math != CGS_MATH_TF32_TENSOR || (debug_flags() & 65536) || en.upd) return 0;
+  if (math != CGS_MATH_TF32_TENSOR || (debug_flags() & CGS_DEBUG_NO_EDGE_PAIR) || en.upd) return 0;
   if (!use_scatter(ln, backward) || !use_window(lw, backward)) return 0;
   EdgeNarrowParams qn;
   if (!make_edge_narrow(ln, backward, B, in, mid, en, false, backward ? ln.kcols_bwd : ln.kcols_fwd, qn)) return 0;
@@ -973,17 +973,17 @@ static int build_chain(const cgs_net_desc* gtail, const cgs_net_desc* d, Chain& 
 }
 
 // Image-like tensors of the chain live in the s2d layout when both image-edge layers run on the tcgen05 edge kernels
-// (edge_tc.cu): G's last deconv (64 -> <= 3 channels) and D's first conv (<= 3 -> 64 channels), rows of >= 16 pixels.
-// CGS_DEBUG bits 4096 (general lowerings) and 2097152 (mma.sync edge kernels) keep the pitched layout.
+// (edge_tc.cu): G's last deconv (64 -> <= 3 channels) and D's first conv (<= 3 -> 64 channels), on a row width those
+// kernels take.  CGS_DEBUG_EDGE_GENERAL keeps the pitched layout.
 static bool chain_s2d(const Chain& c, int math) {
-  if (math != CGS_MATH_TF32_TENSOR || (debug_flags() & (4096 | 2097152))) return false;
+  if (math != CGS_MATH_TF32_TENSOR || !edge_kernels_enabled()) return false;
   if (c.n_gtail < 1 || c.n_gtail >= c.n) return false;
   const cgs_layer_desc& Ln = c.layers[c.n_gtail - 1];
   const cgs_layer_desc& Lw = c.layers[c.n_gtail];
   if (Ln.type != CGS_LAYER_DECONV || Lw.type != CGS_LAYER_CONV) return false;
   if (Ln.cin != 64 || Ln.cout > 3 || Lw.cout != 64 || Lw.cin != Ln.cout) return false;
   if ((Ln.k != 4 && Ln.k != 5) || (Lw.k != 4 && Lw.k != 5)) return false;
-  if (Ln.win < 16 || Ln.win > 64 || Ln.hin != Ln.win || Lw.hin != 2 * Ln.hin || Lw.win != 2 * Ln.win) return false;
+  if (!edge_tc_width_supported(Ln.win) || Ln.hin != Ln.win || Lw.hin != 2 * Ln.hin || Lw.win != 2 * Ln.win) return false;
   if (same_pad_before(Lw.hin, Lw.k) != 1 || same_pad_before(2 * Ln.hin, Ln.k) != 1) return false;
   return true;
 }
@@ -1030,10 +1030,10 @@ static void carve(const Chain& c, int64_t B, void* base, Workspace& w) {
 }
 
 // The last hidden layer runs split-K and nothing but the head reads its output: the head kernel then adds the partial
-// sums itself and the activation is never written (CGS_DEBUG bit 131072 keeps the separate reduce kernel).
+// sums itself and the activation is never written (CGS_DEBUG_NO_HEAD_PARTIALS keeps the separate reduce kernel).
 static bool head_takes_partials(const Chain& c, const Workspace& w, int64_t B, int math) {
   const cgs_layer_desc& L = c.layers[c.n - 1];
-  return use_fc_split(L, false, B, math, w.col) && !(debug_flags() & 131072) && cstride(L.cout) == c.head.cin;
+  return use_fc_split(L, false, B, math, w.col) && !(debug_flags() & CGS_DEBUG_NO_HEAD_PARTIALS) && cstride(L.cout) == c.head.cin;
 }
 
 static int run_forward(const Chain& c, const Workspace& w, int64_t B, int math, cudaStream_t st,
@@ -1361,7 +1361,7 @@ static int layer_pass_dense(const cgs_layer_desc& L, bool backward, int math, in
     // the image-like input is re-laid out first (inside the chain it is produced in that layout: no copy there)
     ConvGemmParams wp;
     EdgeWideParams q;
-    const bool tc = math == CGS_MATH_TF32_TENSOR && !(debug_flags() & (4096 | 2097152)) && w >= 32 && w <= 128 &&
+    const bool tc = math == CGS_MATH_TF32_TENSOR && edge_kernels_enabled() && w >= 32 && w <= 128 &&
                     make_window_params(L, backward, B, in, out, wp) == CGS_OK && make_edge_wide(L, backward, B, in, out, e, wp, q) &&
                     edge_wide_tc_supported(q);
     if (tc) {

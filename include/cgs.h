@@ -248,22 +248,45 @@ CGS_API int cgs_layer_backward(const cgs_layer_desc* L, int math, int64_t B, con
                                const float* x_fwd, int prev_act, void* workspace, size_t workspace_bytes,
                                cgs_stream_t stream);
 
-/* Developer aid: read (and reset) the CTA-0 pipeline event trace recorded when env CGS_DEBUG has bit 256 set. */
+/* Developer knobs (env CGS_DEBUG at first use, or cgs_debug_set_flags): a bit set of the values below.
+ * A lowering knob picks another implementation of the same pass; every one of them gives the same results
+ * (bit-identical or within the stated tolerance, see tests/test_conv_gpu.py).  A profiling knob skips part of the
+ * work to bound where time goes: its results are wrong by design. */
+enum cgs_debug_flag {
+  /* profiling */
+  CGS_DEBUG_SKIP_A_GATHER = 1,            /* tcgen05 GEMM in gather mode: no A-tile copies */
+  CGS_DEBUG_SKIP_WEIGHT_TMA = 2,          /* tcgen05 GEMM: no weight-tile loads */
+  CGS_DEBUG_SKIP_MMA = 4,                 /* tcgen05 GEMM / edge_wide_tc: no MMA issue */
+  CGS_DEBUG_SKIP_A_TMA = 8,               /* tcgen05 GEMM: no A-tile loads; edge_wide_tc: no patch loads */
+  CGS_DEBUG_SKIP_EPILOGUE = 16,           /* tcgen05 GEMM: no epilogue work after the TMEM loads */
+  CGS_DEBUG_TRACE = 256,                  /* CTA-0 event trace (cgs_debug_trace, cgs_debug_trace_tc) */
+  CGS_DEBUG_GATHER_A = 512,               /* tcgen05 GEMM: cp.async gather of the A tiles instead of TMA boxes */
+  CGS_DEBUG_SKIP_STORES = 1024,           /* tcgen05 GEMM / edge_wide_tc: no output stores */
+  CGS_DEBUG_NO_PREFETCH = 2048,           /* tcgen05 GEMM: no epilogue operand prefetch; edge_wide_tc: no operand loads */
+  /* lowering choices */
+  CGS_DEBUG_EDGE_GENERAL = 4096,          /* image-edge passes on the general tcgen05 lowerings, not csrc/edge_*.cu */
+  CGS_DEBUG_NO_FC_SPLIT = 16384,          /* no split-K on the long fc forward */
+  CGS_DEBUG_PDL_ON = 32768,               /* programmatic dependent launch on everywhere (default: per refinement call) */
+  CGS_DEBUG_NO_EDGE_PAIR = 65536,         /* image-edge passes as separate kernels instead of the paired kernel */
+  CGS_DEBUG_NO_HEAD_PARTIALS = 131072,    /* separate split-K reduce kernel before the head */
+  CGS_DEBUG_NO_FUSION = 524288,           /* no class-fused tcgen05 tiles for the transposed-type passes */
+  CGS_DEBUG_FORCE_FUSION = 1048576,       /* class-fused tiles whenever legal, whatever the tile count */
+  CGS_DEBUG_NO_MTILE_PAIRS = 4194304,     /* no M-tile pairs (two M tiles per CTA sharing the weight atoms) */
+  CGS_DEBUG_FORCE_MTILE_PAIRS = 8388608,  /* M-tile pairs whenever legal */
+  CGS_DEBUG_NO_CTA_PAIRS = 16777216,      /* no CTA pairs (clusters of two, tcgen05 cta_group::2) */
+  CGS_DEBUG_FORCE_CTA_PAIRS = 33554432,   /* CTA pairs whenever legal */
+  CGS_DEBUG_MLP2D_ONE_THREAD = 134217728, /* 2-D refinement with one thread per point, not the four-thread split form */
+  CGS_DEBUG_PDL_OFF = 536870912           /* programmatic dependent launch off everywhere (wins over PDL_ON) */
+  /* retired, never reused: 262144, 2097152 */
+};
+
+/* Developer aid: read (and reset) the CTA-0 pipeline event trace recorded under CGS_DEBUG_TRACE. */
 CGS_API int cgs_debug_trace(unsigned long long* out_host, int capacity);
-/* Developer aid: CTA-0 event clocks of the last edge_wide_tc launch run with CGS_DEBUG bit 256 ([8 roles][64 tiles] int64). */
+/* Developer aid: CTA-0 event clocks of the last edge_wide_tc launch run under CGS_DEBUG_TRACE ([8 roles][64 tiles] int64). */
 CGS_API int cgs_debug_trace_tc(long long* out_host);
 /* Developer aid OUTSIDE the drop-in contract (process-wide atomic; the product never calls it -- only the parity
- * tests do, to keep alternative lowerings covered): replace the CGS_DEBUG knobs at run time; returns the previous
- * value.  Every lowering a knob selects produces the same results (bit-identical or within the stated tolerance, see
- * tests/test_conv_gpu.py).  Bit 4096 routes the image-edge
- * passes (first D conv / last G deconv and their data-gradients) through the general tcgen05 lowerings instead of
- * the fused streaming kernels of csrc/edge_conv.cu; 65536 runs the edge passes as separate kernels instead of the
- * paired ones; 16384 disables split-K on the long fc forward; 32768 forces programmatic dependent launch on everywhere / 536870912 off
- * (default: per refinement call, from its average work per launch); 262144
- * keeps the column-buffer form of the narrow edge kernel; 524288 disables / 1048576 forces the class-fused tcgen05
- * tiles of the transposed-type passes; 4194304 disables / 8388608 forces M-tile pairs; 16777216 disables / 33554432
- * forces CTA pairs (clusters of two, tcgen05 cta_group::2); 134217728 runs the 2-D refinement with one thread per
- * point instead of the four-thread split form (bit-identical). */
+ * tests do, to keep alternative lowerings covered): replace the CGS_DEBUG knobs (cgs_debug_flag) at run time;
+ * returns the previous value. */
 CGS_API int cgs_debug_set_flags(int flags);
 
 #ifdef __cplusplus

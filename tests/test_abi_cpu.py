@@ -26,6 +26,21 @@ def test_every_declared_symbol_is_exported(cgs_lib):
     assert cgs_lib.cgs_version() == 1
 
 
+def declared_debug_flags():
+    text = open(os.path.join(ROOT, "include", "cgs.h")).read()
+    body = re.search(r"enum cgs_debug_flag \{(.*?)\};", text, re.S).group(1)
+    return {name: int(v) for name, v in re.findall(r"\bCGS_(DEBUG_[A-Z0-9_]+)\s*=\s*(\d+)", body)}
+
+
+def test_debug_flags_mirror_the_header():
+    from cgs import lib
+    flags = declared_debug_flags()
+    assert len(flags) >= 20 and len(set(flags.values())) == len(flags)
+    assert all(v & (v - 1) == 0 for v in flags.values())          # one bit each
+    mirrored = {n: getattr(lib, n) for n in dir(lib) if n.startswith("DEBUG_") and isinstance(getattr(lib, n), int)}
+    assert mirrored == flags
+
+
 def test_sass_is_blackwell_native():
     import subprocess
     so = os.path.join(ROOT, "collaborative-gan-sampling_b200", "cgs", "libcgs.so")

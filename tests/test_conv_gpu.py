@@ -29,12 +29,26 @@ def pad_c(x, cs):
     return out
 
 
+def _refine(spec, h0, flags, K=3):
+    """K refinement steps of h0 under the CGS_DEBUG knobs `flags`: (refined, optimal_logit, current_feature,
+    optimal_step)."""
+    from cgs import lib as L
+    from cgs import nets as N
+    from sampling.collaborator import Refiner
+    with L.debug_flags(flags):
+        r = Refiner(K, 0.1)
+        r.set_env(N.discriminator_spec(spec), N.feature_to_data_spec(spec), N.loss_refine)
+        x = r.build_refiner(h0)
+        torch.cuda.synchronize()
+        return x.clone(), r.optimal_logit.clone(), r.current_feature.clone(), r.optimal_step.clone()
+
+
 @pytest.fixture
 def general_lowering(cgs_lib):
-    """Route the image-edge passes through the general tcgen05 lowerings (CGS_DEBUG bit 4096) for one test."""
-    old = cgs_lib.cgs_debug_set_flags(4096)
-    yield
-    cgs_lib.cgs_debug_set_flags(old)
+    """Route the image-edge passes through the general tcgen05 lowerings (DEBUG_EDGE_GENERAL) for one test."""
+    from cgs import lib as L
+    with L.debug_flags(L.DEBUG_EDGE_GENERAL):
+        yield
 
 
 @pytest.mark.parametrize("arch_name,B", [("mnist", 5), ("mnist", 67), ("dcgan64_l2", 2)])
@@ -45,10 +59,10 @@ def test_edge_layers_general_lowering(cgs_lib, cuda_device, general_lowering, ar
 
 @pytest.fixture
 def forced_fusion(cgs_lib):
-    """Class-fused tcgen05 tiles whenever they are legal (CGS_DEBUG bit 1048576), whatever the tile count."""
-    old = cgs_lib.cgs_debug_set_flags(1048576)
-    yield
-    cgs_lib.cgs_debug_set_flags(old)
+    """Class-fused tcgen05 tiles whenever they are legal (DEBUG_FORCE_FUSION), whatever the tile count."""
+    from cgs import lib as L
+    with L.debug_flags(L.DEBUG_FORCE_FUSION):
+        yield
 
 
 @pytest.mark.parametrize("arch_name,B", [("dcgan32_l1", 3), ("dcgan32_l2", 40), ("dcgan64_l2", 9), ("dcgan64_l1", 2)])
@@ -63,83 +77,50 @@ def test_layers_class_fused_tiles(cgs_lib, cuda_device, forced_fusion, arch_name
 def test_class_fusion_is_bit_identical(cgs_lib, cuda_device, arch_name, B, gain):
     """Fused tiles accumulate every class in the same (tap, channel block) order as the one-class tiles, so the choice
     (which depends on the tile count, i.e. on the batch) never changes a bit: shard invariance is preserved."""
-    from cgs import nets as N
-    from sampling.collaborator import Refiner
+    from cgs import lib as L
     arch, w, spec = _make(arch_name, 5, gain, cuda_device, "tf32")
     h0 = torch.relu(torch.randn(B, *arch["feature_shape"], generator=torch.Generator().manual_seed(4))).to(cuda_device)
 
-    def run(flags):
-        old = cgs_lib.cgs_debug_set_flags(flags)
-        try:
-            r = Refiner(3, 0.1)
-            r.set_env(N.discriminator_spec(spec), N.feature_to_data_spec(spec), N.loss_refine)
-            x = r.build_refiner(h0)
-            torch.cuda.synchronize()
-            return x.clone(), r.optimal_logit.clone(), r.current_feature.clone()
-        finally:
-            cgs_lib.cgs_debug_set_flags(old)
-
-    fused, plain = run(1048576), run(524288)
+    fused, plain = _refine(spec, h0, L.DEBUG_FORCE_FUSION), _refine(spec, h0, L.DEBUG_NO_FUSION)
     assert all(torch.equal(a, b) for a, b in zip(fused, plain))
 
 
 @pytest.mark.parametrize("arch_name,B,gain", [("mnist", 40, 3.0), ("mnist", 300, 3.0), ("dcgan32_l2", 7, 2.5), ("dcgan64_l1", 3, 2.5),
                                                ("dcgan32_l1", 1024, 2.5)])
 def test_m_tile_pairs_are_bit_identical(cgs_lib, cuda_device, arch_name, B, gain):
-    """Two M tiles per CTA sharing the weight atoms (CGS_DEBUG 8388608 forces them, 4194304 forbids them): every
-    accumulator sees the same MMA sequence, so the results are bit-identical, incl. odd tile counts (half-empty last
-    pair) and several pairs per CTA."""
-    from cgs import nets as N
-    from sampling.collaborator import Refiner
+    """Two M tiles per CTA sharing the weight atoms (DEBUG_FORCE_MTILE_PAIRS forces them, DEBUG_NO_MTILE_PAIRS forbids
+    them): every accumulator sees the same MMA sequence, so the results are bit-identical, incl. odd tile counts
+    (half-empty last pair) and several pairs per CTA."""
+    from cgs import lib as L
     arch, w, spec = _make(arch_name, 5, gain, cuda_device, "tf32")
     h0 = torch.relu(torch.randn(B, *arch["feature_shape"], generator=torch.Generator().manual_seed(4))).to(cuda_device)
 
-    def run(flags):
-        old = cgs_lib.cgs_debug_set_flags(flags)
-        try:
-            r = Refiner(3, 0.1)
-            r.set_env(N.discriminator_spec(spec), N.feature_to_data_spec(spec), N.loss_refine)
-            x = r.build_refiner(h0)
-            torch.cuda.synchronize()
-            return x.clone(), r.optimal_logit.clone(), r.current_feature.clone()
-        finally:
-            cgs_lib.cgs_debug_set_flags(old)
-
-    paired, single = run(8388608 | 524288), run(4194304 | 524288)      # class fusion off in both: pairs everywhere legal
+    # class fusion off in both: pairs everywhere legal
+    paired = _refine(spec, h0, L.DEBUG_FORCE_MTILE_PAIRS | L.DEBUG_NO_FUSION)
+    single = _refine(spec, h0, L.DEBUG_NO_MTILE_PAIRS | L.DEBUG_NO_FUSION)
     assert all(torch.equal(a, b) for a, b in zip(paired, single))
-    default = run(0)
+    default = _refine(spec, h0, 0)
     assert all(torch.equal(a, b) for a, b in zip(default, single))
 
 
 @pytest.mark.parametrize("arch_name,B,gain", [("dcgan32_l2", 7, 2.5), ("dcgan64_l1", 3, 2.5), ("dcgan64_l3", 5, 2.5),
                                                ("dcgan32_l1", 1024, 2.5), ("dcgan32_l2", 601, 2.5)])
 def test_cta_pairs_are_bit_identical(cgs_lib, cuda_device, arch_name, B, gain):
-    """CTA pairs (cluster of two, tcgen05 cta_group::2, M = 256; CGS_DEBUG 33554432 forces them, 16777216 forbids them):
-    every accumulator row sees the same K order as in a single-CTA tile, so the results are bit-identical -- with
-    class-fused tiles and 256-wide tiles, odd tile counts (the pair's second tile past the batch) and several units per
-    pair."""
-    from cgs import nets as N
-    from sampling.collaborator import Refiner
+    """CTA pairs (cluster of two, tcgen05 cta_group::2, M = 256; DEBUG_FORCE_CTA_PAIRS forces them, DEBUG_NO_CTA_PAIRS
+    forbids them): every accumulator row sees the same K order as in a single-CTA tile, so the results are
+    bit-identical -- with class-fused tiles and 256-wide tiles, odd tile counts (the pair's second tile past the batch)
+    and several units per pair."""
+    from cgs import lib as L
     arch, w, spec = _make(arch_name, 5, gain, cuda_device, "tf32")
     h0 = torch.relu(torch.randn(B, *arch["feature_shape"], generator=torch.Generator().manual_seed(4))).to(cuda_device)
 
-    def run(flags):
-        old = cgs_lib.cgs_debug_set_flags(flags)
-        try:
-            r = Refiner(3, 0.1)
-            r.set_env(N.discriminator_spec(spec), N.feature_to_data_spec(spec), N.loss_refine)
-            x = r.build_refiner(h0)
-            torch.cuda.synchronize()
-            return x.clone(), r.optimal_logit.clone(), r.current_feature.clone()
-        finally:
-            cgs_lib.cgs_debug_set_flags(old)
-
-    paired, single = run(33554432 | 1048576), run(16777216 | 1048576)   # class fusion forced in both
+    paired = _refine(spec, h0, L.DEBUG_FORCE_CTA_PAIRS | L.DEBUG_FORCE_FUSION)   # class fusion forced in both
+    single = _refine(spec, h0, L.DEBUG_NO_CTA_PAIRS | L.DEBUG_FORCE_FUSION)
     assert all(torch.equal(a, b) for a, b in zip(paired, single))
-    default = run(0)
+    default = _refine(spec, h0, 0)
     assert all(torch.equal(a, b) for a, b in zip(default, single))
     # M-tile pairs INSIDE CTA pairs (units of four M tiles; class fusion off so the 128-wide passes take them)
-    quad = run(33554432 | 8388608 | 524288)
+    quad = _refine(spec, h0, L.DEBUG_FORCE_CTA_PAIRS | L.DEBUG_FORCE_MTILE_PAIRS | L.DEBUG_NO_FUSION)
     assert all(torch.equal(a, b) for a, b in zip(quad, single))
 
 
@@ -225,7 +206,10 @@ def test_forward_logits_and_grad(cgs_lib, cuda_device, arch_name, B, gain, math)
                                                         ("dcgan64_l1", 2, 3, "momentum", 2.5),
                                                         # refinement at the last map: the policy step is fused into the
                                                         # wide image-edge pass (edge_wide_tc EPI_UPDATE in TF32 mode)
-                                                        ("dcgan32_l4", 5, 3, "momentum", 2.5), ("dcgan64_l4", 2, 2, "sgd", 2.5)])
+                                                        ("dcgan32_l4", 5, 3, "momentum", 2.5), ("dcgan64_l4", 2, 2, "sgd", 2.5),
+                                                        # 24-pixel rows at the image edge: no tcgen05 edge kernel takes
+                                                        # them, the chain keeps the pitched image layout
+                                                        ("dcgan48_l1", 2, 3, "momentum", 2.5)])
 def test_build_refiner_matches_oracle(cgs_lib, cuda_device, arch_name, B, K, method, gain, math):
     from cgs import nets as N
     from sampling.collaborator import Refiner
@@ -299,35 +283,24 @@ def test_cuda_graph_replay_is_bit_identical(cgs_lib, cuda_device):
 
 
 def test_launch_and_lowering_knobs_do_not_change_results(cgs_lib, cuda_device):
-    """Programmatic dependent launch (bit 32768) and where the split-K partial sums are added (head kernel or a separate
-    reduce kernel, bit 131072) change nothing: bit-identical.  The fc split-K lowering (off with
-    bit 16384), the fused edge kernels (off with bit 4096) and their pairing into one kernel (off with bit 65536) only
-    change summation order or nothing at all: same refined batch within the TF32 tolerance and the same best step for
-    nearly every sample."""
-    from cgs import nets as N
-    from sampling.collaborator import Refiner
+    """Programmatic dependent launch (DEBUG_PDL_ON) and where the split-K partial sums are added (head kernel or a
+    separate reduce kernel, DEBUG_NO_HEAD_PARTIALS) change nothing: bit-identical.  The fc split-K lowering (off with
+    DEBUG_NO_FC_SPLIT), the fused edge kernels (off with DEBUG_EDGE_GENERAL) and their pairing into one kernel (off with
+    DEBUG_NO_EDGE_PAIR) only change summation order or nothing at all: same refined batch within the TF32 tolerance and
+    the same best step for nearly every sample."""
+    from cgs import lib as L
     arch, w, spec = _make("mnist", 5, 3.0, cuda_device, "tf32")
     h0 = torch.relu(torch.randn(40, *arch["feature_shape"], generator=torch.Generator().manual_seed(4))).to(cuda_device)
 
-    def run(flags):
-        old = cgs_lib.cgs_debug_set_flags(flags)
-        try:
-            r = Refiner(5, 0.1)
-            r.set_env(N.discriminator_spec(spec), N.feature_to_data_spec(spec), N.loss_refine)
-            x = r.build_refiner(h0)
-            torch.cuda.synchronize()
-            return x.clone(), r.optimal_logit.clone(), r.optimal_step.clone()
-        finally:
-            cgs_lib.cgs_debug_set_flags(old)
-
-    base = run(0)
-    for same in (32768, 131072):                             # PDL; separate split-K reduce kernel instead of the head's
-        assert all(torch.equal(a, b) for a, b in zip(base, run(same))), same
-    for flags in (16384, 4096, 65536, 16384 | 4096):         # 65536: the two edge pairs as four separate kernels
-        x, logit, step = run(flags)
+    base = _refine(spec, h0, 0, K=5)
+    for same in (L.DEBUG_PDL_ON, L.DEBUG_NO_HEAD_PARTIALS):  # PDL; separate split-K reduce kernel instead of the head's
+        assert all(torch.equal(a, b) for a, b in zip(base, _refine(spec, h0, same, K=5))), same
+    # DEBUG_NO_EDGE_PAIR: the two edge pairs as four separate kernels
+    for flags in (L.DEBUG_NO_FC_SPLIT, L.DEBUG_EDGE_GENERAL, L.DEBUG_NO_EDGE_PAIR, L.DEBUG_NO_FC_SPLIT | L.DEBUG_EDGE_GENERAL):
+        x, logit, _, step = _refine(spec, h0, flags, K=5)
         assert rel_l2(x.cpu().numpy(), base[0].cpu().numpy()) <= 1e-2
         assert float((logit - base[1]).abs().max()) <= 1.5e-2
-        assert float((step == base[2]).float().mean()) >= 0.9
+        assert float((step == base[3]).float().mean()) >= 0.9
 
 
 def test_mnist_layer2_and_chunked_batches(cgs_lib, cuda_device, monkeypatch):
@@ -402,6 +375,7 @@ def test_early_exit_is_identical_across_tile_lowerings(cgs_lib, cuda_device, arc
     and M-tile pairs inside CTA pairs all read the live-image count and schedule tiles from it; units whose second /
     third / fourth M tile lies past the live images must neither be stored nor disturb the others.  Same bits as the
     plain one-tile-per-CTA lowering, eager and replayed as a CUDA graph."""
+    from cgs import lib as L
     from cgs import nets as N
     from sampling.collaborator import Refiner
     arch, w, spec = _make(arch_name, 9, 2.5, cuda_device, "tf32")
@@ -412,21 +386,19 @@ def test_early_exit_is_identical_across_tile_lowerings(cgs_lib, cuda_device, arc
     thr = float(torch.median(probe.optimal_logit))            # about half of the batch has left by step K / 2
 
     def run(flags, graph):
-        old = cgs_lib.cgs_debug_set_flags(flags)
-        try:
+        with L.debug_flags(flags):
             r = Refiner(K, 0.1, cuda_graph=graph)
             r.set_env(N.discriminator_spec(spec), N.feature_to_data_spec(spec), N.loss_refine)
             r.early_exit_logit = thr
             x = r.build_refiner(h0, keep_optimal_feature=True)
             torch.cuda.synchronize()
             return x.clone(), r.optimal_logit.clone(), r.current_feature.clone(), r.optimal_step.clone(), r.optimal_feature.clone()
-        finally:
-            cgs_lib.cgs_debug_set_flags(old)
 
-    plain = run(524288 | 4194304 | 16777216, False)           # no fusion, no M-tile pairs, no CTA pairs
+    plain = run(L.DEBUG_NO_FUSION | L.DEBUG_NO_MTILE_PAIRS | L.DEBUG_NO_CTA_PAIRS, False)   # the one-tile-per-CTA lowering
     steps = plain[3].cpu().numpy()
     assert 0 < (steps < K).sum()                               # some samples did stop early
-    for flags in (1048576, 8388608 | 524288, 33554432 | 1048576, 33554432 | 8388608 | 524288, 0):
+    for flags in (L.DEBUG_FORCE_FUSION, L.DEBUG_FORCE_MTILE_PAIRS | L.DEBUG_NO_FUSION, L.DEBUG_FORCE_CTA_PAIRS | L.DEBUG_FORCE_FUSION,
+                  L.DEBUG_FORCE_CTA_PAIRS | L.DEBUG_FORCE_MTILE_PAIRS | L.DEBUG_NO_FUSION, 0):
         for graph in (False, True):
             got = run(flags, graph)
             assert all(torch.equal(a, b) for a, b in zip(got, plain)), (flags, graph)
@@ -435,16 +407,16 @@ def test_early_exit_is_identical_across_tile_lowerings(cgs_lib, cuda_device, arc
 def test_programmatic_dependent_launch_is_bit_identical_at_scale(cgs_lib, cuda_device):
     """At batches where the refinement loop switches programmatic dependent launch on by itself (average pass >= 12
     GFLOP: DCGAN-64 from 157 rows) the kernels' set-up overlaps the previous kernel's drain; every kernel waits for its
-    predecessor before touching activation memory, so the bits equal those of plain stream order (bit 536870912),
+    predecessor before touching activation memory, so the bits equal those of plain stream order (DEBUG_PDL_OFF),
     eager and replayed as a CUDA graph."""
+    from cgs import lib as L
     from cgs import nets as N
     from sampling.collaborator import Refiner
     arch, w, spec = _make("dcgan64_l1", 5, 2.5, cuda_device, "tf32")
     h0 = torch.relu(torch.randn(208, *arch["feature_shape"], generator=torch.Generator().manual_seed(8))).to(cuda_device)
 
     def run(flags, graph):
-        old = cgs_lib.cgs_debug_set_flags(flags)
-        try:
+        with L.debug_flags(flags):
             r = Refiner(3, 0.1, cuda_graph=graph)
             r.set_env(N.discriminator_spec(spec), N.feature_to_data_spec(spec), N.loss_refine)
             outs = []
@@ -454,11 +426,9 @@ def test_programmatic_dependent_launch_is_bit_identical_at_scale(cgs_lib, cuda_d
                 outs.append((x.clone(), r.optimal_logit.clone(), r.current_feature.clone(), r.optimal_step.clone()))
             assert all(torch.equal(a, b) for a, b in zip(*outs))
             return outs[0]
-        finally:
-            cgs_lib.cgs_debug_set_flags(old)
 
-    plain = run(536870912, False)
-    for flags, graph in ((0, False), (0, True), (32768, True)):
+    plain = run(L.DEBUG_PDL_OFF, False)
+    for flags, graph in ((0, False), (0, True), (L.DEBUG_PDL_ON, True)):
         assert all(torch.equal(a, b) for a, b in zip(run(flags, graph), plain)), (flags, graph)
 
 

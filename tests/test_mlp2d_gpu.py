@@ -87,9 +87,10 @@ def test_probabilistic_returns_float64_trajectory_rows(cgs_lib, cuda_device):
                                                 ("ladam", 5, 20001, 2), ("ladam", 4, 300, 8)])
 def test_split_refine_kernel_is_bit_identical(cgs_lib, cuda_device, method, K, n, nlayers):
     """The split form (four threads per point, 16-wide layer slices exchanged through shared memory) accumulates every
-    element in the order of the one-thread form (CGS_DEBUG bit 134217728 selects the latter): same bits for the best
+    element in the order of the one-thread form (DEBUG_MLP2D_ONE_THREAD selects the latter): same bits for the best
     point, its loss and step, and the whole trajectory -- at the benchmark size, ragged sizes, a single point, more
     than 96 points per CTA round, the shallowest and the deepest MLP."""
+    from cgs import lib as L
     from sampling.refiner_cpu import MlpSpec, Refiner
     ws = onets.init_mlp2d(64, nlayers, seed=7, gain=1.5)
     mlp = MlpSpec(ws, cuda_device)
@@ -99,8 +100,7 @@ def test_split_refine_kernel_is_bit_identical(cgs_lib, cuda_device, method, K, n
     rate = 0.1 if method == "ladam" else 50.0
 
     def run(flags):
-        old = cgs_lib.cgs_debug_set_flags(flags)
-        try:
+        with L.debug_flags(flags):
             ref = Refiner(types.SimpleNamespace(rollout_steps=K, rollout_rate=rate, rollout_method=method))
             ref.set_env(mlp, None, _Data(real))
             np.random.seed(3)
@@ -109,9 +109,7 @@ def test_split_refine_kernel_is_bit_identical(cgs_lib, cuda_device, method, K, n
             np.random.seed(3)
             prob = ref.manipulate_sample(x0, "probabilistic")          # reads the full trajectory
             return det, step, loss, prob
-        finally:
-            cgs_lib.cgs_debug_set_flags(old)
 
-    a, b = run(0), run(134217728)
+    a, b = run(0), run(L.DEBUG_MLP2D_ONE_THREAD)
     for u, v in zip(a, b):
         assert np.array_equal(np.asarray(u), np.asarray(v))

@@ -11,20 +11,21 @@ from sampling.collaborator import Refiner
 lib = L.load()
 dev = torch.device("cuda", 0)
 # default rules / class-fused tiles whenever legal / class fusion + M-tile pairs / CTA pairs (cta_group::2) whenever legal
-for flags, name, B, thr in ((0, "dcgan64_l1", 5, None), (1048576, "dcgan64_l1", 5, None), (1048576, "dcgan32_l2", 6, None),
-                            (1048576 | 8388608, "dcgan64_l3", 3, 0.0), (8388608, "dcgan32_l4", 4, None),
-                            (1048576 | 33554432, "dcgan64_l1", 5, None), (33554432, "dcgan32_l2", 7, 0.0),
-                            (33554432 | 8388608 | 524288, "dcgan64_l2", 9, None),
-                            (1048576, "mnist", 20, 0.1)):
-    lib.cgs_debug_set_flags(flags)
-    arch = N.get_arch(name)
-    spec = N.NetSpec(arch, S.init_weights(arch, gain=3.0 if name == "mnist" else 2.5), dev)
-    r = Refiner(3, 0.1)
-    r.set_env(N.discriminator_spec(spec), N.feature_to_data_spec(spec), N.loss_refine)
-    r.early_exit_logit = thr
-    h0 = torch.from_numpy(S.proposal_features(arch, B, seed=1)).to(dev)
-    x = r.build_refiner(h0)
-    torch.cuda.synchronize()
+FUSE, MPAIR, CPAIR = L.DEBUG_FORCE_FUSION, L.DEBUG_FORCE_MTILE_PAIRS, L.DEBUG_FORCE_CTA_PAIRS
+for flags, name, B, thr in ((0, "dcgan64_l1", 5, None), (FUSE, "dcgan64_l1", 5, None), (FUSE, "dcgan32_l2", 6, None),
+                            (FUSE | MPAIR, "dcgan64_l3", 3, 0.0), (MPAIR, "dcgan32_l4", 4, None),
+                            (FUSE | CPAIR, "dcgan64_l1", 5, None), (CPAIR, "dcgan32_l2", 7, 0.0),
+                            (CPAIR | MPAIR | L.DEBUG_NO_FUSION, "dcgan64_l2", 9, None),
+                            (FUSE, "mnist", 20, 0.1)):
+    with L.debug_flags(flags):
+        arch = N.get_arch(name)
+        spec = N.NetSpec(arch, S.init_weights(arch, gain=3.0 if name == "mnist" else 2.5), dev)
+        r = Refiner(3, 0.1)
+        r.set_env(N.discriminator_spec(spec), N.feature_to_data_spec(spec), N.loss_refine)
+        r.early_exit_logit = thr
+        h0 = torch.from_numpy(S.proposal_features(arch, B, seed=1)).to(dev)
+        x = r.build_refiner(h0)
+        torch.cuda.synchronize()
     print(flags, name, "ok", tuple(x.shape), float(r.optimal_logit.mean()))
 # 2-D refinement: split form (four threads per point, named barriers) and the one-thread form
 import types
@@ -42,11 +43,10 @@ class _Data:
 
 rng = np.random.RandomState(0)
 mlp = MlpSpec(S.init_mlp2d(64, 6, seed=3, gain=1.5), dev)
-for flags, n in ((0, 333), (0, 20000), (134217728, 333)):
-    lib.cgs_debug_set_flags(flags)
-    r2 = Refiner2d(types.SimpleNamespace(rollout_steps=4, rollout_rate=0.1, rollout_method="ladam"))
-    r2.set_env(mlp, None, _Data((rng.randn(n, 2) * 3).astype(np.float32)))
-    out = r2.manipulate_sample((rng.randn(n, 2) * 4).astype(np.float32), "probabilistic")
+for flags, n in ((0, 333), (0, 20000), (L.DEBUG_MLP2D_ONE_THREAD, 333)):
+    with L.debug_flags(flags):
+        r2 = Refiner2d(types.SimpleNamespace(rollout_steps=4, rollout_rate=0.1, rollout_method="ladam"))
+        r2.set_env(mlp, None, _Data((rng.randn(n, 2) * 3).astype(np.float32)))
+        out = r2.manipulate_sample((rng.randn(n, 2) * 4).astype(np.float32), "probabilistic")
     print(flags, "2-D", n, "ok", out.shape)
-lib.cgs_debug_set_flags(0)
 print("launches", lib.cgs_launch_count())

@@ -1,4 +1,4 @@
-"""Run one layer pass with the CTA-0 pipeline trace on (CGS_DEBUG |= 256) and print per-role event timelines.
+"""Run one layer pass with the CTA-0 pipeline trace on (CGS_DEBUG_TRACE) and print per-role event timelines.
 
 The trace code is compiled out of the product build: rebuild first with
     CGS_NVCC_EXTRA=-DCGS_TRACE python collaborative-gan-sampling_b200/build.py -f
@@ -9,12 +9,13 @@ import ctypes as C
 import os
 import sys
 
-os.environ["CGS_DEBUG"] = str(int(os.environ.get("CGS_DEBUG", "0")) | 256)
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "collaborative-gan-sampling_b200"))
 import numpy as np  # noqa: E402
 import torch  # noqa: E402
 from cgs import lib as L, nets as N, synthetic as S  # noqa: E402
+
+os.environ["CGS_DEBUG"] = str(int(os.environ.get("CGS_DEBUG", "0")) | L.DEBUG_TRACE)   # read when libcgs loads
 
 ap = argparse.ArgumentParser()
 ap.add_argument("--workload", default="mnist")

@@ -1,4 +1,4 @@
-"""Per-tile event clocks of CTA 0 of edge_wide_tc (CGS_DEBUG bit 256): where a band's time goes."""
+"""Per-tile event clocks of CTA 0 of edge_wide_tc (CGS_DEBUG_TRACE): where a band's time goes."""
 import ctypes as C
 import os
 import sys
@@ -9,7 +9,7 @@ import torch
 from cgs import lib as L, nets as N, synthetic as S
 
 lib = L.load()
-lib.cgs_debug_set_flags(256 | int(os.environ.get("EXTRA", "0")))
+lib.cgs_debug_set_flags(L.DEBUG_TRACE | int(os.environ.get("EXTRA", "0")))
 dev = torch.device("cuda", 0)
 arch = N.get_arch("dcgan64_l1")
 spec = N.NetSpec(arch, S.init_weights(arch, gain=2.5), dev)
