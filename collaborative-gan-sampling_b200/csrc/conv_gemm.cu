@@ -604,16 +604,16 @@ conv_gemm_tc_kernel(const __grid_constant__ ConvGemmParams p, const __grid_const
         if (EPI == EPI_BWD) {
 #pragma unroll
           for (int ps = 0; ps < PASSES; ++ps)
-            if (ro[ps] >= 0) x0[ps] = __ldg(reinterpret_cast<const float4*>(p.aux + ro[ps] + n));
+            if (ro[ps] >= 0) x0[ps] = __ldg(reinterpret_cast<const float4*>(p.ep.aux + ro[ps] + n));
         } else if (EPI == EPI_UPDATE) {
 #pragma unroll
           for (int ps = 0; ps < PASSES; ++ps)
             if (ro[ps] >= 0) {
               x0[ps] = *reinterpret_cast<const float4*>(p.out + ro[ps] + n);
-              if (!p.sgd && !p.first) x1[ps] = *reinterpret_cast<const float4*>(p.mom + ro[ps] + n);
+              if (!p.ep.sgd && !p.ep.first) x1[ps] = *reinterpret_cast<const float4*>(p.ep.mom + ro[ps] + n);
             }
         } else if (EPI == EPI_FWD) {
-          x0[0] = p.bias ? __ldg(reinterpret_cast<const float4*>(p.bias + n)) : make_float4(0.f, 0.f, 0.f, 0.f);
+          x0[0] = p.ep.bias ? __ldg(reinterpret_cast<const float4*>(p.ep.bias + n)) : make_float4(0.f, 0.f, 0.f, 0.f);
         }
       };
       prefetch(chunk_first);                       // in flight while the main loop of this tile still runs
@@ -667,7 +667,7 @@ conv_gemm_tc_kernel(const __grid_constant__ ConvGemmParams p, const __grid_const
           float4 o[PASSES];
 #pragma unroll
           for (int ps = 0; ps < PASSES; ++ps)
-            if (ro[ps] >= 0 && n_ok) o[ps] = epilogue4_t<EPI>(p, ro[ps] + n, a[ps], EPI == EPI_FWD ? x0[0] : x0[ps], x1[ps]);
+            if (ro[ps] >= 0 && n_ok) o[ps] = epilogue4_t<EPI>(p.ep, ro[ps] + n, a[ps], EPI == EPI_FWD ? x0[0] : x0[ps], x1[ps]);
           if (warp == 0 && lane == 0) trace(p, 4, 1, tile_count * 8 + ch);
           if (!dbg_no_prefetch) prefetch(ch + chunk_groups);   // operands of the next chunk: overlap with these stores
 #pragma unroll
@@ -750,14 +750,9 @@ conv_gemm_simt_kernel(const __grid_constant__ ConvGemmParams p, const float* __r
     }
     const int row_off = ((b * p.OH + j * p.os + gc.oy0) * p.OW + (i * p.os + gc.ox0)) * p.ON;
     const int off = row_off + ng * 4;
-    float4 x0 = make_float4(0.f, 0.f, 0.f, 0.f), x1 = x0;
-    if (p.epi == EPI_FWD) { if (p.bias) x0 = __ldg(reinterpret_cast<const float4*>(p.bias + ng * 4)); }
-    else if (p.epi == EPI_BWD) x0 = __ldg(reinterpret_cast<const float4*>(p.aux + off));
-    else if (p.epi == EPI_UPDATE) {
-      x0 = *reinterpret_cast<const float4*>(p.out + off);
-      if (!p.sgd && !p.first) x1 = *reinterpret_cast<const float4*>(p.mom + off);
-    }
-    *reinterpret_cast<float4*>(p.out + off) = epilogue4(p, off, make_float4(acc[0], acc[1], acc[2], acc[3]), x0, x1);
+    float4 x0, x1;
+    epilogue_operands4(p.ep, p.out, off, ng * 4, x0, x1);
+    *reinterpret_cast<float4*>(p.out + off) = epilogue4(p.ep, off, make_float4(acc[0], acc[1], acc[2], acc[3]), x0, x1);
   }
 }
 
@@ -1038,7 +1033,7 @@ int launch_tc_epi(ConvGemmParams p, const float* w, int w_rows, int w_cols, cuda
 
 template <int BN, int NS = 1, int MT = 1, int CG = 1>
 int launch_tc(const ConvGemmParams& p, const float* w, int w_rows, int w_cols, cudaStream_t stream) {
-  switch (p.epi) {                          // the epilogue mode is compiled into the kernel
+  switch (p.ep.mode) {                      // the epilogue mode is compiled into the kernel
     case EPI_FWD: return launch_tc_epi<BN, EPI_FWD, NS, MT, CG>(p, w, w_rows, w_cols, stream);
     case EPI_BWD: return launch_tc_epi<BN, EPI_BWD, NS, MT, CG>(p, w, w_rows, w_cols, stream);
     case EPI_UPDATE: return launch_tc_epi<BN, EPI_UPDATE, NS, MT, CG>(p, w, w_rows, w_cols, stream);
@@ -1054,11 +1049,6 @@ bool use_cta_pairs(const ConvGemmParams& p, long long units_total, int num_sms) 
   if (p.cblocks <= 0 || p.window) return false;
   if (debug_flags() & CGS_DEBUG_FORCE_CTA_PAIRS) return true;
   return 2 * units_total >= (num_sms & ~1);
-}
-
-void derive_act(ConvGemmParams& p) {
-  p.act_tanh = (p.act == ACT_TANH);
-  p.slope = p.act == ACT_RELU ? 0.f : (p.act == ACT_LRELU ? 0.2f : 1.f);
 }
 
 int validate(const ConvGemmParams& p, int w_cols) {
@@ -1077,7 +1067,6 @@ int validate(const ConvGemmParams& p, int w_cols) {
 }  // namespace
 
 int plan_fusion(ConvGemmParams& p) {
-  derive_act(p);
   const int ns = fusion_slots(p, pick_bn(p.N));
   if (ns) build_fusion(p, ns);
   return ns;
@@ -1092,9 +1081,7 @@ int debug_trace_read(unsigned long long* out, int cap) {
   return n;
 }
 
-int launch_conv_gemm_tc(const ConvGemmParams& p_in, const float* w, int w_rows, int w_cols, cudaStream_t stream) {
-  ConvGemmParams p = p_in;
-  derive_act(p);
+int launch_conv_gemm_tc(const ConvGemmParams& p, const float* w, int w_rows, int w_cols, cudaStream_t stream) {
   if (int rc = validate(p, w_cols)) return rc;
   if (p.M <= 0) return CGS_OK;
   const int num_sms = device_num_sms();
@@ -1154,10 +1141,8 @@ int launch_conv_gemm_tc(const ConvGemmParams& p_in, const float* w, int w_rows, 
   }
 }
 
-int launch_conv_gemm_simt(const ConvGemmParams& p_in, const float* w, int w_rows, int w_cols, cudaStream_t stream) {
+int launch_conv_gemm_simt(const ConvGemmParams& p, const float* w, int w_rows, int w_cols, cudaStream_t stream) {
   (void)w_rows;
-  ConvGemmParams p = p_in;
-  derive_act(p);
   if (int rc = validate(p, w_cols)) return rc;
   if (p.M <= 0) return CGS_OK;
   const long long total = (long long)p.nclasses * p.M * (p.ON / 4);

@@ -62,12 +62,33 @@ struct GemmClass {
   signed char dx[kMaxTaps];
 };
 
+// What a layer pass does to its accumulator: the one description every pass kernel's epilogue reads (epilogue4 /
+// epilogue1 below).  Member order matters: the EPI_UPDATE tensor-core instances sit at the register cap, and their
+// allocation follows how these fields pair into 8-byte parameter loads.
+struct Epilogue {
+  const float* bias;  // EPI_FWD (null = no bias)
+  const float* aux;   // EPI_BWD: forward OUTPUT of the layer being differentiated
+  float* mom;         // EPI_UPDATE: momentum, same layout as out
+  int first, clip, sgd;                 // EPI_UPDATE policy constants (sampling/policy.py:27-37, collaborator.py:69-70)
+  float rate, alpha, vmin, vmax;
+  float slope;        // relu 0, lrelu 0.2, none 1 (branch-free: max(v, slope * v) and its derivative)
+  int act_tanh;       // the activation is tanh (slow path)
+  int round_out;      // round results to TF32 (RN) because the next consumer is a kind::tf32 MMA
+  int mode;           // EPI_*
+
+  Epilogue() = default;
+  // host: mode `mode_` (EPI_*) through activation `act` (ACT_*), no operands -- the only place an activation becomes
+  // slope / act_tanh
+  Epilogue(int mode_, int act) : bias(nullptr), aux(nullptr), mom(nullptr), first(0), clip(0), sgd(0), rate(0.f),
+                                 alpha(0.f), vmin(0.f), vmax(0.f),
+                                 slope(act == ACT_RELU ? 0.f : (act == ACT_LRELU ? 0.2f : 1.f)),
+                                 act_tanh(act == ACT_TANH), round_out(0), mode(mode_) {}
+};
+
 struct ConvGemmParams {
   const float* in;
   float* out;
-  const float* bias;
-  const float* aux;
-  float* mom;
+  Epilogue ep;
   int IH, IW, Cs;     // input image, channel stride (floats per pixel)
   int cblocks;        // Cin / 32 in block mode; 0 in pixel mode
   int MH, MW, S;      // rows per image = MH*MW; input pixel = (j*S+dy, i*S+dx)
@@ -85,12 +106,6 @@ struct ConvGemmParams {
   // kernel width carry zero weights.  One TMA box per K block through an overlapping-window tensor map.
   int window, win_k, win_x0, in_pitch_px;
   int nclasses;
-  int epi, act;
-  int first, clip, sgd;
-  float rate, alpha, vmin, vmax;
-  float slope;        // derived from act by the launcher: relu 0, lrelu 0.2, none 1 (branch-free epilogue)
-  int act_tanh;       // act == tanh (slow path)
-  int round_out;      // round results to TF32 (RN) because the next consumer is a kind::tf32 MMA
   int force_bn;       // 0 = tile-width heuristic, else the BN instance to launch
   // early exit (device-resident batch size): when non-null, only the first *live images are processed -- tiles past
   // them are never scheduled, rows past them never stored.  Grids stay sized for the full batch, so the launch
@@ -108,24 +123,6 @@ struct ConvGemmParams {
   unsigned long long fd_tiles_per_class, fd_n_tiles, fd_hy_tiles;
   GemmClass cls[kMaxClasses];
 };
-
-__device__ __forceinline__ float act_apply(float v, int act) {
-  switch (act) {
-    case ACT_RELU: return fmaxf(v, 0.f);
-    case ACT_LRELU: return fmaxf(v, 0.2f * v);   // nsgan/ops.py:69-70
-    case ACT_TANH: return tanhf(v);
-    default: return v;
-  }
-}
-// derivative expressed through the layer OUTPUT y = act(pre)
-__device__ __forceinline__ float act_grad_from_output(float y, int act) {
-  switch (act) {
-    case ACT_RELU: return y > 0.f ? 1.f : 0.f;
-    case ACT_LRELU: return y > 0.f ? 1.f : 0.2f;
-    case ACT_TANH: return 1.f - y * y;
-    default: return 1.f;
-  }
-}
 
 // n / d by multiply-high with magic = ceil(2^64 / d) (0 encodes d == 1): with magic * d = 2^64 + e, 0 <= e < d, the
 // excess n * e / (d * 2^64) stays below 1 / d for every 32-bit n, so the floor is exact
@@ -164,25 +161,33 @@ __device__ __forceinline__ float tf32_rn(float x) {
   return __uint_as_float(r);
 }
 
-// Four consecutive output channels.  `off` = element offset in mom; x0 / x1 are the operands the caller has already
-// fetched (so that many loads can be in flight): FWD x0 = bias; BWD x0 = forward output of the differentiated layer;
-// UPDATE x0 = current feature, x1 = momentum.  EPI is a compile-time constant in the tensor-core kernel (the epilogue
-// runs per 64-byte row segment: no run-time mode switches there) and p.epi in the other callers.
+// ---------------------------------------------------------------------------------------------
+// The epilogue formulas, once: a vector form (four consecutive output channels) and a scalar form (one channel) with
+// the same expressions, so a layer's result does not depend on which lowering ran it.  x0 / x1 are the operands the
+// caller has already fetched (so that many loads can be in flight):
+//   FWD     out = act(acc + x0)          x0 = bias
+//   BWD     out = acc * act'(x0)         x0 = forward output of the differentiated layer (act' through the output)
+//   UPDATE  momentum / sgd step          x0 = current feature, x1 = momentum; the new momentum goes to e.mom
+//   RAW     out = acc
+// FWD / BWD / RAW results are rounded to TF32 when e.round_out.  EPI is a compile-time constant where the epilogue is
+// hot (no run-time mode switches there); epilogue4 / epilogue1 dispatch on e.mode.
+// ---------------------------------------------------------------------------------------------
+// `off` = element offset of the four channels in e.mom
 template <int EPI>
-__device__ __forceinline__ float4 epilogue4_t(const ConvGemmParams& p, int off, float4 a, float4 x0, float4 x1) {
+__device__ __forceinline__ float4 epilogue4_t(const Epilogue& e, int off, float4 a, float4 x0, float4 x1) {
   float4 o = a;
   if (EPI == EPI_FWD) {
     const float vx = a.x + x0.x, vy = a.y + x0.y, vz = a.z + x0.z, vw = a.w + x0.w;
-    if (!p.act_tanh) {          // relu / lrelu / none: max(v, slope * v)
-      o.x = fmaxf(vx, vx * p.slope); o.y = fmaxf(vy, vy * p.slope);
-      o.z = fmaxf(vz, vz * p.slope); o.w = fmaxf(vw, vw * p.slope);
+    if (!e.act_tanh) {          // relu / lrelu / none: max(v, slope * v)
+      o.x = fmaxf(vx, vx * e.slope); o.y = fmaxf(vy, vy * e.slope);
+      o.z = fmaxf(vz, vz * e.slope); o.w = fmaxf(vw, vw * e.slope);
     } else {
       o.x = tanhf(vx); o.y = tanhf(vy); o.z = tanhf(vz); o.w = tanhf(vw);
     }
   } else if (EPI == EPI_BWD) {
-    if (!p.act_tanh) {          // derivative through the forward output: 1 where it is positive, slope elsewhere
-      o.x = a.x * (x0.x > 0.f ? 1.f : p.slope); o.y = a.y * (x0.y > 0.f ? 1.f : p.slope);
-      o.z = a.z * (x0.z > 0.f ? 1.f : p.slope); o.w = a.w * (x0.w > 0.f ? 1.f : p.slope);
+    if (!e.act_tanh) {          // derivative through the forward output: 1 where it is positive, slope elsewhere
+      o.x = a.x * (x0.x > 0.f ? 1.f : e.slope); o.y = a.y * (x0.y > 0.f ? 1.f : e.slope);
+      o.z = a.z * (x0.z > 0.f ? 1.f : e.slope); o.w = a.w * (x0.w > 0.f ? 1.f : e.slope);
     } else {
       o.x = a.x * (1.f - x0.x * x0.x); o.y = a.y * (1.f - x0.y * x0.y);
       o.z = a.z * (1.f - x0.z * x0.z); o.w = a.w * (1.f - x0.w * x0.w);
@@ -190,33 +195,76 @@ __device__ __forceinline__ float4 epilogue4_t(const ConvGemmParams& p, int off, 
   } else if (EPI == EPI_UPDATE) {
     // sampling/policy.py:27-37; separately rounded multiplies / adds like the reference's un-fused TF ops
     float4 m;
-    m.x = __fmul_rn(p.rate, a.x); m.y = __fmul_rn(p.rate, a.y); m.z = __fmul_rn(p.rate, a.z); m.w = __fmul_rn(p.rate, a.w);
-    if (!p.sgd) {
-      if (!p.first) {
-        m.x = __fadd_rn(__fmul_rn(p.alpha, x1.x), m.x);
-        m.y = __fadd_rn(__fmul_rn(p.alpha, x1.y), m.y);
-        m.z = __fadd_rn(__fmul_rn(p.alpha, x1.z), m.z);
-        m.w = __fadd_rn(__fmul_rn(p.alpha, x1.w), m.w);
+    m.x = __fmul_rn(e.rate, a.x); m.y = __fmul_rn(e.rate, a.y); m.z = __fmul_rn(e.rate, a.z); m.w = __fmul_rn(e.rate, a.w);
+    if (!e.sgd) {
+      if (!e.first) {
+        m.x = __fadd_rn(__fmul_rn(e.alpha, x1.x), m.x);
+        m.y = __fadd_rn(__fmul_rn(e.alpha, x1.y), m.y);
+        m.z = __fadd_rn(__fmul_rn(e.alpha, x1.z), m.z);
+        m.w = __fadd_rn(__fmul_rn(e.alpha, x1.w), m.w);
       }
-      *reinterpret_cast<float4*>(p.mom + off) = m;
+      *reinterpret_cast<float4*>(e.mom + off) = m;
     }
     o.x = __fsub_rn(x0.x, m.x); o.y = __fsub_rn(x0.y, m.y); o.z = __fsub_rn(x0.z, m.z); o.w = __fsub_rn(x0.w, m.w);
-    if (p.clip) {                                                    // collaborator.py:69-70
-      o.x = fminf(fmaxf(o.x, p.vmin), p.vmax); o.y = fminf(fmaxf(o.y, p.vmin), p.vmax);
-      o.z = fminf(fmaxf(o.z, p.vmin), p.vmax); o.w = fminf(fmaxf(o.w, p.vmin), p.vmax);
+    if (e.clip) {                                                    // collaborator.py:69-70
+      o.x = fminf(fmaxf(o.x, e.vmin), e.vmax); o.y = fminf(fmaxf(o.y, e.vmin), e.vmax);
+      o.z = fminf(fmaxf(o.z, e.vmin), e.vmax); o.w = fminf(fmaxf(o.w, e.vmin), e.vmax);
     }
     return o;
   }
-  if (p.round_out) { o.x = tf32_rn(o.x); o.y = tf32_rn(o.y); o.z = tf32_rn(o.z); o.w = tf32_rn(o.w); }
+  if (e.round_out) { o.x = tf32_rn(o.x); o.y = tf32_rn(o.y); o.z = tf32_rn(o.z); o.w = tf32_rn(o.w); }
   return o;
 }
 
-__device__ __forceinline__ float4 epilogue4(const ConvGemmParams& p, int off, float4 a, float4 x0, float4 x1) {
-  switch (p.epi) {
-    case EPI_FWD: return epilogue4_t<EPI_FWD>(p, off, a, x0, x1);
-    case EPI_BWD: return epilogue4_t<EPI_BWD>(p, off, a, x0, x1);
-    case EPI_UPDATE: return epilogue4_t<EPI_UPDATE>(p, off, a, x0, x1);
-    default: return epilogue4_t<EPI_RAW>(p, off, a, x0, x1);
+__device__ __forceinline__ float4 epilogue4(const Epilogue& e, int off, float4 a, float4 x0, float4 x1) {
+  switch (e.mode) {
+    case EPI_FWD: return epilogue4_t<EPI_FWD>(e, off, a, x0, x1);
+    case EPI_BWD: return epilogue4_t<EPI_BWD>(e, off, a, x0, x1);
+    case EPI_UPDATE: return epilogue4_t<EPI_UPDATE>(e, off, a, x0, x1);
+    default: return epilogue4_t<EPI_RAW>(e, off, a, x0, x1);
+  }
+}
+
+// The new momentum goes to *m_out instead (the caller stores it with its neighbours).  EPI / TANH / ROUND: -1 = read
+// e.mode / e.act_tanh / e.round_out at run time, else known at compile time (kernels with one instance per mode).
+// (e.mode is re-read at each test rather than copied once: the copy changed the register allocation of the
+// mma.sync edge kernels)
+template <int EPI = -1, int TANH = -1, int ROUND = -1>
+__device__ __forceinline__ float epilogue1_t(const Epilogue& e, float a, float x0, float x1, float* m_out) {
+  float o = a;
+  if ((EPI < 0 ? e.mode : EPI) == EPI_FWD) {
+    const float v = a + x0;
+    o = (TANH < 0 ? e.act_tanh : TANH) ? tanhf(v) : fmaxf(v, v * e.slope);
+  } else if ((EPI < 0 ? e.mode : EPI) == EPI_BWD) {
+    o = (TANH < 0 ? e.act_tanh : TANH) ? a * (1.f - x0 * x0) : a * (x0 > 0.f ? 1.f : e.slope);
+  } else if ((EPI < 0 ? e.mode : EPI) == EPI_UPDATE) {
+    float m = __fmul_rn(e.rate, a);
+    if (!e.sgd) {
+      if (!e.first) m = __fadd_rn(__fmul_rn(e.alpha, x1), m);
+      *m_out = m;
+    }
+    o = __fsub_rn(x0, m);
+    if (e.clip) o = fminf(fmaxf(o, e.vmin), e.vmax);
+    return o;
+  }
+  return (ROUND < 0 ? e.round_out : ROUND) ? tf32_rn(o) : o;
+}
+
+__device__ __forceinline__ float epilogue1(const Epilogue& e, float a, float x0, float x1, float* m_out) {
+  return epilogue1_t<>(e, a, x0, x1, m_out);
+}
+
+// The operands of epilogue4 for four output channels at element `off` of out / aux / mom and channel n of the bias,
+// for the kernels without a tuned load schedule of their own
+__device__ __forceinline__ void epilogue_operands4(const Epilogue& e, const float* out, int off, int n, float4& x0,
+                                                   float4& x1) {
+  x0 = make_float4(0.f, 0.f, 0.f, 0.f);
+  x1 = x0;
+  if (e.mode == EPI_FWD) { if (e.bias) x0 = __ldg(reinterpret_cast<const float4*>(e.bias + n)); }
+  else if (e.mode == EPI_BWD) x0 = __ldg(reinterpret_cast<const float4*>(e.aux + off));
+  else if (e.mode == EPI_UPDATE) {
+    x0 = *reinterpret_cast<const float4*>(out + off);
+    if (!e.sgd && !e.first) x1 = *reinterpret_cast<const float4*>(e.mom + off);
   }
 }
 

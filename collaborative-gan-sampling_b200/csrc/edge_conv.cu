@@ -25,27 +25,6 @@ __device__ __forceinline__ void mma_tf32(float (&c)[4], uint32_t a0, uint32_t a1
       : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
 }
 
-// Scalar twin of epilogue4 (conv_gemm.cuh): same formulas, same separately rounded policy arithmetic.
-__device__ __forceinline__ float epilogue1(const EdgeEpi& e, float a, float x0, float x1, float* m_out) {
-  float o = a;
-  if (e.epi == EPI_FWD) {
-    const float v = a + x0;
-    o = e.act_tanh ? tanhf(v) : fmaxf(v, v * e.slope);
-  } else if (e.epi == EPI_BWD) {
-    o = e.act_tanh ? a * (1.f - x0 * x0) : a * (x0 > 0.f ? 1.f : e.slope);
-  } else if (e.epi == EPI_UPDATE) {
-    float m = __fmul_rn(e.rate, a);                                   // sampling/policy.py:27-37
-    if (!e.sgd) {
-      if (!e.first) m = __fadd_rn(__fmul_rn(e.alpha, x1), m);
-      *m_out = m;
-    }
-    o = __fsub_rn(x0, m);
-    if (e.clip) o = fminf(fmaxf(o, e.vmin), e.vmax);                  // collaborator.py:69-70
-    return o;
-  }
-  return e.round_out ? tf32_rn(o) : o;
-}
-
 // ---------------------------------------------------------------------------------------------
 // edge_wide: per tile (image b, band of RO output rows <= 256 pixels) the input rows the band needs are staged in
 // shared memory by cp.async (rows outside the image zero-filled), double-buffered so the next tile's rows arrive
@@ -64,17 +43,10 @@ constexpr int EW_TILE_PX = EW_THREADS;   // 32 pixels per warp
 enum : int { EM_FWD_SLOPE = 0, EM_BWD_SLOPE = 1, EM_UPDATE = 2, EM_GENERIC = 3 };
 
 template <int MODE, bool ROUND>
-__device__ __forceinline__ float epi_fast(const EdgeEpi& e, float a, float x0, float x1, float* m_out) {
-  float o;
-  if (MODE == EM_FWD_SLOPE) {
-    const float v = a + x0;
-    o = fmaxf(v, v * e.slope);
-  } else if (MODE == EM_BWD_SLOPE) {
-    o = a * (x0 > 0.f ? 1.f : e.slope);
-  } else {
-    return epilogue1(e, a, x0, x1, m_out);
-  }
-  return ROUND ? tf32_rn(o) : o;
+__device__ __forceinline__ float epi_fast(const Epilogue& e, float a, float x0, float x1, float* m_out) {
+  if (MODE == EM_FWD_SLOPE) return epilogue1_t<EPI_FWD, 0, ROUND>(e, a, x0, x1, m_out);
+  if (MODE == EM_BWD_SLOPE) return epilogue1_t<EPI_BWD, 0, ROUND>(e, a, x0, x1, m_out);
+  return epilogue1(e, a, x0, x1, m_out);
 }
 
 // One-time set-up of an edge_wide CTA: k -> patch offset table, bias, weights in mma fragment order.
@@ -92,7 +64,7 @@ __device__ __forceinline__ void wide_setup(const EdgeWideParams& p, int ksteps, 
     }
     koff_s[kk] = off;
   }
-  if (tid < EW_NT * 8) bias_s[tid] = (p.e.epi == EPI_FWD && p.e.bias && tid < p.N) ? __ldg(p.e.bias + tid) : 0.f;
+  if (tid < EW_NT * 8) bias_s[tid] = (p.ep.mode == EPI_FWD && p.ep.bias && tid < p.N) ? __ldg(p.ep.bias + tid) : 0.f;
   for (int idx = tid; idx < ksteps * EW_NT * 32; idx += EW_THREADS) {
     const int l = idx & 31, nt = (idx >> 5) % EW_NT, ks = idx / (EW_NT * 32);
     const int n = nt * 8 + (l >> 2);
@@ -166,14 +138,14 @@ __device__ __forceinline__ void wide_band(const EdgeWideParams& p, int ksteps, c
           if (MODE == EM_FWD_SLOPE) {
             x0[q] = *reinterpret_cast<const float2*>(bias_s + nt * 8 + 2 * t);
           } else if (MODE == EM_BWD_SLOPE) {
-            x0[q] = __ldg(reinterpret_cast<const float2*>(p.e.aux + ro + nt * 8));
+            x0[q] = __ldg(reinterpret_cast<const float2*>(p.ep.aux + ro + nt * 8));
           } else {
             x0[q] = *reinterpret_cast<const float2*>(bias_s + nt * 8 + 2 * t);
-            if (p.e.epi == EPI_BWD) {
-              x0[q] = __ldg(reinterpret_cast<const float2*>(p.e.aux + ro + nt * 8));
-            } else if (p.e.epi == EPI_UPDATE) {
+            if (p.ep.mode == EPI_BWD) {
+              x0[q] = __ldg(reinterpret_cast<const float2*>(p.ep.aux + ro + nt * 8));
+            } else if (p.ep.mode == EPI_UPDATE) {
               x0[q] = *reinterpret_cast<const float2*>(orow + nt * 8);
-              if (!p.e.sgd && !p.e.first) x1[q] = *reinterpret_cast<const float2*>(p.e.mom + ro + nt * 8);
+              if (!p.ep.sgd && !p.ep.first) x1[q] = *reinterpret_cast<const float2*>(p.ep.mom + ro + nt * 8);
             }
           }
         }
@@ -181,9 +153,9 @@ __device__ __forceinline__ void wide_band(const EdgeWideParams& p, int ksteps, c
         for (int q = 0; q < EW_NT / 2; ++q) {
           const int nt = half * (EW_NT / 2) + q;
           float2 m2 = make_float2(0.f, 0.f), o;
-          o.x = epi_fast<MODE, ROUND>(p.e, acc[nt][2 * h], x0[q].x, x1[q].x, &m2.x);
-          o.y = epi_fast<MODE, ROUND>(p.e, acc[nt][2 * h + 1], x0[q].y, x1[q].y, &m2.y);
-          if (MODE >= EM_UPDATE && p.e.epi == EPI_UPDATE && !p.e.sgd) *reinterpret_cast<float2*>(p.e.mom + ro + nt * 8) = m2;
+          o.x = epi_fast<MODE, ROUND>(p.ep, acc[nt][2 * h], x0[q].x, x1[q].x, &m2.x);
+          o.y = epi_fast<MODE, ROUND>(p.ep, acc[nt][2 * h + 1], x0[q].y, x1[q].y, &m2.y);
+          if (MODE >= EM_UPDATE && p.ep.mode == EPI_UPDATE && !p.ep.sgd) *reinterpret_cast<float2*>(p.ep.mom + ro + nt * 8) = m2;
           *reinterpret_cast<float2*>(orow + nt * 8) = o;
         }
       }
@@ -221,7 +193,7 @@ __global__ void __launch_bounds__(EW_THREADS, 4) edge_wide_kernel(const EdgeWide
 
   pdl_launch_dependents();
   pdl_wait();                                // tables and weights above are constants; activations from here on
-  if (p.e.live) ntiles = min(ntiles, live_images(p.e.live, ntiles / bands) * bands);
+  if (p.live) ntiles = min(ntiles, live_images(p.live, ntiles / bands) * bands);
   int tile = blockIdx.x;
   if (tile < ntiles) stage_patch(tile, 0);
   cp_async_commit();
@@ -321,8 +293,8 @@ __device__ __forceinline__ void narrow_col2im(const EdgeNarrowParams& p, const f
                                               int y_lo, int y_hi, float* out, float4* patch, int patch_row0) {
   constexpr int CP = NT * 8 + 4;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const float4 bias4 = (p.e.epi == EPI_FWD && p.e.bias) ? __ldg(reinterpret_cast<const float4*>(p.e.bias))
-                                                        : make_float4(0.f, 0.f, 0.f, 0.f);
+  const float4 bias4 = (p.ep.mode == EPI_FWD && p.ep.bias) ? __ldg(reinterpret_cast<const float4*>(p.ep.bias))
+                                                          : make_float4(0.f, 0.f, 0.f, 0.f);
   for (int y = y_lo + warp; y < y_hi; y += EN_THREADS / 32) {
     const int ky0 = (y + p.pad_y) & 1;
     const size_t grow = ((size_t)b * p.OH + y) * p.out_pitch * 4;
@@ -346,11 +318,11 @@ __device__ __forceinline__ void narrow_col2im(const EdgeNarrowParams& p, const f
           }
         }
         float4 x0 = bias4;
-        if (p.e.epi == EPI_BWD) x0 = __ldg(reinterpret_cast<const float4*>(p.e.aux + grow + xc * 4));
+        if (p.ep.mode == EPI_BWD) x0 = __ldg(reinterpret_cast<const float4*>(p.ep.aux + grow + xc * 4));
         const float xs[3] = {x0.x, x0.y, x0.z};
         float unused;
 #pragma unroll
-        for (int c = 0; c < CI; ++c) o[c] = epilogue1(p.e, a[c], xs[c], 0.f, &unused);
+        for (int c = 0; c < CI; ++c) o[c] = epilogue1(p.ep, a[c], xs[c], 0.f, &unused);
       }
       const float4 v = make_float4(o[0], o[1], o[2], o[3]);
       if (out) *reinterpret_cast<float4*>(out + grow + xc * 4) = v;
@@ -368,7 +340,7 @@ __global__ void __launch_bounds__(EN_THREADS) edge_narrow_kernel(const EdgeNarro
   __syncthreads();
   pdl_launch_dependents();
   pdl_wait();                                // weights above are constants; activations from here on
-  if (p.e.live) ntiles = min(ntiles, live_images(p.e.live, p.B) * p.bands);
+  if (p.live) ntiles = min(ntiles, live_images(p.live, p.B) * p.bands);
 
   for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
     const int b = tile / p.bands;
@@ -414,7 +386,7 @@ __global__ void __launch_bounds__(EN_THREADS, 4) edge_pair_kernel(const EdgeNarr
   pdl_launch_dependents();
   pdl_wait();
   const int npx = pw.OH * pw.OW;
-  const int B_live = live_images(pw.e.live, pn.B);
+  const int B_live = live_images(pw.live, pn.B);
   for (int b = blockIdx.x; b < B_live; b += gridDim.x) {
     narrow_mma<NT>(pn.in + (size_t)b * pn.IH * pn.IW * pn.K, pn.K, pn.IH * pn.IW, bfrag_n, col_s);
     __syncthreads();
@@ -492,12 +464,12 @@ int launch_edge_wide(const EdgeWideParams& p, cudaStream_t st) {
   if (p.M * p.ON >= (1ll << 31)) return set_error(CGS_ERR_UNSUPPORTED, "batch too large for 32-bit indexing; split the batch");
   if (p.OW > EW_TILE_PX) return set_error(CGS_ERR_UNSUPPORTED, "edge_wide: output row wider than a tile");
   const int B = (int)(p.M / ((long long)p.OH * p.OW));
-  const bool rnd = p.e.round_out != 0;
-  if (p.e.epi == EPI_FWD && !p.e.act_tanh)
+  const bool rnd = p.ep.round_out != 0;
+  if (p.ep.mode == EPI_FWD && !p.ep.act_tanh)
     return rnd ? launch_wide_mode<EM_FWD_SLOPE, true>(p, B, st) : launch_wide_mode<EM_FWD_SLOPE, false>(p, B, st);
-  if (p.e.epi == EPI_BWD && !p.e.act_tanh)
+  if (p.ep.mode == EPI_BWD && !p.ep.act_tanh)
     return rnd ? launch_wide_mode<EM_BWD_SLOPE, true>(p, B, st) : launch_wide_mode<EM_BWD_SLOPE, false>(p, B, st);
-  if (p.e.epi == EPI_UPDATE) return launch_wide_mode<EM_UPDATE, false>(p, B, st);
+  if (p.ep.mode == EPI_UPDATE) return launch_wide_mode<EM_UPDATE, false>(p, B, st);
   return launch_wide_mode<EM_GENERIC, false>(p, B, st);
 }
 
@@ -557,14 +529,14 @@ int launch_pair_inst(const EdgeNarrowParams& pn, const EdgeWideParams& pw, int s
 
 template <int NT, int CI>
 int launch_pair_mode(const EdgeNarrowParams& pn, const EdgeWideParams& pw, int store_image, cudaStream_t st) {
-  const bool rnd = pw.e.round_out != 0;
-  if (pw.e.epi == EPI_FWD && !pw.e.act_tanh)
+  const bool rnd = pw.ep.round_out != 0;
+  if (pw.ep.mode == EPI_FWD && !pw.ep.act_tanh)
     return rnd ? launch_pair_inst<NT, CI, EM_FWD_SLOPE, true>(pn, pw, store_image, st)
                : launch_pair_inst<NT, CI, EM_FWD_SLOPE, false>(pn, pw, store_image, st);
-  if (pw.e.epi == EPI_BWD && !pw.e.act_tanh)
+  if (pw.ep.mode == EPI_BWD && !pw.ep.act_tanh)
     return rnd ? launch_pair_inst<NT, CI, EM_BWD_SLOPE, true>(pn, pw, store_image, st)
                : launch_pair_inst<NT, CI, EM_BWD_SLOPE, false>(pn, pw, store_image, st);
-  if (pw.e.epi == EPI_UPDATE) return launch_pair_inst<NT, CI, EM_UPDATE, false>(pn, pw, store_image, st);
+  if (pw.ep.mode == EPI_UPDATE) return launch_pair_inst<NT, CI, EM_UPDATE, false>(pn, pw, store_image, st);
   return launch_pair_inst<NT, CI, EM_GENERIC, false>(pn, pw, store_image, st);
 }
 }  // namespace

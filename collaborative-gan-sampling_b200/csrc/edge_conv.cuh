@@ -10,20 +10,9 @@
 #pragma once
 #include <cuda_runtime.h>
 
-namespace cgs {
+#include "conv_gemm.cuh"
 
-struct EdgeEpi {
-  int epi;            // EPI_FWD / EPI_BWD / EPI_UPDATE / EPI_RAW (conv_gemm.cuh)
-  int act_tanh;
-  float slope;        // relu 0, lrelu 0.2, none 1
-  int round_out;
-  int first, clip, sgd;
-  float rate, alpha, vmin, vmax;
-  const float* bias;
-  const float* aux;
-  float* mom;
-  const int* live;    // early exit: device-resident number of images still in the batch (null = all of them)
-};
+namespace cgs {
 
 // images a kernel of the chain has to process (grids stay sized for the full batch; see ConvGemmParams::live)
 __device__ __forceinline__ int live_images(const int* live, int B) {
@@ -38,7 +27,8 @@ struct EdgeWideParams {
   const float* w;     // window layout: [N][k*32], element (n, ky*32 + kx*4 + c)
   int IH, pitch, xoff, OH, OW, ON, N, k, cimg, pad_y, pad_x;
   long long M;        // B*OH*OW
-  EdgeEpi e;
+  Epilogue ep;
+  const int* live;    // early exit: device-resident number of images still in the batch (null = all of them)
 };
 
 struct EdgeNarrowParams {
@@ -47,8 +37,9 @@ struct EdgeNarrowParams {
   const float* w;     // scatter layout: [k*k*4][K], row (ky*k + kx)*4 + c
   int B, IH, IW, K, OH, OW, k, cimg, pad_y, pad_x, out_pitch, out_xoff;
   int R, halo_lo, halo_hi, bands;   // input rows per tile, extra rows read above / below, tiles per image
-  int s2d;            // 1: out (and e.aux) are in the space-to-depth image layout [B][IH][IW][16] (see edge_tc.cu)
-  EdgeEpi e;
+  int s2d;            // 1: out (and ep.aux) are in the space-to-depth image layout [B][IH][IW][16] (see edge_tc.cu)
+  Epilogue ep;
+  const int* live;    // early exit: device-resident number of images still in the batch (null = all of them)
 };
 
 bool edge_wide_supported(int N, int k, int cimg);

@@ -46,18 +46,6 @@ struct NarrowTcParams {
   int stage_bytes, nstages, ntiles;
 };
 
-// scalar epilogue of an image-edge pass (same formulas as epilogue4 in conv_gemm.cuh; no policy step here)
-__device__ __forceinline__ float epilogue1_tc(const EdgeEpi& e, float a, float x0, float*) {
-  float o = a;
-  if (e.epi == EPI_FWD) {
-    const float v = a + x0;
-    o = e.act_tanh ? tanhf(v) : fmaxf(v, v * e.slope);
-  } else if (e.epi == EPI_BWD) {
-    o = e.act_tanh ? a * (1.f - x0 * x0) : a * (x0 > 0.f ? 1.f : e.slope);
-  }
-  return e.round_out ? tf32_rn(o) : o;
-}
-
 // PW (patch pitch = IW + 2) is a template parameter so that every per-MMA descriptor offset is an immediate: the
 // single MMA-issuing thread is the serial resource of this kernel (216 MMAs per band), and with run-time offsets each
 // MMA cost ~50 cycles of 64-bit address arithmetic and register -> uniform-register moves (11 k cycles per band).
@@ -99,7 +87,7 @@ edge_narrow_tc_kernel(const __grid_constant__ NarrowTcParams q, const __grid_con
   pdl_launch_dependents();
   pdl_wait();
   int ntiles = q.ntiles;
-  if (p.e.live) ntiles = min(ntiles, live_images(p.e.live, p.B) * q.bands);
+  if (p.live) ntiles = min(ntiles, live_images(p.live, p.B) * q.bands);
 
   if (warp == 0) {
     // ------------------------------------------------------------------ TMA producer
@@ -162,9 +150,16 @@ edge_narrow_tc_kernel(const __grid_constant__ NarrowTcParams q, const __grid_con
     const int quarter = warp & 3;
     const int group = (warp - 2) >> 2;
     constexpr int NGROUPS = TC_EPI_WARPS / 4;
-    const bool bwd = p.e.epi == EPI_BWD;
-    const float4 bias4 = (p.e.epi == EPI_FWD && p.e.bias) ? __ldg(reinterpret_cast<const float4*>(p.e.bias))
-                                                          : make_float4(0.f, 0.f, 0.f, 0.f);
+    const bool bwd = p.ep.mode == EPI_BWD;
+    const float4 bias4 = (p.ep.mode == EPI_FWD && p.ep.bias) ? __ldg(reinterpret_cast<const float4*>(p.ep.bias))
+                                                            : make_float4(0.f, 0.f, 0.f, 0.f);
+    // the scalar epilogue without the policy step, which this pass never carries (edge_narrow_tc_supported)
+    auto epi = [&](float v, float x0) {
+      float unused;
+      return bwd ? epilogue1_t<EPI_BWD>(p.ep, v, x0, 0.f, &unused)
+                 : p.ep.mode == EPI_FWD ? epilogue1_t<EPI_FWD>(p.ep, v, x0, 0.f, &unused)
+                                        : epilogue1_t<EPI_RAW>(p.ep, v, x0, 0.f, &unused);
+    };
     uint32_t tile_count = 0;
     for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x, ++tile_count) {
       const int b = tile / q.bands;
@@ -183,7 +178,7 @@ edge_narrow_tc_kernel(const __grid_constant__ NarrowTcParams q, const __grid_con
         // derivative operand (the forward image at the four output pixels): in flight while the MMAs still run
         float4 aux[2][2];
         if (bwd && valid) {
-          const float* abase = p.e.aux + (obase - p.out);
+          const float* abase = p.ep.aux + (obase - p.out);
 #pragma unroll
           for (int py = 0; py < 2; ++py)
 #pragma unroll
@@ -210,11 +205,10 @@ edge_narrow_tc_kernel(const __grid_constant__ NarrowTcParams q, const __grid_con
             for (int px = 0; px < 2; ++px) {
               const int n0 = (py * 2 + px) * 4;
               const float4 x0 = bwd ? aux[py][px] : bias4;
-              float unused;
               float4 o;
-              o.x = epilogue1_tc(p.e, __uint_as_float(a[n0]), x0.x, &unused);
-              o.y = p.cimg > 1 ? epilogue1_tc(p.e, __uint_as_float(a[n0 + 1]), x0.y, &unused) : 0.f;
-              o.z = p.cimg > 2 ? epilogue1_tc(p.e, __uint_as_float(a[n0 + 2]), x0.z, &unused) : 0.f;
+              o.x = epi(__uint_as_float(a[n0]), x0.x);
+              o.y = p.cimg > 1 ? epi(__uint_as_float(a[n0 + 1]), x0.y) : 0.f;
+              o.z = p.cimg > 2 ? epi(__uint_as_float(a[n0 + 2]), x0.z) : 0.f;
               o.w = 0.f;
               *reinterpret_cast<float4*>(orow + px * 4) = o;
             }
@@ -265,7 +259,7 @@ bool edge_tc_width_supported(int w) { return w == 16 || w == 32 || w == 64; }
 
 bool edge_narrow_tc_supported(const EdgeNarrowParams& p) {
   return p.K == 64 && p.pad_y == 1 && p.pad_x == 1 && edge_tc_width_supported(p.IW) && (p.k == 4 || p.k == 5) &&
-         p.OW == 2 * p.IW && p.OH == 2 * p.IH && p.e.epi != EPI_UPDATE && p.cimg >= 1 && p.cimg <= 3;
+         p.OW == 2 * p.IW && p.OH == 2 * p.IH && p.ep.mode != EPI_UPDATE && p.cimg >= 1 && p.cimg <= 3;
 }
 
 int launch_edge_narrow_tc(const EdgeNarrowParams& p, cudaStream_t st) {
@@ -370,7 +364,9 @@ struct WideTcParams {
   int B, H2, W2, k, cimg, pad;
   int R, bands, MT, PW, PR, stage_bytes, nstages, ntiles;
   const int* live;
-  ConvGemmParams ep;       // epilogue description (out / bias / aux / mom / policy constants), see epilogue4
+  float* out;              // [B][H2][W2][64]
+  Epilogue ep;
+  int debug;               // debug_flags() at launch: CGS_DEBUG_SKIP_*, _NO_PREFETCH, _TRACE
 };
 
 __device__ __forceinline__ uint64_t make_smem_desc_sw64(uint32_t smem_addr) {
@@ -401,7 +397,6 @@ edge_wide_tc_kernel(const __grid_constant__ WideTcParams q, const __grid_constan
   __shared__ uint64_t full_bar[8], empty_bar[8], tmem_full_bar[2], tmem_empty_bar[2];
   __shared__ uint32_t tmem_ptr_smem;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const ConvGemmParams& ep = q.ep;
 
   // weights -> [tile = ks / 4][n][32 floats], SWIZZLE_128B; k-step ks = shift * 2 + h holds s2d channels h*8 .. h*8+7
   for (int idx = threadIdx.x; idx < 5 * 64 * 8; idx += WT_THREADS) {
@@ -448,8 +443,8 @@ edge_wide_tc_kernel(const __grid_constant__ WideTcParams q, const __grid_constan
         const uint32_t s = stage, ph = phase;
         if (++stage == (uint32_t)q.nstages) { stage = 0; phase ^= 1u; }
         mbar_wait(&empty_bar[s], ph ^ 1);
-        tc_trace(ep.debug, 0, (unsigned)((tile - blockIdx.x) / gridDim.x));
-        if (ep.debug & CGS_DEBUG_SKIP_A_TMA) { mbar_arrive(&full_bar[s]); continue; }   // profiling knob: no loads
+        tc_trace(q.debug, 0, (unsigned)((tile - blockIdx.x) / gridDim.x));
+        if (q.debug & CGS_DEBUG_SKIP_A_TMA) { mbar_arrive(&full_bar[s]); continue; }   // profiling knob: no loads
         mbar_arrive_expect_tx(&full_bar[s], bytes);
         tma_load_4d(smem_u32(smem_a) + s * q.stage_bytes, &tmap_in, &full_bar[s], 0, -1, j0 - 1, b);
       }
@@ -463,14 +458,14 @@ edge_wide_tc_kernel(const __grid_constant__ WideTcParams q, const __grid_constan
       for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x, ++tile_count) {
         const uint32_t acc = tile_count & 1, acc_ph = (tile_count >> 1) & 1;
         mbar_wait(&tmem_empty_bar[acc], acc_ph ^ 1);
-        tc_trace(ep.debug, 1, tile_count);
+        tc_trace(q.debug, 1, tile_count);
         const uint32_t s = stage;
         mbar_wait(&full_bar[s], phase);
-        tc_trace(ep.debug, 2, tile_count);
+        tc_trace(q.debug, 2, tile_count);
         if (++stage == (uint32_t)q.nstages) { stage = 0; phase ^= 1u; }
         tcgen05_fence_after();
         const uint64_t da_stage = da0 + (uint64_t)((s * (uint32_t)q.stage_bytes) >> 4);
-        const bool no_mma = (ep.debug & CGS_DEBUG_SKIP_MMA) != 0;             // profiling knob
+        const bool no_mma = (q.debug & CGS_DEBUG_SKIP_MMA) != 0;             // profiling knob
         for (int mt = 0; mt < q.MT; ++mt) {
           const uint32_t tmem_d = tmem_base + (acc * TC_MAX_MT + mt) * 64;
           const uint64_t da_mt = da_stage + (uint64_t)(mt * ((128 * 64) >> 4));
@@ -486,7 +481,7 @@ edge_wide_tc_kernel(const __grid_constant__ WideTcParams q, const __grid_constan
         }
         umma_commit(&empty_bar[s]);
         umma_commit(&tmem_full_bar[acc]);
-        tc_trace(ep.debug, 3, tile_count);
+        tc_trace(q.debug, 3, tile_count);
       }
     }
   } else {
@@ -523,18 +518,18 @@ edge_wide_tc_kernel(const __grid_constant__ WideTcParams q, const __grid_constan
           if (EPI == EPI_BWD) {
 #pragma unroll
             for (int ps = 0; ps < 4; ++ps)
-              x0[ch][ps] = (ro[ps] >= 0 && !(ep.debug & CGS_DEBUG_NO_PREFETCH)) ? __ldg(reinterpret_cast<const float4*>(ep.aux + ro[ps] + n))
+              x0[ch][ps] = (ro[ps] >= 0 && !(q.debug & CGS_DEBUG_NO_PREFETCH)) ? __ldg(reinterpret_cast<const float4*>(q.ep.aux + ro[ps] + n))
                                                               : make_float4(1.f, 1.f, 1.f, 1.f);   // knob 2048: no operand loads
           } else if (EPI == EPI_FWD) {
-            x0[ch][0] = ep.bias ? __ldg(reinterpret_cast<const float4*>(ep.bias + n)) : make_float4(0.f, 0.f, 0.f, 0.f);
+            x0[ch][0] = q.ep.bias ? __ldg(reinterpret_cast<const float4*>(q.ep.bias + n)) : make_float4(0.f, 0.f, 0.f, 0.f);
           }
         }
         if (!waited) {
-          if (warp == 2 && lane == 0) tc_trace(ep.debug, 4, tile_count);
+          if (warp == 2 && lane == 0) tc_trace(q.debug, 4, tile_count);
           mbar_wait(&tmem_full_bar[acc], acc_ph);
           tcgen05_fence_after();
           waited = true;
-          if (warp == 2 && lane == 0) tc_trace(ep.debug, 5, tile_count);
+          if (warp == 2 && lane == 0) tc_trace(q.debug, 5, tile_count);
         }
         const uint32_t taddr = tmem_base + (acc * TC_MAX_MT + mt) * 64 + (static_cast<uint32_t>(quarter * 32) << 16);
 #pragma unroll
@@ -566,18 +561,18 @@ edge_wide_tc_kernel(const __grid_constant__ WideTcParams q, const __grid_constan
               if (ro[ps] >= 0) {
                 float4 xa = EPI == EPI_FWD ? x0[ch][0] : x0[ch][ps], xb = make_float4(0.f, 0.f, 0.f, 0.f);
                 if (EPI == EPI_UPDATE) {         // policy step (only when the G tail is this single layer): not prefetched
-                  xa = *reinterpret_cast<const float4*>(ep.out + ro[ps] + n);
-                  if (!ep.sgd && !ep.first) xb = *reinterpret_cast<const float4*>(ep.mom + ro[ps] + n);
+                  xa = *reinterpret_cast<const float4*>(q.out + ro[ps] + n);
+                  if (!q.ep.sgd && !q.ep.first) xb = *reinterpret_cast<const float4*>(q.ep.mom + ro[ps] + n);
                 }
-                const float4 o = epilogue4_t<EPI>(ep, ro[ps] + n, v, xa, xb);
-                if (!(ep.debug & CGS_DEBUG_SKIP_STORES)) *reinterpret_cast<float4*>(ep.out + ro[ps] + n) = o;
+                const float4 o = epilogue4_t<EPI>(q.ep, ro[ps] + n, v, xa, xb);
+                if (!(q.debug & CGS_DEBUG_SKIP_STORES)) *reinterpret_cast<float4*>(q.out + ro[ps] + n) = o;
               }
             }
           }
           __syncwarp();
         }
       }
-      if (warp == 2 && lane == 0) tc_trace(ep.debug, 6, tile_count);
+      if (warp == 2 && lane == 0) tc_trace(q.debug, 6, tile_count);
       if (!waited || group >= q.MT) {
         // a group without an M tile in this band still owes the buffer its arrivals
         if (!waited) { mbar_wait(&tmem_full_bar[acc], acc_ph); tcgen05_fence_after(); }
@@ -638,7 +633,7 @@ int launch_edge_wide_tc(const EdgeWideParams& p, int B, cudaStream_t st) {
   WideTcParams q;
   std::memset(&q, 0, sizeof(q));
   q.in = p.in; q.w = p.w; q.B = B; q.H2 = p.OH; q.W2 = p.OW; q.k = p.k; q.cimg = p.cimg; q.pad = p.pad_y;
-  q.live = p.e.live;
+  q.live = p.live;
   q.PW = q.W2 + 2;
   int bestR = 1;
   double best = 1e30;
@@ -663,12 +658,9 @@ int launch_edge_wide_tc(const EdgeWideParams& p, int B, cudaStream_t st) {
   const long long tiles = (long long)B * q.bands;
   if (tiles >= (1ll << 31) || (long long)B * q.H2 * q.W2 * 64 >= (1ll << 31)) return set_error(CGS_ERR_UNSUPPORTED, "batch too large; split the batch");
   q.ntiles = (int)tiles;
-  // epilogue description in the GEMM kernels' terms
-  ConvGemmParams& ep = q.ep;
-  ep.out = p.out; ep.bias = p.e.bias; ep.aux = p.e.aux; ep.mom = p.e.mom;
-  ep.epi = p.e.epi; ep.act_tanh = p.e.act_tanh; ep.slope = p.e.slope; ep.round_out = p.e.round_out;
-  ep.first = p.e.first; ep.clip = p.e.clip; ep.sgd = p.e.sgd; ep.rate = p.e.rate; ep.alpha = p.e.alpha; ep.vmin = p.e.vmin; ep.vmax = p.e.vmax;
-  ep.debug = debug_flags();
+  q.out = p.out;
+  q.ep = p.ep;
+  q.debug = debug_flags();
   PFN_encodeTiledTc enc = encode_fn();
   if (!enc) return set_error(CGS_ERR_CUDA, "cuTensorMapEncodeTiled entry point not available");
   CUtensorMap tmap;
@@ -691,11 +683,11 @@ int launch_edge_wide_tc(const EdgeWideParams& p, int B, cudaStream_t st) {
       le = launch_pdl(edge_wide_tc_kernel<PWV, EPIV>, dim3((unsigned)grid), dim3(WT_THREADS), smem, st, q, tmap);       \
   } break;
 #define CGS_WIDE_TC_PW(PWV) CGS_WIDE_TC_CASE(PWV, EPI_FWD) CGS_WIDE_TC_CASE(PWV, EPI_BWD) CGS_WIDE_TC_CASE(PWV, EPI_UPDATE) CGS_WIDE_TC_CASE(PWV, EPI_RAW)
-  switch (q.PW * 8 + ep.epi) {
+  switch (q.PW * 8 + q.ep.mode) {
     CGS_WIDE_TC_PW(18)
     CGS_WIDE_TC_PW(34)
     CGS_WIDE_TC_PW(66)
-    default: return set_error(CGS_ERR_UNSUPPORTED, "edge_wide_tc: row width %d / epilogue %d", q.W2, ep.epi);
+    default: return set_error(CGS_ERR_UNSUPPORTED, "edge_wide_tc: row width %d / epilogue %d", q.W2, q.ep.mode);
   }
 #undef CGS_WIDE_TC_PW
 #undef CGS_WIDE_TC_CASE

@@ -22,12 +22,11 @@ inline int same_pad_before(int in_size, int k) {      // TF SAME, stride 2 (SURV
 }
 
 struct LayerShape {
-  int hout, wout, cs_in, cs_out;
+  int hout, wout, cs_out;
 };
 
 LayerShape layer_shape(const cgs_layer_desc& L) {
   LayerShape s;
-  s.cs_in = cstride(L.cin);
   s.cs_out = cstride(L.cout);
   if (L.type == CGS_LAYER_CONV) {
     s.hout = (L.hin + 1) / 2;
@@ -39,6 +38,41 @@ LayerShape layer_shape(const cgs_layer_desc& L) {
     s.hout = s.wout = 1;
   }
   return s;
+}
+
+// The fixed facts of one pass of a layer, forward or data-gradient (the pass that maps the gradient w.r.t. the
+// layer's pre-activation output back to its input).  The strided type (conv forward, deconv data-gradient) reads
+// input pixels (2j + ky - pad, 2i + kx - pad); the transposed type (deconv forward, conv data-gradient) is its
+// adjoint.  Either way the TF SAME pads are those of the stride-2 conv over the finer of the two grids.
+struct PassShape {
+  int ih, iw, oh, ow;     // input and output grid (fc: 1 x 1)
+  int kch, nch;           // reduced (K-side) and produced (N-side) channel counts
+  int pad_y, pad_x;       // 0 for fc
+  bool strided;           // strided type; else transposed type or fc
+  const float* w;         // packed weights of the pass: rows x cols
+  int rows, cols;
+  const float* bias;      // forward only
+};
+
+PassShape pass_shape(const cgs_layer_desc& L, bool backward) {
+  const LayerShape s = layer_shape(L);
+  PassShape p;
+  p.ih = backward ? s.hout : L.hin;
+  p.iw = backward ? s.wout : L.win;
+  p.oh = backward ? L.hin : s.hout;
+  p.ow = backward ? L.win : s.wout;
+  if (L.type == CGS_LAYER_FC) p.ih = p.iw = p.oh = p.ow = 1;
+  p.kch = backward ? L.cout : L.cin;
+  p.nch = backward ? L.cin : L.cout;
+  p.strided = (L.type == CGS_LAYER_CONV && !backward) || (L.type == CGS_LAYER_DECONV && backward);
+  const bool conv = L.type == CGS_LAYER_CONV;
+  p.pad_y = L.type == CGS_LAYER_FC ? 0 : same_pad_before(conv ? L.hin : s.hout, L.k);
+  p.pad_x = L.type == CGS_LAYER_FC ? 0 : same_pad_before(conv ? L.win : s.wout, L.k);
+  p.w = backward ? L.w_bwd : L.w_fwd;
+  p.rows = backward ? L.rows_bwd : L.rows_fwd;
+  p.cols = backward ? L.kcols_bwd : L.kcols_fwd;
+  p.bias = backward ? nullptr : L.bias;
+  return p;
 }
 
 int check_layer(const cgs_layer_desc& L) {
@@ -139,86 +173,39 @@ void fill_transposed(ConvGemmParams& p, int k, int pad_y, int pad_x, int cin_k) 
 
 }  // namespace
 
-// Parameters of the forward pass of one layer.
-int make_forward_params(const cgs_layer_desc& L, int64_t B, const float* x, float* y, ConvGemmParams& p) {
+// Gathered-GEMM parameters of one layer pass (forward: x -> y; data-gradient: dy -> dx); the epilogue is the caller's.
+int make_pass_params(const cgs_layer_desc& L, bool backward, int64_t B, const float* in, float* out, ConvGemmParams& p) {
   if (int rc = check_layer(L)) return rc;
+  if (L.type == CGS_LAYER_FC && backward && L.cout % 32)
+    return set_error(CGS_ERR_UNSUPPORTED, "fc output size %d must be a multiple of 32", L.cout);
   std::memset(&p, 0, sizeof(p));
-  const LayerShape s = layer_shape(L);
-  p.in = x;
-  p.out = y;
-  p.bias = L.bias;
-  p.epi = EPI_FWD;
-  p.act = L.act;
-  p.N = L.cout;
-  p.ON = s.cs_out;
-  p.OH = s.hout;
-  p.OW = s.wout;
-  p.IH = L.hin;
-  p.IW = L.win;
-  p.Cs = s.cs_in;
-  if (L.type == CGS_LAYER_CONV) {
-    fill_strided(p, L.k, same_pad_before(L.hin, L.k), same_pad_before(L.win, L.k), s.cs_in);
-    p.MH = s.hout;
-    p.MW = s.wout;
-  } else if (L.type == CGS_LAYER_DECONV) {
-    fill_transposed(p, L.k, same_pad_before(s.hout, L.k), same_pad_before(s.wout, L.k), L.cin);
-    p.MH = L.hin;
-    p.MW = L.win;
-  } else {
+  const PassShape sh = pass_shape(L, backward);
+  p.in = in;
+  p.out = out;
+  p.N = sh.nch;
+  p.ON = cstride(sh.nch);
+  p.OH = sh.oh;
+  p.OW = sh.ow;
+  p.IH = sh.ih;
+  p.IW = sh.iw;
+  p.Cs = cstride(sh.kch);
+  if (L.type == CGS_LAYER_FC) {
     p.nclasses = 1;
     p.cls[0].ntaps = 1;
     p.cls[0].nkx = 1;
-    p.cblocks = L.cin / 32;
+    p.cblocks = sh.kch / 32;
     p.cls[0].nkb = p.cblocks;
     p.S = 1;
     p.os = 1;
     p.MH = p.MW = 1;
-    p.IH = p.IW = 1;
-    p.Cs = L.cin;
-  }
-  p.M = (int)(B * p.MH * p.MW);
-  return CGS_OK;
-}
-
-// Parameters of the data-gradient pass of one layer: dy (grad w.r.t. the layer's pre-activation output) -> dx.
-int make_backward_params(const cgs_layer_desc& L, int64_t B, const float* dy, float* dx, ConvGemmParams& p) {
-  if (int rc = check_layer(L)) return rc;
-  std::memset(&p, 0, sizeof(p));
-  const LayerShape s = layer_shape(L);
-  p.in = dy;
-  p.out = dx;
-  p.epi = EPI_RAW;
-  p.N = L.cin;
-  p.ON = s.cs_in;
-  p.OH = L.hin;
-  p.OW = L.win;
-  p.IH = s.hout;
-  p.IW = s.wout;
-  p.Cs = s.cs_out;
-  if (L.type == CGS_LAYER_CONV) {
-    // conv data-gradient is a transposed-type pass over dy
-    fill_transposed(p, L.k, same_pad_before(L.hin, L.k), same_pad_before(L.win, L.k), L.cout);
-    p.MH = s.hout;
-    p.MW = s.wout;
-  } else if (L.type == CGS_LAYER_DECONV) {
-    // deconv data-gradient is a strided-type pass over dy (== conv fprop with the same filter)
-    fill_strided(p, L.k, same_pad_before(s.hout, L.k), same_pad_before(s.wout, L.k), s.cs_out);
-    p.MH = L.hin;
-    p.MW = L.win;
+  } else if (sh.strided) {
+    fill_strided(p, L.k, sh.pad_y, sh.pad_x, cstride(sh.kch));
+    p.MH = sh.oh;
+    p.MW = sh.ow;
   } else {
-    if (L.cout % 32) return set_error(CGS_ERR_UNSUPPORTED, "fc output size %d must be a multiple of 32", L.cout);
-    p.nclasses = 1;
-    p.cls[0].ntaps = 1;
-    p.cls[0].nkx = 1;
-    p.cblocks = L.cout / 32;
-    p.cls[0].nkb = p.cblocks;
-    p.S = 1;
-    p.os = 1;
-    p.MH = p.MW = 1;
-    p.IH = p.IW = 1;
-    p.OH = p.OW = 1;
-    p.Cs = L.cout;
-    p.ON = L.cin;
+    fill_transposed(p, L.k, sh.pad_y, sh.pad_x, sh.kch);
+    p.MH = sh.ih;
+    p.MW = sh.iw;
   }
   p.M = (int)(B * p.MH * p.MW);
   return CGS_OK;
@@ -253,32 +240,27 @@ int make_window_params(const cgs_layer_desc& L, bool backward, int64_t B, const 
   if (int rc = check_layer(L)) return rc;
   if (L.k > 8) return set_error(CGS_ERR_UNSUPPORTED, "window lowering needs k <= 8");
   std::memset(&p, 0, sizeof(p));
-  const LayerShape s = layer_shape(L);
-  const int ih = backward ? s.hout : L.hin, iw = backward ? s.wout : L.win;      // image-like input
-  const int oh = backward ? L.hin : s.hout, ow = backward ? L.win : s.wout;      // output grid = M-space
-  const int pad_y = same_pad_before(ih, L.k), pad_x = same_pad_before(iw, L.k);
-  if (pad_x > IMG_XOFF) return set_error(CGS_ERR_UNSUPPORTED, "horizontal padding %d exceeds the image margin", pad_x);
+  const PassShape sh = pass_shape(L, backward);      // image-like input, output grid = M-space
+  if (sh.pad_x > IMG_XOFF) return set_error(CGS_ERR_UNSUPPORTED, "horizontal padding %d exceeds the image margin", sh.pad_x);
   p.in = in;
   p.out = out;
-  p.bias = backward ? nullptr : L.bias;
-  p.epi = EPI_RAW;
-  p.N = backward ? L.cin : L.cout;
+  p.N = sh.nch;
   p.ON = cstride(p.N);
-  p.OH = oh; p.OW = ow;
-  p.IH = ih; p.IW = iw;
+  p.OH = sh.oh; p.OW = sh.ow;
+  p.IH = sh.ih; p.IW = sh.iw;
   p.Cs = 4;
   p.cblocks = 1;
-  p.MH = oh; p.MW = ow;
+  p.MH = sh.oh; p.MW = sh.ow;
   p.S = 2; p.os = 1;
   p.nclasses = 1;
   GemmClass& g = p.cls[0];
   g.k0 = 0; g.oy0 = g.ox0 = 0;
   g.ntaps = L.k; g.nkx = 1; g.nkb = L.k;
-  for (int ky = 0; ky < L.k; ++ky) { g.dy[ky] = (signed char)(ky - pad_y); g.dx[ky] = 0; }
+  for (int ky = 0; ky < L.k; ++ky) { g.dy[ky] = (signed char)(ky - sh.pad_y); g.dx[ky] = 0; }
   p.window = 1;
   p.win_k = L.k;
-  p.win_x0 = IMG_XOFF - pad_x;
-  p.in_pitch_px = img_pitch(iw);
+  p.win_x0 = IMG_XOFF - sh.pad_x;
+  p.in_pitch_px = img_pitch(sh.iw);
   p.M = (int)(B * p.MH * p.MW);
   return CGS_OK;
 }
@@ -341,9 +323,8 @@ inline bool use_fc_split(const cgs_layer_desc& L, bool backward, int64_t B, int 
 size_t scatter_col_elems(const cgs_layer_desc& L, bool backward) {     // per-sample elements of the pass scratch buffer
   if (fc_split(L, backward) > 1) return (size_t)fc_split(L, backward) * cstride(L.cout);
   if (!use_scatter(L, backward)) return 0;
-  const LayerShape s = layer_shape(L);
-  const size_t pixels = backward ? (size_t)s.hout * s.wout : (size_t)L.hin * L.win;   // stage-1 rows per sample
-  return pixels * scatter_cols(L);
+  const PassShape sh = pass_shape(L, backward);
+  return (size_t)sh.ih * sh.iw * scatter_cols(L);          // stage-1 rows (input pixels) per sample
 }
 
 // stage 1 as a 1-tap "fc over pixels": rows = B * pixels, K = big channel count, N = k*k*4
@@ -351,12 +332,12 @@ int make_scatter_gemm_params(const cgs_layer_desc& L, bool backward, int64_t B, 
                              ConvGemmParams& p) {
   if (int rc = check_layer(L)) return rc;
   std::memset(&p, 0, sizeof(p));
-  const LayerShape s = layer_shape(L);
-  const int kch = backward ? L.cout : L.cin;                   // reduced (big) channel count
-  const int64_t pixels = backward ? (int64_t)s.hout * s.wout : (int64_t)L.hin * L.win;
+  const PassShape sh = pass_shape(L, backward);
+  const int kch = sh.kch;                                      // reduced (big) channel count
+  const int64_t pixels = (int64_t)sh.ih * sh.iw;
   p.in = in;
   p.out = col;
-  p.epi = EPI_RAW;
+  p.ep = Epilogue(EPI_RAW, ACT_NONE);
   p.N = scatter_cols(L);
   p.ON = scatter_cols(L);
   p.OH = p.OW = 1;
@@ -378,10 +359,8 @@ int make_scatter_gemm_params(const cgs_layer_desc& L, bool backward, int64_t B, 
 struct Col2imParams {
   const float* col;
   float* out;
-  const float* bias;
-  const float* aux;
+  Epilogue ep;
   int IH, IW, OH, OW, k, pad_y, pad_x, pitch;
-  int epi, act, round_out;
   int out_pitch, out_xoff;   // row pitch (pixels) and first data column of out / aux (dense: OW, 0)
   long long pixels;          // B * OH * out_pitch (pad columns are written as zeros)
   const int* live;           // early exit: images still in the batch (null = all)
@@ -420,48 +399,11 @@ __global__ void __launch_bounds__(256) col2im_kernel(const Col2imParams p) {
         a.x += v.x; a.y += v.y; a.z += v.z; a.w += v.w;
       }
     }
-    float4 o = a;
-    if (p.epi == EPI_FWD) {
-      const float4 bb = p.bias ? __ldg(reinterpret_cast<const float4*>(p.bias)) : make_float4(0.f, 0.f, 0.f, 0.f);
-      o.x = act_apply(a.x + bb.x, p.act); o.y = act_apply(a.y + bb.y, p.act);
-      o.z = act_apply(a.z + bb.z, p.act); o.w = act_apply(a.w + bb.w, p.act);
-    } else if (p.epi == EPI_BWD) {
-      const float4 yv = __ldg(reinterpret_cast<const float4*>(p.aux + idx * 4));
-      o.x = a.x * act_grad_from_output(yv.x, p.act); o.y = a.y * act_grad_from_output(yv.y, p.act);
-      o.z = a.z * act_grad_from_output(yv.z, p.act); o.w = a.w * act_grad_from_output(yv.w, p.act);
-    }
-    if (p.round_out) { o.x = tf32_rn(o.x); o.y = tf32_rn(o.y); o.z = tf32_rn(o.z); o.w = tf32_rn(o.w); }
-    *reinterpret_cast<float4*>(p.out + idx * 4) = o;
+    float4 x0 = make_float4(0.f, 0.f, 0.f, 0.f);     // no policy step in this lowering (run_pass)
+    if (p.ep.mode == EPI_FWD && p.ep.bias) x0 = __ldg(reinterpret_cast<const float4*>(p.ep.bias));
+    else if (p.ep.mode == EPI_BWD) x0 = __ldg(reinterpret_cast<const float4*>(p.ep.aux + idx * 4));
+    *reinterpret_cast<float4*>(p.out + idx * 4) = epilogue4(p.ep, 0, a, x0, x0);
   }
-}
-
-struct PassEpi {
-  int epi = EPI_RAW;
-  int act = ACT_NONE;
-  const float* aux = nullptr;
-  int round_out = 0;
-  const ConvGemmParams* upd = nullptr;   // EPI_UPDATE fields
-  const int* live = nullptr;             // early exit: device-resident count of the images still in the batch
-};
-
-// Epilogue description of an image-edge kernel (edge_conv.cuh) from the pass epilogue.
-EdgeEpi make_edge_epi(const PassEpi& e, const float* bias) {
-  EdgeEpi x;
-  std::memset(&x, 0, sizeof(x));
-  x.epi = e.epi;
-  x.act_tanh = (e.act == ACT_TANH);
-  x.slope = e.act == ACT_RELU ? 0.f : (e.act == ACT_LRELU ? 0.2f : 1.f);
-  x.round_out = e.round_out;
-  x.bias = (e.epi == EPI_FWD) ? bias : nullptr;
-  x.aux = e.aux;
-  x.live = e.live;
-  if (e.upd) {
-    x.epi = EPI_UPDATE;
-    x.mom = e.upd->mom; x.first = e.upd->first; x.sgd = e.upd->sgd; x.rate = e.upd->rate; x.alpha = e.upd->alpha;
-    x.clip = e.upd->clip; x.vmin = e.upd->vmin; x.vmax = e.upd->vmax;
-    x.round_out = 0;
-  }
-  return x;
 }
 
 // CGS_DEBUG_EDGE_GENERAL: keep the image-edge passes on the general tcgen05 lowerings
@@ -490,20 +432,13 @@ __global__ void __launch_bounds__(256) splitk_reduce_kernel(const __grid_constan
       const float4 v = __ldg(reinterpret_cast<const float4*>(part + ((size_t)b * S + s) * p.ON + ng * 4));
       a.x += v.x; a.y += v.y; a.z += v.z; a.w += v.w;
     }
-    float4 x0 = make_float4(0.f, 0.f, 0.f, 0.f), x1 = x0;
-    if (p.epi == EPI_FWD) { if (p.bias) x0 = __ldg(reinterpret_cast<const float4*>(p.bias + ng * 4)); }
-    else if (p.epi == EPI_BWD) x0 = __ldg(reinterpret_cast<const float4*>(p.aux + off));
-    else if (p.epi == EPI_UPDATE) {
-      x0 = *reinterpret_cast<const float4*>(p.out + off);
-      if (!p.sgd && !p.first) x1 = *reinterpret_cast<const float4*>(p.mom + off);
-    }
-    *reinterpret_cast<float4*>(p.out + off) = epilogue4(p, off, a, x0, x1);
+    float4 x0, x1;
+    epilogue_operands4(p.ep, p.out, off, ng * 4, x0, x1);
+    *reinterpret_cast<float4*>(p.out + off) = epilogue4(p.ep, off, a, x0, x1);
   }
 }
 
-int launch_splitk_reduce(ConvGemmParams pe, const float* part, int S, int64_t B, cudaStream_t st) {
-  pe.act_tanh = (pe.act == ACT_TANH);
-  pe.slope = pe.act == ACT_RELU ? 0.f : (pe.act == ACT_LRELU ? 0.2f : 1.f);
+int launch_splitk_reduce(const ConvGemmParams& pe, const float* part, int S, int64_t B, cudaStream_t st) {
   const long long total4 = (long long)B * (pe.ON / 4);
   long long blocks = (total4 + 255) / 256;
   if (blocks > 148 * 8) blocks = 148 * 8;
@@ -515,41 +450,39 @@ int launch_splitk_reduce(ConvGemmParams pe, const float* part, int S, int64_t B,
 
 // Parameters of the fused image-edge kernels (edge_conv.cuh) for a scatter- / window-lowered pass; false when the
 // shape is not covered (the general tcgen05 lowering runs instead) or the kernels are switched off.
-bool make_edge_narrow(const cgs_layer_desc& L, bool backward, int64_t B, const float* in, float* out, const PassEpi& e,
-                      int img_mode, int w_cols, EdgeNarrowParams& q) {
-  const LayerShape s = layer_shape(L);
-  const int kch = backward ? L.cout : L.cin, cimg = backward ? L.cin : L.cout;
-  const int iw = backward ? s.wout : L.win;
-  if (!edge_kernels_enabled() || !use_scatter(L, backward) || !edge_narrow_supported(kch, L.k, cimg, iw) || w_cols != kch)
+bool make_edge_narrow(const cgs_layer_desc& L, bool backward, int64_t B, const float* in, float* out, const Epilogue& e,
+                      const int* live, int img_mode, EdgeNarrowParams& q) {
+  const PassShape sh = pass_shape(L, backward);
+  if (!edge_kernels_enabled() || !use_scatter(L, backward) || !edge_narrow_supported(sh.kch, L.k, sh.nch, sh.iw) ||
+      sh.cols != sh.kch)
     return false;
   std::memset(&q, 0, sizeof(q));
-  q.in = in; q.out = out; q.w = backward ? L.w_bwd : L.w_fwd;
-  q.B = (int)B; q.K = kch; q.k = L.k; q.cimg = cimg;
-  if (!backward) {
-    q.IH = L.hin; q.IW = L.win; q.OH = s.hout; q.OW = s.wout;
-    q.pad_y = same_pad_before(s.hout, L.k); q.pad_x = same_pad_before(s.wout, L.k);
-  } else {
-    q.IH = s.hout; q.IW = s.wout; q.OH = L.hin; q.OW = L.win;
-    q.pad_y = same_pad_before(L.hin, L.k); q.pad_x = same_pad_before(L.win, L.k);
-  }
+  q.in = in; q.out = out; q.w = sh.w;
+  q.B = (int)B; q.K = sh.kch; q.k = L.k; q.cimg = sh.nch;
+  q.IH = sh.ih; q.IW = sh.iw; q.OH = sh.oh; q.OW = sh.ow;
+  q.pad_y = sh.pad_y; q.pad_x = sh.pad_x;
   q.out_pitch = img_mode == IMG_PITCHED ? img_pitch(q.OW) : q.OW;
   q.out_xoff = img_mode == IMG_PITCHED ? IMG_XOFF : 0;
   q.s2d = img_mode == IMG_S2D;
-  q.e = make_edge_epi(e, L.bias);
+  q.ep = e;
+  q.ep.bias = sh.bias;
+  q.live = live;
   return true;
 }
 
-bool make_edge_wide(const cgs_layer_desc& L, bool backward, int64_t B, const float* in, float* out, const PassEpi& e,
-                    const ConvGemmParams& wp, EdgeWideParams& q) {     // wp = make_window_params of the same pass
-  const int cimg = backward ? L.cout : L.cin;
-  if (!edge_kernels_enabled() || !edge_wide_supported(wp.N, L.k, cimg) || wp.ON != wp.N) return false;
+bool make_edge_wide(const cgs_layer_desc& L, bool backward, int64_t B, const float* in, float* out, const Epilogue& e,
+                    const int* live, const ConvGemmParams& wp, EdgeWideParams& q) {   // wp = make_window_params of the same pass
+  const PassShape sh = pass_shape(L, backward);
+  if (!edge_kernels_enabled() || !edge_wide_supported(wp.N, L.k, sh.kch) || wp.ON != wp.N) return false;
   std::memset(&q, 0, sizeof(q));
-  q.in = in; q.out = out; q.w = backward ? L.w_bwd : L.w_fwd;
+  q.in = in; q.out = out; q.w = sh.w;
   q.IH = wp.IH; q.pitch = wp.in_pitch_px; q.xoff = IMG_XOFF; q.OH = wp.OH; q.OW = wp.OW; q.ON = wp.ON; q.N = wp.N;
-  q.k = L.k; q.cimg = cimg;
-  q.pad_y = same_pad_before(wp.IH, L.k); q.pad_x = same_pad_before(wp.IW, L.k);
+  q.k = L.k; q.cimg = sh.kch;
+  q.pad_y = sh.pad_y; q.pad_x = sh.pad_x;
   q.M = (long long)B * wp.OH * wp.OW;
-  q.e = make_edge_epi(e, backward ? nullptr : L.bias);
+  q.ep = e;
+  q.ep.bias = sh.bias;
+  q.live = live;
   return true;
 }
 
@@ -557,35 +490,38 @@ bool make_edge_wide(const cgs_layer_desc& L, bool backward, int64_t B, const flo
 // first conv; backward: their data-gradients in the opposite order) as ONE kernel when both fit a one-image tile.
 // Returns 1 when the pair was launched, 0 when the caller should run the two passes separately, < 0 on error.
 int try_edge_pair(const cgs_layer_desc& ln, const cgs_layer_desc& lw, bool backward, int64_t B, const float* in,
-                  float* mid, float* out, const PassEpi& en, const PassEpi& ew, int store_mid, int math, cudaStream_t st) {
-  if (math != CGS_MATH_TF32_TENSOR || (debug_flags() & CGS_DEBUG_NO_EDGE_PAIR) || en.upd) return 0;
+                  float* mid, float* out, const Epilogue& en, const Epilogue& ew, const int* live, int store_mid, int math,
+                  cudaStream_t st) {
+  if (math != CGS_MATH_TF32_TENSOR || (debug_flags() & CGS_DEBUG_NO_EDGE_PAIR) || en.mode == EPI_UPDATE) return 0;
   if (!use_scatter(ln, backward) || !use_window(lw, backward)) return 0;
   EdgeNarrowParams qn;
-  if (!make_edge_narrow(ln, backward, B, in, mid, en, false, backward ? ln.kcols_bwd : ln.kcols_fwd, qn)) return 0;
+  if (!make_edge_narrow(ln, backward, B, in, mid, en, live, IMG_PITCHED, qn)) return 0;
   ConvGemmParams wp;
   if (make_window_params(lw, backward, B, mid, out, wp) != CGS_OK) return 0;
-  if ((backward ? lw.rows_bwd : lw.rows_fwd) != (backward ? lw.cin : lw.cout) ||
-      (backward ? lw.kcols_bwd : lw.kcols_fwd) != window_kcols(lw)) return 0;
+  const PassShape shw = pass_shape(lw, backward);
+  if (shw.rows != shw.nch || shw.cols != window_kcols(lw)) return 0;
   EdgeWideParams qw;
-  if (!make_edge_wide(lw, backward, B, mid, out, ew, wp, qw)) return 0;
+  if (!make_edge_wide(lw, backward, B, mid, out, ew, live, wp, qw)) return 0;
   if (!edge_pair_supported(qn, qw)) return 0;
   if (int rc = launch_edge_pair(qn, qw, store_mid, st)) return rc;
   return 1;
 }
 
-// One layer pass (forward or data-gradient) with its fused epilogue; picks the gather or the scatter lowering.
-int run_pass(const cgs_layer_desc& L, bool backward, int64_t B, const float* in, float* out, const PassEpi& e,
-             float* col, int math, cudaStream_t st, int img_mode = IMG_PITCHED, bool defer_reduce = false) {
-  const float* w = backward ? L.w_bwd : L.w_fwd;
-  const int rows = backward ? L.rows_bwd : L.rows_fwd;
-  const int cols = backward ? L.kcols_bwd : L.kcols_fwd;
-  if (!w) return set_error(CGS_ERR_INVALID, "layer has no packed %s weights", backward ? "backward" : "forward");
+// One layer pass (forward or data-gradient) with its fused epilogue `e` (its bias is the layer's, set here); picks
+// the gather or the scatter lowering.
+int run_pass(const cgs_layer_desc& L, bool backward, int64_t B, const float* in, float* out, const Epilogue& e,
+             const int* live, float* col, int math, cudaStream_t st, int img_mode = IMG_PITCHED, bool defer_reduce = false) {
+  const PassShape sh = pass_shape(L, backward);
+  if (!sh.w) return set_error(CGS_ERR_INVALID, "layer has no packed %s weights", backward ? "backward" : "forward");
+  Epilogue ep = e;
+  ep.bias = sh.bias;
   if (use_scatter(L, backward)) {
     if (!col) return set_error(CGS_ERR_WORKSPACE, "scatter pass needs a column workspace");
-    if (rows != scatter_cols(L)) return set_error(CGS_ERR_INVALID, "weights of this pass must be in scatter layout (%d rows)", scatter_cols(L));
+    if (e.mode == EPI_UPDATE) return set_error(CGS_ERR_UNSUPPORTED, "the policy step is not fused into a scatter-lowered pass");
+    if (sh.rows != scatter_cols(L)) return set_error(CGS_ERR_INVALID, "weights of this pass must be in scatter layout (%d rows)", scatter_cols(L));
     {
       EdgeNarrowParams q;
-      if (math == CGS_MATH_TF32_TENSOR && !e.upd && make_edge_narrow(L, backward, B, in, out, e, img_mode, cols, q))
+      if (math == CGS_MATH_TF32_TENSOR && e.mode != EPI_UPDATE && make_edge_narrow(L, backward, B, in, out, e, live, img_mode, q))
         return launch_edge_narrow(q, st);
       if (img_mode == IMG_S2D) return set_error(CGS_ERR_UNSUPPORTED, "s2d image layout needs the tcgen05 edge kernels");
     }
@@ -593,29 +529,19 @@ int run_pass(const cgs_layer_desc& L, bool backward, int64_t B, const float* in,
     if (int rc = make_scatter_gemm_params(L, backward, B, in, col, p)) return rc;
     // (early exit: the 1-tap GEMM over pixels runs over the full batch -- its rows are pixels, not images; the
     //  col2im below stops at the live images)
-    if (int rc = launch_gemm(p, w, rows, cols, math, st)) return rc;
-    const LayerShape s = layer_shape(L);
+    if (int rc = launch_gemm(p, sh.w, sh.rows, sh.cols, math, st)) return rc;
     Col2imParams c;
     c.col = col;
     c.out = out;
-    c.bias = (e.epi == EPI_FWD) ? L.bias : nullptr;
-    c.aux = e.aux;
+    c.ep = ep;
     c.k = L.k;
     c.pitch = scatter_cols(L);
-    c.epi = e.epi;
-    c.act = e.act;
-    c.round_out = e.round_out;
-    if (!backward) {           // deconv forward: col over the input grid, out = 2x grid
-      c.IH = L.hin; c.IW = L.win; c.OH = s.hout; c.OW = s.wout;
-      c.pad_y = same_pad_before(s.hout, L.k); c.pad_x = same_pad_before(s.wout, L.k);
-    } else {                   // conv data-gradient: col over the conv-output grid, out = conv-input grid
-      c.IH = s.hout; c.IW = s.wout; c.OH = L.hin; c.OW = L.win;
-      c.pad_y = same_pad_before(L.hin, L.k); c.pad_x = same_pad_before(L.win, L.k);
-    }
+    c.IH = sh.ih; c.IW = sh.iw; c.OH = sh.oh; c.OW = sh.ow;   // col over the input grid, out = 2x grid
+    c.pad_y = sh.pad_y; c.pad_x = sh.pad_x;
     c.out_pitch = img_mode == IMG_PITCHED ? img_pitch(c.OW) : c.OW;
     c.out_xoff = img_mode == IMG_PITCHED ? IMG_XOFF : 0;
     c.pixels = (long long)B * c.OH * c.out_pitch;
-    c.live = e.live;
+    c.live = live;
     long long blocks = (c.pixels + 255) / 256;
     if (blocks > 148 * 16) blocks = 148 * 16;
     col2im_kernel<<<(int)blocks, 256, 0, st>>>(c); count_launch();
@@ -623,21 +549,13 @@ int run_pass(const cgs_layer_desc& L, bool backward, int64_t B, const float* in,
   }
   ConvGemmParams p;
   if (const int S = fc_split(L, backward); use_fc_split(L, backward, B, math, col)) {
-    if (int rc = make_forward_params(L, B, in, col, p)) return rc;
+    if (int rc = make_pass_params(L, false, B, in, col, p)) return rc;
     ConvGemmParams pe = p;                    // epilogue description of the real output
     pe.out = out;
-    pe.bias = L.bias;
-    pe.epi = e.epi; pe.act = e.act; pe.aux = e.aux; pe.round_out = e.round_out;
-    if (e.upd) {
-      pe.epi = EPI_UPDATE;
-      pe.mom = e.upd->mom; pe.first = e.upd->first; pe.sgd = e.upd->sgd; pe.rate = e.upd->rate; pe.alpha = e.upd->alpha;
-      pe.clip = e.upd->clip; pe.vmin = e.upd->vmin; pe.vmax = e.upd->vmax;
-      pe.round_out = 0;
-    }
-    p.bias = nullptr;
-    p.epi = EPI_RAW;
-    p.live = e.live;
-    pe.live = e.live;
+    pe.ep = ep;
+    pe.live = live;
+    p.ep = Epilogue(EPI_RAW, ACT_NONE);
+    p.live = live;
     p.nclasses = S;
     p.cblocks = L.cin / 32 / S;
     for (int c = 0; c < S; ++c) {
@@ -652,37 +570,27 @@ int run_pass(const cgs_layer_desc& L, bool backward, int64_t B, const float* in,
     }
     p.OH = S;
     { static const int bn = env_int("CGS_FC_BN", 256); p.force_bn = bn; }
-    if (int rc = launch_gemm(p, w, rows, cols, math, st)) return rc;
+    if (int rc = launch_gemm(p, sh.w, sh.rows, sh.cols, math, st)) return rc;
     if (defer_reduce) return CGS_OK;          // the head kernel adds the partial sums itself (head_takes_partials)
     return launch_splitk_reduce(pe, col, S, B, st);
   }
   if (use_window(L, backward)) {
-    if (rows != (backward ? L.cin : L.cout) || cols != window_kcols(L))
+    if (sh.rows != sh.nch || sh.cols != window_kcols(L))
       return set_error(CGS_ERR_INVALID, "weights of this pass must be in window layout (%d columns)", window_kcols(L));
     if (int rc = make_window_params(L, backward, B, in, out, p)) return rc;
     EdgeWideParams q;
     if (img_mode == IMG_S2D) {               // image-like input in s2d layout: tcgen05 resident-patch kernel
-      if (math == CGS_MATH_TF32_TENSOR && make_edge_wide(L, backward, B, in, out, e, p, q) && edge_wide_tc_supported(q))
+      if (math == CGS_MATH_TF32_TENSOR && make_edge_wide(L, backward, B, in, out, e, live, p, q) && edge_wide_tc_supported(q))
         return launch_edge_wide_tc(q, (int)B, st);
       return set_error(CGS_ERR_UNSUPPORTED, "s2d image layout needs the tcgen05 edge kernels");
     }
-    if (math == CGS_MATH_TF32_TENSOR && make_edge_wide(L, backward, B, in, out, e, p, q)) return launch_edge_wide(q, st);
-  } else if (int rc = backward ? make_backward_params(L, B, in, out, p) : make_forward_params(L, B, in, out, p)) {
+    if (math == CGS_MATH_TF32_TENSOR && make_edge_wide(L, backward, B, in, out, e, live, p, q)) return launch_edge_wide(q, st);
+  } else if (int rc = make_pass_params(L, backward, B, in, out, p)) {
     return rc;
   }
-  if (!backward) p.bias = L.bias;
-  p.epi = e.epi;
-  p.act = e.act;
-  p.aux = e.aux;
-  p.round_out = e.round_out;
-  p.live = e.live;
-  if (e.upd) {
-    p.epi = EPI_UPDATE;
-    p.mom = e.upd->mom; p.first = e.upd->first; p.sgd = e.upd->sgd; p.rate = e.upd->rate; p.alpha = e.upd->alpha;
-    p.clip = e.upd->clip; p.vmin = e.upd->vmin; p.vmax = e.upd->vmax;
-    p.round_out = 0;
-  }
-  return launch_gemm(p, w, rows, cols, math, st);
+  p.ep = ep;
+  p.live = live;
+  return launch_gemm(p, sh.w, sh.rows, sh.cols, math, st);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -698,7 +606,6 @@ struct HeadParams {
   const float* w;       // [K]
   const float* bias;    // [1] device scalar (folded)
   int K;
-  int act;              // activation of the producer of feat
   float* dpre;          // [B, K] or nullptr (no backward wanted)
   const float* img;     // [B, img_elems] current image
   float* best_img;      // [B, img_elems]
@@ -719,12 +626,11 @@ struct HeadParams {
   float* final_feature; // [B_orig, feat_elems]: state of a sample at the step it exits (early-exit) or nullptr
   float exit_logit;
   int round_out;        // round dpre to TF32 (RN): it feeds a kind::tf32 MMA
-  // split-K producer (fc_split): feat is not materialised; feat[b][k] = act(sum_s part[b][s][k] + fc_bias[k])
+  // split-K producer (fc_split): feat is not materialised; feat[b][k] = act(sum_s part[b][s][k] + bias[k])
   const float* part;    // [B][S][K] partial sums or nullptr
   int S;
-  const float* fc_bias;
-  float fc_slope;       // relu 0, lrelu 0.2, none 1 (same expression as the GEMM epilogue: bit-identical)
-  int fc_tanh;
+  // the forward epilogue of the producer of feat (its activation; its bias when feat is given as partial sums)
+  Epilogue feat_ep;
   const int* live;      // early exit: device-resident count of the rows still in the batch (null = gridDim.x)
 };
 
@@ -738,11 +644,8 @@ __device__ __forceinline__ float4 head_feat4(const HeadParams& p, const float* f
     const float4 v = __ldg(reinterpret_cast<const float4*>(pr + (size_t)s * p.K));
     a.x += v.x; a.y += v.y; a.z += v.z; a.w += v.w;
   }
-  const float4 bb = p.fc_bias ? __ldg(reinterpret_cast<const float4*>(p.fc_bias + k)) : make_float4(0.f, 0.f, 0.f, 0.f);
-  const float vx = a.x + bb.x, vy = a.y + bb.y, vz = a.z + bb.z, vw = a.w + bb.w;
-  if (p.fc_tanh) return make_float4(tanhf(vx), tanhf(vy), tanhf(vz), tanhf(vw));
-  return make_float4(fmaxf(vx, vx * p.fc_slope), fmaxf(vy, vy * p.fc_slope), fmaxf(vz, vz * p.fc_slope),
-                     fmaxf(vw, vw * p.fc_slope));
+  const float4 bb = p.feat_ep.bias ? __ldg(reinterpret_cast<const float4*>(p.feat_ep.bias + k)) : make_float4(0.f, 0.f, 0.f, 0.f);
+  return epilogue4_t<EPI_FWD>(p.feat_ep, 0, a, bb, bb);
 }
 
 __global__ void __launch_bounds__(256) head_kernel(const HeadParams p) {
@@ -809,11 +712,7 @@ __global__ void __launch_bounds__(256) head_kernel(const HeadParams p) {
     for (int k = threadIdx.x * 4; k < p.K; k += 256 * 4) {
       const float4 a = (k < 256 * 4) ? a_first : head_feat4(p, f, b, k);
       const float4 ww = __ldg(reinterpret_cast<const float4*>(p.w + k));
-      float4 o;
-      o.x = dl * ww.x * act_grad_from_output(a.x, p.act);
-      o.y = dl * ww.y * act_grad_from_output(a.y, p.act);
-      o.z = dl * ww.z * act_grad_from_output(a.z, p.act);
-      o.w = dl * ww.w * act_grad_from_output(a.w, p.act);
+      float4 o = epilogue4_t<EPI_BWD>(p.feat_ep, 0, make_float4(dl * ww.x, dl * ww.y, dl * ww.z, dl * ww.w), a, a);
       if (p.round_out) { o.x = tf32_rn(o.x); o.y = tf32_rn(o.y); o.z = tf32_rn(o.z); o.w = tf32_rn(o.w); }
       *reinterpret_cast<float4*>(d + k) = o;
     }
@@ -984,7 +883,7 @@ static bool chain_s2d(const Chain& c, int math) {
   if (Ln.cin != 64 || Ln.cout > 3 || Lw.cout != 64 || Lw.cin != Ln.cout) return false;
   if ((Ln.k != 4 && Ln.k != 5) || (Lw.k != 4 && Lw.k != 5)) return false;
   if (!edge_tc_width_supported(Ln.win) || Ln.hin != Ln.win || Lw.hin != 2 * Ln.hin || Lw.win != 2 * Ln.win) return false;
-  if (same_pad_before(Lw.hin, Lw.k) != 1 || same_pad_before(2 * Ln.hin, Ln.k) != 1) return false;
+  if (pass_shape(Lw, false).pad_y != 1 || pass_shape(Ln, false).pad_y != 1) return false;
   return true;
 }
 
@@ -1039,68 +938,54 @@ static bool head_takes_partials(const Chain& c, const Workspace& w, int64_t B, i
 static int run_forward(const Chain& c, const Workspace& w, int64_t B, int math, cudaStream_t st,
                        const int* live = nullptr) {
   const int img_mode = chain_s2d(c, math) ? IMG_S2D : IMG_PITCHED;
-  for (int i = 0; i < c.n; ++i) {
-    PassEpi e;
-    e.live = live;
-    e.epi = EPI_FWD;
-    e.act = c.layers[i].act;
-    // TF32 path: activations that feed another MMA are rounded to TF32 (RN) where they are produced, so the
-    // tensor core's operand truncation is exact; the image (returned to the caller) and the head input stay FP32
+  // TF32 path: activations that feed another MMA are rounded to TF32 (RN) where they are produced, so the tensor
+  // core's operand truncation is exact; the image (returned to the caller) and the head input stay FP32
+  auto epi = [&](int i) {
+    Epilogue e(EPI_FWD, c.layers[i].act);
     e.round_out = (math == CGS_MATH_TF32_TENSOR) && (i != c.n_gtail - 1) && (i != c.n - 1);
+    return e;
+  };
+  for (int i = 0; i < c.n; ++i) {
     if (i == c.n_gtail - 1 && i + 1 < c.n && img_mode == IMG_PITCHED) {
       // generator's last deconv + discriminator's first conv on the same image: one kernel when the shapes allow
-      PassEpi e2;
-      e2.live = live;
-      e2.epi = EPI_FWD;
-      e2.act = c.layers[i + 1].act;
-      e2.round_out = (math == CGS_MATH_TF32_TENSOR) && (i + 1 != c.n - 1);
-      const int rc = try_edge_pair(c.layers[i], c.layers[i + 1], false, B, w.act[i], w.act[i + 1], w.act[i + 2], e, e2, 1, math, st);
+      const int rc = try_edge_pair(c.layers[i], c.layers[i + 1], false, B, w.act[i], w.act[i + 1], w.act[i + 2], epi(i),
+                                   epi(i + 1), live, 1, math, st);
       if (rc < 0) return rc;
       if (rc == 1) { ++i; continue; }
     }
     const bool defer = (i == c.n - 1) && head_takes_partials(c, w, B, math);
-    if (int rc = run_pass(c.layers[i], false, B, w.act[i], w.act[i + 1], e, w.col, math, st, img_mode, defer)) return rc;
+    if (int rc = run_pass(c.layers[i], false, B, w.act[i], w.act[i + 1], epi(i), live, w.col, math, st, img_mode, defer))
+      return rc;
   }
   return CGS_OK;
 }
 
-// Backward from dpre[c.n-1] (already in w.g[0]) down to the feature.  `upd` != null fuses the policy step into
-// the last GEMM's epilogue; otherwise the raw gradient is written to grad_out.
-static int run_backward(const Chain& c, const Workspace& w, int64_t B, int math, const ConvGemmParams* upd,
+// Backward from dpre[c.n-1] (already in w.g[0]) down to the feature.  `upd` != null is the policy step fused into
+// the last pass's epilogue; otherwise the raw gradient is written to grad_out.
+static int run_backward(const Chain& c, const Workspace& w, int64_t B, int math, const Epilogue* upd,
                         float* grad_out, cudaStream_t st, const int* live = nullptr) {
   const int img_mode = chain_s2d(c, math) ? IMG_S2D : IMG_PITCHED;
+  // pass i: times the derivative of the activation that produced its input, the policy step or nothing (i = 0)
+  auto epi = [&](int i) {
+    if (i == 0) return upd ? *upd : Epilogue(EPI_RAW, ACT_NONE);
+    Epilogue e(EPI_BWD, c.layers[i - 1].act);
+    e.aux = w.act[i];
+    e.round_out = (math == CGS_MATH_TF32_TENSOR);
+    return e;
+  };
   int cur = 0;
   for (int i = c.n - 1; i >= 0; --i) {
     float* dst = (i == 0) ? (upd ? w.act[0] : grad_out) : w.g[cur ^ 1];
-    PassEpi e;
-    e.live = live;
-    if (i > 0) {
-      e.epi = EPI_BWD;
-      e.aux = w.act[i];
-      e.act = c.layers[i - 1].act;
-      e.round_out = (math == CGS_MATH_TF32_TENSOR);
-    } else {
-      e.upd = upd;
-    }
     if (i == c.n_gtail && i >= 1 && img_mode == IMG_PITCHED) {
       // data-gradients of D's first conv and G's last deconv: one kernel, the image gradient never leaves the SM
-      PassEpi e2;
-      e2.live = live;
       float* dst2 = (i - 1 == 0) ? (upd ? w.act[0] : grad_out) : w.g[cur ^ 1];
-      if (i - 1 > 0) {
-        e2.epi = EPI_BWD;
-        e2.aux = w.act[i - 1];
-        e2.act = c.layers[i - 2].act;
-        e2.round_out = (math == CGS_MATH_TF32_TENSOR);
-      } else {
-        e2.upd = upd;
-      }
       // the intermediate (image gradient) buffer is only described, never written: any valid pointer of that size
-      const int rc = try_edge_pair(c.layers[i], c.layers[i - 1], true, B, w.g[cur], w.g[cur ^ 1], dst2, e, e2, 0, math, st);
+      const int rc = try_edge_pair(c.layers[i], c.layers[i - 1], true, B, w.g[cur], w.g[cur ^ 1], dst2, epi(i), epi(i - 1),
+                                   live, 0, math, st);
       if (rc < 0) return rc;
       if (rc == 1) { --i; cur ^= 1; continue; }
     }
-    if (int rc = run_pass(c.layers[i], true, B, w.g[cur], dst, e, w.col, math, st, img_mode)) return rc;
+    if (int rc = run_pass(c.layers[i], true, B, w.g[cur], dst, epi(i), live, w.col, math, st, img_mode)) return rc;
     cur ^= 1;
   }
   return CGS_OK;
@@ -1132,14 +1017,12 @@ static int head_launch(const Chain& c, const Workspace& w, int64_t B, HeadParams
     const cgs_layer_desc& L = c.layers[c.n - 1];
     hp.part = w.col;
     hp.S = fc_split(L, false);
-    hp.fc_bias = L.bias;
-    hp.fc_slope = L.act == ACT_RELU ? 0.f : (L.act == ACT_LRELU ? 0.2f : 1.f);
-    hp.fc_tanh = (L.act == ACT_TANH);
   }
+  hp.feat_ep = Epilogue(EPI_FWD, c.layers[c.n - 1].act);
+  hp.feat_ep.bias = hp.part ? c.layers[c.n - 1].bias : nullptr;
   hp.w = c.head.w_fwd;
   hp.bias = c.head.bias;
   hp.K = c.head.cin;
-  hp.act = c.layers[c.n - 1].act;
   hp.img = w.act[c.n_gtail];
   {
     const cgs_layer_desc& Li = c.layers[c.n_gtail - 1];          // producer of the image
@@ -1237,8 +1120,7 @@ extern "C" int cgs_refine_conv(const cgs_net_desc* gtail, const cgs_net_desc* d,
   hp.step = -1;
   hp.dpre = K > 0 ? w.g[0] : nullptr;
   if (int rc = head_launch(c, w, B, hp, cfg->math, st)) return rc;
-  ConvGemmParams upd;
-  std::memset(&upd, 0, sizeof(upd));
+  Epilogue upd(EPI_UPDATE, ACT_NONE);
   upd.sgd = cfg->method == CGS_POLICY_SGD;
   upd.rate = cfg->rate;
   upd.alpha = cfg->alpha;
@@ -1329,8 +1211,8 @@ extern "C" int cgs_forward_logits_and_grad(const cgs_net_desc* gtail, const cgs_
 
 static size_t layer_stage_elems(const cgs_layer_desc& L, bool backward) {   // pitched copy of an image-like input
   if (!use_window(L, backward)) return 0;
-  const LayerShape s = layer_shape(L);
-  return backward ? tensor_elems(s.hout, s.wout, L.cout) : tensor_elems(L.hin, L.win, L.cin);
+  const PassShape sh = pass_shape(L, backward);
+  return tensor_elems(sh.ih, sh.iw, sh.kch);
 }
 
 extern "C" size_t cgs_layer_workspace_bytes(const cgs_layer_desc* L, int64_t B) {
@@ -1345,7 +1227,7 @@ extern "C" size_t cgs_layer_workspace_bytes(const cgs_layer_desc* L, int64_t B) 
 // The single-layer entry points take and return DENSE tensors; image-like inputs of window-lowered passes are
 // re-laid out into the workspace first (inside the refinement chain they are produced pitched, no copy).
 static int layer_pass_dense(const cgs_layer_desc& L, bool backward, int math, int64_t B, const float* in, float* out,
-                            const PassEpi& e, void* workspace, size_t workspace_bytes, cudaStream_t st) {
+                            const Epilogue& e, void* workspace, size_t workspace_bytes, cudaStream_t st) {
   const bool needs_ws = use_scatter(L, backward) || use_window(L, backward);
   if (needs_ws && (!workspace || workspace_bytes < cgs_layer_workspace_bytes(&L, B)))
     return set_error(CGS_ERR_WORKSPACE, "workspace too small");
@@ -1356,14 +1238,15 @@ static int layer_pass_dense(const cgs_layer_desc& L, bool backward, int math, in
   float* stage = base + ((ce * (size_t)B + 63) & ~size_t(63));
   int img_mode = IMG_DENSE;
   if (use_window(L, backward)) {
-    const LayerShape s = layer_shape(L);
-    const int h = backward ? s.hout : L.hin, w = backward ? s.wout : L.win;
+    const PassShape sh = pass_shape(L, backward);
+    const int h = sh.ih, w = sh.iw;
     // the image-like input is re-laid out first (inside the chain it is produced in that layout: no copy there)
     ConvGemmParams wp;
     EdgeWideParams q;
-    const bool tc = math == CGS_MATH_TF32_TENSOR && edge_kernels_enabled() && w >= 32 && w <= 128 &&
-                    make_window_params(L, backward, B, in, out, wp) == CGS_OK && make_edge_wide(L, backward, B, in, out, e, wp, q) &&
-                    edge_wide_tc_supported(q);
+    const bool tc = math == CGS_MATH_TF32_TENSOR && edge_kernels_enabled() &&
+                    make_window_params(L, backward, B, in, out, wp) == CGS_OK &&
+                    make_edge_wide(L, backward, B, in, out, e, nullptr, wp, q) && edge_wide_tc_supported(q) &&
+                    w == 2 * q.OW;            // the s2d layout pairs image columns: an odd width has no s2d form
     if (tc) {
       if (int rc = image_to_s2d(in, stage, B, h, w, st)) return rc;
       img_mode = IMG_S2D;
@@ -1373,17 +1256,15 @@ static int layer_pass_dense(const cgs_layer_desc& L, bool backward, int math, in
     }
     in = stage;
   }
-  return run_pass(L, backward, B, in, out, e, col, math, st, img_mode);
+  return run_pass(L, backward, B, in, out, e, nullptr, col, math, st, img_mode);
 }
 
 extern "C" int cgs_layer_forward(const cgs_layer_desc* L, int math, int64_t B, const float* x, float* y,
                                  void* workspace, size_t workspace_bytes, cgs_stream_t stream) {
   if (int rc = require_sm100()) return rc;
   if (!L || !x || !y) return set_error(CGS_ERR_INVALID, "null argument");
-  PassEpi e;
-  e.epi = EPI_FWD;
-  e.act = L->act;
-  return layer_pass_dense(*L, false, math, B, x, y, e, workspace, workspace_bytes, (cudaStream_t)stream);
+  return layer_pass_dense(*L, false, math, B, x, y, Epilogue(EPI_FWD, L->act), workspace, workspace_bytes,
+                          (cudaStream_t)stream);
 }
 
 extern "C" int cgs_layer_backward(const cgs_layer_desc* L, int math, int64_t B, const float* dy, float* dx,
@@ -1391,11 +1272,10 @@ extern "C" int cgs_layer_backward(const cgs_layer_desc* L, int math, int64_t B, 
                                   cgs_stream_t stream) {
   if (int rc = require_sm100()) return rc;
   if (!L || !dy || !dx) return set_error(CGS_ERR_INVALID, "null argument");
-  PassEpi e;
+  Epilogue e(EPI_RAW, ACT_NONE);
   if (x_fwd && prev_act != CGS_ACT_NONE) {
-    e.epi = EPI_BWD;
+    e = Epilogue(EPI_BWD, prev_act);
     e.aux = x_fwd;
-    e.act = prev_act;
   }
   return layer_pass_dense(*L, true, math, B, dy, dx, e, workspace, workspace_bytes, (cudaStream_t)stream);
 }
@@ -1416,8 +1296,7 @@ extern "C" int64_t cgs_pack_map(const cgs_layer_desc* L, int backward, int32_t* 
                                 int64_t capacity) {
   if (!L) return set_error(CGS_ERR_INVALID, "null layer");
   ConvGemmParams p;
-  int rc = backward ? make_backward_params(*L, 1, nullptr, nullptr, p) : make_forward_params(*L, 1, nullptr, nullptr, p);
-  if (rc) return rc;
+  if (int rc = make_pass_params(*L, backward != 0, 1, nullptr, nullptr, p)) return rc;
   int64_t total = 0;
   for (int c = 0; c < p.nclasses; ++c) total += (int64_t)p.cls[c].nkb * 32;
   if (!ky || !kx || !ch) return total;
@@ -1427,10 +1306,9 @@ extern "C" int64_t cgs_pack_map(const cgs_layer_desc* L, int backward, int32_t* 
     return total;
   }
   // recover (ky,kx) from (dy,dx): strided pass dy = ky - pad ; transposed pass dy = (py + pad - ky)/2
-  const bool strided = (p.S == 2);
-  const int size_for_pad = (L->type == CGS_LAYER_CONV) ? L->hin : L->hin * 2;
-  const int size_for_pad_x = (L->type == CGS_LAYER_CONV) ? L->win : L->win * 2;
-  const int pad_y = same_pad_before(size_for_pad, L->k), pad_x = same_pad_before(size_for_pad_x, L->k);
+  const PassShape sh = pass_shape(*L, backward != 0);
+  const bool strided = sh.strided;
+  const int pad_y = sh.pad_y, pad_x = sh.pad_x;
   for (int c = 0; c < p.nclasses; ++c) {
     const GemmClass& g = p.cls[c];
     const int cin_k = p.cblocks ? p.cblocks * 32 : 4;
@@ -1461,8 +1339,7 @@ extern "C" int64_t cgs_debug_fusion_plan(const cgs_layer_desc* L, int backward, 
   if (!L) return set_error(CGS_ERR_INVALID, "null layer");
   if (use_window(*L, backward != 0) || use_scatter(*L, backward != 0)) return 0;
   ConvGemmParams p;
-  int rc = backward ? make_backward_params(*L, B, nullptr, nullptr, p) : make_forward_params(*L, B, nullptr, nullptr, p);
-  if (rc) return rc;
+  if (int rc = make_pass_params(*L, backward != 0, B, nullptr, nullptr, p)) return rc;
   const int ns = plan_fusion(p);
   if (!ns) return 0;
   int nshf = 0;
@@ -1498,7 +1375,7 @@ extern "C" int64_t cgs_debug_gemm_params(const cgs_layer_desc* L, int backward, 
   ConvGemmParams p;
   int rc = use_window(*L, backward != 0) ? make_window_params(*L, backward != 0, B, nullptr, nullptr, p)
            : use_scatter(*L, backward != 0) ? make_scatter_gemm_params(*L, backward != 0, B, nullptr, nullptr, p)
-           : backward ? make_backward_params(*L, B, nullptr, nullptr, p) : make_forward_params(*L, B, nullptr, nullptr, p);
+           : make_pass_params(*L, backward != 0, B, nullptr, nullptr, p);
   if (rc) return rc;
   const int64_t need = 18 + (int64_t)p.nclasses * (5 + 2 * kMaxTaps);
   if (!out) return need;

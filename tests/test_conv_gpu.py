@@ -127,9 +127,25 @@ def test_cta_pairs_are_bit_identical(cgs_lib, cuda_device, arch_name, B, gain):
 @pytest.mark.parametrize("math", ["fp32", "tf32"])
 @pytest.mark.parametrize("arch_name,B", [("mnist", 5), ("mnist", 67), ("dcgan32_l1", 3), ("dcgan64_l2", 2), ("dcgan64_l2", 9)])
 def test_layers_forward_backward(cgs_lib, cuda_device, arch_name, B, math):
+    from cgs import nets as N
+    _layer_parity(cgs_lib, cuda_device, N.get_arch(arch_name), B, math)
+
+
+@pytest.mark.parametrize("win", [31, 63])
+def test_odd_width_image_layer(cgs_lib, cuda_device, win):
+    """An image-input conv whose width is odd has no space-to-depth form: cgs_layer_forward must not take the s2d
+    tcgen05 edge kernel for it (its output rows would be read W / 2 pixels wide) and still match the oracle."""
+    from cgs import nets as N
+    arch = N.get_arch("mnist")
+    arch["d"] = [dict(arch["d"][0], hin=32, win=win)] + arch["d"][1:]   # k = 4: pad 1, 16 x (win + 1) / 2 outputs
+    _layer_parity(cgs_lib, cuda_device, arch, 3, "tf32", names={"d_conv1"})
+
+
+def _layer_parity(cgs_lib, cuda_device, arch, B, math, names=None):
+    """cgs_layer_forward / cgs_layer_backward of every GEMM layer of `arch` (or of the layers in `names`) vs the
+    oracle."""
     from cgs import lib as L
     from cgs import nets as N
-    arch = N.get_arch(arch_name)
     w = onets.init_weights(arch, seed=11)
     spec = N.NetSpec(arch, w, cuda_device, math=math)
     rng = np.random.RandomState(1)
@@ -137,6 +153,8 @@ def test_layers_forward_backward(cgs_lib, cuda_device, arch_name, B, math):
             [("discriminator", l, spec.d.layer_desc(i)) for i, l in enumerate(arch["d"][:-1])]
     worst = {}
     for scope, layer, desc in chain:
+        if names is not None and layer["name"] not in names:
+            continue
         cin, cout = layer["cin"], layer["cout"]
         shp = (B, cin) if layer["type"] == "fc" else (B, layer["hin"], layer["win"], cin)
         x = rng.standard_normal(shp).astype(np.float32)
@@ -167,7 +185,7 @@ def test_layers_forward_backward(cgs_lib, cuda_device, arch_name, B, math):
         e = rel_l2(gotg[..., :cin], dx.numpy())
         worst[layer["name"] + ".bwd"] = e
         assert e <= TOL[math], (layer["name"], "bwd", e)
-    print(arch_name, math, {k: "%.2e" % v for k, v in worst.items()})
+    print(arch["name"], math, {k: "%.2e" % v for k, v in worst.items()})
 
 
 def _make(arch_name, seed, gain, cuda_device, math="fp32"):
