@@ -423,12 +423,12 @@ int launch_narrow_nt(const EdgeNarrowParams& p, cudaStream_t st) {
 
 }  // namespace
 
-bool edge_wide_supported(int N, int k, int cimg) {
-  return N == 64 && k >= 1 && k <= 5 && cimg >= 1 && cimg <= 4;
+bool edge_wide_supported(const EdgeWideParams& p) {
+  return p.N == 64 && p.ON == p.N && p.k >= 1 && p.k <= 5 && p.cimg >= 1 && p.cimg <= 4;
 }
 
-bool edge_narrow_supported(int K, int k, int cimg, int IW) {
-  return K == 64 && (k == 4 || k == 5) && (cimg == 1 || cimg == 3) && IW <= EN_ROWS / 4;
+bool edge_narrow_supported(const EdgeNarrowParams& p) {
+  return p.K == 64 && (p.k == 4 || p.k == 5) && (p.cimg == 1 || p.cimg == 3) && p.IW <= EN_ROWS / 4;
 }
 
 template <int MODE, bool ROUND>
@@ -541,13 +541,12 @@ int launch_pair_mode(const EdgeNarrowParams& pn, const EdgeWideParams& pw, int s
 }
 }  // namespace
 
-// One image per tile in both passes, single-channel image, same pitched layout on both sides; the shared-memory
-// footprint (column buffer + staged image + two weight tiles) must leave room for three CTAs per SM.
+// Of two passes edge_route gives a fused kernel: one image per tile in both, single-channel image, same pitched layout
+// on both sides; the shared-memory footprint (column buffer + staged image + two weights) leaves room for 3 CTAs / SM.
 bool edge_pair_supported(const EdgeNarrowParams& pn, const EdgeWideParams& pw) {
-  if (!edge_narrow_supported(pn.K, pn.k, pn.cimg, pn.IW) || !edge_wide_supported(pw.N, pw.k, pw.cimg)) return false;
   if (pn.cimg != 1 || pw.cimg != 1) return false;
   if (pn.IH * pn.IW > EN_ROWS || pw.OH * pw.OW > EW_TILE_PX) return false;
-  if (pn.OH != pw.IH || pn.out_pitch != pw.pitch || pn.out_xoff != pw.xoff || pw.ON != pw.N) return false;
+  if (pn.OH != pw.IH || pn.out_pitch != pw.pitch || pn.out_xoff != pw.xoff) return false;
   return true;
 }
 
@@ -562,9 +561,6 @@ int launch_edge_pair(EdgeNarrowParams pn, const EdgeWideParams& pw, int store_im
 
 int launch_edge_narrow(EdgeNarrowParams p, cudaStream_t st) {
   if (p.B <= 0) return CGS_OK;
-  // tcgen05 form with the input patch resident in shared memory (edge_tc.cu), else the column-buffer kernel
-  if (edge_narrow_tc_supported(p)) return launch_edge_narrow_tc(p, st);
-  if (p.s2d) return set_error(CGS_ERR_UNSUPPORTED, "s2d image layout needs the tcgen05 edge kernels");
   if (int rc = narrow_geometry(p)) return rc;
   if (p.k == 4 && p.cimg == 1) return launch_narrow_nt<2, 1>(p, st);
   if (p.k == 5 && p.cimg == 1) return launch_narrow_nt<4, 1>(p, st);

@@ -42,19 +42,17 @@ struct EdgeNarrowParams {
   const int* live;    // early exit: device-resident number of images still in the batch (null = all of them)
 };
 
-bool edge_wide_supported(int N, int k, int cimg);
-bool edge_narrow_supported(int K, int k, int cimg, int IW);
+bool edge_wide_supported(const EdgeWideParams& p);
+bool edge_narrow_supported(const EdgeNarrowParams& p);
 int launch_edge_wide(const EdgeWideParams& p, cudaStream_t st);
 int launch_edge_narrow(EdgeNarrowParams p, cudaStream_t st);
-// the row widths the tcgen05 edge kernels take (narrow pass input = wide pass output = s2d grid width)
-bool edge_tc_width_supported(int w);
 // the same pass on tcgen05 with the input patch resident in shared memory (edge_tc.cu)
 bool edge_narrow_tc_supported(const EdgeNarrowParams& p);
 int launch_edge_narrow_tc(const EdgeNarrowParams& p, cudaStream_t st);
 // the wide pass (image-like input -> 64 channels, stride-2 strided type) on tcgen05 over the SPACE-TO-DEPTH image
 // layout [B][H/2][W/2][16], channel (ry * 2 + rx) * 4 + c = image pixel (2j + ry, 2i + rx, c): the k x k stride-2 conv
 // becomes a 3 x 3 stride-1 conv over 16 channels, which the resident-patch / shifted-descriptor scheme covers
-bool edge_wide_tc_supported(const EdgeWideParams& p);
+bool edge_wide_tc_supported(const EdgeWideParams& p, int image_w);   // image_w: width of the image-like input
 int launch_edge_wide_tc(const EdgeWideParams& p, int B, cudaStream_t st);
 // dense [B][H][W][4] <-> space-to-depth [B][H/2][W/2][16]
 int image_to_s2d(const float* dense, float* s2d, long long B, int H, int W, cudaStream_t st);

@@ -153,7 +153,7 @@ edge_narrow_tc_kernel(const __grid_constant__ NarrowTcParams q, const __grid_con
     const bool bwd = p.ep.mode == EPI_BWD;
     const float4 bias4 = (p.ep.mode == EPI_FWD && p.ep.bias) ? __ldg(reinterpret_cast<const float4*>(p.ep.bias))
                                                             : make_float4(0.f, 0.f, 0.f, 0.f);
-    // the scalar epilogue without the policy step, which this pass never carries (edge_narrow_tc_supported)
+    // the scalar epilogue without the policy step, which no scatter-lowered pass carries (run_pass refuses it)
     auto epi = [&](float v, float x0) {
       float unused;
       return bwd ? epilogue1_t<EPI_BWD>(p.ep, v, x0, 0.f, &unused)
@@ -255,11 +255,11 @@ PFN_encodeTiledTc encode_fn() {
 
 }  // namespace
 
-bool edge_tc_width_supported(int w) { return w == 16 || w == 32 || w == 64; }
+static bool edge_tc_width_supported(int w) { return w == 16 || w == 32 || w == 64; }   // s2d grid row widths
 
 bool edge_narrow_tc_supported(const EdgeNarrowParams& p) {
   return p.K == 64 && p.pad_y == 1 && p.pad_x == 1 && edge_tc_width_supported(p.IW) && (p.k == 4 || p.k == 5) &&
-         p.OW == 2 * p.IW && p.OH == 2 * p.IH && p.ep.mode != EPI_UPDATE && p.cimg >= 1 && p.cimg <= 3;
+         p.OW == 2 * p.IW && p.OH == 2 * p.IH && p.cimg >= 1 && p.cimg <= 3;
 }
 
 int launch_edge_narrow_tc(const EdgeNarrowParams& p, cudaStream_t st) {
@@ -622,9 +622,9 @@ int debug_trace_tc(long long* out_host) {
   return cudaMemcpyFromSymbol(out_host, g_tc_trace, sizeof(long long) * 8 * 64) == cudaSuccess ? 8 * 64 : -1;
 }
 
-bool edge_wide_tc_supported(const EdgeWideParams& p) {
+bool edge_wide_tc_supported(const EdgeWideParams& p, int image_w) {
   return p.N == 64 && p.ON == 64 && (p.k == 4 || p.k == 5) && p.cimg >= 1 && p.cimg <= 3 && p.pad_y == 1 && p.pad_x == 1 &&
-         (p.IH % 2) == 0 && p.OH * 2 == p.IH && edge_tc_width_supported(p.OW);
+         p.OH * 2 == p.IH && p.OW * 2 == image_w && edge_tc_width_supported(p.OW);
 }
 
 // p.in must be the s2d form of the image-like input; p.pitch / p.xoff are ignored

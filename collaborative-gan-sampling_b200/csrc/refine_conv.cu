@@ -406,9 +406,6 @@ __global__ void __launch_bounds__(256) col2im_kernel(const Col2imParams p) {
   }
 }
 
-// CGS_DEBUG_EDGE_GENERAL: keep the image-edge passes on the general tcgen05 lowerings
-bool edge_kernels_enabled() { return !(debug_flags() & CGS_DEBUG_EDGE_GENERAL); }
-
 int launch_gemm(const ConvGemmParams& p, const float* w, int rows, int cols, int math, cudaStream_t stream) {
   if (math == CGS_MATH_FP32_SIMT) return launch_conv_gemm_simt(p, w, rows, cols, stream);
   if (math == CGS_MATH_TF32_TENSOR) return launch_conv_gemm_tc(p, w, rows, cols, stream);
@@ -448,14 +445,22 @@ int launch_splitk_reduce(const ConvGemmParams& pe, const float* part, int S, int
   return check_launch("splitk_reduce_kernel");
 }
 
-// Parameters of the fused image-edge kernels (edge_conv.cuh) for a scatter- / window-lowered pass; false when the
-// shape is not covered (the general tcgen05 lowering runs instead) or the kernels are switched off.
-bool make_edge_narrow(const cgs_layer_desc& L, bool backward, int64_t B, const float* in, float* out, const Epilogue& e,
-                      const int* live, int img_mode, EdgeNarrowParams& q) {
+// The packed weights of a pass are in the layout cgs_pass_layout gives it.
+int check_weights(const cgs_layer_desc& L, bool backward) {
   const PassShape sh = pass_shape(L, backward);
-  if (!edge_kernels_enabled() || !use_scatter(L, backward) || !edge_narrow_supported(sh.kch, L.k, sh.nch, sh.iw) ||
-      sh.cols != sh.kch)
-    return false;
+  if (!sh.w) return set_error(CGS_ERR_INVALID, "layer has no packed %s weights", backward ? "backward" : "forward");
+  if (use_scatter(L, backward) && (sh.rows != scatter_cols(L) || sh.cols != sh.kch))
+    return set_error(CGS_ERR_INVALID, "weights of this pass must be in scatter layout (%d x %d)", scatter_cols(L), sh.kch);
+  if (use_window(L, backward) && (sh.rows != sh.nch || sh.cols != window_kcols(L)))
+    return set_error(CGS_ERR_INVALID, "weights of this pass must be in window layout (%d columns)", window_kcols(L));
+  return CGS_OK;
+}
+
+// Parameters of the fused image-edge kernels (edge_conv.cuh) for a scatter- (narrow) / window-lowered (wide) pass.
+EdgeNarrowParams make_edge_narrow(const cgs_layer_desc& L, bool backward, int64_t B, const float* in, float* out,
+                                  const Epilogue& e, const int* live, int img_mode) {
+  const PassShape sh = pass_shape(L, backward);
+  EdgeNarrowParams q;
   std::memset(&q, 0, sizeof(q));
   q.in = in; q.out = out; q.w = sh.w;
   q.B = (int)B; q.K = sh.kch; q.k = L.k; q.cimg = sh.nch;
@@ -467,23 +472,44 @@ bool make_edge_narrow(const cgs_layer_desc& L, bool backward, int64_t B, const f
   q.ep = e;
   q.ep.bias = sh.bias;
   q.live = live;
-  return true;
+  return q;
 }
 
-bool make_edge_wide(const cgs_layer_desc& L, bool backward, int64_t B, const float* in, float* out, const Epilogue& e,
-                    const int* live, const ConvGemmParams& wp, EdgeWideParams& q) {   // wp = make_window_params of the same pass
+EdgeWideParams make_edge_wide(const cgs_layer_desc& L, bool backward, int64_t B, const float* in, float* out,
+                              const Epilogue& e, const int* live) {
   const PassShape sh = pass_shape(L, backward);
-  if (!edge_kernels_enabled() || !edge_wide_supported(wp.N, L.k, sh.kch) || wp.ON != wp.N) return false;
+  EdgeWideParams q;
   std::memset(&q, 0, sizeof(q));
   q.in = in; q.out = out; q.w = sh.w;
-  q.IH = wp.IH; q.pitch = wp.in_pitch_px; q.xoff = IMG_XOFF; q.OH = wp.OH; q.OW = wp.OW; q.ON = wp.ON; q.N = wp.N;
+  q.IH = sh.ih; q.pitch = img_pitch(sh.iw); q.xoff = IMG_XOFF; q.OH = sh.oh; q.OW = sh.ow; q.ON = cstride(sh.nch); q.N = sh.nch;
   q.k = L.k; q.cimg = sh.kch;
   q.pad_y = sh.pad_y; q.pad_x = sh.pad_x;
-  q.M = (long long)B * wp.OH * wp.OW;
+  q.M = (long long)B * sh.oh * sh.ow;
   q.ep = e;
   q.ep.bias = sh.bias;
   q.live = live;
-  return true;
+  return q;
+}
+
+// How an image-edge pass (scatter- or window-lowered: the generated image is its output or its input) runs.
+enum EdgeRoute : int {
+  ROUTE_GENERAL,   // scatter GEMM + col2im_kernel / window GEMM (no route for a wide pass over the s2d image)
+  ROUTE_MMA,       // mma.sync: edge_narrow (column buffer) / edge_wide over the pitched image (edge_conv.cu)
+  ROUTE_TC,        // tcgen05: edge_narrow_tc / edge_wide_tc, the wide pass over the s2d image (edge_tc.cu)
+};
+
+// The route of pass (L, backward) with epilogue e, its image-like tensor in layout img_mode, from the kernels' own
+// predicates; the only code that reads CGS_DEBUG_EDGE_GENERAL and the math mode for these passes.
+EdgeRoute edge_route(const cgs_layer_desc& L, bool backward, int math, const Epilogue& e, int img_mode) {
+  if (math != CGS_MATH_TF32_TENSOR || (debug_flags() & CGS_DEBUG_EDGE_GENERAL)) return ROUTE_GENERAL;
+  if (use_scatter(L, backward)) {
+    const EdgeNarrowParams q = make_edge_narrow(L, backward, 0, nullptr, nullptr, e, nullptr, img_mode);
+    return !edge_narrow_supported(q) ? ROUTE_GENERAL : edge_narrow_tc_supported(q) ? ROUTE_TC : ROUTE_MMA;
+  }
+  const EdgeWideParams q = make_edge_wide(L, backward, 0, nullptr, nullptr, e, nullptr);
+  if (!use_window(L, backward) || !edge_wide_supported(q)) return ROUTE_GENERAL;
+  if (img_mode != IMG_S2D) return ROUTE_MMA;
+  return edge_wide_tc_supported(q, pass_shape(L, backward).iw) ? ROUTE_TC : ROUTE_GENERAL;
 }
 
 // The narrow pass of layer `ln` followed by the wide pass of layer `lw` on its output (forward: G's last deconv + D's
@@ -492,40 +518,46 @@ bool make_edge_wide(const cgs_layer_desc& L, bool backward, int64_t B, const flo
 int try_edge_pair(const cgs_layer_desc& ln, const cgs_layer_desc& lw, bool backward, int64_t B, const float* in,
                   float* mid, float* out, const Epilogue& en, const Epilogue& ew, const int* live, int store_mid, int math,
                   cudaStream_t st) {
-  if (math != CGS_MATH_TF32_TENSOR || (debug_flags() & CGS_DEBUG_NO_EDGE_PAIR) || en.mode == EPI_UPDATE) return 0;
-  if (!use_scatter(ln, backward) || !use_window(lw, backward)) return 0;
-  EdgeNarrowParams qn;
-  if (!make_edge_narrow(ln, backward, B, in, mid, en, live, IMG_PITCHED, qn)) return 0;
-  ConvGemmParams wp;
-  if (make_window_params(lw, backward, B, mid, out, wp) != CGS_OK) return 0;
-  const PassShape shw = pass_shape(lw, backward);
-  if (shw.rows != shw.nch || shw.cols != window_kcols(lw)) return 0;
-  EdgeWideParams qw;
-  if (!make_edge_wide(lw, backward, B, mid, out, ew, live, wp, qw)) return 0;
+  if ((debug_flags() & CGS_DEBUG_NO_EDGE_PAIR) || edge_route(ln, backward, math, en, IMG_PITCHED) == ROUTE_GENERAL ||
+      edge_route(lw, backward, math, ew, IMG_PITCHED) == ROUTE_GENERAL)
+    return 0;
+  const EdgeNarrowParams qn = make_edge_narrow(ln, backward, B, in, mid, en, live, IMG_PITCHED);
+  const EdgeWideParams qw = make_edge_wide(lw, backward, B, mid, out, ew, live);
   if (!edge_pair_supported(qn, qw)) return 0;
+  if (int rc = check_weights(ln, backward)) return rc;
+  if (int rc = check_weights(lw, backward)) return rc;
   if (int rc = launch_edge_pair(qn, qw, store_mid, st)) return rc;
   return 1;
 }
 
-// One layer pass (forward or data-gradient) with its fused epilogue `e` (its bias is the layer's, set here); picks
-// the gather or the scatter lowering.
+// One layer pass (forward or data-gradient) with its fused epilogue `e` (its bias is the layer's, set here); an
+// image-edge pass on its route, any other on the gathered GEMM.
 int run_pass(const cgs_layer_desc& L, bool backward, int64_t B, const float* in, float* out, const Epilogue& e,
              const int* live, float* col, int math, cudaStream_t st, int img_mode = IMG_PITCHED, bool defer_reduce = false) {
+  if (int rc = check_weights(L, backward)) return rc;
   const PassShape sh = pass_shape(L, backward);
-  if (!sh.w) return set_error(CGS_ERR_INVALID, "layer has no packed %s weights", backward ? "backward" : "forward");
-  Epilogue ep = e;
-  ep.bias = sh.bias;
-  if (use_scatter(L, backward)) {
+  const bool scatter = use_scatter(L, backward), window = use_window(L, backward);
+  ConvGemmParams p;
+  if (scatter) {
     if (!col) return set_error(CGS_ERR_WORKSPACE, "scatter pass needs a column workspace");
     if (e.mode == EPI_UPDATE) return set_error(CGS_ERR_UNSUPPORTED, "the policy step is not fused into a scatter-lowered pass");
-    if (sh.rows != scatter_cols(L)) return set_error(CGS_ERR_INVALID, "weights of this pass must be in scatter layout (%d rows)", scatter_cols(L));
-    {
-      EdgeNarrowParams q;
-      if (math == CGS_MATH_TF32_TENSOR && e.mode != EPI_UPDATE && make_edge_narrow(L, backward, B, in, out, e, live, img_mode, q))
-        return launch_edge_narrow(q, st);
-      if (img_mode == IMG_S2D) return set_error(CGS_ERR_UNSUPPORTED, "s2d image layout needs the tcgen05 edge kernels");
-    }
-    ConvGemmParams p;
+  } else if (int rc = window ? make_window_params(L, backward, B, in, out, p) : make_pass_params(L, backward, B, in, out, p)) {
+    return rc;
+  }
+  const EdgeRoute r = edge_route(L, backward, math, e, img_mode);
+  if ((scatter || window) && img_mode == IMG_S2D && r != ROUTE_TC)
+    return set_error(CGS_ERR_UNSUPPORTED, "s2d image layout needs the tcgen05 edge kernels");
+  if (r != ROUTE_GENERAL && scatter) {
+    const EdgeNarrowParams q = make_edge_narrow(L, backward, B, in, out, e, live, img_mode);
+    return r == ROUTE_TC ? launch_edge_narrow_tc(q, st) : launch_edge_narrow(q, st);
+  }
+  if (r != ROUTE_GENERAL) {
+    const EdgeWideParams q = make_edge_wide(L, backward, B, in, out, e, live);
+    return r == ROUTE_TC ? launch_edge_wide_tc(q, (int)B, st) : launch_edge_wide(q, st);
+  }
+  Epilogue ep = e;
+  ep.bias = sh.bias;
+  if (scatter) {
     if (int rc = make_scatter_gemm_params(L, backward, B, in, col, p)) return rc;
     // (early exit: the 1-tap GEMM over pixels runs over the full batch -- its rows are pixels, not images; the
     //  col2im below stops at the live images)
@@ -547,11 +579,9 @@ int run_pass(const cgs_layer_desc& L, bool backward, int64_t B, const float* in,
     col2im_kernel<<<(int)blocks, 256, 0, st>>>(c); count_launch();
     return check_launch("col2im_kernel");
   }
-  ConvGemmParams p;
   if (const int S = fc_split(L, backward); use_fc_split(L, backward, B, math, col)) {
-    if (int rc = make_pass_params(L, false, B, in, col, p)) return rc;
     ConvGemmParams pe = p;                    // epilogue description of the real output
-    pe.out = out;
+    p.out = col;
     pe.ep = ep;
     pe.live = live;
     p.ep = Epilogue(EPI_RAW, ACT_NONE);
@@ -573,20 +603,6 @@ int run_pass(const cgs_layer_desc& L, bool backward, int64_t B, const float* in,
     if (int rc = launch_gemm(p, sh.w, sh.rows, sh.cols, math, st)) return rc;
     if (defer_reduce) return CGS_OK;          // the head kernel adds the partial sums itself (head_takes_partials)
     return launch_splitk_reduce(pe, col, S, B, st);
-  }
-  if (use_window(L, backward)) {
-    if (sh.rows != sh.nch || sh.cols != window_kcols(L))
-      return set_error(CGS_ERR_INVALID, "weights of this pass must be in window layout (%d columns)", window_kcols(L));
-    if (int rc = make_window_params(L, backward, B, in, out, p)) return rc;
-    EdgeWideParams q;
-    if (img_mode == IMG_S2D) {               // image-like input in s2d layout: tcgen05 resident-patch kernel
-      if (math == CGS_MATH_TF32_TENSOR && make_edge_wide(L, backward, B, in, out, e, live, p, q) && edge_wide_tc_supported(q))
-        return launch_edge_wide_tc(q, (int)B, st);
-      return set_error(CGS_ERR_UNSUPPORTED, "s2d image layout needs the tcgen05 edge kernels");
-    }
-    if (math == CGS_MATH_TF32_TENSOR && make_edge_wide(L, backward, B, in, out, e, live, p, q)) return launch_edge_wide(q, st);
-  } else if (int rc = make_pass_params(L, backward, B, in, out, p)) {
-    return rc;
   }
   p.ep = ep;
   p.live = live;
@@ -831,6 +847,7 @@ struct Chain {
   cgs_layer_desc head;
   size_t max_elems;
   size_t col_elems;              // per-sample elements of the scatter column buffer (0 if unused)
+  int img_mode;                  // layout of the image-like tensors: IMG_S2D or IMG_PITCHED (choose_image_layout)
 };
 
 static int build_chain(const cgs_net_desc* gtail, const cgs_net_desc* d, Chain& c) {
@@ -871,20 +888,34 @@ static int build_chain(const cgs_net_desc* gtail, const cgs_net_desc* d, Chain& 
   return CGS_OK;
 }
 
-// Image-like tensors of the chain live in the s2d layout when both image-edge layers run on the tcgen05 edge kernels
-// (edge_tc.cu): G's last deconv (64 -> <= 3 channels) and D's first conv (<= 3 -> 64 channels), on a row width those
-// kernels take.  CGS_DEBUG_EDGE_GENERAL keeps the pitched layout.
-static bool chain_s2d(const Chain& c, int math) {
-  if (math != CGS_MATH_TF32_TENSOR || !edge_kernels_enabled()) return false;
-  if (c.n_gtail < 1 || c.n_gtail >= c.n) return false;
-  const cgs_layer_desc& Ln = c.layers[c.n_gtail - 1];
-  const cgs_layer_desc& Lw = c.layers[c.n_gtail];
-  if (Ln.type != CGS_LAYER_DECONV || Lw.type != CGS_LAYER_CONV) return false;
-  if (Ln.cin != 64 || Ln.cout > 3 || Lw.cout != 64 || Lw.cin != Ln.cout) return false;
-  if ((Ln.k != 4 && Ln.k != 5) || (Lw.k != 4 && Lw.k != 5)) return false;
-  if (!edge_tc_width_supported(Ln.win) || Ln.hin != Ln.win || Lw.hin != 2 * Ln.hin || Lw.win != 2 * Ln.win) return false;
-  if (pass_shape(Lw, false).pad_y != 1 || pass_shape(Ln, false).pad_y != 1) return false;
-  return true;
+// Forward pass i.  TF32 path: activations that feed another MMA are rounded to TF32 (RN) where they are produced, so
+// the tensor core's operand truncation is exact; the image (returned to the caller) and the head input stay FP32.
+static Epilogue forward_epi(const Chain& c, int i, int math) {
+  Epilogue e(EPI_FWD, c.layers[i].act);
+  e.round_out = (math == CGS_MATH_TF32_TENSOR) && (i != c.n_gtail - 1) && (i != c.n - 1);
+  return e;
+}
+
+// Epilogue of data-gradient pass i: times the derivative of the activation that produced its input x, the policy
+// step `upd` or nothing (i = 0).
+static Epilogue backward_epi(const Chain& c, int i, int math, const Epilogue* upd, const float* x) {
+  if (i == 0) return upd ? *upd : Epilogue(EPI_RAW, ACT_NONE);
+  Epilogue e(EPI_BWD, c.layers[i - 1].act);
+  e.aux = x;
+  e.round_out = (math == CGS_MATH_TF32_TENSOR);
+  return e;
+}
+
+// The image-like tensors of the chain are in the s2d layout exactly when all four image-edge passes (G's last deconv
+// and D's first conv, forward and data-gradient, with the epilogues of a refinement step) take the tcgen05 route over
+// it; pitched otherwise.
+static void choose_image_layout(Chain& c, int math) {
+  Epilogue upd(EPI_UPDATE, ACT_NONE);
+  c.img_mode = IMG_S2D;
+  for (int i = c.n_gtail - 1; i <= c.n_gtail; ++i)
+    if (edge_route(c.layers[i], false, math, forward_epi(c, i, math), IMG_S2D) != ROUTE_TC ||
+        edge_route(c.layers[i], true, math, backward_epi(c, i, math, &upd, nullptr), IMG_S2D) != ROUTE_TC)
+      c.img_mode = IMG_PITCHED;
 }
 
 static inline size_t align256(size_t x) { return (x + 255) & ~size_t(255); }
@@ -937,16 +968,9 @@ static bool head_takes_partials(const Chain& c, const Workspace& w, int64_t B, i
 
 static int run_forward(const Chain& c, const Workspace& w, int64_t B, int math, cudaStream_t st,
                        const int* live = nullptr) {
-  const int img_mode = chain_s2d(c, math) ? IMG_S2D : IMG_PITCHED;
-  // TF32 path: activations that feed another MMA are rounded to TF32 (RN) where they are produced, so the tensor
-  // core's operand truncation is exact; the image (returned to the caller) and the head input stay FP32
-  auto epi = [&](int i) {
-    Epilogue e(EPI_FWD, c.layers[i].act);
-    e.round_out = (math == CGS_MATH_TF32_TENSOR) && (i != c.n_gtail - 1) && (i != c.n - 1);
-    return e;
-  };
+  auto epi = [&](int i) { return forward_epi(c, i, math); };
   for (int i = 0; i < c.n; ++i) {
-    if (i == c.n_gtail - 1 && i + 1 < c.n && img_mode == IMG_PITCHED) {
+    if (i == c.n_gtail - 1 && i + 1 < c.n && c.img_mode == IMG_PITCHED) {
       // generator's last deconv + discriminator's first conv on the same image: one kernel when the shapes allow
       const int rc = try_edge_pair(c.layers[i], c.layers[i + 1], false, B, w.act[i], w.act[i + 1], w.act[i + 2], epi(i),
                                    epi(i + 1), live, 1, math, st);
@@ -954,7 +978,7 @@ static int run_forward(const Chain& c, const Workspace& w, int64_t B, int math, 
       if (rc == 1) { ++i; continue; }
     }
     const bool defer = (i == c.n - 1) && head_takes_partials(c, w, B, math);
-    if (int rc = run_pass(c.layers[i], false, B, w.act[i], w.act[i + 1], epi(i), live, w.col, math, st, img_mode, defer))
+    if (int rc = run_pass(c.layers[i], false, B, w.act[i], w.act[i + 1], epi(i), live, w.col, math, st, c.img_mode, defer))
       return rc;
   }
   return CGS_OK;
@@ -964,19 +988,11 @@ static int run_forward(const Chain& c, const Workspace& w, int64_t B, int math, 
 // the last pass's epilogue; otherwise the raw gradient is written to grad_out.
 static int run_backward(const Chain& c, const Workspace& w, int64_t B, int math, const Epilogue* upd,
                         float* grad_out, cudaStream_t st, const int* live = nullptr) {
-  const int img_mode = chain_s2d(c, math) ? IMG_S2D : IMG_PITCHED;
-  // pass i: times the derivative of the activation that produced its input, the policy step or nothing (i = 0)
-  auto epi = [&](int i) {
-    if (i == 0) return upd ? *upd : Epilogue(EPI_RAW, ACT_NONE);
-    Epilogue e(EPI_BWD, c.layers[i - 1].act);
-    e.aux = w.act[i];
-    e.round_out = (math == CGS_MATH_TF32_TENSOR);
-    return e;
-  };
+  auto epi = [&](int i) { return backward_epi(c, i, math, upd, w.act[i]); };
   int cur = 0;
   for (int i = c.n - 1; i >= 0; --i) {
     float* dst = (i == 0) ? (upd ? w.act[0] : grad_out) : w.g[cur ^ 1];
-    if (i == c.n_gtail && i >= 1 && img_mode == IMG_PITCHED) {
+    if (i == c.n_gtail && i >= 1 && c.img_mode == IMG_PITCHED) {
       // data-gradients of D's first conv and G's last deconv: one kernel, the image gradient never leaves the SM
       float* dst2 = (i - 1 == 0) ? (upd ? w.act[0] : grad_out) : w.g[cur ^ 1];
       // the intermediate (image gradient) buffer is only described, never written: any valid pointer of that size
@@ -985,7 +1001,7 @@ static int run_backward(const Chain& c, const Workspace& w, int64_t B, int math,
       if (rc < 0) return rc;
       if (rc == 1) { --i; cur ^= 1; continue; }
     }
-    if (int rc = run_pass(c.layers[i], true, B, w.g[cur], dst, epi(i), live, w.col, math, st, img_mode)) return rc;
+    if (int rc = run_pass(c.layers[i], true, B, w.g[cur], dst, epi(i), live, w.col, math, st, c.img_mode)) return rc;
     cur ^= 1;
   }
   return CGS_OK;
@@ -1034,10 +1050,7 @@ static int head_launch(const Chain& c, const Workspace& w, int64_t B, HeadParams
     hp.img_pitch4 = (pitched ? img_pitch(si.wout) : si.wout) * c4;
     hp.img_xoff4 = pitched ? IMG_XOFF * c4 : 0;
     hp.img_elems = si.hout * si.wout * si.cs_out;
-    if (chain_s2d(c, math)) {
-      hp.img_s2d = 1;
-      hp.img_w4 = si.wout;                      // one float4 per pixel
-    }
+    hp.img_s2d = c.img_mode == IMG_S2D;
   }
   hp.feature = w.act[0];
   hp.feat_elems = (int)c.act_elems[0];
@@ -1063,6 +1076,7 @@ extern "C" int cgs_refine_conv(const cgs_net_desc* gtail, const cgs_net_desc* d,
     return set_error(CGS_ERR_UNSUPPORTED, "unknown mode %d", cfg->mode);
   Chain c;
   if (int rc = build_chain(gtail, d, c)) return rc;
+  choose_image_layout(c, cfg->math);
   // programmatic dependent launch for this call's kernels when the average pass is large (common.h launch_pdl):
   // forward + data-gradient FLOPs of one iteration over its 2 n + 1 launches
   double macs = 0.0;
@@ -1173,6 +1187,7 @@ extern "C" int cgs_forward_logits_and_grad(const cgs_net_desc* gtail, const cgs_
   if (B <= 0) return B == 0 ? CGS_OK : set_error(CGS_ERR_INVALID, "negative batch");
   Chain c;
   if (int rc = build_chain(gtail, d, c)) return rc;
+  choose_image_layout(c, math);
   Workspace w;
   carve(c, B, (void*)(((uintptr_t)workspace + 255) & ~uintptr_t(255)), w);
   if (!workspace || w.total + 256 > workspace_bytes) return set_error(CGS_ERR_WORKSPACE, "workspace too small");
@@ -1195,12 +1210,11 @@ extern "C" int cgs_forward_logits_and_grad(const cgs_net_desc* gtail, const cgs_
   if (img_out) {
     const cgs_layer_desc& Li = c.layers[c.n_gtail - 1];
     const LayerShape si = layer_shape(Li);
-    if (Li.cout <= 4 && chain_s2d(c, math)) {
-      if (int rc = s2d_to_image(w.act[c.n_gtail], img_out, B, si.hout, si.wout, st)) return rc;
-    } else if (Li.cout <= 4) {
-      if (int rc = unpad_image(w.act[c.n_gtail], img_out, B, si.hout, si.wout, st)) return rc;
-    } else {
+    if (Li.cout > 4) {
       cudaMemcpyAsync(img_out, w.act[c.n_gtail], (size_t)B * c.act_elems[c.n_gtail] * 4, cudaMemcpyDeviceToDevice, st);
+    } else if (int rc = c.img_mode == IMG_S2D ? s2d_to_image(w.act[c.n_gtail], img_out, B, si.hout, si.wout, st)
+                                              : unpad_image(w.act[c.n_gtail], img_out, B, si.hout, si.wout, st)) {
+      return rc;
     }
   }
   if (grad_out) {
@@ -1238,22 +1252,11 @@ static int layer_pass_dense(const cgs_layer_desc& L, bool backward, int math, in
   float* stage = base + ((ce * (size_t)B + 63) & ~size_t(63));
   int img_mode = IMG_DENSE;
   if (use_window(L, backward)) {
-    const PassShape sh = pass_shape(L, backward);
-    const int h = sh.ih, w = sh.iw;
     // the image-like input is re-laid out first (inside the chain it is produced in that layout: no copy there)
-    ConvGemmParams wp;
-    EdgeWideParams q;
-    const bool tc = math == CGS_MATH_TF32_TENSOR && edge_kernels_enabled() &&
-                    make_window_params(L, backward, B, in, out, wp) == CGS_OK &&
-                    make_edge_wide(L, backward, B, in, out, e, nullptr, wp, q) && edge_wide_tc_supported(q) &&
-                    w == 2 * q.OW;            // the s2d layout pairs image columns: an odd width has no s2d form
-    if (tc) {
-      if (int rc = image_to_s2d(in, stage, B, h, w, st)) return rc;
-      img_mode = IMG_S2D;
-    } else {
-      if (int rc = pad_image(in, stage, B, h, w, st)) return rc;
-      img_mode = IMG_PITCHED;                 // (the window passes read the pitched layout; their output is not image-like)
-    }
+    const PassShape sh = pass_shape(L, backward);
+    img_mode = edge_route(L, backward, math, e, IMG_S2D) == ROUTE_TC ? IMG_S2D : IMG_PITCHED;
+    if (int rc = img_mode == IMG_S2D ? image_to_s2d(in, stage, B, sh.ih, sh.iw, st) : pad_image(in, stage, B, sh.ih, sh.iw, st))
+      return rc;
     in = stage;
   }
   return run_pass(L, backward, B, in, out, e, nullptr, col, math, st, img_mode);
