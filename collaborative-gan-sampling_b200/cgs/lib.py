@@ -48,6 +48,7 @@ DEBUG_NO_CTA_PAIRS = 16777216
 DEBUG_FORCE_CTA_PAIRS = 33554432
 DEBUG_MLP2D_ONE_THREAD = 134217728
 DEBUG_PDL_OFF = 536870912
+DEBUG_TF32_OPERANDS = 1073741824
 
 
 class PolicyCfg(C.Structure):
@@ -69,7 +70,7 @@ class LayerDesc(C.Structure):
                 ("win", C.c_int), ("act", C.c_int),
                 ("w_fwd", C.c_void_p), ("rows_fwd", C.c_int), ("kcols_fwd", C.c_int),
                 ("w_bwd", C.c_void_p), ("rows_bwd", C.c_int), ("kcols_bwd", C.c_int),
-                ("bias", C.c_void_p)]
+                ("bias", C.c_void_p), ("w16_fwd", C.c_void_p), ("w16_bwd", C.c_void_p)]
 
 
 class NetDesc(C.Structure):

@@ -213,6 +213,9 @@ def pack_layer(layer, w, b):
     return w_fwd, w_bwd, bias
 
 
+FP16_MAX = 65504.0
+
+
 def round_tf32(t):
     """Round-to-nearest (ties away, like cvt.rna.tf32.f32) to a 10-bit mantissa, so that the tensor core's operand
     truncation is exact instead of a systematic shrink."""
@@ -248,6 +251,12 @@ class PackedNet:
                 wb = wb.to(self.device)
                 self.tensors.append(wb)
                 d.w_bwd, d.rows_bwd, d.kcols_bwd = wb.data_ptr(), wb.shape[0], wb.shape[1]
+                if math == "tf32" and max(float(wf.abs().max()), float(wb.abs().max())) <= FP16_MAX:
+                    # FP16 copies of the TF32-rounded matrices (the same values: same 10-bit mantissa, inside FP16's
+                    # range); whether a chain runs on them is the library's decision (choose_operand_type)
+                    wf16, wb16 = wf.half(), wb.half()
+                    self.tensors += [wf16, wb16]
+                    d.w16_fwd, d.w16_bwd = wf16.data_ptr(), wb16.data_ptr()
             self.desc.layers[i] = d
 
     def layer_desc(self, i):

@@ -1,4 +1,4 @@
-// tcgen05 / TMEM implicit-GEMM kernel (TF32 inputs, FP32 accumulate) + an FP32 SIMT twin used by the
+// tcgen05 / TMEM implicit-GEMM kernel (TF32 or FP16 inputs, FP32 accumulate) + an FP32 SIMT twin used by the
 // parity tests and as the exact-FP32 mode.  See conv_gemm.cuh for the contraction it computes.
 //
 // CTA = 15 warps, persistent over output tiles (128 rows x BN channels):
@@ -8,7 +8,8 @@
 //               group owns whole tiles, at BN = 256 the three groups split one tile's 16-column chunks.
 //               Gather mode (pixel layout, <= 4 channels): A producers, cp.async gather of 128 rows x 128 B per K
 //               block into SWIZZLE_128B smem
-//   warp  12    MMA issuer (one elected lane of a warp-uniform loop): 4 x tcgen05.mma.kind::tf32 (K=8) per K atom
+//   warp  12    MMA issuer (one elected lane of a warp-uniform loop): 4 x tcgen05.mma.kind::tf32 (K=8) or kind::f16
+//               (K=16) per K atom
 //   warp  13    TMA producer for the weight tile (one 3-D box {32, BN, KB} per stage, SWIZZLE_128B)
 //   warp  14    TMA producer for the A tile (one 4-D box per K atom with traversal strides, or the window map)
 // Pipelines: full/empty mbarriers per smem stage (3-8 stages, 1-2 K atoms each), tmem_full/tmem_empty per
@@ -58,9 +59,18 @@ constexpr int EPI_PITCH = 20;                // floats per staged row (16-byte a
 constexpr int kMaxEpiWarps = kEpiWarps + kProdWarps;              // producer warps help in TMA mode
 constexpr int EPI_STAGE_BYTES = kMaxEpiWarps * 32 * EPI_PITCH * 4;   // 30 KB
 
-template <int CG>
+constexpr int K_STEPS = 4;                   // MMAs per K atom: 32 bytes each (K = 8 TF32 or K = 16 FP16)
+
+template <int CG, bool F16>
 __device__ __forceinline__ void umma(uint32_t tmem_d, uint64_t da, uint64_t db, uint32_t idesc, uint32_t accumulate) {
-  if (CG == 2) umma_tf32_ss_cg2(tmem_d, da, db, idesc, accumulate); else umma_tf32_ss(tmem_d, da, db, idesc, accumulate);
+  if (F16) {
+    if (CG == 2) umma_f16_ss_cg2(tmem_d, da, db, idesc, accumulate); else umma_f16_ss(tmem_d, da, db, idesc, accumulate);
+  } else {
+    if (CG == 2) umma_tf32_ss_cg2(tmem_d, da, db, idesc, accumulate); else umma_tf32_ss(tmem_d, da, db, idesc, accumulate);
+  }
+}
+__host__ __device__ constexpr uint32_t make_idesc(bool f16, uint32_t M, uint32_t N) {
+  return f16 ? make_idesc_f16(M, N) : make_idesc_tf32(M, N);
 }
 template <int CG>
 __device__ __forceinline__ void commit(uint64_t* bar) {
@@ -100,11 +110,17 @@ struct Cfg {
   static constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + EPI_STAGE_BYTES + 1024 /*align*/ + 256 /*barriers*/;
 };
 
-template <int BN, int EPI, int NS, int MT, int CG>
-__global__ void __launch_bounds__(kThreads, 1)
-conv_gemm_tc_kernel(const __grid_constant__ ConvGemmParams p, const __grid_constant__ CUtensorMap tmap_w,
-                    const __grid_constant__ CUtensorMap tmap_a) {
+// F16: FP16 operands on kind::f16.  A 128-byte K atom holds 64 channels instead of 32, and one K = 16 MMA step covers
+// the same 32 bytes as a K = 8 TF32 step: stages, ring, TMEM plan and descriptor stepping are those of the TF32 form,
+// each stage simply carries twice the K.  The epilogue reads FP16 act' operands and stores FP16 where the output
+// feeds another MMA (Epilogue::out16); the policy step removes the head's per-sample gradient scale (Epilogue::gexp).
+// OPS: 0 = TF32 operands, FP32 outputs (the form every chain without FP16 operands runs); 1 = TF32 operands in an FP16
+// chain (layer 0's forward pass: its output may be FP16); 2 = FP16 operands
+template <int BN, int EPI, int NS, int MT, int CG, int OPS>
+__device__ __forceinline__ void conv_gemm_tc_body(const ConvGemmParams& p, const CUtensorMap& tmap_w, const CUtensorMap& tmap_a) {
   using C = Cfg<BN, NS, MT, CG>;
+  constexpr bool F16 = OPS == 2;
+  constexpr int AK = F16 ? 64 : BK;            // channels per K atom
   constexpr bool FUSED = NS > 1;
   constexpr bool PAIR = MT > 1;
   constexpr bool CG2 = CG == 2;
@@ -303,7 +319,7 @@ conv_gemm_tc_kernel(const __grid_constant__ ConvGemmParams p, const __grid_const
         const int ci = fast_div(tile, fd_tpc);
         const int rem = tile - ci * tiles_per_class;
         const int n_tile = rem - fast_div(rem, p.fd_n_tiles) * p.n_tiles;
-        const int katom0 = p.cls[ci].k0 / BK;
+        const int katom0 = p.cls[ci].k0 / AK;
         const int nkb = p.cls[ci].nkb;
         for (int kb = 0; kb < nkb; kb += C::KB, ++it_global) {
           const uint32_t s = stage, ph = phase;
@@ -352,10 +368,10 @@ conv_gemm_tc_kernel(const __grid_constant__ ConvGemmParams p, const __grid_const
                   if (leader) mbar_arrive(&full_bar[s]);
                 } else if (CG2) {
                   if (leader) mbar_arrive_expect_tx(&full_bar[s], 2u * a_bytes);
-                  tma_load_4d_cg2(smem_a_u32 + s * C::A_STAGE_BYTES, &tmap_a, &full_bar[s], cb * BK, sh.dx, y_tile + sh.dy, b0);
+                  tma_load_4d_cg2(smem_a_u32 + s * C::A_STAGE_BYTES, &tmap_a, &full_bar[s], cb * AK, sh.dx, y_tile + sh.dy, b0);
                 } else {
                   mbar_arrive_expect_tx(&full_bar[s], a_bytes);
-                  tma_load_4d(smem_a_u32 + s * C::A_STAGE_BYTES, &tmap_a, &full_bar[s], cb * BK, sh.dx, y_tile + sh.dy, b0);
+                  tma_load_4d(smem_a_u32 + s * C::A_STAGE_BYTES, &tmap_a, &full_bar[s], cb * AK, sh.dx, y_tile + sh.dy, b0);
                 }
               }
             }
@@ -380,14 +396,14 @@ conv_gemm_tc_kernel(const __grid_constant__ ConvGemmParams p, const __grid_const
                 if (leader) mbar_arrive(&full_bar[s]);
               } else if (CG2) {
                 if (leader) mbar_arrive_expect_tx(&full_bar[s], 4u * a_bytes);
-                tma_load_4d_cg2(smem_a_u32 + s * C::A_STAGE_BYTES, &tmap_a, &full_bar[s], (cb + cb0) * BK, gc.dx[t], yA + gc.dy[t], b0A);
-                tma_load_4d_cg2(smem_a_u32 + s * C::A_STAGE_BYTES + A_ATOM_BYTES, &tmap_a, &full_bar[s], (cb + cb0) * BK, gc.dx[t],
+                tma_load_4d_cg2(smem_a_u32 + s * C::A_STAGE_BYTES, &tmap_a, &full_bar[s], (cb + cb0) * AK, gc.dx[t], yA + gc.dy[t], b0A);
+                tma_load_4d_cg2(smem_a_u32 + s * C::A_STAGE_BYTES + A_ATOM_BYTES, &tmap_a, &full_bar[s], (cb + cb0) * AK, gc.dx[t],
                                 yB + gc.dy[t], b0B);
               } else {
                 mbar_arrive_expect_tx(&full_bar[s], second ? 2u * a_bytes : a_bytes);
-                tma_load_4d(smem_a_u32 + s * C::A_STAGE_BYTES, &tmap_a, &full_bar[s], (cb + cb0) * BK, gc.dx[t], yA + gc.dy[t], b0A);
+                tma_load_4d(smem_a_u32 + s * C::A_STAGE_BYTES, &tmap_a, &full_bar[s], (cb + cb0) * AK, gc.dx[t], yA + gc.dy[t], b0A);
                 if (second)
-                  tma_load_4d(smem_a_u32 + s * C::A_STAGE_BYTES + A_ATOM_BYTES, &tmap_a, &full_bar[s], (cb + cb0) * BK, gc.dx[t],
+                  tma_load_4d(smem_a_u32 + s * C::A_STAGE_BYTES + A_ATOM_BYTES, &tmap_a, &full_bar[s], (cb + cb0) * AK, gc.dx[t],
                               yB + gc.dy[t], b0B);
               }
               if (++cb == cblocks) { cb = 0; ++t; }
@@ -411,10 +427,10 @@ conv_gemm_tc_kernel(const __grid_constant__ ConvGemmParams p, const __grid_const
               if (!skip) {
                 if (CG2)
                   tma_load_4d_cg2(smem_a_u32 + s * C::A_STAGE_BYTES + a * A_ATOM_BYTES, &tmap_a, &full_bar[s],
-                                  (cb + cb0) * BK, gc.dx[t], y_tile + gc.dy[t], b0);
+                                  (cb + cb0) * AK, gc.dx[t], y_tile + gc.dy[t], b0);
                 else
                 tma_load_4d(smem_a_u32 + s * C::A_STAGE_BYTES + a * A_ATOM_BYTES, &tmap_a, &full_bar[s],
-                            (cb + cb0) * BK, gc.dx[t], y_tile + gc.dy[t], b0);
+                            (cb + cb0) * AK, gc.dx[t], y_tile + gc.dy[t], b0);
               }
               if (++cb == cblocks) {
                 cb = 0;
@@ -428,7 +444,7 @@ conv_gemm_tc_kernel(const __grid_constant__ ConvGemmParams p, const __grid_const
   } else if (warp == kMmaWarp) {
     // ------------------------------------------------------------------ MMA issuer
     // whole warp walks the loop (uniform control flow); one elected lane issues the tcgen05 instructions
-    constexpr uint32_t idesc = make_idesc_tf32(BM * CG, BN);
+    constexpr uint32_t idesc = make_idesc(F16, BM * CG, BN);
     const uint64_t da0 = make_smem_desc_sw128(smem_u32(smem_a));
     const uint64_t db0 = make_smem_desc_sw128(smem_u32(smem_b));
     // The loop body is kept minimal (ring position kept incrementally, parameters hoisted, no trace code unless
@@ -460,7 +476,7 @@ conv_gemm_tc_kernel(const __grid_constant__ ConvGemmParams p, const __grid_const
             const uint32_t slot = sh.run_slot[r];
             r_tm[r] = slot * BN;
             r_db[r] = slot * (C::B_ATOM_BYTES >> 4);
-            r_idesc[r] = make_idesc_tf32(BM * CG, BN * sh.run_len[r]);
+            r_idesc[r] = make_idesc(F16, BM * CG, BN * sh.run_len[r]);
             r_acc[r] = sh.run_acc[r];
           }
           for (int cb = 0; cb < p.cblocks; ++cb, ++it_global) {
@@ -480,8 +496,8 @@ conv_gemm_tc_kernel(const __grid_constant__ ConvGemmParams p, const __grid_const
                 // adjacent weight atoms in the stage, the A tile is read once for all of them
                 const uint32_t had = (cb > 0) ? 1u : r_acc[r];
 #pragma unroll
-                for (int k = 0; k < BK / 8; ++k)
-                  umma<CG>(tmem_d + r_tm[r], da + 2 * k, db + r_db[r] + 2 * k, r_idesc[r], (had || k > 0) ? 1u : 0u);
+                for (int k = 0; k < K_STEPS; ++k)
+                  umma<CG, F16>(tmem_d + r_tm[r], da + 2 * k, db + r_db[r] + 2 * k, r_idesc[r], (had || k > 0) ? 1u : 0u);
               }
             }
             commit<CG>(&empty_bar[s]);
@@ -510,13 +526,13 @@ conv_gemm_tc_kernel(const __grid_constant__ ConvGemmParams p, const __grid_const
           for (int a = 0; a < C::KB; ++a) {
             if (a >= na) break;
 #pragma unroll
-            for (int k = 0; k < BK / 8; ++k)
-              umma<CG>(tmem_d, da + a * (A_ATOM_BYTES >> 4) + 2 * k, db + a * (C::B_ATOM_BYTES >> 4) + 2 * k, idesc,
+            for (int k = 0; k < K_STEPS; ++k)
+              umma<CG, F16>(tmem_d, da + a * (A_ATOM_BYTES >> 4) + 2 * k, db + a * (C::B_ATOM_BYTES >> 4) + 2 * k, idesc,
                        (kb > 0 || a > 0 || k > 0) ? 1u : 0u);
             if (PAIR) {                        // second M tile of the pair: its own A atom, the SAME weight atom
 #pragma unroll
-              for (int k = 0; k < BK / 8; ++k)
-                umma<CG>(tmem_d + BN, da + (A_ATOM_BYTES >> 4) + 2 * k, db + 2 * k, idesc, (kb > 0 || k > 0) ? 1u : 0u);
+              for (int k = 0; k < K_STEPS; ++k)
+                umma<CG, F16>(tmem_d + BN, da + (A_ATOM_BYTES >> 4) + 2 * k, db + 2 * k, idesc, (kb > 0 || k > 0) ? 1u : 0u);
             }
           }
         }
@@ -604,7 +620,9 @@ conv_gemm_tc_kernel(const __grid_constant__ ConvGemmParams p, const __grid_const
         if (EPI == EPI_BWD) {
 #pragma unroll
           for (int ps = 0; ps < PASSES; ++ps)
-            if (ro[ps] >= 0) x0[ps] = __ldg(reinterpret_cast<const float4*>(p.ep.aux + ro[ps] + n));
+            if (ro[ps] >= 0)
+              x0[ps] = F16 ? unpack_half4(__ldg(reinterpret_cast<const uint2*>(reinterpret_cast<const __half*>(p.ep.aux) + ro[ps] + n)))
+                           : __ldg(reinterpret_cast<const float4*>(p.ep.aux + ro[ps] + n));
         } else if (EPI == EPI_UPDATE) {
 #pragma unroll
           for (int ps = 0; ps < PASSES; ++ps)
@@ -622,6 +640,14 @@ conv_gemm_tc_kernel(const __grid_constant__ ConvGemmParams p, const __grid_const
         if (warp == 0 && lane == 0) trace(p, 3, 0, tile_count);
         tcgen05_fence_after();
         waited = true;
+      }
+      // FP16 chains: the gradient of this lane's TMEM row (sample b) carries the head's scale 2^gexp[b]; it is removed
+      // (exactly) as the row is staged, before the policy step.  The factor waits in the staging row's padding column
+      // (EPI_PITCH > EPI_CH), not in a register held across the chunk loop.
+      if (F16 && (EPI == EPI_UPDATE || EPI == EPI_RAW)) {
+        const int r = quarter * 32 + lane, b = b0 + (multi_img ? r / rows_per_img_tile : 0);
+        stage[lane * EPI_PITCH + EPI_CH] =
+            (p.ep.gexp && tile_live && r < p.rows_valid && b < B_live) ? exp2_neg(__ldg(p.ep.gexp + b)) : 1.f;
       }
       const uint32_t taddr = tmem_base + acc * C::ACC_COLS + ((FUSED || PAIR) ? slot * BN : 0) + (static_cast<uint32_t>(quarter * 32) << 16);
       bool released = false;
@@ -652,11 +678,15 @@ conv_gemm_tc_kernel(const __grid_constant__ ConvGemmParams p, const __grid_const
           if (ch >= nch) break;
           if (dbg_skip_epi) continue;                          // warp-uniform
           // lane = row: stage 32 rows x 16 columns, then re-read with lane = (row group, 16-byte column)
+          const float gscale = (F16 && (EPI == EPI_UPDATE || EPI == EPI_RAW)) ? stage[lane * EPI_PITCH + EPI_CH] : 1.f;
 #pragma unroll
           for (int q4 = 0; q4 < Q; ++q4)
             *reinterpret_cast<float4*>(stage + lane * EPI_PITCH + q4 * 4) =
-                make_float4(__uint_as_float(v[u][4 * q4]), __uint_as_float(v[u][4 * q4 + 1]),
-                            __uint_as_float(v[u][4 * q4 + 2]), __uint_as_float(v[u][4 * q4 + 3]));
+                (F16 && (EPI == EPI_UPDATE || EPI == EPI_RAW))
+                    ? make_float4(__uint_as_float(v[u][4 * q4]) * gscale, __uint_as_float(v[u][4 * q4 + 1]) * gscale,
+                                  __uint_as_float(v[u][4 * q4 + 2]) * gscale, __uint_as_float(v[u][4 * q4 + 3]) * gscale)
+                    : make_float4(__uint_as_float(v[u][4 * q4]), __uint_as_float(v[u][4 * q4 + 1]),
+                                  __uint_as_float(v[u][4 * q4 + 2]), __uint_as_float(v[u][4 * q4 + 3]));
           __syncwarp();
           const int n = n0 + ch * EPI_CH + c4 * 4;
           const bool n_ok = n < p.ON;                // ON is a multiple of 4
@@ -672,7 +702,12 @@ conv_gemm_tc_kernel(const __grid_constant__ ConvGemmParams p, const __grid_const
           if (!dbg_no_prefetch) prefetch(ch + chunk_groups);   // operands of the next chunk: overlap with these stores
 #pragma unroll
           for (int ps = 0; ps < PASSES; ++ps)
-            if (ro[ps] >= 0 && n_ok && !dbg_skip_store) *reinterpret_cast<float4*>(p.out + ro[ps] + n) = o[ps];
+            if (ro[ps] >= 0 && n_ok && !dbg_skip_store) {
+              if (OPS > 0 && (EPI == EPI_FWD || EPI == EPI_BWD) && p.ep.out16)
+                *reinterpret_cast<uint2*>(reinterpret_cast<__half*>(p.out) + ro[ps] + n) = pack_half4(o[ps]);
+              else
+                *reinterpret_cast<float4*>(p.out + ro[ps] + n) = o[ps];
+            }
           if (warp == 0 && lane == 0) trace(p, 4, 2, tile_count * 8 + ch);
           __syncwarp();
           if (warp == 0 && lane == 0) trace(p, 4, 3, tile_count * 8 + ch);
@@ -688,6 +723,34 @@ conv_gemm_tc_kernel(const __grid_constant__ ConvGemmParams p, const __grid_const
   if (CG2) cluster_sync_all();                   // the leader's MMAs write this CTA's TMEM and barriers until its last commit
   if (warp == kMmaWarp) {
     if (CG2) tmem_dealloc_cg2(tmem_base, C::TMEM_COLS); else tmem_dealloc(tmem_base, C::TMEM_COLS);
+  }
+}
+
+// One kernel name per tile shape and epilogue mode, two overloads: the passes of an FP16-operand chain take the one
+// whose parameter is F16ChainParams, every other pass keeps the TF32-only code unchanged (a kernel that also held the
+// FP16 body measured 59.7 k instead of 62.6 k samples/s on the MNIST-sized chain, B200).  In an FP16 chain only the
+// forward pass of layer 0 runs TF32 operands (its input is the FP32 feature), and the policy step / raw gradient
+// ends a data-gradient chain of strided passes, never a class-fused one: chain_instance() lists the bodies compiled.
+struct F16ChainParams { ConvGemmParams p; };
+__host__ __device__ constexpr bool chain_instance(int epi, int ns, bool f16) {
+  return epi == EPI_FWD || (f16 && (epi == EPI_BWD || ns == 1));
+}
+
+template <int BN, int EPI, int NS, int MT, int CG>
+__global__ void __launch_bounds__(kThreads, 1)
+conv_gemm_tc_kernel(const __grid_constant__ ConvGemmParams p, const __grid_constant__ CUtensorMap tmap_w,
+                    const __grid_constant__ CUtensorMap tmap_a) {
+  conv_gemm_tc_body<BN, EPI, NS, MT, CG, 0>(p, tmap_w, tmap_a);
+}
+template <int BN, int EPI, int NS, int MT, int CG>
+__global__ void __launch_bounds__(kThreads, 1)
+conv_gemm_tc_kernel(const __grid_constant__ F16ChainParams q, const __grid_constant__ CUtensorMap tmap_w,
+                    const __grid_constant__ CUtensorMap tmap_a) {
+  if constexpr (EPI == EPI_FWD) {
+    if (q.p.f16) conv_gemm_tc_body<BN, EPI, NS, MT, CG, 2>(q.p, tmap_w, tmap_a);
+    else conv_gemm_tc_body<BN, EPI, NS, MT, CG, 1>(q.p, tmap_w, tmap_a);
+  } else if constexpr (chain_instance(EPI, NS, true)) {
+    conv_gemm_tc_body<BN, EPI, NS, MT, CG, 2>(q.p, tmap_w, tmap_a);
   }
 }
 
@@ -805,7 +868,8 @@ int pick_bn_for(const ConvGemmParams& p, int num_sms) {
 // Class-fusion tables of a transposed-type pass (see FuseShift): NS slots per tile; NS == 4 puts all four parity
 // classes into one group, NS == 2 makes one group per output-row parity (heavier group first).
 void build_fusion(ConvGemmParams& p, int NS) {
-  const int C = p.cblocks * BK;
+  const int ak = p.f16 ? 64 : BK;               // channels per K atom
+  const int C = p.cblocks * ak;
   p.fuse = NS;
   p.ngroups = 0;
   int nshf = 0;
@@ -854,7 +918,7 @@ void build_fusion(ConvGemmParams& p, int NS) {
         for (int t = 0; t < gc.ntaps; ++t)
           if (gc.dy[t] == sh.dy && gc.dx[t] == sh.dx) {
             sh.slot[sh.ncls] = (unsigned char)q;
-            sh.katom0[sh.ncls] = (gc.k0 + t * C) / BK;
+            sh.katom0[sh.ncls] = (gc.k0 + t * C) / ak;
             ++sh.ncls;
           }
       }
@@ -898,7 +962,7 @@ int fusion_slots(const ConvGemmParams& p, int bn) {
   if (debug_flags() & (CGS_DEBUG_NO_FUSION | CGS_DEBUG_GATHER_A)) return 0;
   if (p.nclasses != 4 || p.S != 1 || p.os != 2 || p.cblocks <= 0 || p.window || bn != p.N) return 0;
   for (int c = 0; c < 4; ++c) {
-    if (p.cls[c].cb0 != 0 || p.cls[c].k0 % BK) return 0;
+    if (p.cls[c].cb0 != 0 || p.cls[c].k0 % (p.f16 ? 64 : BK)) return 0;
     for (int t = 0; t < p.cls[c].ntaps; ++t)
       if (p.cls[c].dy[t] < -1 || p.cls[c].dy[t] > 1 || p.cls[c].dx[t] < -1 || p.cls[c].dx[t] > 1) return 0;
   }
@@ -942,19 +1006,22 @@ bool cluster_pair_fits(K kernel, size_t smem, int threads) {
   return st > 0;
 }
 
-template <int BN, int EPI, int NS = 1, int MT = 1, int CG = 1>
-int launch_tc_epi(ConvGemmParams p, const float* w, int w_rows, int w_cols, cudaStream_t stream) {
+template <int BN, int EPI, int NS = 1, int MT = 1, int CG = 1, bool F16 = false>
+int launch_tc_epi(ConvGemmParams p, const void* w, int w_rows, int w_cols, cudaStream_t stream) {
   using C = Cfg<BN, NS, MT, CG>;
+  constexpr int AK = F16 ? 64 : BK;                     // elements per 128-byte K atom
+  constexpr size_t ES = F16 ? 2 : 4;                    // bytes per element
+  const CUtensorMapDataType dtype = F16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
   const ConvGemmParams p_in = p;
   PFN_encodeTiled enc = get_encode_fn();
   if (!enc) return set_error(CGS_ERR_CUDA, "cuTensorMapEncodeTiled entry point not available");
   CUtensorMap tmap;
-  // weights [rows][K] viewed as {32 (k inside an atom), rows, K/32 (atom)}: a box {32, BN, KB} lands as KB atom tiles
-  cuuint64_t gdim[3] = {(cuuint64_t)BK, (cuuint64_t)w_rows, (cuuint64_t)(w_cols / BK)};
-  cuuint64_t gstride[2] = {(cuuint64_t)w_cols * sizeof(float), (cuuint64_t)BK * sizeof(float)};
-  cuuint32_t box[3] = {(cuuint32_t)BK, (cuuint32_t)(BN / CG), (cuuint32_t)C::KB};   // CTA pair: half an atom per box
+  // weights [rows][K] viewed as {AK (k inside an atom), rows, K/AK (atom)}: a box {AK, BN, KB} lands as KB atom tiles
+  cuuint64_t gdim[3] = {(cuuint64_t)AK, (cuuint64_t)w_rows, (cuuint64_t)(w_cols / AK)};
+  cuuint64_t gstride[2] = {(cuuint64_t)w_cols * ES, (cuuint64_t)AK * ES};
+  cuuint32_t box[3] = {(cuuint32_t)AK, (cuuint32_t)(BN / CG), (cuuint32_t)C::KB};   // CTA pair: half an atom per box
   cuuint32_t estr[3] = {1, 1, 1};
-  CUresult r = enc(&tmap, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(w), gdim, gstride, box, estr,
+  CUresult r = enc(&tmap, dtype, 3, const_cast<void*>(w), gdim, gstride, box, estr,
                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) return set_error(CGS_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d)", (int)r);
@@ -975,6 +1042,7 @@ int launch_tc_epi(ConvGemmParams p, const float* w, int w_rows, int w_cols, cuda
   p.rows_valid = p.BB * p.BH * p.MW;
   p.m_tiles = ((p.B + p.BB - 1) / p.BB) * p.hy_tiles;
   p.a_tma = (p.cblocks > 0) && !(p.debug & CGS_DEBUG_GATHER_A);
+  if (F16 && (!p.a_tma || p.window)) return set_error(CGS_ERR_UNSUPPORTED, "FP16 operands need the TMA'd A operand");
   CUtensorMap tmap_a;
   std::memset(&tmap_a, 0, sizeof(tmap_a));
   if (p.window) {
@@ -996,22 +1064,29 @@ int launch_tc_epi(ConvGemmParams p, const float* w, int w_rows, int w_cols, cuda
     // {32 ch, MW*S, BH*S, BB} lands as BB*BH*MW rows of 128 bytes; out-of-range coordinates read zeros
     if (p.MW * p.S > 256 || p.BH * p.S > 256) return set_error(CGS_ERR_UNSUPPORTED, "TMA box too large");
     cuuint64_t adim[4] = {(cuuint64_t)p.Cs, (cuuint64_t)p.IW, (cuuint64_t)p.IH, (cuuint64_t)p.B};
-    cuuint64_t astr[3] = {(cuuint64_t)p.Cs * 4, (cuuint64_t)p.IW * p.Cs * 4, (cuuint64_t)p.IH * p.IW * p.Cs * 4};
-    cuuint32_t abox[4] = {(cuuint32_t)BK, (cuuint32_t)(p.MW * p.S), (cuuint32_t)(p.BH * p.S), (cuuint32_t)p.BB};
+    cuuint64_t astr[3] = {(cuuint64_t)p.Cs * ES, (cuuint64_t)p.IW * p.Cs * ES, (cuuint64_t)p.IH * p.IW * p.Cs * ES};
+    cuuint32_t abox[4] = {(cuuint32_t)AK, (cuuint32_t)(p.MW * p.S), (cuuint32_t)(p.BH * p.S), (cuuint32_t)p.BB};
     cuuint32_t aest[4] = {1, (cuuint32_t)p.S, (cuuint32_t)p.S, 1};
-    CUresult ra = enc(&tmap_a, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<float*>(p.in), adim, astr, abox, aest,
+    CUresult ra = enc(&tmap_a, dtype, 4, const_cast<float*>(p.in), adim, astr, abox, aest,
                       CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                       CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (ra != CUDA_SUCCESS) return set_error(CGS_ERR_CUDA, "cuTensorMapEncodeTiled (A operand) failed (%d)", (int)ra);
   }
   const int num_sms = device_num_sms();
+  void (*const k_plain)(ConvGemmParams, CUtensorMap, CUtensorMap) = conv_gemm_tc_kernel<BN, EPI, NS, MT, CG>;
+  void (*const k_chain)(F16ChainParams, CUtensorMap, CUtensorMap) = conv_gemm_tc_kernel<BN, EPI, NS, MT, CG>;
+  const bool chain16 = p.f16 || p.ep.out16;    // a pass of an FP16-operand chain
+  if (chain16 && !chain_instance(EPI, NS, p.f16 != 0))
+    return set_error(CGS_ERR_UNSUPPORTED, "no FP16-chain form of this pass (epilogue %d, %d classes per tile)", EPI, NS);
   {
-    static DynSmemCache smem_cache;            // per kernel instantiation, per device
-    cudaError_t e = ensure_dyn_smem(conv_gemm_tc_kernel<BN, EPI, NS, MT, CG>, (size_t)C::SMEM_BYTES, smem_cache);
+    static DynSmemCache smem_cache[2];         // per kernel, per device
+    cudaError_t e = chain16 ? ensure_dyn_smem(k_chain, (size_t)C::SMEM_BYTES, smem_cache[1])
+                            : ensure_dyn_smem(k_plain, (size_t)C::SMEM_BYTES, smem_cache[0]);
     if (e != cudaSuccess) return set_error(CGS_ERR_CUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
   }
-  if (CG > 1 && !cluster_pair_fits(conv_gemm_tc_kernel<BN, EPI, NS, MT, CG>, (size_t)C::SMEM_BYTES, kThreads))
-    return launch_tc_epi<BN, EPI, NS, MT, 1>(p_in, w, w_rows, w_cols, stream);
+  if (CG > 1 && !(chain16 ? cluster_pair_fits(k_chain, (size_t)C::SMEM_BYTES, kThreads)
+                          : cluster_pair_fits(k_plain, (size_t)C::SMEM_BYTES, kThreads)))
+    return launch_tc_epi<BN, EPI, NS, MT, 1, F16>(p_in, w, w_rows, w_cols, stream);
   if (NS > 1) build_fusion(p, NS); else p.fuse = 0;
   p.m2 = MT * CG;                             // adjacent M tiles per scheduling unit
   const int m_units = (p.m_tiles + p.m2 - 1) / p.m2;
@@ -1023,21 +1098,23 @@ int launch_tc_epi(ConvGemmParams p, const float* w, int w_rows, int w_cols, cuda
   p.fd_hy_tiles = fast_div_magic((unsigned)p.hy_tiles);
   // CTA pairs: one cluster of two per unit, at most one CTA per SM (148 = 2 x 74 TPCs)
   const int grid = CG > 1 ? (2 * total < (num_sms & ~1) ? 2 * total : (num_sms & ~1)) : (total < num_sms ? total : num_sms);
-  cudaError_t e = launch_pdl_cluster(conv_gemm_tc_kernel<BN, EPI, NS, MT, CG>, dim3(grid), dim3(kThreads), (size_t)C::SMEM_BYTES,
-                                     stream, CG, p, tmap, tmap_a);
+  cudaError_t e = chain16 ? launch_pdl_cluster(k_chain, dim3(grid), dim3(kThreads), (size_t)C::SMEM_BYTES, stream, CG,
+                                                F16ChainParams{p}, tmap, tmap_a)
+                          : launch_pdl_cluster(k_plain, dim3(grid), dim3(kThreads), (size_t)C::SMEM_BYTES, stream, CG, p,
+                                                tmap, tmap_a);
   count_launch();
   if (e == cudaSuccess) e = cudaGetLastError();
   if (e != cudaSuccess) return set_error(CGS_ERR_CUDA, "conv_gemm_tc launch: %s", cudaGetErrorString(e));
   return CGS_OK;
 }
 
-template <int BN, int NS = 1, int MT = 1, int CG = 1>
-int launch_tc(const ConvGemmParams& p, const float* w, int w_rows, int w_cols, cudaStream_t stream) {
+template <bool F16, int BN, int NS = 1, int MT = 1, int CG = 1>
+int launch_tc(const ConvGemmParams& p, const void* w, int w_rows, int w_cols, cudaStream_t stream) {
   switch (p.ep.mode) {                      // the epilogue mode is compiled into the kernel
-    case EPI_FWD: return launch_tc_epi<BN, EPI_FWD, NS, MT, CG>(p, w, w_rows, w_cols, stream);
-    case EPI_BWD: return launch_tc_epi<BN, EPI_BWD, NS, MT, CG>(p, w, w_rows, w_cols, stream);
-    case EPI_UPDATE: return launch_tc_epi<BN, EPI_UPDATE, NS, MT, CG>(p, w, w_rows, w_cols, stream);
-    default: return launch_tc_epi<BN, EPI_RAW, NS, MT, CG>(p, w, w_rows, w_cols, stream);
+    case EPI_FWD: return launch_tc_epi<BN, EPI_FWD, NS, MT, CG, F16>(p, w, w_rows, w_cols, stream);
+    case EPI_BWD: return launch_tc_epi<BN, EPI_BWD, NS, MT, CG, F16>(p, w, w_rows, w_cols, stream);
+    case EPI_UPDATE: return launch_tc_epi<BN, EPI_UPDATE, NS, MT, CG, F16>(p, w, w_rows, w_cols, stream);
+    default: return launch_tc_epi<BN, EPI_RAW, NS, MT, CG, F16>(p, w, w_rows, w_cols, stream);
   }
 }
 
@@ -1052,6 +1129,7 @@ bool use_cta_pairs(const ConvGemmParams& p, long long units_total, int num_sms) 
 }
 
 int validate(const ConvGemmParams& p, int w_cols) {
+  const int ak = p.f16 ? 64 : BK;
   if (p.ON % 4 != 0) return set_error(CGS_ERR_INVALID, "output channel stride %d must be a multiple of 4", p.ON);
   if (p.cblocks == 0 && p.Cs != 4) return set_error(CGS_ERR_INVALID, "pixel mode needs channel stride 4");
   if (p.window && (p.cblocks != 1 || p.in_pitch_px <= 0)) return set_error(CGS_ERR_INVALID, "bad window-mode parameters");
@@ -1059,7 +1137,7 @@ int validate(const ConvGemmParams& p, int w_cols) {
   if (w_cols % 32 != 0) return set_error(CGS_ERR_INVALID, "weight row length must be a multiple of 32 floats");
   for (int c = 0; c < p.nclasses; ++c) {
     if (p.cls[c].ntaps > kMaxTaps) return set_error(CGS_ERR_INVALID, "too many taps");
-    if (p.cls[c].k0 + p.cls[c].nkb * BK > w_cols) return set_error(CGS_ERR_INVALID, "class K range exceeds weight matrix");
+    if (p.cls[c].k0 + p.cls[c].nkb * ak > w_cols) return set_error(CGS_ERR_INVALID, "class K range exceeds weight matrix");
   }
   return CGS_OK;
 }
@@ -1081,7 +1159,8 @@ int debug_trace_read(unsigned long long* out, int cap) {
   return n;
 }
 
-int launch_conv_gemm_tc(const ConvGemmParams& p, const float* w, int w_rows, int w_cols, cudaStream_t stream) {
+template <bool F16>
+int launch_conv_gemm_tc_t(const ConvGemmParams& p, const void* w, int w_rows, int w_cols, cudaStream_t stream) {
   if (int rc = validate(p, w_cols)) return rc;
   if (p.M <= 0) return CGS_OK;
   const int num_sms = device_num_sms();
@@ -1099,9 +1178,9 @@ int launch_conv_gemm_tc(const ConvGemmParams& p, const float* w, int w_rows, int
     if (ns && ((debug_flags() & CGS_DEBUG_FORCE_FUSION) || count_m_tiles(p) * (ns == 2 ? 2 : 1) >= num_sms)) {
       const bool pairs = use_cta_pairs(p, (long long)((count_m_tiles(p) + 1) / 2) * (ns == 2 ? 2 : 1), num_sms);
       switch (ns * 1000 + bn_full) {
-        case 4032: return launch_tc<32, 4>(p, w, w_rows, w_cols, stream);
-        case 4064: return pairs ? launch_tc<64, 4, 1, 2>(p, w, w_rows, w_cols, stream) : launch_tc<64, 4>(p, w, w_rows, w_cols, stream);
-        case 2128: return pairs ? launch_tc<128, 2, 1, 2>(p, w, w_rows, w_cols, stream) : launch_tc<128, 2>(p, w, w_rows, w_cols, stream);
+        case 4032: return launch_tc<F16, 32, 4>(p, w, w_rows, w_cols, stream);
+        case 4064: return pairs ? launch_tc<F16, 64, 4, 1, 2>(p, w, w_rows, w_cols, stream) : launch_tc<F16, 64, 4>(p, w, w_rows, w_cols, stream);
+        case 2128: return pairs ? launch_tc<F16, 128, 2, 1, 2>(p, w, w_rows, w_cols, stream) : launch_tc<F16, 128, 2>(p, w, w_rows, w_cols, stream);
         default: break;
       }
     }
@@ -1124,21 +1203,25 @@ int launch_conv_gemm_tc(const ConvGemmParams& p, const float* w, int w_rows, int
       // M-tile pairs inside CTA pairs: 40 KB instead of 48 KB of L2 -> SM traffic per 512 tensor cycles (BN = 128) on
       // passes that sit at the L2 throughput ceiling
       if (use_cta_pairs(p, quads, num_sms))
-        return bn == 64 ? launch_tc<64, 1, 2, 2>(p, w, w_rows, w_cols, stream) : launch_tc<128, 1, 2, 2>(p, w, w_rows, w_cols, stream);
+        return bn == 64 ? launch_tc<F16, 64, 1, 2, 2>(p, w, w_rows, w_cols, stream) : launch_tc<F16, 128, 1, 2, 2>(p, w, w_rows, w_cols, stream);
       if (bn == 128 || forced)
-        return bn == 64 ? launch_tc<64, 1, 2>(p, w, w_rows, w_cols, stream) : launch_tc<128, 1, 2>(p, w, w_rows, w_cols, stream);
+        return bn == 64 ? launch_tc<F16, 64, 1, 2>(p, w, w_rows, w_cols, stream) : launch_tc<F16, 128, 1, 2>(p, w, w_rows, w_cols, stream);
     }
   }
   switch (bn) {
-    case 16: return launch_tc<16>(p, w, w_rows, w_cols, stream);
-    case 32: return launch_tc<32>(p, w, w_rows, w_cols, stream);
-    case 64: return launch_tc<64>(p, w, w_rows, w_cols, stream);
-    case 128: return launch_tc<128>(p, w, w_rows, w_cols, stream);
+    case 16: return launch_tc<F16, 16>(p, w, w_rows, w_cols, stream);
+    case 32: return launch_tc<F16, 32>(p, w, w_rows, w_cols, stream);
+    case 64: return launch_tc<F16, 64>(p, w, w_rows, w_cols, stream);
+    case 128: return launch_tc<F16, 128>(p, w, w_rows, w_cols, stream);
     default:
       if (use_cta_pairs(p, (long long)((count_m_tiles(p) + 1) / 2) * ((p.N + 255) / 256) * p.nclasses, num_sms))
-        return launch_tc<256, 1, 1, 2>(p, w, w_rows, w_cols, stream);
-      return launch_tc<256>(p, w, w_rows, w_cols, stream);
+        return launch_tc<F16, 256, 1, 1, 2>(p, w, w_rows, w_cols, stream);
+      return launch_tc<F16, 256>(p, w, w_rows, w_cols, stream);
   }
+}
+
+int launch_conv_gemm_tc(const ConvGemmParams& p, const void* w, int w_rows, int w_cols, cudaStream_t stream) {
+  return p.f16 ? launch_conv_gemm_tc_t<true>(p, w, w_rows, w_cols, stream) : launch_conv_gemm_tc_t<false>(p, w, w_rows, w_cols, stream);
 }
 
 int launch_conv_gemm_simt(const ConvGemmParams& p, const float* w, int w_rows, int w_cols, cudaStream_t stream) {

@@ -12,6 +12,7 @@
 // for the 1-/3-channel image layers.
 #pragma once
 #include <cstdint>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 
 namespace cgs {
@@ -75,6 +76,9 @@ struct Epilogue {
   int act_tanh;       // the activation is tanh (slow path)
   int round_out;      // round results to TF32 (RN) because the next consumer is a kind::tf32 MMA
   int mode;           // EPI_*
+  // FP16 operand chains (choose_operand_type in refine_conv.cu):
+  int out16;          // FWD / BWD: the output is stored as FP16 (it feeds a kind::f16 MMA); aux is FP16 there too
+  const int* gexp;    // UPDATE / RAW: the accumulator is d loss / d x times 2^gexp[b] (head_kernel), null = unscaled
 
   Epilogue() = default;
   // host: mode `mode_` (EPI_*) through activation `act` (ACT_*), no operands -- the only place an activation becomes
@@ -82,7 +86,8 @@ struct Epilogue {
   Epilogue(int mode_, int act) : bias(nullptr), aux(nullptr), mom(nullptr), first(0), clip(0), sgd(0), rate(0.f),
                                  alpha(0.f), vmin(0.f), vmax(0.f),
                                  slope(act == ACT_RELU ? 0.f : (act == ACT_LRELU ? 0.2f : 1.f)),
-                                 act_tanh(act == ACT_TANH), round_out(0), mode(mode_) {}
+                                 act_tanh(act == ACT_TANH), round_out(0), mode(mode_),
+                                 out16(0), gexp(nullptr) {}
 };
 
 struct ConvGemmParams {
@@ -119,6 +124,7 @@ struct ConvGemmParams {
   FuseGroup grp[2];
   FuseShift shf[kMaxShifts];
   int debug;          // debug_flags() at launch: the profiling knobs of cgs_debug_flag (CGS_DEBUG_SKIP_*, _TRACE)
+  int f16;            // FP16 operands on kind::f16: cblocks / nkb / cb0 count 64-channel atoms (host: to_f16_atoms)
   // exact division of the persistent tile index by multiply-shift (filled by the launcher; see fast_div)
   unsigned long long fd_tiles_per_class, fd_n_tiles, fd_hy_tiles;
   GemmClass cls[kMaxClasses];
@@ -160,6 +166,21 @@ __device__ __forceinline__ float tf32_rn(float x) {
   asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
   return __uint_as_float(r);
 }
+
+// FP16 operands: four values -> four halves (RN, saturating to +-65504 instead of overflowing to inf), and back
+__device__ __forceinline__ uint2 pack_half4(float4 v) {
+  uint32_t lo, hi;
+  asm("cvt.rn.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(lo) : "f"(v.y), "f"(v.x));
+  asm("cvt.rn.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(hi) : "f"(v.w), "f"(v.z));
+  return make_uint2(lo, hi);
+}
+__device__ __forceinline__ float4 unpack_half4(uint2 u) {
+  const float2 a = __half22float2(*reinterpret_cast<const __half2*>(&u.x));
+  const float2 b = __half22float2(*reinterpret_cast<const __half2*>(&u.y));
+  return make_float4(a.x, a.y, b.x, b.y);
+}
+// 2^-e exactly (0 <= e < 127): removes the per-sample gradient scale of head_kernel
+__device__ __forceinline__ float exp2_neg(int e) { return __int_as_float((127 - e) << 23); }
 
 // ---------------------------------------------------------------------------------------------
 // The epilogue formulas, once: a vector form (four consecutive output channels) and a scalar form (one channel) with
@@ -269,7 +290,8 @@ __device__ __forceinline__ void epilogue_operands4(const Epilogue& e, const floa
 }
 
 // host launchers (conv_gemm.cu)
-int launch_conv_gemm_tc(const ConvGemmParams& p, const float* w, int w_rows, int w_cols, cudaStream_t stream);
+// p.f16: FP16 operands (p.in, w and the FP16 outputs of the epilogue are __half; K counted in 64-channel atoms)
+int launch_conv_gemm_tc(const ConvGemmParams& p, const void* w, int w_rows, int w_cols, cudaStream_t stream);
 int launch_conv_gemm_simt(const ConvGemmParams& p, const float* w, int w_rows, int w_cols, cudaStream_t stream);
 // host only: fills p.grp / p.shf the way the class-fused launch would and returns the slots per tile (0 = this pass
 // is never class-fused).  No device state is touched (cgs_debug_fusion_plan).

@@ -364,7 +364,7 @@ struct WideTcParams {
   int B, H2, W2, k, cimg, pad;
   int R, bands, MT, PW, PR, stage_bytes, nstages, ntiles;
   const int* live;
-  float* out;              // [B][H2][W2][64]
+  float* out;              // [B][H2][W2][64], FP16 when ep.out16 (it feeds a kind::f16 MMA)
   Epilogue ep;
   int debug;               // debug_flags() at launch: CGS_DEBUG_SKIP_*, _NO_PREFETCH, _TRACE
 };
@@ -532,6 +532,8 @@ edge_wide_tc_kernel(const __grid_constant__ WideTcParams q, const __grid_constan
           if (warp == 2 && lane == 0) tc_trace(q.debug, 5, tile_count);
         }
         const uint32_t taddr = tmem_base + (acc * TC_MAX_MT + mt) * 64 + (static_cast<uint32_t>(quarter * 32) << 16);
+        // policy step / raw gradient of an FP16 operand chain: remove the head's scale 2^gexp[b] of this image
+        const float gscale = ((EPI == EPI_UPDATE || EPI == EPI_RAW) && q.ep.gexp) ? exp2_neg(__ldg(q.ep.gexp + b)) : 1.f;
 #pragma unroll
         for (int cp = 0; cp < 2; ++cp) {                        // two 16-channel chunks per round
           uint32_t a[2][16];
@@ -557,7 +559,8 @@ edge_wide_tc_kernel(const __grid_constant__ WideTcParams q, const __grid_constan
             const int n = ch * 16 + c4 * 4;
 #pragma unroll
             for (int ps = 0; ps < 4; ++ps) {
-              const float4 v = lds_f4(stg + ((u * 32 + ps * 8 + rsub) * WT_PITCH + c4 * 4) * 4);
+              float4 v = lds_f4(stg + ((u * 32 + ps * 8 + rsub) * WT_PITCH + c4 * 4) * 4);
+              if (EPI == EPI_UPDATE || EPI == EPI_RAW) { v.x *= gscale; v.y *= gscale; v.z *= gscale; v.w *= gscale; }
               if (ro[ps] >= 0) {
                 float4 xa = EPI == EPI_FWD ? x0[ch][0] : x0[ch][ps], xb = make_float4(0.f, 0.f, 0.f, 0.f);
                 if (EPI == EPI_UPDATE) {         // policy step (only when the G tail is this single layer): not prefetched
@@ -565,7 +568,11 @@ edge_wide_tc_kernel(const __grid_constant__ WideTcParams q, const __grid_constan
                   if (!q.ep.sgd && !q.ep.first) xb = *reinterpret_cast<const float4*>(q.ep.mom + ro[ps] + n);
                 }
                 const float4 o = epilogue4_t<EPI>(q.ep, ro[ps] + n, v, xa, xb);
-                if (!(q.debug & CGS_DEBUG_SKIP_STORES)) *reinterpret_cast<float4*>(q.out + ro[ps] + n) = o;
+                if (q.debug & CGS_DEBUG_SKIP_STORES) continue;
+                if ((EPI == EPI_FWD || EPI == EPI_BWD) && q.ep.out16)
+                  *reinterpret_cast<uint2*>(reinterpret_cast<__half*>(q.out) + ro[ps] + n) = pack_half4(o);
+                else
+                  *reinterpret_cast<float4*>(q.out + ro[ps] + n) = o;
               }
             }
           }

@@ -156,6 +156,19 @@ __device__ __forceinline__ void umma_tf32_ss(uint32_t tmem_d, uint64_t desc_a, u
       "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
       : "memory");
 }
+// D[tmem] (+)= A[smem] * B[smem], FP16 inputs, FP32 accumulate, single-CTA (K = 16 per instruction: 32 bytes of a
+// 128-byte K-major row, the same step as one K = 8 kind::tf32 instruction).
+__device__ __forceinline__ void umma_f16_ss(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
+                                            uint32_t accumulate) {
+  asm volatile(
+      "{\n\t"
+      ".reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t"
+      "}\n" ::"r"(tmem_d),
+      "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
 // Arrive on an mbarrier once all previously issued tcgen05.mma of this thread have completed.
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
@@ -219,6 +232,17 @@ __device__ __forceinline__ void umma_tf32_ss_cg2(uint32_t tmem_d, uint64_t desc_
       "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
       : "memory");
 }
+__device__ __forceinline__ void umma_f16_ss_cg2(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
+                                                uint32_t accumulate) {
+  asm volatile(
+      "{\n\t"
+      ".reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t"
+      "}\n" ::"r"(tmem_d),
+      "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
 // Arrive on the barrier at this offset in BOTH CTAs once all previously issued MMAs have completed.
 __device__ __forceinline__ void umma_commit_cg2(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
@@ -258,6 +282,10 @@ __device__ __forceinline__ uint64_t make_smem_desc_sw128(uint32_t smem_addr) {
 // Instruction descriptor for kind::tf32, FP32 accumulate, both operands K-major (cute::UMMA::InstrDescriptor).
 __host__ __device__ constexpr uint32_t make_idesc_tf32(uint32_t M, uint32_t N) {
   return (1u << 4) | (2u << 7) | (2u << 10) | ((N >> 3) << 17) | ((M >> 4) << 24);
+}
+// Instruction descriptor for kind::f16 with FP16 A and B (format 0), FP32 accumulate, both operands K-major.
+__host__ __device__ constexpr uint32_t make_idesc_f16(uint32_t M, uint32_t N) {
+  return (1u << 4) | ((N >> 3) << 17) | ((M >> 4) << 24);
 }
 
 }  // namespace cgs

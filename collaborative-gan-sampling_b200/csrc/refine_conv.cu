@@ -532,8 +532,10 @@ int try_edge_pair(const cgs_layer_desc& ln, const cgs_layer_desc& lw, bool backw
 
 // One layer pass (forward or data-gradient) with its fused epilogue `e` (its bias is the layer's, set here); an
 // image-edge pass on its route, any other on the gathered GEMM.
+// w16: FP16 copy of the pass's packed weights -- the pass runs on kind::f16 over FP16 operands (choose_operand_type)
 int run_pass(const cgs_layer_desc& L, bool backward, int64_t B, const float* in, float* out, const Epilogue& e,
-             const int* live, float* col, int math, cudaStream_t st, int img_mode = IMG_PITCHED, bool defer_reduce = false) {
+             const int* live, float* col, int math, cudaStream_t st, int img_mode = IMG_PITCHED, bool defer_reduce = false,
+             const __half* w16 = nullptr) {
   if (int rc = check_weights(L, backward)) return rc;
   const PassShape sh = pass_shape(L, backward);
   const bool scatter = use_scatter(L, backward), window = use_window(L, backward);
@@ -606,6 +608,13 @@ int run_pass(const cgs_layer_desc& L, bool backward, int64_t B, const float* in,
   }
   p.ep = ep;
   p.live = live;
+  if (w16) {
+    if (math != CGS_MATH_TF32_TENSOR || p.cblocks % 2) return set_error(CGS_ERR_UNSUPPORTED, "FP16 operands need 64-channel blocks");
+    p.f16 = 1;                                // K counted in 64-channel atoms
+    p.cblocks /= 2;
+    for (int c = 0; c < p.nclasses; ++c) { p.cls[c].nkb /= 2; p.cls[c].cb0 /= 2; }
+    return launch_conv_gemm_tc(p, w16, sh.rows, sh.cols, st);
+  }
   return launch_gemm(p, sh.w, sh.rows, sh.cols, math, st);
 }
 
@@ -642,6 +651,8 @@ struct HeadParams {
   float* final_feature; // [B_orig, feat_elems]: state of a sample at the step it exits (early-exit) or nullptr
   float exit_logit;
   int round_out;        // round dpre to TF32 (RN): it feeds a kind::tf32 MMA
+  int dpre16;           // dpre is FP16, scaled per sample by 2^gexp[b] (it feeds a kind::f16 MMA)
+  int* gexp;            // [B] that exponent: |dl| * 2^gexp in [1, 2), 0 where dl == 0
   // split-K producer (fc_split): feat is not materialised; feat[b][k] = act(sum_s part[b][s][k] + bias[k])
   const float* part;    // [B][S][K] partial sums or nullptr
   int S;
@@ -723,12 +734,25 @@ __global__ void __launch_bounds__(256) head_kernel(const HeadParams p) {
   const float logit = s_logit;
   if (p.dpre) {
     // d softplus(-l)/dl = sigmoid(l) - 1
-    const float dl = 1.f / (1.f + expf(-logit)) - 1.f;
+    float dl = 1.f / (1.f + expf(-logit)) - 1.f;
+    if (p.dpre16) {
+      // The data-gradient chain is linear and homogeneous in dl per sample (masks and tanh' from the forward pass, no
+      // bias), so a power of two set here and removed by the policy step changes no FP32 value.  dl is 0 or at least
+      // 2^-24 in magnitude; scaled to [1, 2) it keeps the whole chain inside FP16's normal range (DESIGN §2).
+      int e = 0;
+      if (dl != 0.f) { (void)frexpf(dl, &e); e = 1 - e; }
+      dl = ldexpf(dl, e);
+      if (threadIdx.x == 0) p.gexp[b] = e;
+    }
     float* d = p.dpre + (size_t)b * p.K;
     for (int k = threadIdx.x * 4; k < p.K; k += 256 * 4) {
       const float4 a = (k < 256 * 4) ? a_first : head_feat4(p, f, b, k);
       const float4 ww = __ldg(reinterpret_cast<const float4*>(p.w + k));
       float4 o = epilogue4_t<EPI_BWD>(p.feat_ep, 0, make_float4(dl * ww.x, dl * ww.y, dl * ww.z, dl * ww.w), a, a);
+      if (p.dpre16) {
+        *reinterpret_cast<uint2*>(reinterpret_cast<__half*>(p.dpre) + (size_t)b * p.K + k) = pack_half4(o);
+        continue;
+      }
       if (p.round_out) { o.x = tf32_rn(o.x); o.y = tf32_rn(o.y); o.z = tf32_rn(o.z); o.w = tf32_rn(o.w); }
       *reinterpret_cast<float4*>(d + k) = o;
     }
@@ -848,13 +872,39 @@ struct Chain {
   size_t max_elems;
   size_t col_elems;              // per-sample elements of the scatter column buffer (0 if unused)
   int img_mode;                  // layout of the image-like tensors: IMG_S2D or IMG_PITCHED (choose_image_layout)
+  int f16;                       // MMA operands of the GEMM layers are FP16 on kind::f16 (choose_operand_type)
 };
+
+// G's last deconv / D's first conv: the passes that produce or read the image (edge kernels / general lowerings)
+static bool edge_layer(const cgs_layer_desc& L) { return use_scatter(L, false) || use_window(L, false); }
+
+// Every pass of every other layer can take FP16 operands: plain gathered GEMMs (no split-K) whose reduced channel
+// count fills whole 64-channel atoms, with FP16 copies of both packed weight matrices in the descriptor.
+static bool f16_capable(const Chain& c) {
+  for (int i = 0; i < c.n; ++i) {
+    const cgs_layer_desc& L = c.layers[i];
+    if (edge_layer(L)) continue;
+    if (!L.w16_fwd || !L.w16_bwd) return false;
+    for (int bw = 0; bw < 2; ++bw)
+      if (use_scatter(L, bw != 0) || use_window(L, bw != 0) || fc_split(L, bw != 0) > 1 || pass_shape(L, bw != 0).kch % 64)
+        return false;
+  }
+  return true;
+}
+
+// In an FP16 chain the tensor that layer j's data-gradient pass reduces is FP16 exactly when layer j is a GEMM layer,
+// and so is the forward input of such a layer, except the refined feature itself (j = 0): it stays FP32, because
+// momentum integrates steps below its last TF32 bit, and layer 0's forward pass keeps kind::tf32 over it.  The edge
+// kernels' 64-channel side towards the narrow kernel stays FP32 too.
+static bool feeds16(const Chain& c, int j) { return c.f16 && j >= 0 && j < c.n && !edge_layer(c.layers[j]); }
+static bool fwd16(const Chain& c, int i) { return i > 0 && feeds16(c, i); }
 
 static int build_chain(const cgs_net_desc* gtail, const cgs_net_desc* d, Chain& c) {
   if (!gtail || !d) return set_error(CGS_ERR_INVALID, "null network descriptor");
   if (gtail->n_layers < 1 || gtail->n_layers > CGS_MAX_LAYERS || d->n_layers < 2 || d->n_layers > CGS_MAX_LAYERS)
     return set_error(CGS_ERR_INVALID, "bad layer counts (%d, %d)", gtail->n_layers, d->n_layers);
   c.n = 0;
+  c.f16 = 0;
   for (int i = 0; i < gtail->n_layers; ++i) c.layers[c.n++] = gtail->layers[i];
   c.n_gtail = gtail->n_layers;
   for (int i = 0; i < d->n_layers - 1; ++i) c.layers[c.n++] = d->layers[i];
@@ -892,7 +942,8 @@ static int build_chain(const cgs_net_desc* gtail, const cgs_net_desc* d, Chain& 
 // the tensor core's operand truncation is exact; the image (returned to the caller) and the head input stay FP32.
 static Epilogue forward_epi(const Chain& c, int i, int math) {
   Epilogue e(EPI_FWD, c.layers[i].act);
-  e.round_out = (math == CGS_MATH_TF32_TENSOR) && (i != c.n_gtail - 1) && (i != c.n - 1);
+  e.out16 = fwd16(c, i + 1);
+  e.round_out = (math == CGS_MATH_TF32_TENSOR) && !e.out16 && (i != c.n_gtail - 1) && (i != c.n - 1);
   return e;
 }
 
@@ -902,7 +953,8 @@ static Epilogue backward_epi(const Chain& c, int i, int math, const Epilogue* up
   if (i == 0) return upd ? *upd : Epilogue(EPI_RAW, ACT_NONE);
   Epilogue e(EPI_BWD, c.layers[i - 1].act);
   e.aux = x;
-  e.round_out = (math == CGS_MATH_TF32_TENSOR);
+  e.out16 = feeds16(c, i - 1);
+  e.round_out = (math == CGS_MATH_TF32_TENSOR) && !e.out16;
   return e;
 }
 
@@ -916,6 +968,14 @@ static void choose_image_layout(Chain& c, int math) {
     if (edge_route(c.layers[i], false, math, forward_epi(c, i, math), IMG_S2D) != ROUTE_TC ||
         edge_route(c.layers[i], true, math, backward_epi(c, i, math, &upd, nullptr), IMG_S2D) != ROUTE_TC)
       c.img_mode = IMG_PITCHED;
+}
+
+// FP16 operands (half the bytes of the TF32-rounded FP32 ones, same 10-bit mantissa; kind::f16 at twice the kind::tf32
+// rate) for the DCGAN-shaped chains: s2d image layout, every other layer a plain tcgen05 GEMM with 64-channel atoms.
+// CGS_DEBUG_TF32_OPERANDS keeps the TF32 path for A/B comparisons; the gather-mode knob has no FP16 form.
+static void choose_operand_type(Chain& c, int math) {
+  c.f16 = math == CGS_MATH_TF32_TENSOR && c.img_mode == IMG_S2D && f16_capable(c) &&
+          !(debug_flags() & (CGS_DEBUG_TF32_OPERANDS | CGS_DEBUG_GATHER_A));
 }
 
 static inline size_t align256(size_t x) { return (x + 255) & ~size_t(255); }
@@ -934,6 +994,7 @@ struct Workspace {
   int* orig[2];
   int* idx;
   int* count;            // count[0], count[1]: live rows, ping-pong per step
+  int* gexp;             // FP16 operand chains: per-sample gradient scale (head_kernel)
   size_t total;
 };
 
@@ -956,6 +1017,7 @@ static void carve(const Chain& c, int64_t B, void* base, Workspace& w) {
   w.orig[1] = (int*)take((size_t)B * 4);
   w.idx = (int*)take((size_t)B * 4);
   w.count = (int*)take(16);
+  w.gexp = (int*)take((size_t)B * 4);
   w.total = off;
 }
 
@@ -978,7 +1040,8 @@ static int run_forward(const Chain& c, const Workspace& w, int64_t B, int math, 
       if (rc == 1) { ++i; continue; }
     }
     const bool defer = (i == c.n - 1) && head_takes_partials(c, w, B, math);
-    if (int rc = run_pass(c.layers[i], false, B, w.act[i], w.act[i + 1], epi(i), live, w.col, math, st, c.img_mode, defer))
+    if (int rc = run_pass(c.layers[i], false, B, w.act[i], w.act[i + 1], epi(i), live, w.col, math, st, c.img_mode, defer,
+                          fwd16(c, i) ? (const __half*)c.layers[i].w16_fwd : nullptr))
       return rc;
   }
   return CGS_OK;
@@ -1001,7 +1064,11 @@ static int run_backward(const Chain& c, const Workspace& w, int64_t B, int math,
       if (rc < 0) return rc;
       if (rc == 1) { --i; cur ^= 1; continue; }
     }
-    if (int rc = run_pass(c.layers[i], true, B, w.g[cur], dst, epi(i), live, w.col, math, st, c.img_mode)) return rc;
+    Epilogue e = epi(i);
+    if (i == 0 && c.f16) e.gexp = w.gexp;    // the policy step / raw gradient removes the head's per-sample scale
+    if (int rc = run_pass(c.layers[i], true, B, w.g[cur], dst, e, live, w.col, math, st, c.img_mode, false,
+                          feeds16(c, i) ? (const __half*)c.layers[i].w16_bwd : nullptr))
+      return rc;
     cur ^= 1;
   }
   return CGS_OK;
@@ -1055,6 +1122,8 @@ static int head_launch(const Chain& c, const Workspace& w, int64_t B, HeadParams
   hp.feature = w.act[0];
   hp.feat_elems = (int)c.act_elems[0];
   hp.cur_logit = w.cur_logit;
+  hp.dpre16 = feeds16(c, c.n - 1);
+  hp.gexp = w.gexp;
   cudaError_t le = launch_pdl(head_kernel, dim3((unsigned)B), dim3(256), (size_t)0, st, hp);
   count_launch();
   if (le != cudaSuccess) return set_error(CGS_ERR_CUDA, "head_kernel: %s", cudaGetErrorString(le));
@@ -1077,6 +1146,7 @@ extern "C" int cgs_refine_conv(const cgs_net_desc* gtail, const cgs_net_desc* d,
   Chain c;
   if (int rc = build_chain(gtail, d, c)) return rc;
   choose_image_layout(c, cfg->math);
+  choose_operand_type(c, cfg->math);
   // programmatic dependent launch for this call's kernels when the average pass is large (common.h launch_pdl):
   // forward + data-gradient FLOPs of one iteration over its 2 n + 1 launches
   double macs = 0.0;
@@ -1188,6 +1258,7 @@ extern "C" int cgs_forward_logits_and_grad(const cgs_net_desc* gtail, const cgs_
   Chain c;
   if (int rc = build_chain(gtail, d, c)) return rc;
   choose_image_layout(c, math);
+  choose_operand_type(c, math);
   Workspace w;
   carve(c, B, (void*)(((uintptr_t)workspace + 255) & ~uintptr_t(255)), w);
   if (!workspace || w.total + 256 > workspace_bytes) return set_error(CGS_ERR_WORKSPACE, "workspace too small");

@@ -163,6 +163,10 @@ typedef struct cgs_layer_desc {
   const float* w_fwd; int rows_fwd, kcols_fwd;
   const float* w_bwd; int rows_bwd, kcols_bwd;
   const float* bias; /* folded bias, padded with zeros to the output channel stride */
+  /* optional FP16 copies (__half, same layout) of w_fwd / w_bwd: with them on every GEMM layer, the DCGAN-shaped
+     refinement chains run their MMAs on FP16 operands (kind::f16); null = TF32 operands */
+  const void* w16_fwd;
+  const void* w16_bwd;
 } cgs_layer_desc;
 
 #define CGS_MAX_LAYERS 8
@@ -276,7 +280,8 @@ enum cgs_debug_flag {
   CGS_DEBUG_NO_CTA_PAIRS = 16777216,      /* no CTA pairs (clusters of two, tcgen05 cta_group::2) */
   CGS_DEBUG_FORCE_CTA_PAIRS = 33554432,   /* CTA pairs whenever legal */
   CGS_DEBUG_MLP2D_ONE_THREAD = 134217728, /* 2-D refinement with one thread per point, not the four-thread split form */
-  CGS_DEBUG_PDL_OFF = 536870912           /* programmatic dependent launch off everywhere (wins over PDL_ON) */
+  CGS_DEBUG_PDL_OFF = 536870912,          /* programmatic dependent launch off everywhere (wins over PDL_ON) */
+  CGS_DEBUG_TF32_OPERANDS = 1073741824    /* DCGAN refinement chain on TF32 (FP32-stored) MMA operands, not FP16 */
   /* retired, never reused: 262144, 2097152 */
 };
 
