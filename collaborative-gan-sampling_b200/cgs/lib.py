@@ -47,6 +47,7 @@ DEBUG_FORCE_MTILE_PAIRS = 8388608
 DEBUG_NO_CTA_PAIRS = 16777216
 DEBUG_FORCE_CTA_PAIRS = 33554432
 DEBUG_MLP2D_ONE_THREAD = 134217728
+DEBUG_MLP2D_CLUSTER = 268435456
 DEBUG_PDL_OFF = 536870912
 DEBUG_TF32_OPERANDS = 1073741824
 

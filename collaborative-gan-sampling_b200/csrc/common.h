@@ -115,6 +115,13 @@ inline cudaError_t launch_pdl_cluster(void (*kernel)(KArgs...), dim3 grid, dim3 
   return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
 }
 
+// cluster form of the 2-D MLP kernels, any nhidden = 16..256 divisible by 16 (mlp2d_cluster.cu); the descriptor is
+// already checked, inv_n = 1 / n_mean
+int mlp2d_cluster_score(const cgs_mlp_desc& d, const float* x, int64_t n, float inv_n, float* sig_out,
+                        float* logit_out, float* sal_out, cudaStream_t st);
+int mlp2d_cluster_refine(const cgs_mlp_desc& d, const cgs_refine2d_cfg& cfg, float inv_n, const float* x_in, int64_t n,
+                         float* best_x, float* best_loss, float* best_step, float* traj, cudaStream_t st);
+
 // shared device utilities (sampling_kernels.cu)
 int compact_flags(const unsigned char* flags, long n, int* block_counts, int* idx_out, int* count_out, cudaStream_t st);
 int gather_rows(const void* src, long row_bytes, const int* idx, const int* count, long max_rows, void* dst,

@@ -11,7 +11,7 @@
 namespace cgs {
 namespace {
 
-constexpr int H = 64;                 // nhidden supported by this build
+constexpr int H = 64;                 // nhidden of these kernels; every other width runs the cluster form (mlp2d_cluster.cu)
 constexpr int kMlpThreads = 128;
 
 struct MlpSmem {
@@ -139,8 +139,6 @@ __device__ __forceinline__ float mlp_point(const MlpSmem& s, int nlayers, float 
   gy = ay;
   return logit;
 }
-
-__device__ __forceinline__ float sigmoid_f32(float l) { return 1.f / (1.f + expf(-l)); }
 
 __global__ void __launch_bounds__(kMlpThreads, 1)
 mlp2d_score_kernel(const cgs_mlp_desc d, const float* __restrict__ x, int64_t n, float inv_n,
@@ -424,12 +422,16 @@ mlp2d_refine_split_kernel(const cgs_mlp_desc d, PolicyConsts pc, int steps, floa
 
 int check_mlp(const cgs_mlp_desc* d) {
   if (!d) return set_error(CGS_ERR_INVALID, "null mlp descriptor");
-  if (d->nhidden != H) return set_error(CGS_ERR_UNSUPPORTED, "nhidden %d: this build keeps the MLP in shared memory for nhidden == 64 only", d->nhidden);
+  if (d->nhidden < 16 || d->nhidden > 256 || d->nhidden % 16)
+    return set_error(CGS_ERR_UNSUPPORTED, "nhidden %d: this build runs the multiples of 16 from 16 to 256", d->nhidden);
   if (d->nlayers < 2 || d->nlayers > CGS_MLP_MAX_LAYERS) return set_error(CGS_ERR_UNSUPPORTED, "nlayers %d (2..8)", d->nlayers);   // synthetic/GAN.py:32 range(nlayers-2)
   for (int l = 0; l < d->nlayers; ++l)
     if (!d->weights[l] || !d->biases[l]) return set_error(CGS_ERR_INVALID, "null weights for layer %d", l);
   return CGS_OK;
 }
+
+// nhidden == 64 runs the kernels above; every other width, and 64 under CGS_DEBUG_MLP2D_CLUSTER, the cluster form
+bool use_cluster_form(const cgs_mlp_desc& d) { return d.nhidden != H || (debug_flags() & CGS_DEBUG_MLP2D_CLUSTER); }
 
 size_t mlp_smem_bytes(int nlayers, int threads) {
   const size_t wf = 2 * H + H + (size_t)(nlayers - 2) * (H * H + H) + H + 4;
@@ -462,6 +464,8 @@ extern "C" int cgs_mlp2d_score(const cgs_mlp_desc* d, const float* x, int64_t n,
   if (n == 0) return CGS_OK;
   if (!x || !sigmoid_out) return set_error(CGS_ERR_INVALID, "null argument");
   if (n_mean <= 0) n_mean = n;
+  if (use_cluster_form(*d))
+    return mlp2d_cluster_score(*d, x, n, 1.0f / (float)n_mean, sigmoid_out, logit_out, saliency_out, (cudaStream_t)stream);
   const LaunchShape s = mlp_launch_shape(d->nlayers, n);
   cudaError_t e = cudaFuncSetAttribute(mlp2d_score_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s.smem);
   if (e != cudaSuccess) return set_error(CGS_ERR_CUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
@@ -484,6 +488,9 @@ extern "C" int cgs_refine_mlp2d(const cgs_mlp_desc* d, const cgs_refine2d_cfg* c
   if (n == 0) return CGS_OK;
   if (!x_in || !best_x || !best_loss || !best_step) return set_error(CGS_ERR_INVALID, "null argument");
   const int64_t n_mean = cfg->n_mean > 0 ? cfg->n_mean : n;
+  if (use_cluster_form(*d))
+    return mlp2d_cluster_refine(*d, *cfg, 1.0f / (float)n_mean, x_in, n, best_x, best_loss, best_step, traj_out,
+                                (cudaStream_t)stream);
   if (!(debug_flags() & CGS_DEBUG_MLP2D_ONE_THREAD)) {
     // split form: four threads per point; the points are dealt evenly over the SMs (at most 96 per CTA round)
     const int sms = device_num_sms();

@@ -54,4 +54,7 @@ __device__ __forceinline__ float ladam_update(const PolicyConsts& c, float theta
   return __fsub_rn(theta, __fmul_rn(dx, r2));
 }
 
+// the discriminator's score (synthetic/GAN.py:108), shared by every form of the 2-D refiner so they agree bit for bit
+__device__ __forceinline__ float sigmoid_f32(float l) { return 1.f / (1.f + expf(-l)); }
+
 }  // namespace cgs

@@ -271,6 +271,13 @@ __device__ __forceinline__ void mbar_arrive_cluster(uint64_t* bar, uint32_t cta)
   asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(ra) : "r"(smem_u32(bar)), "r"(cta));
   asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(ra) : "memory");
 }
+// 16-byte store into the shared memory of CTA `cta` of the cluster, at the offset `p` has in this CTA
+__device__ __forceinline__ void st_cluster_v4(const void* p, uint32_t cta, float4 v) {
+  uint32_t ra;
+  asm("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(ra) : "r"(smem_u32(p)), "r"(cta));
+  asm volatile("st.shared::cluster.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(ra), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w)
+               : "memory");
+}
 
 // Shared-memory matrix descriptor: K-major operand, SWIZZLE_128B, rows of 128 bytes, 8-row groups 1024 B apart.
 // Field layout = cute::UMMA::SmemDescriptor (version_=1 for sm_100, layout_type 2 = SWIZZLE_128B).

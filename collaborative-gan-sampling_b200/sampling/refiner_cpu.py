@@ -44,6 +44,13 @@ class MlpSpec:
         self.desc.nhidden = self.nhidden
         if self.nlayers > L.MLP_MAX_LAYERS:
             raise NotImplementedError("at most %d layers" % L.MLP_MAX_LAYERS)
+        # the kernels read every layer at the shape nlayers and nhidden imply: check it before they do
+        nh = self.nhidden
+        for i, (k, b) in enumerate(layers):
+            want = (2 if i == 0 else nh, 1 if i == self.nlayers - 1 else nh)
+            ks, bs = tuple(np.shape(k)), tuple(np.shape(b))
+            if ks != want or bs != want[1:]:
+                raise ValueError("layer %d: kernel %s and bias %s, expected %s and %s" % (i, ks, bs, want, want[1:]))
         for i, (k, b) in enumerate(layers):
             kt, _ = R.to_device(k, torch.float32, dev)
             bt, _ = R.to_device(b, torch.float32, dev)

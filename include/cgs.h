@@ -120,7 +120,8 @@ CGS_API int cgs_gather_rows(const void* src, int64_t row_bytes, const int32_t* i
 #define CGS_MLP_MAX_LAYERS 8
 typedef struct cgs_mlp_desc {
   int nlayers;  /* --nlayers (synthetic/main.py), 2..8 ; layer 0 is 2->nhidden, last is nhidden->1 */
-  int nhidden;  /* --nhidden, must be 64 in this build */
+  int nhidden;  /* --nhidden, a multiple of 16 from 16 to 256; at 64 every CTA holds the whole MLP, every other width
+                   is held across a thread-block cluster of nhidden / 16 CTAs */
   const float* weights[CGS_MLP_MAX_LAYERS];
   const float* biases[CGS_MLP_MAX_LAYERS];
 } cgs_mlp_desc;
@@ -279,7 +280,10 @@ enum cgs_debug_flag {
   CGS_DEBUG_FORCE_MTILE_PAIRS = 8388608,  /* M-tile pairs whenever legal */
   CGS_DEBUG_NO_CTA_PAIRS = 16777216,      /* no CTA pairs (clusters of two, tcgen05 cta_group::2) */
   CGS_DEBUG_FORCE_CTA_PAIRS = 33554432,   /* CTA pairs whenever legal */
-  CGS_DEBUG_MLP2D_ONE_THREAD = 134217728, /* 2-D refinement with one thread per point, not the four-thread split form */
+  CGS_DEBUG_MLP2D_ONE_THREAD = 134217728, /* 2-D refinement with one thread per point, not the four-thread split form
+                                             (nhidden == 64 only) */
+  CGS_DEBUG_MLP2D_CLUSTER = 268435456,    /* 2-D score and refinement at nhidden == 64 on the cluster form that runs
+                                             every other width (wins over MLP2D_ONE_THREAD) */
   CGS_DEBUG_PDL_OFF = 536870912,          /* programmatic dependent launch off everywhere (wins over PDL_ON) */
   CGS_DEBUG_TF32_OPERANDS = 1073741824    /* DCGAN refinement chain on TF32 (FP32-stored) MMA operands, not FP16 */
   /* retired, never reused: 262144, 2097152 */
