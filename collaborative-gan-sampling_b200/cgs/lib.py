@@ -78,6 +78,10 @@ class NetDesc(C.Structure):
     _fields_ = [("n_layers", C.c_int), ("layers", LayerDesc * MAX_LAYERS)]
 
 
+class BatchnormDesc(C.Structure):
+    _fields_ = [("n_layers", C.c_int), ("gamma", C.c_void_p * MAX_LAYERS), ("beta", C.c_void_p * MAX_LAYERS)]
+
+
 class RefineCfg(C.Structure):
     _fields_ = [("steps", C.c_int), ("rate", C.c_double), ("method", C.c_int), ("alpha", C.c_double),
                 ("mode", C.c_int), ("clip", C.c_int), ("vmin", C.c_float), ("vmax", C.c_float),
@@ -118,6 +122,19 @@ _SIGNATURES = {
     "cgs_forward_logits_and_grad": (C.c_int, [C.POINTER(NetDesc), C.POINTER(NetDesc), C.c_int, C.c_int64,
                                               C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                               C.c_size_t, C.c_void_p]),
+    "cgs_refine_workspace_bytes_bn": (C.c_size_t, [C.POINTER(NetDesc), C.POINTER(NetDesc), C.POINTER(BatchnormDesc),
+                                                   C.c_int64]),
+    "cgs_refine_conv_bn": (C.c_int, [C.POINTER(NetDesc), C.POINTER(NetDesc), C.POINTER(BatchnormDesc),
+                                     C.POINTER(RefineCfg), C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                     C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "cgs_forward_logits_and_grad_bn": (C.c_int, [C.POINTER(NetDesc), C.POINTER(NetDesc), C.POINTER(BatchnormDesc),
+                                                 C.c_int, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                 C.c_void_p, C.c_size_t, C.c_void_p]),
+    "cgs_batchnorm_workspace_bytes": (C.c_size_t, [C.c_int64, C.c_int]),
+    "cgs_batchnorm_forward": (C.c_int, [C.c_int64, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p,
+                                        C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "cgs_batchnorm_backward": (C.c_int, [C.c_int64, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                         C.c_void_p, C.c_size_t, C.c_void_p]),
     "cgs_pack_map": (C.c_int64, [C.POINTER(LayerDesc), C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64]),
     "cgs_debug_gemm_params": (C.c_int64, [C.POINTER(LayerDesc), C.c_int, C.c_int64, C.c_void_p, C.c_int64]),
     "cgs_debug_fusion_plan": (C.c_int64, [C.POINTER(LayerDesc), C.c_int, C.c_int64, C.c_void_p, C.c_int64]),

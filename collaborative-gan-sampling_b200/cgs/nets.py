@@ -110,14 +110,15 @@ def _as_t(v):
     return v.detach().to("cpu", torch.float32) if isinstance(v, torch.Tensor) else torch.from_numpy(np.asarray(v, np.float32))
 
 
-def fold_layer(layer, scope, weights):
-    """Inference-mode BN folded into the layer: returns (W_tf_layout_scaled, bias_folded)."""
+def fold_layer(layer, scope, weights, fold_bn=True):
+    """Inference-mode BN folded into the layer: returns (W_tf_layout_scaled, bias_folded).  fold_bn=False: the layer's
+    own (W, bias), for a batch-statistic BN applied after it."""
     p = "%s/%s/" % (scope, layer["name"])
     if layer["type"] == "fc":
         w, b = _as_t(weights[p + "Matrix"]).clone(), _as_t(weights[p + "bias"]).clone()
     else:
         w, b = _as_t(weights[p + "w"]).clone(), _as_t(weights[p + "biases"]).clone()
-    if layer["bn"]:
+    if layer["bn"] and fold_bn:
         q = "%s/%s/" % (scope, layer["bn"])
         s = _as_t(weights[q + "gamma"]).double() / torch.sqrt(_as_t(weights[q + "moving_variance"]).double() + BN_EPS)
         t = _as_t(weights[q + "beta"]).double() - _as_t(weights[q + "moving_mean"]).double() * s
@@ -225,9 +226,12 @@ def round_tf32(t):
 
 
 class PackedNet:
-    """A chain of packed layers resident on one device + the cgs_net_desc that points at them."""
+    """A chain of packed layers resident on one device + the cgs_net_desc that points at them.
 
-    def __init__(self, layers, scope, weights, device, math="tf32"):
+    fold_bn=False packs the layers without their BN (training mode): ``bn_desc`` (cgs_batchnorm_desc) then points at
+    device copies of every BN's gamma / beta, which the library applies with the statistics of the batch."""
+
+    def __init__(self, layers, scope, weights, device, math="tf32", fold_bn=True):
         if len(layers) > L.MAX_LAYERS:
             raise ValueError("too many layers")
         self.layers = [dict(l) for l in layers]
@@ -236,8 +240,17 @@ class PackedNet:
         self.tensors = []
         self.desc = L.NetDesc()
         self.desc.n_layers = len(layers)
+        self.bn_desc = None
+        if not fold_bn:
+            self.bn_desc = L.BatchnormDesc()
+            self.bn_desc.n_layers = len(layers)
         for i, layer in enumerate(layers):
-            w, b = fold_layer(layer, scope, weights)
+            w, b = fold_layer(layer, scope, weights, fold_bn)
+            if not fold_bn and layer["bn"]:
+                q = "%s/%s/" % (scope, layer["bn"])
+                gamma, beta = (_as_t(weights[q + k]).to(self.device) for k in ("gamma", "beta"))
+                self.tensors += [gamma, beta]
+                self.bn_desc.gamma[i], self.bn_desc.beta[i] = gamma.data_ptr(), beta.data_ptr()
             wf, wb, bias = pack_layer(layer, w, b)
             if math == "tf32" and wb is not None:       # GEMM layers only; the 1-logit head stays FP32
                 wf, wb = round_tf32(wf), round_tf32(wb)
@@ -251,7 +264,7 @@ class PackedNet:
                 wb = wb.to(self.device)
                 self.tensors.append(wb)
                 d.w_bwd, d.rows_bwd, d.kcols_bwd = wb.data_ptr(), wb.shape[0], wb.shape[1]
-                if math == "tf32" and max(float(wf.abs().max()), float(wb.abs().max())) <= FP16_MAX:
+                if math == "tf32" and fold_bn and max(float(wf.abs().max()), float(wb.abs().max())) <= FP16_MAX:
                     # FP16 copies of the TF32-rounded matrices (the same values: same 10-bit mantissa, inside FP16's
                     # range); whether a chain runs on them is the library's decision (choose_operand_type)
                     wf16, wb16 = wf.half(), wb.half()
@@ -276,6 +289,16 @@ class NetSpec:
         self.gtail = PackedNet(arch["gtail"], "generator", weights, self.device, math)
         self.d = PackedNet(arch["d"], "discriminator", weights, self.device, math)
         self.role = role
+        self._weights = weights
+        self._d_batch = None
+
+    @property
+    def d_batch(self):
+        """D packed for training-mode BN (``discriminator_spec(spec, is_training=True)``): unfolded weights and the
+        BN parameters, packed on first use; ``d`` (inference mode, BN folded) is unchanged."""
+        if self._d_batch is None:
+            self._d_batch = PackedNet(self.arch["d"], "discriminator", self._weights, self.device, self.math, fold_bn=False)
+        return self._d_batch
 
     @classmethod
     def from_variables(cls, arch, variables, device="cuda", math="tf32", layout="tf"):
@@ -308,12 +331,15 @@ class NetSpec:
 class _Role:
     """View of a NetSpec playing one of the two set_env roles (discriminator / feature_to_data)."""
 
-    def __init__(self, spec, role):
-        self.spec, self.role = spec, role
+    def __init__(self, spec, role, is_training=False):
+        self.spec, self.role, self.is_training = spec, role, bool(is_training)
 
 
-def discriminator_spec(spec):
-    return _Role(spec, "discriminator")
+def discriminator_spec(spec, is_training=False):
+    """``partial(self.discriminator, is_training=..., reuse=True)`` (nsgan/GAN.py:175).  False (the default): BN in
+    inference mode, folded into the weights.  True: the reference's mode, BN with the statistics of the batch being
+    refined and the gradient through them (the moving averages are not updated)."""
+    return _Role(spec, "discriminator", is_training)
 
 
 def feature_to_data_spec(spec):

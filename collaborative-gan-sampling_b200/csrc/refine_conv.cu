@@ -1,5 +1,6 @@
 // Image-path refinement: layer -> gathered-GEMM parameter mapping, the fused head kernel (logit GEMV +
 // BCE gradient + best-of-K select + image keep), and the K-step loop of sampling/collaborator.py:41-88.
+#include "batchnorm.cuh"
 #include "common.h"
 #include "conv_gemm.cuh"
 #include "edge_conv.cuh"
@@ -873,6 +874,10 @@ struct Chain {
   size_t col_elems;              // per-sample elements of the scatter column buffer (0 if unused)
   int img_mode;                  // layout of the image-like tensors: IMG_S2D or IMG_PITCHED (choose_image_layout)
   int f16;                       // MMA operands of the GEMM layers are FP16 on kind::f16 (choose_operand_type)
+  // batch-statistic BN after layer i's GEMM (D layers only; null = none); batch_bn: any layer has it
+  const float* bn_gamma[2 * CGS_MAX_LAYERS];
+  const float* bn_beta[2 * CGS_MAX_LAYERS];
+  int batch_bn;
 };
 
 // G's last deconv / D's first conv: the passes that produce or read the image (edge kernels / general lowerings)
@@ -899,12 +904,14 @@ static bool f16_capable(const Chain& c) {
 static bool feeds16(const Chain& c, int j) { return c.f16 && j >= 0 && j < c.n && !edge_layer(c.layers[j]); }
 static bool fwd16(const Chain& c, int i) { return i > 0 && feeds16(c, i); }
 
-static int build_chain(const cgs_net_desc* gtail, const cgs_net_desc* d, Chain& c) {
+static int build_chain(const cgs_net_desc* gtail, const cgs_net_desc* d, const cgs_batchnorm_desc* bn, Chain& c) {
   if (!gtail || !d) return set_error(CGS_ERR_INVALID, "null network descriptor");
   if (gtail->n_layers < 1 || gtail->n_layers > CGS_MAX_LAYERS || d->n_layers < 2 || d->n_layers > CGS_MAX_LAYERS)
     return set_error(CGS_ERR_INVALID, "bad layer counts (%d, %d)", gtail->n_layers, d->n_layers);
   c.n = 0;
   c.f16 = 0;
+  c.batch_bn = 0;
+  for (int i = 0; i < 2 * CGS_MAX_LAYERS; ++i) c.bn_gamma[i] = c.bn_beta[i] = nullptr;
   for (int i = 0; i < gtail->n_layers; ++i) c.layers[c.n++] = gtail->layers[i];
   c.n_gtail = gtail->n_layers;
   for (int i = 0; i < d->n_layers - 1; ++i) c.layers[c.n++] = d->layers[i];
@@ -935,6 +942,22 @@ static int build_chain(const cgs_net_desc* gtail, const cgs_net_desc* d, Chain& 
   }
   if ((size_t)c.head.cin != c.act_elems[c.n]) return set_error(CGS_ERR_INVALID, "head input size mismatch");
   if (c.head.cin % 4) return set_error(CGS_ERR_UNSUPPORTED, "head input size must be a multiple of 4");
+  if (!bn) return CGS_OK;
+  if (bn->n_layers != d->n_layers)
+    return set_error(CGS_ERR_INVALID, "batchnorm descriptor has %d layers, the discriminator %d", bn->n_layers, d->n_layers);
+  for (int j = 0; j < d->n_layers; ++j) {
+    if (!bn->gamma[j]) continue;
+    if (!bn->beta[j]) return set_error(CGS_ERR_INVALID, "batch BN of D layer %d has gamma but no beta", j);
+    if (((uintptr_t)bn->gamma[j] | (uintptr_t)bn->beta[j]) & 15)
+      return set_error(CGS_ERR_INVALID, "gamma / beta of D layer %d must be 16-byte aligned", j);
+    if (j == d->n_layers - 1) return set_error(CGS_ERR_UNSUPPORTED, "batch BN on the 1-logit head is not built");
+    const int i = c.n_gtail + j;
+    if (edge_layer(c.layers[i])) return set_error(CGS_ERR_UNSUPPORTED, "batch BN on the image-edge layer %d of D is not built", j);
+    if (c.layers[i].cout % 4) return set_error(CGS_ERR_UNSUPPORTED, "batch BN needs a multiple of 4 channels (%d)", c.layers[i].cout);
+    c.bn_gamma[i] = bn->gamma[j];
+    c.bn_beta[i] = bn->beta[j];
+    c.batch_bn = 1;
+  }
   return CGS_OK;
 }
 
@@ -954,7 +977,8 @@ static Epilogue backward_epi(const Chain& c, int i, int math, const Epilogue* up
   Epilogue e(EPI_BWD, c.layers[i - 1].act);
   e.aux = x;
   e.out16 = feeds16(c, i - 1);
-  e.round_out = (math == CGS_MATH_TF32_TENSOR) && !e.out16;
+  // a batch-BN layer's gradient feeds bn_backward, not an MMA: it is rounded after that instead
+  e.round_out = (math == CGS_MATH_TF32_TENSOR) && !e.out16 && !c.bn_gamma[i - 1];
   return e;
 }
 
@@ -972,9 +996,11 @@ static void choose_image_layout(Chain& c, int math) {
 
 // FP16 operands (half the bytes of the TF32-rounded FP32 ones, same 10-bit mantissa; kind::f16 at twice the kind::tf32
 // rate) for the DCGAN-shaped chains: s2d image layout, every other layer a plain tcgen05 GEMM with 64-channel atoms.
-// CGS_DEBUG_TF32_OPERANDS keeps the TF32 path for A/B comparisons; the gather-mode knob has no FP16 form.
+// CGS_DEBUG_TF32_OPERANDS keeps the TF32 path for A/B comparisons; the gather-mode knob has no FP16 form.  A batch-BN
+// chain keeps TF32 operands: the per-sample gradient scale relies on the data-gradient chain being linear per sample,
+// and the BN backward mixes the samples.
 static void choose_operand_type(Chain& c, int math) {
-  c.f16 = math == CGS_MATH_TF32_TENSOR && c.img_mode == IMG_S2D && f16_capable(c) &&
+  c.f16 = math == CGS_MATH_TF32_TENSOR && c.img_mode == IMG_S2D && f16_capable(c) && !c.batch_bn &&
           !(debug_flags() & (CGS_DEBUG_TF32_OPERANDS | CGS_DEBUG_GATHER_A));
 }
 
@@ -995,8 +1021,15 @@ struct Workspace {
   int* idx;
   int* count;            // count[0], count[1]: live rows, ping-pong per step
   int* gexp;             // FP16 operand chains: per-sample gradient scale (head_kernel)
+  // batch-BN layers: their pre-BN output y (act[i + 1]'s layout), per-channel state, the FP64 partial sums
+  float* pre[2 * CGS_MAX_LAYERS];
+  float* bn_stat[2 * CGS_MAX_LAYERS];
+  double* bn_part;
   size_t total;
 };
+
+// rows of the [rows, C] tensor a batch-BN layer normalises over
+static long long bn_rows(const Chain& c, int i, int64_t B) { return (long long)B * (long long)(c.act_elems[i + 1] / cstride(c.layers[i].cout)); }
 
 // act[0] is the caller's feature buffer; everything else is carved out of the workspace.
 static void carve(const Chain& c, int64_t B, void* base, Workspace& w) {
@@ -1018,14 +1051,31 @@ static void carve(const Chain& c, int64_t B, void* base, Workspace& w) {
   w.idx = (int*)take((size_t)B * 4);
   w.count = (int*)take(16);
   w.gexp = (int*)take((size_t)B * 4);
+  size_t part_bytes = 0;
+  for (int i = 0; i < c.n; ++i) {
+    w.pre[i] = nullptr;
+    w.bn_stat[i] = nullptr;
+    if (!c.bn_gamma[i]) continue;
+    w.pre[i] = (float*)take((size_t)B * c.act_elems[i + 1] * 4);
+    w.bn_stat[i] = (float*)take((size_t)5 * c.layers[i].cout * 4);
+    const size_t pb = bn_partial_bytes(bn_rows(c, i, B), c.layers[i].cout);
+    if (pb > part_bytes) part_bytes = pb;
+  }
+  w.bn_part = part_bytes ? (double*)take(part_bytes) : nullptr;
   w.total = off;
 }
 
 // The last hidden layer runs split-K and nothing but the head reads its output: the head kernel then adds the partial
 // sums itself and the activation is never written (CGS_DEBUG_NO_HEAD_PARTIALS keeps the separate reduce kernel).
+// (A batch-BN layer's output needs the statistics of the whole sum first.)
 static bool head_takes_partials(const Chain& c, const Workspace& w, int64_t B, int math) {
   const cgs_layer_desc& L = c.layers[c.n - 1];
-  return use_fc_split(L, false, B, math, w.col) && !(debug_flags() & CGS_DEBUG_NO_HEAD_PARTIALS) && cstride(L.cout) == c.head.cin;
+  return use_fc_split(L, false, B, math, w.col) && !(debug_flags() & CGS_DEBUG_NO_HEAD_PARTIALS) &&
+         cstride(L.cout) == c.head.cin && !c.bn_gamma[c.n - 1];
+}
+
+static BnLayer bn_layer(const Chain& c, const Workspace& w, int i, int64_t B) {
+  return BnLayer{c.bn_gamma[i], c.bn_beta[i], bn_rows(c, i, B), c.layers[i].cout, w.bn_stat[i]};
 }
 
 static int run_forward(const Chain& c, const Workspace& w, int64_t B, int math, cudaStream_t st,
@@ -1040,6 +1090,14 @@ static int run_forward(const Chain& c, const Workspace& w, int64_t B, int math, 
       if (rc == 1) { ++i; continue; }
     }
     const bool defer = (i == c.n - 1) && head_takes_partials(c, w, B, math);
+    if (c.bn_gamma[i]) {
+      // batch BN: the GEMM stores y = conv(x) + b unrounded, the BN kernels normalise it into act[i + 1]
+      if (int rc = run_pass(c.layers[i], false, B, w.act[i], w.pre[i], Epilogue(EPI_FWD, ACT_NONE), live, w.col, math, st,
+                            c.img_mode))
+        return rc;
+      if (int rc = bn_forward(bn_layer(c, w, i, B), w.pre[i], w.act[i + 1], epi(i), w.bn_part, st)) return rc;
+      continue;
+    }
     if (int rc = run_pass(c.layers[i], false, B, w.act[i], w.act[i + 1], epi(i), live, w.col, math, st, c.img_mode, defer,
                           fwd16(c, i) ? (const __half*)c.layers[i].w16_fwd : nullptr))
       return rc;
@@ -1055,6 +1113,11 @@ static int run_backward(const Chain& c, const Workspace& w, int64_t B, int math,
   int cur = 0;
   for (int i = c.n - 1; i >= 0; --i) {
     float* dst = (i == 0) ? (upd ? w.act[0] : grad_out) : w.g[cur ^ 1];
+    if (c.bn_gamma[i]) {
+      // g[cur] is d loss / d (the BN output before the activation): through the batch statistics to d loss / d y, in place
+      if (int rc = bn_backward(bn_layer(c, w, i, B), w.pre[i], w.g[cur], w.g[cur], math == CGS_MATH_TF32_TENSOR, w.bn_part, st))
+        return rc;
+    }
     if (i == c.n_gtail && i >= 1 && c.img_mode == IMG_PITCHED) {
       // data-gradients of D's first conv and G's last deconv: one kernel, the image gradient never leaves the SM
       float* dst2 = (i - 1 == 0) ? (upd ? w.act[0] : grad_out) : w.g[cur ^ 1];
@@ -1081,17 +1144,22 @@ using namespace cgs;
 // Largest batch one call can take (rows are indexed with 32 bits); larger batches are refined in chunks by the caller.
 extern "C" int64_t cgs_refine_max_batch(const cgs_net_desc* gtail, const cgs_net_desc* d) {
   Chain c;
-  if (int rc = build_chain(gtail, d, c)) return rc;
+  if (int rc = build_chain(gtail, d, nullptr, c)) return rc;
   const size_t per = c.max_elems > c.col_elems ? c.max_elems : c.col_elems;
   return (int64_t)(((1ull << 31) - 1) / per) - 1;
 }
 
-extern "C" size_t cgs_refine_workspace_bytes(const cgs_net_desc* gtail, const cgs_net_desc* d, int64_t B) {
+extern "C" size_t cgs_refine_workspace_bytes_bn(const cgs_net_desc* gtail, const cgs_net_desc* d,
+                                                 const cgs_batchnorm_desc* bn, int64_t B) {
   Chain c;
-  if (build_chain(gtail, d, c) != CGS_OK || B < 0) return 0;
+  if (build_chain(gtail, d, bn, c) != CGS_OK || B < 0) return 0;
   Workspace w;
   carve(c, B, nullptr, w);
   return w.total + 256;
+}
+
+extern "C" size_t cgs_refine_workspace_bytes(const cgs_net_desc* gtail, const cgs_net_desc* d, int64_t B) {
+  return cgs_refine_workspace_bytes_bn(gtail, d, nullptr, B);
 }
 
 static int head_launch(const Chain& c, const Workspace& w, int64_t B, HeadParams hp, int math, cudaStream_t st) {
@@ -1123,6 +1191,7 @@ static int head_launch(const Chain& c, const Workspace& w, int64_t B, HeadParams
   hp.feat_elems = (int)c.act_elems[0];
   hp.cur_logit = w.cur_logit;
   hp.dpre16 = feeds16(c, c.n - 1);
+  if (c.bn_gamma[c.n - 1]) hp.round_out = 0;           // dpre feeds bn_backward, which rounds its own output
   hp.gexp = w.gexp;
   cudaError_t le = launch_pdl(head_kernel, dim3((unsigned)B), dim3(256), (size_t)0, st, hp);
   count_launch();
@@ -1130,10 +1199,10 @@ static int head_launch(const Chain& c, const Workspace& w, int64_t B, HeadParams
   return check_launch("head_kernel");
 }
 
-extern "C" int cgs_refine_conv(const cgs_net_desc* gtail, const cgs_net_desc* d, const cgs_refine_cfg* cfg,
-                               int64_t B, float* feature, float* best_img, float* best_logit, float* best_step,
-                               float* default_logit, const int32_t* prob_indices, float* best_feature,
-                               void* workspace, size_t workspace_bytes, cgs_stream_t stream) {
+extern "C" int cgs_refine_conv_bn(const cgs_net_desc* gtail, const cgs_net_desc* d, const cgs_batchnorm_desc* bn,
+                                  const cgs_refine_cfg* cfg, int64_t B, float* feature, float* best_img, float* best_logit,
+                                  float* best_step, float* default_logit, const int32_t* prob_indices, float* best_feature,
+                                  void* workspace, size_t workspace_bytes, cgs_stream_t stream) {
   if (int rc = require_sm100()) return rc;
   if (!cfg || !feature || !best_img || !best_logit || !best_step) return set_error(CGS_ERR_INVALID, "null argument");
   if (B <= 0) return B == 0 ? CGS_OK : set_error(CGS_ERR_INVALID, "negative batch");
@@ -1144,7 +1213,9 @@ extern "C" int cgs_refine_conv(const cgs_net_desc* gtail, const cgs_net_desc* d,
   if (cfg->mode != CGS_MODE_PROBABILISTIC && cfg->mode != CGS_MODE_DETERMINISTIC)
     return set_error(CGS_ERR_UNSUPPORTED, "unknown mode %d", cfg->mode);
   Chain c;
-  if (int rc = build_chain(gtail, d, c)) return rc;
+  if (int rc = build_chain(gtail, d, bn, c)) return rc;
+  if (c.batch_bn && cfg->early_exit)
+    return set_error(CGS_ERR_UNSUPPORTED, "early exit with batch BN: leaving rows would change the batch statistics");
   choose_image_layout(c, cfg->math);
   choose_operand_type(c, cfg->math);
   // programmatic dependent launch for this call's kernels when the average pass is large (common.h launch_pdl):
@@ -1249,14 +1320,23 @@ extern "C" int cgs_refine_conv(const cgs_net_desc* gtail, const cgs_net_desc* d,
   return CGS_OK;
 }
 
-extern "C" int cgs_forward_logits_and_grad(const cgs_net_desc* gtail, const cgs_net_desc* d, int math, int64_t B,
-                                           const float* feature, float* logit_out, float* grad_out, float* img_out,
-                                           void* workspace, size_t workspace_bytes, cgs_stream_t stream) {
+extern "C" int cgs_refine_conv(const cgs_net_desc* gtail, const cgs_net_desc* d, const cgs_refine_cfg* cfg,
+                               int64_t B, float* feature, float* best_img, float* best_logit, float* best_step,
+                               float* default_logit, const int32_t* prob_indices, float* best_feature,
+                               void* workspace, size_t workspace_bytes, cgs_stream_t stream) {
+  return cgs_refine_conv_bn(gtail, d, nullptr, cfg, B, feature, best_img, best_logit, best_step, default_logit,
+                            prob_indices, best_feature, workspace, workspace_bytes, stream);
+}
+
+extern "C" int cgs_forward_logits_and_grad_bn(const cgs_net_desc* gtail, const cgs_net_desc* d,
+                                              const cgs_batchnorm_desc* bn, int math, int64_t B, const float* feature,
+                                              float* logit_out, float* grad_out, float* img_out, void* workspace,
+                                              size_t workspace_bytes, cgs_stream_t stream) {
   if (int rc = require_sm100()) return rc;
   if (!feature || !logit_out) return set_error(CGS_ERR_INVALID, "null argument");
   if (B <= 0) return B == 0 ? CGS_OK : set_error(CGS_ERR_INVALID, "negative batch");
   Chain c;
-  if (int rc = build_chain(gtail, d, c)) return rc;
+  if (int rc = build_chain(gtail, d, bn, c)) return rc;
   choose_image_layout(c, math);
   choose_operand_type(c, math);
   Workspace w;
@@ -1292,6 +1372,13 @@ extern "C" int cgs_forward_logits_and_grad(const cgs_net_desc* gtail, const cgs_
     if (int rc = run_backward(c, w, B, math, nullptr, grad_out, st)) return rc;
   }
   return check_launch("cgs_forward_logits_and_grad");
+}
+
+extern "C" int cgs_forward_logits_and_grad(const cgs_net_desc* gtail, const cgs_net_desc* d, int math, int64_t B,
+                                           const float* feature, float* logit_out, float* grad_out, float* img_out,
+                                           void* workspace, size_t workspace_bytes, cgs_stream_t stream) {
+  return cgs_forward_logits_and_grad_bn(gtail, d, nullptr, math, B, feature, logit_out, grad_out, img_out, workspace,
+                                        workspace_bytes, stream);
 }
 
 static size_t layer_stage_elems(const cgs_layer_desc& L, bool backward) {   // pitched copy of an image-like input

@@ -9,7 +9,8 @@ Semantic shift (SURVEY.md §8b): the reference builds a symbolic TF graph from p
 ``discriminator`` / ``feature_to_data`` are network specs (``cgs.nets.discriminator_spec(spec)`` /
 ``feature_to_data_spec(spec)``) and ``build_refiner`` runs eagerly and returns the refined batch.
 ``func_loss`` must be the BCE-with-ones marker ``cgs.nets.loss_refine`` (nsgan/GAN.py:176-177).
-BatchNorm runs in inference mode (folded), see DESIGN.md for the delta to the reference's training-mode D.
+D's BatchNorm runs in inference mode (folded) by default; ``discriminator_spec(spec, is_training=True)`` selects the
+reference's training mode (statistics of the refined batch, nsgan/GAN.py:175), see DESIGN.md.
 """
 from __future__ import annotations
 
@@ -54,13 +55,17 @@ class Refiner():
             raise TypeError("discriminator / feature_to_data must be cgs.nets specs (python callables cannot be fused)")
         if not getattr(func_loss, "is_bce_with_ones", False):
             raise NotImplementedError("only the reference's BCE-with-ones refinement loss is built (nsgan/GAN.py:176-177)")
+        if getattr(feature_to_data, "is_training", False):
+            raise NotImplementedError("G's tail runs in inference mode, as in the reference (nsgan/GAN.py:94)")
         self.discriminator = discriminator
         self.feature_to_data = feature_to_data
         self.func_loss = func_loss
         # captured graphs hold the weight / bias pointers of the previous environment by value: never replay them
         # against another one (their cache entries also keep the specs they were captured with alive)
         self._graphs = {}
-        self._d = spec_d.d
+        self._batch_bn = bool(getattr(discriminator, "is_training", False))
+        self._d = spec_d.d_batch if self._batch_bn else spec_d.d
+        self._bn = C.byref(self._d.bn_desc) if self._batch_bn else None     # NULL: inference mode
         self._g = spec_g.gtail
         self._spec = spec_g
         self._cimg = spec_g.image_shape[2]
@@ -76,7 +81,7 @@ class Refiner():
 
     # ------------------------------------------------------------------------------------------
     def _workspace(self, B, dev):
-        nbytes = L.load().cgs_refine_workspace_bytes(C.byref(self._g.desc), C.byref(self._d.desc), B)
+        nbytes = L.load().cgs_refine_workspace_bytes_bn(C.byref(self._g.desc), C.byref(self._d.desc), self._bn, B)
         if nbytes == 0:
             L.check(-1 if not L.last_error() else -2)
         return self._ws.get(nbytes, dev)
@@ -96,9 +101,9 @@ class Refiner():
         logit = torch.empty(B, dtype=torch.float32, device=dev)
         grad = torch.empty_like(feat)
         ws = self._workspace(B, dev)
-        L.check(L.load().cgs_forward_logits_and_grad(C.byref(self._g.desc), C.byref(self._d.desc), L.MATH_IDS[self.math],
-                                                     B, L.ptr(feat), L.ptr(logit), L.ptr(grad), None, L.ptr(ws),
-                                                     ws.numel(), L.stream_ptr()))
+        L.check(L.load().cgs_forward_logits_and_grad_bn(C.byref(self._g.desc), C.byref(self._d.desc), self._bn,
+                                                        L.MATH_IDS[self.math], B, L.ptr(feat), L.ptr(logit), L.ptr(grad),
+                                                        None, L.ptr(ws), ws.numel(), L.stream_ptr()))
         return logit, grad
 
     def feature_to_image(self, feature):
@@ -109,9 +114,9 @@ class Refiner():
         logit = torch.empty(B, dtype=torch.float32, device=dev)
         img = torch.empty(self._img_shape(B), dtype=torch.float32, device=dev)
         ws = self._workspace(B, dev)
-        L.check(L.load().cgs_forward_logits_and_grad(C.byref(self._g.desc), C.byref(self._d.desc), L.MATH_IDS[self.math],
-                                                     B, L.ptr(feat), L.ptr(logit), None, L.ptr(img), L.ptr(ws),
-                                                     ws.numel(), L.stream_ptr()))
+        L.check(L.load().cgs_forward_logits_and_grad_bn(C.byref(self._g.desc), C.byref(self._d.desc), self._bn,
+                                                        L.MATH_IDS[self.math], B, L.ptr(feat), L.ptr(logit), None,
+                                                        L.ptr(img), L.ptr(ws), ws.numel(), L.stream_ptr()))
         return img[..., :self._cimg], logit
 
     def prefetch(self, fake_feature):
@@ -153,6 +158,13 @@ class Refiner():
         limit = self._max_rows_per_launch()
         if self.chunk_rows:
             limit = max(1, min(limit, int(self.chunk_rows)))
+        if self._batch_bn:
+            # training-mode BN normalises over the whole batch: chunks or leaving rows would change the statistics
+            if B > limit:
+                raise ValueError("a training-mode discriminator refines one batch of at most %d rows in one call "
+                                 "(chunking would change the batch statistics)" % limit)
+            if self.early_exit_logit is not None:
+                raise ValueError("early exit changes the batch the training-mode BN statistics run over")
         if B > limit:
             if prob_indices is None and mode == 'probabilistic':
                 prob_indices = np.random.randint(self.forward_steps + 1, size=B)
@@ -195,10 +207,10 @@ class Refiner():
             return b
 
         def launch(b, ws):
-            L.check(lib.cgs_refine_conv(C.byref(self._g.desc), C.byref(self._d.desc), C.byref(cfg), B, L.ptr(b["feat"]),
-                                        L.ptr(b["best_img"]), L.ptr(b["best_logit"]), L.ptr(b["best_step"]),
-                                        L.ptr(b["default_logit"]), L.ptr(b["idx"]), L.ptr(b["best_feat"]), L.ptr(ws),
-                                        ws.numel(), L.stream_ptr()))
+            L.check(lib.cgs_refine_conv_bn(C.byref(self._g.desc), C.byref(self._d.desc), self._bn, C.byref(cfg), B,
+                                           L.ptr(b["feat"]), L.ptr(b["best_img"]), L.ptr(b["best_logit"]),
+                                           L.ptr(b["best_step"]), L.ptr(b["default_logit"]), L.ptr(b["idx"]),
+                                           L.ptr(b["best_feat"]), L.ptr(ws), ws.numel(), L.stream_ptr()))
 
         if not self.cuda_graph:
             b = buffers()
@@ -209,11 +221,11 @@ class Refiner():
         else:
             # the launch sequence depends only on (shapes, config): capture it once, replay afterwards
             key = (B, mode, cfg.steps, cfg.rate, cfg.method, cfg.alpha, cfg.clip, cfg.vmin, cfg.vmax, cfg.math,
-                   cfg.early_exit, cfg.exit_logit, keep_optimal_feature, id(self._g), id(self._d), str(dev))
+                   cfg.early_exit, cfg.exit_logit, keep_optimal_feature, self._batch_bn, id(self._g), id(self._d), str(dev))
             ent = self._graphs.get(key)
             if ent is None:
                 b = buffers()
-                nbytes = lib.cgs_refine_workspace_bytes(C.byref(self._g.desc), C.byref(self._d.desc), B)
+                nbytes = lib.cgs_refine_workspace_bytes_bn(C.byref(self._g.desc), C.byref(self._d.desc), self._bn, B)
                 ws = torch.empty(int(nbytes), dtype=torch.uint8, device=dev)
                 b["feat"].copy_(feat_in)
                 if idx_host is not None:

@@ -217,6 +217,47 @@ CGS_API int cgs_forward_logits_and_grad(const cgs_net_desc* gtail, const cgs_net
                                 const float* feature, float* logit_out, float* grad_out, float* img_out,
                                 void* workspace, size_t workspace_bytes, cgs_stream_t stream);
 
+/* ------------------------------------------------------------------------------------------------------------
+ * Training-mode discriminator: batch-statistic BatchNorm (nsgan/GAN.py:175 `is_training=True`, nsgan/ops.py:19-26).
+ * For every D layer with a gamma: y = layer(x) + bias, mean / biased variance per channel over all B*H*W rows of
+ * the batch of the call (B rows for fc), out = act(gamma * (y - mean) / sqrt(var + 1e-5) + beta); the gradient flows
+ * through the statistics.  G's tail stays in inference mode, as in the reference (nsgan/GAN.py:94).  The moving
+ * averages are not updated (they change no value the refinement computes) and the weights are never written.
+ * ---------------------------------------------------------------------------------------------------------- */
+typedef struct cgs_batchnorm_desc {
+  int n_layers;                        /* == the D net's n_layers */
+  const float* gamma[CGS_MAX_LAYERS];  /* [cout] per D layer; null = no batch BN after that layer */
+  const float* beta[CGS_MAX_LAYERS];   /* [cout] */
+} cgs_batchnorm_desc;
+
+/* The _bn entry points are the plain ones with a batchnorm descriptor; bn == NULL is exactly the plain call.  With a
+ * non-null bn, `d` carries the UNFOLDED weights of the layers that have a gamma (w * 1, bias = the layer's own).
+ * CGS_ERR_UNSUPPORTED: batch BN with early exit (it would change the batch the statistics run over), on D's
+ * image-edge (first) layer or on the 1-logit head.  The statistics are those of the B rows of one call: the
+ * caller must not split a batch into chunks.  The chain runs on TF32 (FP32-stored) operands in this mode. */
+CGS_API size_t cgs_refine_workspace_bytes_bn(const cgs_net_desc* gtail, const cgs_net_desc* d,
+                                             const cgs_batchnorm_desc* bn, int64_t B);
+CGS_API int cgs_refine_conv_bn(const cgs_net_desc* gtail, const cgs_net_desc* d, const cgs_batchnorm_desc* bn,
+                               const cgs_refine_cfg* cfg, int64_t B, float* feature, float* best_img, float* best_logit,
+                               float* best_step, float* default_logit, const int32_t* prob_indices, float* best_feature,
+                               void* workspace, size_t workspace_bytes, cgs_stream_t stream);
+CGS_API int cgs_forward_logits_and_grad_bn(const cgs_net_desc* gtail, const cgs_net_desc* d,
+                                           const cgs_batchnorm_desc* bn, int math, int64_t B, const float* feature,
+                                           float* logit_out, float* grad_out, float* img_out, void* workspace,
+                                           size_t workspace_bytes, cgs_stream_t stream);
+
+/* The batch-BN kernels alone (per-kernel tests): y, out, dz, dy are [rows, C] FP32, C a multiple of 4; every tensor
+ * (gamma and beta too) 16-byte aligned, else CGS_ERR_INVALID.
+ * forward: out = act(gamma * (y - mean) * rstd + beta), act a cgs_act; mean_out / rstd_out [C] nullable.
+ * backward: dz = d loss / d (gamma * x^ + beta) with x^ = (y - mean) * rstd, the statistics of y recomputed ->
+ *   dy = d loss / d y = rstd * (dz^ - mean(dz^) - x^ * mean(dz^ * x^)), dz^ = gamma * dz. */
+CGS_API size_t cgs_batchnorm_workspace_bytes(int64_t rows, int C);
+CGS_API int cgs_batchnorm_forward(int64_t rows, int C, const float* y, const float* gamma, const float* beta, int act,
+                                  float* out, float* mean_out, float* rstd_out, void* workspace, size_t workspace_bytes,
+                                  cgs_stream_t stream);
+CGS_API int cgs_batchnorm_backward(int64_t rows, int C, const float* y, const float* gamma, const float* dz, float* dy,
+                                   void* workspace, size_t workspace_bytes, cgs_stream_t stream);
+
 /* Host-only helper (no GPU needed): K ordering of a layer's packed weight matrix.  For K index q of the forward
  * (backward != 0: data-gradient) matrix: ky[q], kx[q] = filter tap or -1 for zero padding, ch[q] = reduced channel
  * (forward: input channel; backward: output channel).  Pass NULL arrays to query the K length (multiple of 32). */
