@@ -40,6 +40,7 @@ struct EdgeNarrowParams {
   int s2d;            // 1: out (and ep.aux) are in the space-to-depth image layout [B][IH][IW][16] (see edge_tc.cu)
   Epilogue ep;
   const int* live;    // early exit: device-resident number of images still in the batch (null = all of them)
+  int in16;           // in is FP16 (it was stored for a kind::f16 MMA): only the tcgen05 kernel takes it (edge_tc.cu)
 };
 
 bool edge_wide_supported(const EdgeWideParams& p);

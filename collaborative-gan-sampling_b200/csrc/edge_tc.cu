@@ -16,10 +16,16 @@
 // whose start address is simply advanced by a multiple of 128 bytes (the hardware swizzles on absolute address bits:
 // tools/probes/umma_shift_probe.cu).  Virtual pixels run over the halo columns too; those rows are never stored.
 //
-// CTA = 6 warps, persistent over (image, band) tiles: warp 0 TMA producer (one box per channel half into a ring of
+// CTA = 14 warps, persistent over (image, band) tiles: warp 0 TMA producer (one box per channel half into a ring of
 // half-patch stages), warp 1 MMA issuer (tcgen05.mma kind::tf32, M = 128, N = 16, accumulators in TMEM, double-buffered
-// per band), warps 2-5 epilogue (tcgen05.ld, bias + tanh or x tanh', pitched float4 stores).  HBM-bound by design:
+// per band), warps 2-13 epilogue (tcgen05.ld, bias + tanh or x tanh', pitched float4 stores).  HBM-bound by design:
 // every input byte is read once (+ 2 halo rows per band, L2 hits), every output byte written once.
+//
+// FP16 form (EdgeNarrowParams::in16: the input was stored as FP16 by the pass before it, in an FP16 operand chain): a
+// 128-byte row holds all 64 channels, so one TMA box {64 ch, PW, PR, 1} is a whole band and one ring stage; the
+// weights are [9 shifts][16 rows][64 k] FP16 (18 KB) and each shift is 4 kind::f16 MMAs (M 128, N 16, K 16) -- half
+// the MMAs and half the shared-memory operand reads of the TF32 form over the same row pitch, so the shifted
+// descriptors are unchanged.  The epilogue is the same.
 #include "edge_conv.cuh"
 
 #include <cuda.h>
@@ -38,6 +44,7 @@ constexpr int TC_EPI_WARPS = 12;                // three groups of four epilogue
 constexpr int TC_THREADS = (2 + TC_EPI_WARPS) * 32;
 constexpr int TC_MAX_MT = 4;                   // M tiles (128 virtual pixels) per band
 constexpr int TC_B_BYTES = 9 * 2 * 16 * 128;   // weights: [shift][channel half][16 columns][32 k] = 36 KB
+constexpr int TC_B16_BYTES = 9 * 16 * 128;     // FP16 form: [shift][16 columns][64 k] = 18 KB
 constexpr int TC_SLACK_BYTES = 16 * 1024;      // rows a (never stored) virtual pixel past the band may read
 
 struct NarrowTcParams {
@@ -45,32 +52,49 @@ struct NarrowTcParams {
   int R, bands, MT, PW, PR;                    // rows per band, bands per image, M tiles per band, patch pitch / rows
   int stage_bytes, nstages, ntiles;
 };
+// the FP16 form's kernel parameter: an overload of the same kernel, so the TF32 instances stay exactly what they were
+struct NarrowTc16Params { NarrowTcParams q; };
 
 // PW (patch pitch = IW + 2) is a template parameter so that every per-MMA descriptor offset is an immediate: the
 // single MMA-issuing thread is the serial resource of this kernel (216 MMAs per band), and with run-time offsets each
 // MMA cost ~50 cycles of 64-bit address arithmetic and register -> uniform-register moves (11 k cycles per band).
-template <int PW>
-__global__ void __launch_bounds__(TC_THREADS, 1)
-edge_narrow_tc_kernel(const __grid_constant__ NarrowTcParams q, const __grid_constant__ CUtensorMap tmap_in) {
+// F16: FP16 input and weights on kind::f16 (one stage per band, 108 MMAs per band).
+template <int PW, bool F16>
+__device__ __forceinline__ void edge_narrow_tc_body(const NarrowTcParams& q, const CUtensorMap& tmap_in) {
+  constexpr int NH = F16 ? 1 : 2;                            // ring stages (channel halves) per band
+  constexpr int B_BYTES = F16 ? TC_B16_BYTES : TC_B_BYTES;
   const EdgeNarrowParams& p = q.p;
   extern __shared__ uint8_t tc_smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(tc_smem_raw) + 1023) & ~uintptr_t(1023));
-  uint8_t* smem_b = smem;                                    // [9][2][16 rows][128 B], swizzled
-  uint8_t* smem_a = smem + TC_B_BYTES;                       // ring of half-patch stages (+ slack behind the last)
+  uint8_t* smem_b = smem;                                    // [9][NH][16 rows][128 B], swizzled
+  uint8_t* smem_a = smem + B_BYTES;                          // ring of (half-)patch stages (+ slack behind the last)
   __shared__ uint64_t full_bar[8], empty_bar[8], tmem_full_bar[2], tmem_empty_bar[2];
   __shared__ uint32_t tmem_ptr_smem;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 
   // weights -> SWIZZLE_128B K-major tiles: tile (shift, half), row n = (py * 2 + px) * 4 + c, k = channel in the half
-  for (int idx = threadIdx.x; idx < 9 * 2 * 16 * 8; idx += TC_THREADS) {
-    const int ck = idx & 7, n = (idx >> 3) & 15, h = (idx >> 7) & 1, sh = idx >> 8;
+  // (FP16: tile (shift), k = channel; converted RN here, like every FP16 operand of the chain)
+  for (int idx = threadIdx.x; idx < 9 * NH * 16 * 8; idx += TC_THREADS) {
+    const int ck = idx & 7, n = (idx >> 3) & 15, h = F16 ? 0 : (idx >> 7) & 1, sh = idx >> (F16 ? 7 : 8);
     const int dy = sh / 3 - 1, dx = sh % 3 - 1;
     const int py = n >> 3, px = (n >> 2) & 1, c = n & 3;
     const int ky = py + p.pad_y - 2 * dy, kx = px + p.pad_x - 2 * dx;
-    float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-    if (c < p.cimg && ky >= 0 && ky < p.k && kx >= 0 && kx < p.k)
-      v = __ldg(reinterpret_cast<const float4*>(p.w + (size_t)((ky * p.k + kx) * 4 + c) * p.K + h * 32 + ck * 4));
-    *reinterpret_cast<float4*>(smem_b + ((sh * 2 + h) * 16 + n) * 128 + ((ck ^ (n & 7)) << 4)) = v;
+    const bool tap = c < p.cimg && ky >= 0 && ky < p.k && kx >= 0 && kx < p.k;
+    const float* src = p.w + (size_t)((ky * p.k + kx) * 4 + c) * p.K;
+    uint8_t* dst = smem_b + ((sh * NH + h) * 16 + n) * 128 + ((ck ^ (n & 7)) << 4);
+    if (F16) {
+      uint4 v = make_uint4(0u, 0u, 0u, 0u);
+      if (tap) {
+        const uint2 lo = pack_half4(__ldg(reinterpret_cast<const float4*>(src + ck * 8)));
+        const uint2 hi = pack_half4(__ldg(reinterpret_cast<const float4*>(src + ck * 8 + 4)));
+        v = make_uint4(lo.x, lo.y, hi.x, hi.y);
+      }
+      *reinterpret_cast<uint4*>(dst) = v;
+    } else {
+      float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+      if (tap) v = __ldg(reinterpret_cast<const float4*>(src + h * 32 + ck * 4));
+      *reinterpret_cast<float4*>(dst) = v;
+    }
   }
   if (threadIdx.x == 0) {
     for (int s = 0; s < q.nstages; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], 1); }
@@ -97,12 +121,13 @@ edge_narrow_tc_kernel(const __grid_constant__ NarrowTcParams q, const __grid_con
       for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
         const int b = tile / q.bands;
         const int j0 = (tile - b * q.bands) * q.R;
-        for (int h = 0; h < 2; ++h) {
+        for (int h = 0; h < NH; ++h) {
           const uint32_t s = stage, ph = phase;
           if (++stage == (uint32_t)q.nstages) { stage = 0; phase ^= 1u; }
           mbar_wait(&empty_bar[s], ph ^ 1);
           mbar_arrive_expect_tx(&full_bar[s], bytes);
-          // box {32 channels, PW pixels from x = -1, PR rows from y = j0 - 1, 1 image}; outside the image reads zeros
+          // box {32 channels (FP16: 64), PW pixels from x = -1, PR rows from y = j0 - 1, 1 image}; outside the image
+          // reads zeros
           tma_load_4d(smem_u32(smem_a) + s * q.stage_bytes, &tmap_in, &full_bar[s], h * 32, -1, j0 - 1, b);
         }
       }
@@ -110,35 +135,43 @@ edge_narrow_tc_kernel(const __grid_constant__ NarrowTcParams q, const __grid_con
   } else if (warp == 1) {
     // ------------------------------------------------------------------ MMA issuer
     if (elect_one()) {
-      constexpr uint32_t idesc = make_idesc_tf32(128, 16);
+      constexpr uint32_t idesc = F16 ? make_idesc_f16(128, 16) : make_idesc_tf32(128, 16);
       const uint64_t da0 = make_smem_desc_sw128(smem_u32(smem_a));
       const uint64_t db0 = make_smem_desc_sw128(smem_u32(smem_b));
       uint32_t stage = 0, phase = 0, tile_count = 0;
       for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x, ++tile_count) {
         const uint32_t acc = tile_count & 1, acc_ph = (tile_count >> 1) & 1;
         mbar_wait(&tmem_empty_bar[acc], acc_ph ^ 1);
-        for (int h = 0; h < 2; ++h) {
+        for (int h = 0; h < NH; ++h) {
           const uint32_t s = stage;
           mbar_wait(&full_bar[s], phase);
           if (++stage == (uint32_t)q.nstages) { stage = 0; phase ^= 1u; }
           tcgen05_fence_after();
           const uint64_t da_stage = da0 + (uint64_t)((s * (uint32_t)q.stage_bytes) >> 4);
           const uint64_t db_half = db0 + (uint64_t)(h * ((16 * 128) >> 4));
-          for (int mt = 0; mt < q.MT; ++mt) {
-            const uint32_t tmem_d = tmem_base + (acc * TC_MAX_MT + mt) * 16;
-            const uint64_t da_mt = da_stage + (uint64_t)(mt * ((128 * 128) >> 4));
+          // FP16: the stage holds both channel halves; they are still reduced half after half, in the TF32 form's order
 #pragma unroll
-            for (int sh = 0; sh < 9; ++sh) {
-              // rows of the A tile = stored pixels 128 mt + dyi * PW + dxi ..: descriptor start in 16-byte units
-              constexpr int kRow = 128 >> 4;
-              const uint64_t da = da_mt + (uint64_t)(((sh / 3) * PW + (sh % 3)) * kRow);
-              const uint64_t db = db_half + (uint64_t)(sh * ((2 * 16 * 128) >> 4));
+          for (int hh = 0; hh < (F16 ? 2 : 1); ++hh) {
+            for (int mt = 0; mt < q.MT; ++mt) {
+              const uint32_t tmem_d = tmem_base + (acc * TC_MAX_MT + mt) * 16;
+              const uint64_t da_mt = da_stage + (uint64_t)(mt * ((128 * 128) >> 4));
 #pragma unroll
-              for (int k = 0; k < 4; ++k)
-                umma_tf32_ss(tmem_d, da + 2 * k, db + 2 * k, idesc, (h > 0 || sh > 0 || k > 0) ? 1u : 0u);
+              for (int sh = 0; sh < 9; ++sh) {
+                // rows of the A tile = stored pixels 128 mt + dyi * PW + dxi ..: descriptor start in 16-byte units
+                constexpr int kRow = 128 >> 4;
+                const uint64_t da = da_mt + (uint64_t)(((sh / 3) * PW + (sh % 3)) * kRow);
+                const uint64_t db = db_half + (uint64_t)(sh * ((NH * 16 * 128) >> 4));
+#pragma unroll
+                for (int k = 0; k < (F16 ? 2 : 4); ++k) {      // 32 bytes of the 128-byte row per MMA: K = 8 / 16
+                  const uint32_t accum = (h > 0 || hh > 0 || sh > 0 || k > 0) ? 1u : 0u;
+                  const int ko = 2 * (hh * 2 + k);              // 16-byte units; a channel half is 64 bytes
+                  if (F16) umma_f16_ss(tmem_d, da + ko, db + ko, idesc, accum);
+                  else umma_tf32_ss(tmem_d, da + ko, db + ko, idesc, accum);
+                }
+              }
             }
           }
-          umma_commit(&empty_bar[s]);                          // half-patch stage reusable once these MMAs have read it
+          umma_commit(&empty_bar[s]);                          // stage reusable once these MMAs have read it
         }
         umma_commit(&tmem_full_bar[acc]);                      // all accumulators of the band complete
       }
@@ -237,6 +270,17 @@ edge_narrow_tc_kernel(const __grid_constant__ NarrowTcParams q, const __grid_con
   if (warp == 1) tmem_dealloc(tmem_base, 2 * TC_MAX_MT * 16);
 }
 
+template <int PW>
+__global__ void __launch_bounds__(TC_THREADS, 1)
+edge_narrow_tc_kernel(const __grid_constant__ NarrowTcParams q, const __grid_constant__ CUtensorMap tmap_in) {
+  edge_narrow_tc_body<PW, false>(q, tmap_in);
+}
+template <int PW>
+__global__ void __launch_bounds__(TC_THREADS, 1)
+edge_narrow_tc_kernel(const __grid_constant__ NarrowTc16Params q, const __grid_constant__ CUtensorMap tmap_in) {
+  edge_narrow_tc_body<PW, true>(q.q, tmap_in);
+}
+
 typedef CUresult (*PFN_encodeTiledTc)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
                                       const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
                                       CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
@@ -287,8 +331,9 @@ int launch_edge_narrow_tc(const EdgeNarrowParams& p, cudaStream_t st) {
   q.bands = (p.IH + q.R - 1) / q.R;
   q.PR = q.R + 2;
   q.MT = ((q.R - 1) * q.PW + p.IW + 127) / 128;
-  q.stage_bytes = ((q.PR * q.PW * 128 + 1023) / 1024) * 1024;
-  const int budget = 227 * 1024 - TC_B_BYTES - TC_SLACK_BYTES - 2048;
+  q.stage_bytes = ((q.PR * q.PW * 128 + 1023) / 1024) * 1024;      // 128-byte rows: 32 FP32 or 64 FP16 channels
+  const int b_bytes = p.in16 ? TC_B16_BYTES : TC_B_BYTES;
+  const int budget = 227 * 1024 - b_bytes - TC_SLACK_BYTES - 2048;
   q.nstages = budget / q.stage_bytes;
   if (q.nstages > 8) q.nstages = 8;
   if (q.nstages < 2) return set_error(CGS_ERR_UNSUPPORTED, "edge_narrow_tc: band does not fit shared memory");
@@ -301,23 +346,27 @@ int launch_edge_narrow_tc(const EdgeNarrowParams& p, cudaStream_t st) {
   PFN_encodeTiledTc enc = encode_fn();
   if (!enc) return set_error(CGS_ERR_CUDA, "cuTensorMapEncodeTiled entry point not available");
   CUtensorMap tmap;
+  const cuuint64_t esz = p.in16 ? 2 : 4;
   cuuint64_t gdim[4] = {64, (cuuint64_t)p.IW, (cuuint64_t)p.IH, (cuuint64_t)p.B};
-  cuuint64_t gstr[3] = {64 * 4, (cuuint64_t)p.IW * 64 * 4, (cuuint64_t)p.IH * p.IW * 64 * 4};
-  cuuint32_t box[4] = {32, (cuuint32_t)q.PW, (cuuint32_t)q.PR, 1};
+  cuuint64_t gstr[3] = {64 * esz, (cuuint64_t)p.IW * 64 * esz, (cuuint64_t)p.IH * p.IW * 64 * esz};
+  cuuint32_t box[4] = {p.in16 ? 64u : 32u, (cuuint32_t)q.PW, (cuuint32_t)q.PR, 1};   // one 128-byte row per pixel
   cuuint32_t estr[4] = {1, 1, 1, 1};
-  CUresult r = enc(&tmap, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<float*>(p.in), gdim, gstr, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  CUresult r = enc(&tmap, p.in16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4,
+                   const_cast<float*>(p.in), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                   CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) return set_error(CGS_ERR_CUDA, "cuTensorMapEncodeTiled (edge_narrow_tc) failed (%d)", (int)r);
-  const size_t smem = (size_t)TC_B_BYTES + (size_t)q.nstages * q.stage_bytes + TC_SLACK_BYTES + 1024;
+  const size_t smem = (size_t)b_bytes + (size_t)q.nstages * q.stage_bytes + TC_SLACK_BYTES + 1024;
   long long grid = tiles < device_num_sms() ? tiles : device_num_sms();
   cudaError_t e = cudaSuccess, le = cudaSuccess;
 #define CGS_NARROW_TC_CASE(PWV)                                                                                          \
   case PWV: {                                                                                                            \
-    static DynSmemCache smem_cache;                                                                                      \
-    e = ensure_dyn_smem(edge_narrow_tc_kernel<PWV>, smem, smem_cache);                                                   \
+    void (*const k32)(NarrowTcParams, CUtensorMap) = edge_narrow_tc_kernel<PWV>;                                         \
+    void (*const k16)(NarrowTc16Params, CUtensorMap) = edge_narrow_tc_kernel<PWV>;                                       \
+    static DynSmemCache smem_cache, smem_cache16;                                                                        \
+    e = p.in16 ? ensure_dyn_smem(k16, smem, smem_cache16) : ensure_dyn_smem(k32, smem, smem_cache);                      \
     if (e == cudaSuccess)                                                                                                \
-      le = launch_pdl(edge_narrow_tc_kernel<PWV>, dim3((unsigned)grid), dim3(TC_THREADS), smem, st, q, tmap);           \
+      le = p.in16 ? launch_pdl(k16, dim3((unsigned)grid), dim3(TC_THREADS), smem, st, NarrowTc16Params{q}, tmap)         \
+                  : launch_pdl(k32, dim3((unsigned)grid), dim3(TC_THREADS), smem, st, q, tmap);                          \
   } break;
   switch (q.PW) {
     CGS_NARROW_TC_CASE(18)
@@ -364,7 +413,7 @@ struct WideTcParams {
   int B, H2, W2, k, cimg, pad;
   int R, bands, MT, PW, PR, stage_bytes, nstages, ntiles;
   const int* live;
-  float* out;              // [B][H2][W2][64], FP16 when ep.out16 (it feeds a kind::f16 MMA)
+  float* out;              // [B][H2][W2][64], FP16 when ep.out16 (it feeds a kind::f16 MMA; ep.aux is FP16 then too)
   Epilogue ep;
   int debug;               // debug_flags() at launch: CGS_DEBUG_SKIP_*, _NO_PREFETCH, _TRACE
 };
@@ -385,10 +434,10 @@ __device__ __forceinline__ float4 lds_f4(uint32_t addr) {
 }
 
 // PW: patch pitch (see edge_narrow_tc_kernel); EPI: epilogue mode compiled in (the per-element epilogue is a dependent
-// instruction stream -- a run-time mode switch per float4 doubled its length)
-template <int PW, int EPI>
-__global__ void __launch_bounds__(WT_THREADS, 1)
-edge_wide_tc_kernel(const __grid_constant__ WideTcParams q, const __grid_constant__ CUtensorMap tmap_in) {
+// instruction stream -- a run-time mode switch per float4 doubled its length); AUX16: the data-gradient pass of an FP16
+// operand chain, whose derivative operand is FP16 like its output (Epilogue::out16)
+template <int PW, int EPI, bool AUX16>
+__device__ __forceinline__ void edge_wide_tc_body(const WideTcParams& q, const CUtensorMap& tmap_in) {
   extern __shared__ uint8_t wt_smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(wt_smem_raw) + 1023) & ~uintptr_t(1023));
   uint8_t* smem_b = smem;
@@ -510,16 +559,23 @@ edge_wide_tc_kernel(const __grid_constant__ WideTcParams q, const __grid_constan
           ro[ps] = (i < q.W2 && j < j1) ? (((b * q.H2 + j) * q.W2 + i) * 64) : -1;
         }
         // epilogue operands of all four 16-channel chunks, fetched before the accumulator wait (their latency hides
-        // behind the MMAs of this tile): forward output (derivative) / feature + momentum (policy step) / bias
+        // behind the MMAs of this tile): forward output (derivative; FP16 in the AUX16 form) / feature + momentum
+        // (policy step) / bias
         float4 x0[4][4];
+        uint2 x0h[4][4];
 #pragma unroll
         for (int ch = 0; ch < 4; ++ch) {
           const int n = ch * 16 + c4 * 4;
           if (EPI == EPI_BWD) {
 #pragma unroll
             for (int ps = 0; ps < 4; ++ps)
-              x0[ch][ps] = (ro[ps] >= 0 && !(q.debug & CGS_DEBUG_NO_PREFETCH)) ? __ldg(reinterpret_cast<const float4*>(q.ep.aux + ro[ps] + n))
-                                                              : make_float4(1.f, 1.f, 1.f, 1.f);   // knob 2048: no operand loads
+              if (AUX16)                                        // kept packed until used: the loads stay in flight
+                x0h[ch][ps] = (ro[ps] >= 0 && !(q.debug & CGS_DEBUG_NO_PREFETCH))
+                                  ? __ldg(reinterpret_cast<const uint2*>(reinterpret_cast<const __half*>(q.ep.aux) + ro[ps] + n))
+                                  : make_uint2(0x3C003C00u, 0x3C003C00u);
+              else
+                x0[ch][ps] = (ro[ps] >= 0 && !(q.debug & CGS_DEBUG_NO_PREFETCH)) ? __ldg(reinterpret_cast<const float4*>(q.ep.aux + ro[ps] + n))
+                                                                : make_float4(1.f, 1.f, 1.f, 1.f);   // knob 2048: no operand loads
           } else if (EPI == EPI_FWD) {
             x0[ch][0] = q.ep.bias ? __ldg(reinterpret_cast<const float4*>(q.ep.bias + n)) : make_float4(0.f, 0.f, 0.f, 0.f);
           }
@@ -562,7 +618,8 @@ edge_wide_tc_kernel(const __grid_constant__ WideTcParams q, const __grid_constan
               float4 v = lds_f4(stg + ((u * 32 + ps * 8 + rsub) * WT_PITCH + c4 * 4) * 4);
               if (EPI == EPI_UPDATE || EPI == EPI_RAW) { v.x *= gscale; v.y *= gscale; v.z *= gscale; v.w *= gscale; }
               if (ro[ps] >= 0) {
-                float4 xa = EPI == EPI_FWD ? x0[ch][0] : x0[ch][ps], xb = make_float4(0.f, 0.f, 0.f, 0.f);
+                float4 xa = EPI == EPI_FWD ? x0[ch][0] : AUX16 ? unpack_half4(x0h[ch][ps]) : x0[ch][ps];
+                float4 xb = make_float4(0.f, 0.f, 0.f, 0.f);
                 if (EPI == EPI_UPDATE) {         // policy step (only when the G tail is this single layer): not prefetched
                   xa = *reinterpret_cast<const float4*>(q.out + ro[ps] + n);
                   if (!q.ep.sgd && !q.ep.first) xb = *reinterpret_cast<const float4*>(q.ep.mom + ro[ps] + n);
@@ -592,6 +649,19 @@ edge_wide_tc_kernel(const __grid_constant__ WideTcParams q, const __grid_constan
   tcgen05_fence_before();
   __syncthreads();
   if (warp == 1) tmem_dealloc(tmem_base, 512);
+}
+
+template <int PW, int EPI>
+__global__ void __launch_bounds__(WT_THREADS, 1)
+edge_wide_tc_kernel(const __grid_constant__ WideTcParams q, const __grid_constant__ CUtensorMap tmap_in) {
+  edge_wide_tc_body<PW, EPI, false>(q, tmap_in);
+}
+// the FP16-derivative form (EPI_BWD only): an overload of the same kernel, so the other instances stay what they were
+struct WideTc16Params { WideTcParams q; };
+template <int PW, int EPI>
+__global__ void __launch_bounds__(WT_THREADS, 1)
+edge_wide_tc_kernel(const __grid_constant__ WideTc16Params q, const __grid_constant__ CUtensorMap tmap_in) {
+  edge_wide_tc_body<PW, EPI, true>(q.q, tmap_in);
 }
 
 // dense [B][H][W][4] <-> s2d [B][H/2][W/2][16]: one float4 (pixel) per thread
@@ -682,21 +752,40 @@ int launch_edge_wide_tc(const EdgeWideParams& p, int B, cudaStream_t st) {
   const size_t smem = (size_t)fixed - 2048 + (size_t)q.nstages * q.stage_bytes + 1024;
   long long grid = tiles < device_num_sms() ? tiles : device_num_sms();
   cudaError_t e = cudaSuccess, le = cudaSuccess;
+  const bool aux16 = q.ep.mode == EPI_BWD && q.ep.out16;
 #define CGS_WIDE_TC_CASE(PWV, EPIV)                                                                                      \
   case PWV * 8 + EPIV: {                                                                                                 \
+    void (*const k32)(WideTcParams, CUtensorMap) = edge_wide_tc_kernel<PWV, EPIV>;                                       \
     static DynSmemCache smem_cache;                                                                                      \
-    e = ensure_dyn_smem(edge_wide_tc_kernel<PWV, EPIV>, smem, smem_cache);                                               \
+    e = ensure_dyn_smem(k32, smem, smem_cache);                                                                          \
+    if (e == cudaSuccess) le = launch_pdl(k32, dim3((unsigned)grid), dim3(WT_THREADS), smem, st, q, tmap);               \
+  } break;
+#define CGS_WIDE_TC_CASE16(PWV)                                                                                          \
+  case PWV * 8 + EPI_BWD: {                                                                                              \
+    void (*const k16)(WideTc16Params, CUtensorMap) = edge_wide_tc_kernel<PWV, EPI_BWD>;                                  \
+    static DynSmemCache smem_cache;                                                                                      \
+    e = ensure_dyn_smem(k16, smem, smem_cache);                                                                          \
     if (e == cudaSuccess)                                                                                                \
-      le = launch_pdl(edge_wide_tc_kernel<PWV, EPIV>, dim3((unsigned)grid), dim3(WT_THREADS), smem, st, q, tmap);       \
+      le = launch_pdl(k16, dim3((unsigned)grid), dim3(WT_THREADS), smem, st, WideTc16Params{q}, tmap);                   \
   } break;
 #define CGS_WIDE_TC_PW(PWV) CGS_WIDE_TC_CASE(PWV, EPI_FWD) CGS_WIDE_TC_CASE(PWV, EPI_BWD) CGS_WIDE_TC_CASE(PWV, EPI_UPDATE) CGS_WIDE_TC_CASE(PWV, EPI_RAW)
-  switch (q.PW * 8 + q.ep.mode) {
-    CGS_WIDE_TC_PW(18)
-    CGS_WIDE_TC_PW(34)
-    CGS_WIDE_TC_PW(66)
-    default: return set_error(CGS_ERR_UNSUPPORTED, "edge_wide_tc: row width %d / epilogue %d", q.W2, q.ep.mode);
+  if (aux16) {
+    switch (q.PW * 8 + q.ep.mode) {
+      CGS_WIDE_TC_CASE16(18)
+      CGS_WIDE_TC_CASE16(34)
+      CGS_WIDE_TC_CASE16(66)
+      default: return set_error(CGS_ERR_UNSUPPORTED, "edge_wide_tc: row width %d", q.W2);
+    }
+  } else {
+    switch (q.PW * 8 + q.ep.mode) {
+      CGS_WIDE_TC_PW(18)
+      CGS_WIDE_TC_PW(34)
+      CGS_WIDE_TC_PW(66)
+      default: return set_error(CGS_ERR_UNSUPPORTED, "edge_wide_tc: row width %d / epilogue %d", q.W2, q.ep.mode);
+    }
   }
 #undef CGS_WIDE_TC_PW
+#undef CGS_WIDE_TC_CASE16
 #undef CGS_WIDE_TC_CASE
   if (e != cudaSuccess) return set_error(CGS_ERR_CUDA, "cudaFuncSetAttribute(edge_wide_tc): %s", cudaGetErrorString(e));
   count_launch();

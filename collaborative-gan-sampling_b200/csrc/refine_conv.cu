@@ -459,7 +459,7 @@ int check_weights(const cgs_layer_desc& L, bool backward) {
 
 // Parameters of the fused image-edge kernels (edge_conv.cuh) for a scatter- (narrow) / window-lowered (wide) pass.
 EdgeNarrowParams make_edge_narrow(const cgs_layer_desc& L, bool backward, int64_t B, const float* in, float* out,
-                                  const Epilogue& e, const int* live, int img_mode) {
+                                  const Epilogue& e, const int* live, int img_mode, bool in16 = false) {
   const PassShape sh = pass_shape(L, backward);
   EdgeNarrowParams q;
   std::memset(&q, 0, sizeof(q));
@@ -473,6 +473,7 @@ EdgeNarrowParams make_edge_narrow(const cgs_layer_desc& L, bool backward, int64_
   q.ep = e;
   q.ep.bias = sh.bias;
   q.live = live;
+  q.in16 = in16;
   return q;
 }
 
@@ -533,10 +534,11 @@ int try_edge_pair(const cgs_layer_desc& ln, const cgs_layer_desc& lw, bool backw
 
 // One layer pass (forward or data-gradient) with its fused epilogue `e` (its bias is the layer's, set here); an
 // image-edge pass on its route, any other on the gathered GEMM.
-// w16: FP16 copy of the pass's packed weights -- the pass runs on kind::f16 over FP16 operands (choose_operand_type)
+// in16: `in` is FP16 (choose_operand_type) -- a GEMM pass runs on kind::f16 over the FP16 copy of its packed weights,
+// the narrow image-edge pass takes the FP16 form of edge_narrow_tc
 int run_pass(const cgs_layer_desc& L, bool backward, int64_t B, const float* in, float* out, const Epilogue& e,
              const int* live, float* col, int math, cudaStream_t st, int img_mode = IMG_PITCHED, bool defer_reduce = false,
-             const __half* w16 = nullptr) {
+             bool in16 = false) {
   if (int rc = check_weights(L, backward)) return rc;
   const PassShape sh = pass_shape(L, backward);
   const bool scatter = use_scatter(L, backward), window = use_window(L, backward);
@@ -550,8 +552,10 @@ int run_pass(const cgs_layer_desc& L, bool backward, int64_t B, const float* in,
   const EdgeRoute r = edge_route(L, backward, math, e, img_mode);
   if ((scatter || window) && img_mode == IMG_S2D && r != ROUTE_TC)
     return set_error(CGS_ERR_UNSUPPORTED, "s2d image layout needs the tcgen05 edge kernels");
+  if (in16 && (scatter || window) && !(scatter && r == ROUTE_TC))
+    return set_error(CGS_ERR_UNSUPPORTED, "an FP16 input of an image-edge pass needs the tcgen05 narrow kernel");
   if (r != ROUTE_GENERAL && scatter) {
-    const EdgeNarrowParams q = make_edge_narrow(L, backward, B, in, out, e, live, img_mode);
+    const EdgeNarrowParams q = make_edge_narrow(L, backward, B, in, out, e, live, img_mode, in16);
     return r == ROUTE_TC ? launch_edge_narrow_tc(q, st) : launch_edge_narrow(q, st);
   }
   if (r != ROUTE_GENERAL) {
@@ -609,7 +613,9 @@ int run_pass(const cgs_layer_desc& L, bool backward, int64_t B, const float* in,
   }
   p.ep = ep;
   p.live = live;
-  if (w16) {
+  if (in16) {
+    const __half* w16 = (const __half*)(backward ? L.w16_bwd : L.w16_fwd);
+    if (!w16) return set_error(CGS_ERR_INVALID, "layer has no FP16 copy of its packed %s weights", backward ? "backward" : "forward");
     if (math != CGS_MATH_TF32_TENSOR || p.cblocks % 2) return set_error(CGS_ERR_UNSUPPORTED, "FP16 operands need 64-channel blocks");
     p.f16 = 1;                                // K counted in 64-channel atoms
     p.cblocks /= 2;
@@ -897,12 +903,16 @@ static bool f16_capable(const Chain& c) {
   return true;
 }
 
-// In an FP16 chain the tensor that layer j's data-gradient pass reduces is FP16 exactly when layer j is a GEMM layer,
-// and so is the forward input of such a layer, except the refined feature itself (j = 0): it stays FP32, because
-// momentum integrates steps below its last TF32 bit, and layer 0's forward pass keeps kind::tf32 over it.  The edge
-// kernels' 64-channel side towards the narrow kernel stays FP32 too.
-static bool feeds16(const Chain& c, int j) { return c.f16 && j >= 0 && j < c.n && !edge_layer(c.layers[j]); }
-static bool fwd16(const Chain& c, int i) { return i > 0 && feeds16(c, i); }
+// In an FP16 chain every 64-channel tensor a pass reads is FP16, with two exceptions:
+//  - the refined feature (layer 0's forward input) stays FP32, because momentum integrates steps below its last TF32
+//    bit; layer 0's forward pass keeps kind::tf32 over it (the narrow edge kernel's TF32 form when layer 0 is G's last
+//    deconv, as in the one-layer G tails);
+//  - the generated image act[n_gtail] (returned to the caller) and its gradient stay FP32 in the s2d layout.
+// So both image-edge kernels take FP16 on their 64-channel side, except the narrow forward pass of layer 0.
+// fwd16(i): layer i's forward input act[i] is FP16.  bwd16(j): the tensor layer j's data-gradient pass reduces,
+// d loss / d act[j + 1], is FP16 (and so is act[j + 1], the derivative operand of the pass that produces it).
+static bool fwd16(const Chain& c, int i) { return c.f16 && i > 0 && i < c.n && i != c.n_gtail; }
+static bool bwd16(const Chain& c, int j) { return c.f16 && j >= 0 && j < c.n && j + 1 != c.n_gtail; }
 
 static int build_chain(const cgs_net_desc* gtail, const cgs_net_desc* d, const cgs_batchnorm_desc* bn, Chain& c) {
   if (!gtail || !d) return set_error(CGS_ERR_INVALID, "null network descriptor");
@@ -976,7 +986,7 @@ static Epilogue backward_epi(const Chain& c, int i, int math, const Epilogue* up
   if (i == 0) return upd ? *upd : Epilogue(EPI_RAW, ACT_NONE);
   Epilogue e(EPI_BWD, c.layers[i - 1].act);
   e.aux = x;
-  e.out16 = feeds16(c, i - 1);
+  e.out16 = bwd16(c, i - 1);
   // a batch-BN layer's gradient feeds bn_backward, not an MMA: it is rounded after that instead
   e.round_out = (math == CGS_MATH_TF32_TENSOR) && !e.out16 && !c.bn_gamma[i - 1];
   return e;
@@ -1099,7 +1109,7 @@ static int run_forward(const Chain& c, const Workspace& w, int64_t B, int math, 
       continue;
     }
     if (int rc = run_pass(c.layers[i], false, B, w.act[i], w.act[i + 1], epi(i), live, w.col, math, st, c.img_mode, defer,
-                          fwd16(c, i) ? (const __half*)c.layers[i].w16_fwd : nullptr))
+                          fwd16(c, i)))
       return rc;
   }
   return CGS_OK;
@@ -1129,8 +1139,7 @@ static int run_backward(const Chain& c, const Workspace& w, int64_t B, int math,
     }
     Epilogue e = epi(i);
     if (i == 0 && c.f16) e.gexp = w.gexp;    // the policy step / raw gradient removes the head's per-sample scale
-    if (int rc = run_pass(c.layers[i], true, B, w.g[cur], dst, e, live, w.col, math, st, c.img_mode, false,
-                          feeds16(c, i) ? (const __half*)c.layers[i].w16_bwd : nullptr))
+    if (int rc = run_pass(c.layers[i], true, B, w.g[cur], dst, e, live, w.col, math, st, c.img_mode, false, bwd16(c, i)))
       return rc;
     cur ^= 1;
   }
@@ -1190,7 +1199,7 @@ static int head_launch(const Chain& c, const Workspace& w, int64_t B, HeadParams
   hp.feature = w.act[0];
   hp.feat_elems = (int)c.act_elems[0];
   hp.cur_logit = w.cur_logit;
-  hp.dpre16 = feeds16(c, c.n - 1);
+  hp.dpre16 = bwd16(c, c.n - 1);
   if (c.bn_gamma[c.n - 1]) hp.round_out = 0;           // dpre feeds bn_backward, which rounds its own output
   hp.gexp = w.gexp;
   cudaError_t le = launch_pdl(head_kernel, dim3((unsigned)B), dim3(256), (size_t)0, st, hp);

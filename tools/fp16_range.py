@@ -122,19 +122,24 @@ def analyse(arch_name, batch, steps, gain=2.5, seed=2019, rate=0.1):
                 stat("grad %s output" % names[i]).add(g * view(plain, g))
                 stat("grad %s output, scaled" % names[i]).add(g * view(scaled, g))
     # the matrices the chain converts to FP16: packed, BN folded, TF32 rounded (cgs.nets.PackedNet)
-    wstat = Stat()
+    wstat, nstat = Stat(), Stat()
     for L in layers:
         scope = "generator" if L in arch["gtail"] else "discriminator"
+        wf, wb, _ = N.pack_layer(L, *N.fold_layer(L, scope, w))
         if L["cin"] > 4 and L["cout"] > 4:
-            wf, wb, _ = N.pack_layer(L, *N.fold_layer(L, scope, w))
             wstat.add(N.round_tf32(wf))
             wstat.add(N.round_tf32(wb))
+        elif L["cin"] > 4:                            # G's last deconv: the narrow edge kernel's forward matrix
+            nstat.add(N.round_tf32(wf))
+        else:                                         # D's first conv: the narrow edge kernel's data-gradient matrix
+            nstat.add(N.round_tf32(wb))
     print("\n### %s, B=%d, K=%d (gain %.1f, seed %d)\n" % (arch_name, batch, steps, gain, seed))
     print("| tensor | amax | log2(65504 / amax) | nonzero share < 2^-14 |")
     print("|---|---|---|---|")
     for k, v in st.items():
         print(v.row(k))
     print(wstat.row("packed weights of the GEMM layers (BN folded, TF32 rounded)"))
+    print(nstat.row("packed weights of the narrow image-edge passes (TF32 rounded; FP16 inside edge_narrow_tc)"))
     logit = o["optimal_logit"]
     print("\nlogits: best mean %.2f, max %.2f" % (float(logit.mean()), float(logit.max())))
 
