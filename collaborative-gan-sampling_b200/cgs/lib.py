@@ -138,6 +138,10 @@ _SIGNATURES = {
     "cgs_pack_map": (C.c_int64, [C.POINTER(LayerDesc), C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64]),
     "cgs_debug_gemm_params": (C.c_int64, [C.POINTER(LayerDesc), C.c_int, C.c_int64, C.c_void_p, C.c_int64]),
     "cgs_debug_fusion_plan": (C.c_int64, [C.POINTER(LayerDesc), C.c_int, C.c_int64, C.c_void_p, C.c_int64]),
+    "cgs_debug_chain_layout": (C.c_int64, [C.POINTER(NetDesc), C.POINTER(NetDesc), C.c_int, C.c_void_p, C.c_int64]),
+    "cgs_debug_chain_pass": (C.c_int, [C.POINTER(NetDesc), C.POINTER(NetDesc), C.c_int, C.c_int64, C.c_int, C.c_int,
+                                       C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(RefineCfg),
+                                       C.c_void_p, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p]),
     "cgs_pass_layout": (C.c_int, [C.POINTER(LayerDesc), C.c_int]),
     "cgs_layer_workspace_bytes": (C.c_size_t, [C.POINTER(LayerDesc), C.c_int64]),
     "cgs_layer_forward": (C.c_int, [C.POINTER(LayerDesc), C.c_int, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,

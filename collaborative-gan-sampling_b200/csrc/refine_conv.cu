@@ -1390,6 +1390,102 @@ extern "C" int cgs_forward_logits_and_grad(const cgs_net_desc* gtail, const cgs_
                                         workspace_bytes, stream);
 }
 
+// Host-only introspection (include/cgs.h): dtype and layout of every tensor of the chain, from the chain's own
+// decisions (build_chain, choose_image_layout, choose_operand_type, fwd16 / bwd16).
+extern "C" int64_t cgs_debug_chain_layout(const cgs_net_desc* gtail, const cgs_net_desc* d, int math, int32_t* out,
+                                          int64_t capacity) {
+  Chain c;
+  if (int rc = build_chain(gtail, d, nullptr, c)) return rc;
+  choose_image_layout(c, math);
+  choose_operand_type(c, math);
+  const int64_t need = 4 + (int64_t)(2 * c.n + 1) * 8;
+  if (!out) return need;
+  if (capacity < need) return set_error(CGS_ERR_INVALID, "capacity too small");
+  enum { DENSE = 0, S2D = 1, PITCHED = 2 };
+  const int img = c.img_mode == IMG_S2D ? S2D : PITCHED;
+  int32_t* o = out;
+  *o++ = c.n; *o++ = c.n_gtail; *o++ = img; *o++ = c.f16;
+  auto put = [&](int i, bool f16) {          // act[i] (or the gradient in its place): H, W, channels as produced
+    const cgs_layer_desc& Lp = c.layers[i == 0 ? 0 : i - 1];
+    const LayerShape s = layer_shape(Lp);
+    const int h = i == 0 ? Lp.hin : s.hout, w = i == 0 ? Lp.win : s.wout, ch = i == 0 ? Lp.cin : Lp.cout;
+    const int lay = ch <= 4 ? img : DENSE;
+    *o++ = f16; *o++ = lay; *o++ = h; *o++ = w; *o++ = ch;
+    *o++ = lay == DENSE ? cstride(ch) : lay == S2D ? 16 : 4;                 // values per stored pixel
+    *o++ = lay == DENSE ? w : lay == S2D ? w / 2 : img_pitch(w);             // stored pixels per row
+    *o++ = lay == S2D ? h * w * 4 : (int32_t)c.act_elems[i];                 // s2d samples lie back to back
+  };
+  for (int i = 0; i <= c.n; ++i) put(i, fwd16(c, i));
+  for (int i = 1; i <= c.n; ++i) put(i, bwd16(c, i - 1));
+  return need;
+}
+
+// Developer entry point (include/cgs.h): one pass of the chain, launched exactly as run_forward / run_backward /
+// head_launch launch it, but unpaired (try_edge_pair is not taken) and with the head reading a stored act[n] rather
+// than split-K partial sums.
+extern "C" int cgs_debug_chain_pass(const cgs_net_desc* gtail, const cgs_net_desc* d, int math, int64_t B, int layer,
+                                    int backward, const void* in, void* out, void* aux, int32_t* gexp,
+                                    const cgs_refine_cfg* step_cfg, float* mom, int first, void* workspace,
+                                    size_t workspace_bytes, cgs_stream_t stream) {
+  if (int rc = require_sm100()) return rc;
+  if (!in || !out) return set_error(CGS_ERR_INVALID, "null argument");
+  if (B <= 0) return B == 0 ? CGS_OK : set_error(CGS_ERR_INVALID, "negative batch");
+  Chain c;
+  if (int rc = build_chain(gtail, d, nullptr, c)) return rc;
+  choose_image_layout(c, math);
+  choose_operand_type(c, math);
+  if (layer < 0 || layer > c.n || (layer == c.n && !backward))
+    return set_error(CGS_ERR_INVALID, "pass %d (%s) is not in the chain", layer, backward ? "data-gradient" : "forward");
+  Workspace w;
+  carve(c, B, (void*)(((uintptr_t)workspace + 255) & ~uintptr_t(255)), w);
+  if (!workspace || w.total + 256 > workspace_bytes) return set_error(CGS_ERR_WORKSPACE, "workspace too small");
+  if (B > cgs_refine_max_batch(gtail, d))
+    return set_error(CGS_ERR_UNSUPPORTED, "batch too large for 32-bit row indexing; split it (cgs_refine_max_batch)");
+  cudaStream_t st = (cudaStream_t)stream;
+  const bool scaled = layer == 0 && backward && c.f16;       // the pass that removes the head's per-sample scale
+  if (gexp && !scaled && layer != c.n)
+    return set_error(CGS_ERR_INVALID, "only layer 0's data-gradient pass of an FP16 chain takes a gradient scale");
+  if (layer == c.n) {
+    if (!aux || (bwd16(c, c.n - 1) && !gexp)) return set_error(CGS_ERR_INVALID, "the head needs logit / exponent outputs");
+    HeadParams hp;
+    std::memset(&hp, 0, sizeof(hp));
+    w.act[0] = w.feat2;
+    w.act[c.n] = (float*)in;
+    w.cur_logit = (float*)aux;
+    if (gexp) w.gexp = gexp;
+    w.col = nullptr;                                         // no split-K partials: the head reads `in`
+    hp.best_img = w.g[1];                                    // selection outputs to scratch, as cgs_forward_logits_and_grad
+    hp.best_logit = w.cur_logit;
+    hp.best_step = w.mom;
+    hp.step = -1;
+    hp.round_out = (math == CGS_MATH_TF32_TENSOR);
+    hp.dpre = (float*)out;
+    return head_launch(c, w, B, hp, math, st);
+  }
+  const cgs_layer_desc& L = c.layers[layer];
+  if (!backward)
+    return run_pass(L, false, B, (const float*)in, (float*)out, forward_epi(c, layer, math), nullptr, w.col, math, st,
+                    c.img_mode, false, fwd16(c, layer));
+  Epilogue upd(EPI_UPDATE, ACT_NONE);
+  if (step_cfg) {
+    if (layer != 0) return set_error(CGS_ERR_INVALID, "the policy step is fused into layer 0's data-gradient pass only");
+    if (!mom && step_cfg->method != CGS_POLICY_SGD) return set_error(CGS_ERR_INVALID, "momentum step without momentum");
+    upd.sgd = step_cfg->method == CGS_POLICY_SGD;
+    upd.rate = step_cfg->rate;
+    upd.alpha = step_cfg->alpha;
+    upd.clip = step_cfg->clip;
+    upd.vmin = step_cfg->vmin;
+    upd.vmax = step_cfg->vmax;
+    upd.first = first != 0;
+    upd.mom = mom;
+  }
+  if (layer > 0 && !aux) return set_error(CGS_ERR_INVALID, "a data-gradient pass needs the forward output it differentiates");
+  Epilogue e = backward_epi(c, layer, math, step_cfg ? &upd : nullptr, (const float*)aux);
+  if (scaled) e.gexp = gexp;
+  return run_pass(L, true, B, (const float*)in, (float*)out, e, nullptr, w.col, math, st, c.img_mode, false,
+                  bwd16(c, layer));
+}
+
 static size_t layer_stage_elems(const cgs_layer_desc& L, bool backward) {   // pitched copy of an image-like input
   if (!use_window(L, backward)) return 0;
   const PassShape sh = pass_shape(L, backward);

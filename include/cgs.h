@@ -277,6 +277,38 @@ CGS_API int64_t cgs_debug_gemm_params(const cgs_layer_desc* L, int backward, int
  * NULL `out` queries the length.  Lets tests check the fused walk and the pair split on the CPU. */
 CGS_API int64_t cgs_debug_fusion_plan(const cgs_layer_desc* L, int backward, int64_t B, int32_t* out, int64_t capacity);
 
+/* Host-only introspection of a refinement chain (G tail + D without its head, bn == NULL) under `math` and the current
+ * CGS_DEBUG knobs: where and in which type every tensor lives.  Writes [n, n_gtail, img_mode, f16] and then 8 int32s
+ * per tensor, first act[0 .. n] (act[0] = the refined feature, act[i + 1] = output of layer i), then d loss / d act[1 .. n]
+ * (exactly: the tensor data-gradient pass i - 1 reduces, i.e. the gradient w.r.t. layer i - 1's pre-activation output,
+ * held in act[i]'s layout): [fp16, layout, H, W, C, values per stored pixel, stored pixels per row, elements per sample
+ * (the stride from one sample to the next)].
+ * fp16: 1 = __half, 0 = float.  layout: 0 = dense NHWC (channel stride = C rounded up to 4), 1 = space-to-depth
+ * [H/2][W/2][2][2][4], 2 = pitched [H][W + 8][4] with pixel x at column x + 2 and zeros elsewhere.  img_mode = the
+ * layout (1 or 2) of the <= 4-channel tensors; f16 = the chain's MMA operands are FP16.  NULL `out` queries the length. */
+CGS_API int64_t cgs_debug_chain_layout(const cgs_net_desc* gtail, const cgs_net_desc* d, int math, int32_t* out,
+                                       int64_t capacity);
+/* Developer aid OUTSIDE the drop-in contract: ONE pass of the chain on the caller's tensors, launched as a refinement
+ * call launches it (same kernel route, operand type, layouts and fused epilogue; cgs_debug_chain_layout gives the
+ * layouts), so that each pass can be checked alone.  Tensors are batch-major with cgs_debug_chain_layout's elements
+ * per sample.
+ *   forward (backward == 0), 0 <= layer < n: in = act[layer], out = act[layer + 1].
+ *   data-gradient, 0 < layer < n: in = d loss / d act[layer + 1], aux = act[layer] (the forward output the epilogue
+ *     differentiates through), out = d loss / d act[layer].
+ *   data-gradient, layer 0: in as above; step_cfg NULL: out = the raw gradient w.r.t. the feature; else out is the
+ *     feature, updated in place by the fused policy step of step_cfg (method, rate, alpha, clip, vmin, vmax), with
+ *     `mom` (momentum, read unless `first`, written) and `first`.  gexp (nullable, [B] int32; FP16 chains only): the
+ *     input carries the per-sample factor 2^gexp[b], which the pass removes.
+ *   layer == n, data-gradient: the head.  in = act[n], aux = the [B] logits (out), out = d loss / d act[n] (dpre), gexp =
+ *     the [B] exponents the head writes (required when dpre is FP16).
+ * The workspace is cgs_refine_workspace_bytes(gtail, d, B).  Where a refinement call runs the two image-edge passes as
+ * one paired kernel (pitched image layout), this entry point runs them as the two separate kernels that
+ * CGS_DEBUG_NO_EDGE_PAIR selects; the head never takes split-K partial sums here. */
+CGS_API int cgs_debug_chain_pass(const cgs_net_desc* gtail, const cgs_net_desc* d, int math, int64_t B, int layer,
+                                 int backward, const void* in, void* out, void* aux, int32_t* gexp,
+                                 const cgs_refine_cfg* step_cfg, float* mom, int first, void* workspace,
+                                 size_t workspace_bytes, cgs_stream_t stream);
+
 /* Lowering of a pass: 0 = gather layout (K order given by cgs_pack_map), 1 = scatter layout, 2 = window layout
  * (strided passes reading a <= 4-channel image: rows = large channel, K index = ky*32 + kx*4 + small channel).  Transposed-type
  * passes with <= 4 output channels (deconv -> image forward, first-conv data-gradient) run as one GEMM over the

@@ -147,3 +147,36 @@ def test_class_fusion_plan_and_cta_pair_split(cgs_lib, arch_name):
                     assert covered[c] == [g["k0"] // 32 + t * cb for t in range(g["ntaps"])], (layer["name"], c)
             assert sorted(seen_classes) == [0, 1, 2, 3]
     assert (fused > 0) == (arch_name != "mnist")
+
+
+@pytest.mark.parametrize("arch_name", ["mnist", "mnist_l2", "dcgan32_l1", "dcgan32_l2", "dcgan32_l3", "dcgan32_l4",
+                                       "dcgan64_l1", "dcgan64_l2", "dcgan64_l3", "dcgan64_l4", "dcgan48_l1"])
+def test_chain_layout_follows_the_operand_rule(cgs_lib, arch_name):
+    """cgs_debug_chain_layout against DESIGN.md §2's rule, without a GPU.  DCGAN-32 / -64 chains take FP16 operands:
+    every tensor is FP16 except the refined feature act[0], the image and its gradient (s2d) and the head input act[n];
+    so a one-layer G tail runs layer 0's narrow pass over FP32 (its TF32 form).  MNIST and DCGAN-48 (no tcgen05 edge
+    kernel takes 24-pixel rows: pitched image) and every chain under DEBUG_TF32_OPERANDS are FP32 throughout."""
+    import chain_ref as R
+    from cgs import lib as L
+    from cgs import nets as N
+    arch = N.get_arch(arch_name)
+    spec = N.NetSpec(arch, onets.init_weights(arch, seed=3), "cpu")
+    f16_arch = arch_name.startswith(("dcgan32", "dcgan64"))
+    for flags in (0, L.DEBUG_TF32_OPERANDS):
+        with L.debug_flags(flags):
+            lay = R.chain_layout(spec.gtail.desc, spec.d.desc)
+        n, ng = lay["n"], lay["n_gtail"]
+        assert (n, ng) == (len(arch["gtail"]) + len(arch["d"]) - 1, len(arch["gtail"]))
+        assert lay["img_mode"] == (R.S2D if f16_arch else R.PITCHED)
+        f16 = f16_arch and not flags
+        assert lay["f16"] == f16
+        for kind, i, t in [("act", i, t) for i, t in enumerate(lay["act"])] + \
+                          [("grad", i, t) for i, t in enumerate(lay["grad"]) if t is not None]:
+            fp32 = i == ng or (kind == "act" and i in (0, n))
+            assert t["fp16"] == (f16 and not fp32), (kind, i)
+            image = i == ng
+            assert t["layout"] == (lay["img_mode"] if image else R.DENSE), (kind, i)
+            assert t["C"] <= 4 if image else t["C"] >= 32
+            assert t["elems"] >= t["H"] * t["W"] * t["C"]
+        if arch_name == "dcgan64_l4":                      # layer 0 = G's last deconv, reading the FP32 feature
+            assert ng == 1 and not lay["act"][0]["fp16"] and lay["grad"][2]["fp16"] == f16
